@@ -1,8 +1,9 @@
 #!/usr/bin/env python3
-"""bench.py -- the driver's benchmark contract for the multi-start forward-star sweep.
+"""bench.py -- the benchmark of the multi-start forward-star sweep.
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (also save what the last timed step computed)
 
 Workload (BASELINE.json configs[2] -- the configuration the metric "... 241x241x51 818-FS, 1/2/4/8 B200" is quoted
 on; it fits one GPU): 241x241x51 heterogeneous slowness box (synthetic stand-in, seed 7: the reference's velocity
@@ -15,6 +16,12 @@ rides along under "extras" together with config 1 (3-FS) and the 5-FS star.
 
 Prints ONE JSON line (rank 0).  metric = GRelax/s: in-bounds (node, offset, source) pull
 evaluations executed per second, summed over GPUs; converged sources/s rides along.
+
+--dump-outputs DIR writes the travel-time fields of the last timed step, sampled at the same seeded node set for every
+source (see dump_outputs), as DIR/tt.npy (DIR/tt_rank<r>.npy per rank when N>1).  The inputs are fixed by their seeds,
+so two builds run with the same arguments can be compared output for output.  It applies to --impl ours only: the
+reference arm times the original serial sweepXYZ over slices of the star and never holds a converged field of this
+project to dump.
 """
 import argparse
 import ctypes
@@ -38,6 +45,7 @@ WORKLOADS = {
     "config4": "1201x1201x251 heterogeneous slowness (synthetic, seed 11), 818-FS, 24 sources (start-24 x5) sharded over the GPUs",
 }
 VISITS_PER_SWEEP_818 = 2_246_171_812   # in-bounds (node, offset) visits of one reference sweep of the 241 box (SURVEY 8a)
+DUMP_NODES = 1 << 16   # sampled nodes per source: 111 sources x 64 Ki x 4 B = 29 MB, under the 64 MB a dump may take
 
 
 def parse():
@@ -53,7 +61,15 @@ def parse():
                          "config2: 241 box, 4 sources per GPU (weak); "
                          "config4: 1201x1201x251, 24 sources sharded over the GPUs (strong, device-resident only). "
                          "Config 5 (one source, one huge grid over all GPUs) is tools/config5_bench.py.")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, save a seeded sample of the travel times of the last timed step as "
+                         "float32 .npy files in DIR")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs saves the GPU solve's fields: it needs --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------
@@ -308,6 +324,22 @@ def _golden(label):
 # ------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------
+def dump_outputs(ctx, nsrc, dims, out_dir, name):
+    """Travel times of the context's last solve as out_dir/<name>.npy, float32[nsrc, DUMP_NODES]: row s holds source s's
+    field at DUMP_NODES flat node indices drawn without replacement by numpy's default_rng(0) and sorted -- the same
+    nodes for every source and every run.  (The full fields of config 3 are 1.3 GB.)"""
+    import numpy as np
+    n = int(np.prod(dims))
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_NODES), replace=False))
+    field = np.empty(dims, np.float32)
+    out = np.empty((nsrc, len(idx)), np.float32)
+    for s in range(nsrc):
+        out[s] = ctx.get_tt(s, out=field).ravel()[idx]
+    d = pathlib.Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / f"{name}.npy", out)
+
+
 def timed_resident(P, torch, ctx, stream, flush, steps, warmup, barrier, before_timed=None):
     """W untimed + K timed device-resident solves (CUDA events on the solve stream, L2 flushed in between)."""
     for _ in range(warmup):
@@ -454,6 +486,8 @@ def run_ours(args):
     acc = timed_resident(P, torch, ctx, stream, flush, args.steps, args.warmup, barrier,
                          before_timed=lambda: box.setdefault("sampler", ClockSampler(local) if rank == 0 else None))
     clocks = box["sampler"].stop() if box.get("sampler") else None
+    if args.dump_outputs:
+        dump_outputs(ctx, nsrc, dims, args.dump_outputs, "tt" if world == 1 else f"tt_rank{rank}")
     tot = dispatch.combine(dist, dev, elapsed_ms=acc["dev_ms"], relaxations=acc["relaxations"],
                            sources=nsrc * args.steps, launches=acc["launches"])
     pulls_per_grid_round = ctx.relaxations_per_round   # in-bounds pulls of ONE full round of one source (analytic)

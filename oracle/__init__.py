@@ -2,7 +2,8 @@
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference leg may
 import this package.  `restatement()` is our C restatement; `reference()` is the reference's
-own serial_new program compiled from /root/reference into oracle/_ref (None when absent).
+own serial_new program compiled into oracle/_ref from the checkout of the original project named by
+$SWEEPTT_REFERENCE (None when absent).
 """
 from __future__ import annotations
 

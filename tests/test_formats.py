@@ -1,6 +1,9 @@
 """CPU: file formats of the drop-in surface (csrc/hostio.cpp through the C ABI) against the
-oracle's restatement and -- where oracle/_ref exists -- the reference's own loaders/writers."""
+oracle's restatement, the .vbox bytes recorded in tests/golden/oracle_pins.json and -- where oracle/_ref exists -- the
+reference's own loaders/writers."""
 import ctypes
+import hashlib
+import json
 import struct
 import subprocess
 
@@ -11,12 +14,21 @@ import oracle
 import uoparallel_seismic_project_b200 as P
 from uoparallel_seismic_project_b200 import workloads as W
 
+from conftest import ROOT
+
+VBOX_SHA = json.loads((ROOT / "tests" / "golden" / "oracle_pins.json").read_text())["vbox_sha256"]
+
+
+def _sha(path):
+    return hashlib.sha256(path.read_bytes()).hexdigest()
+
 
 def test_vbox_store_bytes_match_oracle_and_vconvert(tmp_path):
     v = (W.random_field((7, 5, 9), seed=3) - np.float32(0.25)).astype(np.float32)  # negative values: sign-extension matters
     P.vbox_store(tmp_path / "ours.vbox", v, origin=(1, 1, 1))
     oracle.vbox_write(tmp_path / "oracle.vbox", v, origin=(1, 1, 1))
     assert (tmp_path / "ours.vbox").read_bytes() == (tmp_path / "oracle.vbox").read_bytes()
+    assert _sha(tmp_path / "ours.vbox") == VBOX_SHA["vbox_store_random_7x5x9_seed3_minus_quarter"]
     vc = oracle.vconvert_path()
     if vc is not None:  # the reference's own tools/vconvert.c on the same text input
         W.write_text_a(tmp_path / "v.txt", v)
@@ -32,6 +44,7 @@ def test_vconvert_tool_matches_reference_tool(tmp_path):
     assert r.returncode == 0 and "writing new velocity model" in r.stdout
     got, origin, dims = P.vbox_load(tmp_path / "ours.vbox")
     assert origin == (1, 1, 1) and np.array_equal(got, v)
+    assert _sha(tmp_path / "ours.vbox") == VBOX_SHA["vconvert_hetero_5x6x7_seed9"]
     vc = oracle.vconvert_path()
     if vc is not None:
         subprocess.run([str(vc), str(tmp_path / "v.txt"), str(tmp_path / "ref.vbox")], check=True, capture_output=True)
@@ -83,6 +96,13 @@ def test_reference_loader_accepts_our_vbox(tmp_path):
     assert tuple(dims) == (5, 4, 6) and tuple(origin) == (1, 1, 1)
     got = np.ctypeslib.as_array(lib.refh_velocity_ptr(), shape=(v.size,)).reshape(v.shape)
     assert np.array_equal(got, v)
+    assert _sha(tmp_path / "a.vbox") == VBOX_SHA["vbox_store_random_5x4x6_seed8"]
+
+
+def test_vbox_bytes_match_the_recorded_file_the_reference_loader_reads(tmp_path):
+    """The file test_reference_loader_accepts_our_vbox hands to the reference's loader, against the recorded bytes."""
+    P.vbox_store(tmp_path / "a.vbox", W.random_field((5, 4, 6), seed=8), origin=(1, 1, 1))
+    assert _sha(tmp_path / "a.vbox") == VBOX_SHA["vbox_store_random_5x4x6_seed8"]
 
 
 def test_vbox_subset(tmp_path):

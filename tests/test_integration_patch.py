@@ -1,9 +1,10 @@
-"""CPU (only where the reference checkout is present): the binding of INTEGRATION.md 1 applied mechanically to a
-TEMPORARY copy of the reference's serial_new/sweep-tt-multistart.c -- include the header after the file's own struct
-definitions, replace the sweep loop (:150-170) by one sweeptt_solve call -- builds with the reference's flags, links
-against libsweeptt.so, and runs the reference's own main() up to our call: on this GPU-less container the call must fail
-loudly with the library's message; on a GPU box (no reference checkout) the test is skipped and the CLI test covers the
-run.  Nothing of the reference is copied into the repository."""
+"""CPU (only where $SWEEPTT_REFERENCE names a checkout of the original project): the binding of INTEGRATION.md 1
+applied mechanically to a TEMPORARY copy of the reference's serial_new/sweep-tt-multistart.c -- include the header after
+the file's own struct definitions, replace the sweep loop (:150-170) by one sweeptt_solve call -- builds with the
+reference's flags, links against libsweeptt.so, and runs the reference's own main() up to our call: without a GPU the
+call must fail loudly with the library's message, on a GPU machine it must run.  Without the checkout the test is
+skipped and the CLI test covers the run.  Nothing of the reference is copied into the repository."""
+import os
 import pathlib
 import re
 import subprocess
@@ -16,7 +17,8 @@ from uoparallel_seismic_project_b200 import workloads as W
 
 from conftest import ROOT
 
-REF = pathlib.Path("/root/reference/serial_new/sweep-tt-multistart.c")
+REF_DIR = pathlib.Path(os.environ["SWEEPTT_REFERENCE"]) if os.environ.get("SWEEPTT_REFERENCE") else None
+REF = REF_DIR / "serial_new" / "sweep-tt-multistart.c" if REF_DIR else None
 
 CALL = r'''
   {
@@ -36,7 +38,7 @@ CALL = r'''
 '''
 
 
-@pytest.mark.skipif(not REF.exists(), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(REF is None or not os.path.isfile(REF), reason="needs a checkout of the original project in $SWEEPTT_REFERENCE")
 def test_binding_patch_builds_links_and_reaches_our_call(tmp_path):
     src = REF.read_text()
     # 1. our header after the file's own struct definitions
@@ -51,7 +53,7 @@ def test_binding_patch_builds_links_and_reaches_our_call(tmp_path):
     patched.write_text(src)
     exe = tmp_path / "sweep-tt-multistart"
     lib = P.lib_path()
-    subprocess.run(["gcc", "-O3", "-Wfatal-errors", "-w", "-I/root/reference/include", f"-I{ROOT / 'include'}", "-o", str(exe),
+    subprocess.run(["gcc", "-O3", "-Wfatal-errors", "-w", f"-I{REF_DIR / 'include'}", f"-I{ROOT / 'include'}", "-o", str(exe),
                     str(patched), f"-L{lib.parent}", "-lsweeptt", f"-Wl,-rpath,{lib.parent}", "-lm"], check=True)
     v = W.heterogeneous_field((12, 11, 9), 3)
     P.vbox_store(tmp_path / "m.vbox", v, origin=(1, 1, 1))

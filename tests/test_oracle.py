@@ -1,6 +1,8 @@
-"""CPU: the oracle restatement against the reference-generated goldens and (when the build
-container's oracle/_ref exists) against the reference's own code sweep by sweep."""
+"""CPU: the oracle restatement against the reference-generated goldens, against the star distances and per-sweep
+trace recorded in tests/golden/oracle_pins.json and (where oracle/_ref exists) against the reference's own code sweep by
+sweep -- which also checks the recorded values."""
 import hashlib
+import json
 
 import numpy as np
 import pytest
@@ -8,7 +10,9 @@ import pytest
 import oracle
 from uoparallel_seismic_project_b200 import workloads as W
 
-from conftest import assert_bit_equal, make_field
+from conftest import ROOT, assert_bit_equal, make_field
+
+PINS = json.loads((ROOT / "tests" / "golden" / "oracle_pins.json").read_text())
 
 
 def test_restatement_matches_reference_goldens(golden_small):
@@ -20,7 +24,7 @@ def test_restatement_matches_reference_goldens(golden_small):
         assert sweeps == m["ref_sweeps"]
 
 
-@pytest.mark.skipif(oracle.reference() is None, reason="oracle/_ref not built (no /root/reference)")
+@pytest.mark.skipif(oracle.reference() is None, reason="oracle/_ref not built (needs $SWEEPTT_REFERENCE)")
 def test_restatement_sweep_by_sweep_against_reference_code():
     v = W.contrast_field((14, 13, 12), seed=4)
     for name in ("3", "5", "818"):
@@ -33,6 +37,20 @@ def test_restatement_sweep_by_sweep_against_reference_code():
             c = oracle.sweep(v, tt, off, start)
             assert c == c_ref
             assert_bit_equal(tt, t_ref, f"{name}-FS per-sweep state")
+        assert [[c, hashlib.sha256(t.tobytes()).hexdigest()] for c, t in trace] == PINS["trace"][name]
+
+
+def test_restatement_sweep_by_sweep_against_recorded_trace():
+    case = PINS["trace_case"]
+    v = make_field(case["kind"], case["dims"], case["seed"])
+    for name in ("3", "5", "818"):
+        off = W.star(name)
+        tt = oracle.init_tt(v.shape, case["start"])
+        for k, (c_ref, sha_ref) in enumerate(PINS["trace"][name]):
+            c = oracle.sweep(v, tt, off, case["start"])
+            assert c == c_ref, f"{name}-FS sweep {k + 1}: store count"
+            assert hashlib.sha256(tt.tobytes()).hexdigest() == sha_ref, f"{name}-FS sweep {k + 1}: field"
+        assert c_ref == 0
 
 
 @pytest.mark.skipif(oracle.reference() is None, reason="oracle/_ref not built")
@@ -44,6 +62,14 @@ def test_star_distances_match_reference():
         assert lib.refh_set_star(ctypes.c_void_p(off.ctypes.data), len(off))
         d_ref = np.array([lib.refh_star_distance(l) for l in range(len(off))], np.float32)
         assert_bit_equal(oracle.star_distances(off), d_ref)
+        assert [int(x) for x in d_ref.view(np.uint32)] == PINS["star_distance_bits"][name]
+
+
+def test_star_distances_match_recorded():
+    for name in ("3", "5", "818"):
+        want = np.array(PINS["star_distance_bits"][name], np.uint32).view(np.float32)
+        assert len(want) == len(W.star(name))
+        assert_bit_equal(oracle.star_distances(W.star(name)), want, f"{name}-FS")
 
 
 def test_fixed_point_invariant_and_detection(golden_small):

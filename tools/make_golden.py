@@ -7,6 +7,7 @@ serial_new/sweep-tt-multistart.c compiled in the build container).
   python tools/make_golden.py config3_all [P] -> tests/golden/config3_all.json (every other row of start-111, sha256 only)
   python tools/make_golden.py more [P]  -> tests/golden/full_241_more.json (round 2: 9 further config-3 sources,
                                            full-size 5-FS and a scaled config-4-like box; P processes, ~1 h on 6)
+  python tools/make_golden.py pins      -> tests/golden/oracle_pins.json (see pins(); needs no reference)
 
 The GPU box has no /root/reference; the parity tests there compare against these files.
 Small cases: converged float32 fields for seeded boxes.  Full size (BASELINE configs 1 and 2):
@@ -141,5 +142,59 @@ def config3_all():
             print(r["label"], r["ref_sweeps"], r["seconds"], r["tt_sha256"][:16], flush=True)
 
 
+PIN_TRACE = dict(kind="contrast", dims=(14, 13, 12), seed=4, start=(7, 3, 11))
+
+
+def pin_vbox_bytes(tmp):
+    """The .vbox files of the cases tests/test_formats.py compares with the reference's own tools and loaders."""
+    import subprocess
+    import uoparallel_seismic_project_b200 as P
+    tmp = pathlib.Path(tmp)
+    out = {}
+    P.vbox_store(tmp / "a.vbox", (W.random_field((7, 5, 9), seed=3) - np.float32(0.25)).astype(np.float32), origin=(1, 1, 1))
+    out["vbox_store_random_7x5x9_seed3_minus_quarter"] = (tmp / "a.vbox").read_bytes()
+    W.write_text_a(tmp / "v.txt", W.heterogeneous_field((5, 6, 7), seed=9))
+    subprocess.run([str(P.lib_path().parent / "vconvert"), str(tmp / "v.txt"), str(tmp / "b.vbox")], check=True,
+                   capture_output=True)
+    out["vconvert_hetero_5x6x7_seed9"] = (tmp / "b.vbox").read_bytes()
+    P.vbox_store(tmp / "c.vbox", W.random_field((5, 4, 6), seed=8), origin=(1, 1, 1))
+    out["vbox_store_random_5x4x6_seed8"] = (tmp / "c.vbox").read_bytes()
+    return {k: hashlib.sha256(v).hexdigest() for k, v in out.items()}
+
+
+def restatement_trace(star):
+    """(stores, sha256 of the field) after every sweep of the restatement on the PIN_TRACE case, up to the first sweep
+    that stores nothing -- the sequence oracle.ref_solve(per_sweep=...) yields for the reference's own sweepXYZ."""
+    v = field(PIN_TRACE["kind"], PIN_TRACE["dims"], PIN_TRACE["seed"])
+    off = W.star(star)
+    tt = oracle.init_tt(v.shape, PIN_TRACE["start"])
+    trace = []
+    while True:
+        c = oracle.sweep(v, tt, off, PIN_TRACE["start"])
+        trace.append((int(c), hashlib.sha256(tt.tobytes()).hexdigest()))
+        if c == 0:
+            return trace
+
+
+def pins():
+    """tests/golden/oracle_pins.json: the quantities the CPU tests compare with the original project's own code when a
+    checkout of it is at hand (SWEEPTT_REFERENCE) -- star distances, the per-sweep trace of the restatement, .vbox bytes --
+    recorded from the restatement and this project's writers, so that the comparison also runs without the checkout."""
+    import tempfile
+    stars = ("3", "5", "818")
+    with tempfile.TemporaryDirectory() as tmp:
+        vbox = pin_vbox_bytes(tmp)
+    res = {
+        "provenance": "recorded by tools/make_golden.py pins from oracle/sweep_oracle.c and the project's .vbox writers; "
+                      "tests/test_oracle.py and tests/test_formats.py compare the same quantities with the original "
+                      "project's own code when SWEEPTT_REFERENCE names a checkout of it",
+        "star_distance_bits": {s: [int(x) for x in oracle.star_distances(W.star(s)).view(np.uint32)] for s in stars},
+        "trace_case": {k: list(v) if isinstance(v, tuple) else v for k, v in PIN_TRACE.items()},
+        "trace": {s: [list(t) for t in restatement_trace(s)] for s in stars},
+        "vbox_sha256": vbox,
+    }
+    (GOLD / "oracle_pins.json").write_text(json.dumps(res, indent=0) + "\n")
+
+
 if __name__ == "__main__":
-    {"small": small, "full": full, "more": more, "config3_all": config3_all}[sys.argv[1]]()
+    {"small": small, "full": full, "more": more, "config3_all": config3_all, "pins": pins}[sys.argv[1]]()
