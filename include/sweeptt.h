@@ -207,6 +207,47 @@ int sweeptt_put_tt(sweeptt_ctx *ctx, int source, const float *tt_in);
  * old/wavefront-openmp/wave-multistart.c:300-347, for this edge set). 0 <=> converged. */
 int sweeptt_count_violations(sweeptt_ctx *ctx, int source, long long *violations);
 
+/* ---- rays: shortest paths read off a converged field ------------------------ */
+
+/* Status of one traced ray (data, never an error return). */
+enum {
+  SWEEPTT_RAY_OK = 0,              /* the ray reached the start point                                     */
+  SWEEPTT_RAY_UNREACHED = 1,       /* tt[receiver] = +INF                                                  */
+  SWEEPTT_RAY_NOT_FIXED_POINT = 2, /* a candidate on the path is below tt[n]: the field is not converged  */
+  SWEEPTT_RAY_NO_PREDECESSOR = 3,  /* no candidate equals tt[n]: the field is not of this model/star/start */
+  SWEEPTT_RAY_STALLED = 4,         /* the chosen predecessor is not below tt[n] (a zero-delay edge)        */
+  SWEEPTT_RAY_TRUNCATED = 5        /* the ray has more than max_nodes nodes; the first max_nodes are kept  */
+};
+
+/* Traces, for every source s in [source_begin, source_begin+source_count) and every receiver r, the
+ * shortest-path ray from r back to the start point p of s through the field the context holds for s.
+ * Receivers are caller-axis node coordinates like start points.
+ *
+ * Candidate predecessors of a node n != p are exactly the edges the sweep relaxes (o_l: star entries
+ * l < star_used): m = n + o_l, and m = n - o_l unless m == p (the reference skips visits whose centre
+ * is the start); in-bounds m only.  cand(n,m) = fl(fl(hd*fl(v_n+v_m)) + tt[m]) with hd = 0.5f*d, the
+ * sweep's own expression.  At the fixed point every finite tt[n], n != p, equals its smallest candidate.
+ * pred(n): among the candidates with cand == tt[n], the one with the smallest tt[m] (-0 before +0),
+ * then the one with the smallest FLOATBOX index of m.  The rule depends only on the field and the
+ * geometry, never on the relaxation kernel or schedule that produced the field.
+ * The ray is r, pred(r), pred(pred(r)), ..., p; a receiver that is the start gives a ray of one node.
+ * Its status is SWEEPTT_RAY_UNREACHED when tt[r] = +INF; otherwise the first node n != p of the path at
+ * which a candidate is below tt[n] (NOT_FIXED_POINT), no candidate equals tt[n] (NO_PREDECESSOR) or
+ * the chosen tt[m] is not below tt[n] (STALLED) ends the ray with that status, n being its last node.
+ *
+ * Ray (s, r) is stored at q = (s - source_begin)*nrec + r: nodes_out[q*max_nodes + t] (t < length_out[q],
+ * caller axes; past the length (-1,-1,-1) up to the call's longest ray, then left as they were), length_out[q], status_out[q] and
+ * tt_out[q] = tt[r] (whatever the status: a receiver table without copying whole fields).  Any output
+ * may be NULL.  Reads only the model, the field and the start points, so it works after any solve,
+ * after sweeptt_step and after sweeptt_put_tt.  Runs on the context's stream and synchronises it.
+ * stats (may be NULL): solve_ms = device time of the trace, relaxations = candidate evaluations,
+ * kernel_launches, d2h_ms / d2h_bytes. */
+int sweeptt_trace_rays(sweeptt_ctx *ctx, int source_begin, int source_count,
+                       const struct START *receivers, int nrec, int max_nodes,
+                       struct START *nodes_out, /* [source_count*nrec*max_nodes], may be NULL */
+                       int32_t *length_out, int32_t *status_out, float *tt_out, /* [source_count*nrec] */
+                       sweeptt_stats *stats);
+
 /* In-bounds pull evaluations of one full round of one source (analytic). */
 long long sweeptt_relaxations_per_round(sweeptt_ctx *ctx);
 /* Bytes of device memory currently held by the context's pool. */

@@ -8,6 +8,7 @@ raises ``SweepError`` when the extension or a CUDA device is missing.
 """
 from .api import (  # noqa: F401
     FS,
+    Rays,
     START,
     SweepContext,
     SweepError,
@@ -23,6 +24,7 @@ from .api import (  # noqa: F401
     star_load,
     starts_load,
     text_load,
+    trace_rays,
     vbox_load,
     vbox_load_subset,
     vbox_store,

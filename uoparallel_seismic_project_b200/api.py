@@ -21,6 +21,8 @@ _LIB = None
 
 KERNEL_AUTO, KERNEL_SIMPLE, KERNEL_TILED = 0, 1, 2
 LOOP_AUTO, LOOP_BATCHED, LOOP_GRAPH = 0, 1, 2
+# status of a traced ray (SWEEPTT_RAY_*, include/sweeptt.h)
+RAY_OK, RAY_UNREACHED, RAY_NOT_FIXED_POINT, RAY_NO_PREDECESSOR, RAY_STALLED, RAY_TRUNCATED = range(6)
 
 
 class SweepError(RuntimeError):
@@ -89,7 +91,7 @@ _EXPORTS = [
     "sweeptt_host_alloc", "sweeptt_host_free",
     "sweeptt_create", "sweeptt_destroy", "sweeptt_set_stream", "sweeptt_set_model", "sweeptt_set_star",
     "sweeptt_set_sources", "sweeptt_run", "sweeptt_step", "sweeptt_reset", "sweeptt_get_tt", "sweeptt_put_tt",
-    "sweeptt_count_violations", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_solve_slabs",
+    "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
     "sweeptt_vbox_load", "sweeptt_vbox_store", "sweeptt_vbox_load_subset", "sweeptt_text_load",
     "sweeptt_star_load", "sweeptt_starts_load", "sweeptt_write_output_tt", "sweeptt_free",
@@ -134,6 +136,8 @@ def load_library() -> C.CDLL:
     lib.sweeptt_get_tt.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
     lib.sweeptt_put_tt.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
     lib.sweeptt_count_violations.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_longlong)]
+    lib.sweeptt_trace_rays.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(START), C.c_int, C.c_int, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_relaxations_per_round.argtypes = [C.c_void_p]
     lib.sweeptt_relaxations_per_round.restype = C.c_longlong
     lib.sweeptt_pool_bytes.argtypes = [C.c_void_p]
@@ -306,6 +310,22 @@ def solve_raw(v_ptr: int, dims, fs, starts_arr, out_ptrs, opts: _Opts):
     return SweepStats._from(s)
 
 
+@dataclass
+class Rays:
+    """Rays of sources [S] x receivers [R] (SweepContext.trace_rays).  nodes[s, r, :length[s, r]] are the ray's nodes
+    (caller axes) from the receiver to the start; entries past the length are -1.  tt[s, r] = travel time at the
+    receiver whatever the status (RAY_*)."""
+    tt: np.ndarray        # float32[S, R]
+    status: np.ndarray    # int32[S, R]
+    length: np.ndarray    # int32[S, R]
+    nodes: np.ndarray     # int32[S, R, max_nodes, 3]
+    stats: SweepStats
+
+    def path(self, s: int, r: int) -> np.ndarray:
+        """int32[L, 3]: the nodes of ray (s, r), receiver first."""
+        return self.nodes[s, r, : self.length[s, r]]
+
+
 class SweepContext:
     """Device-resident context: padded slowness box + pool of travel-time boxes on one GPU."""
 
@@ -380,6 +400,37 @@ class SweepContext:
         _check(self._lib.sweeptt_count_violations(self._h, source, C.byref(n)), "sweeptt_count_violations")
         return n.value
 
+    def trace_rays(self, receivers, sources=None, max_nodes: int | None = None) -> Rays:
+        """Shortest-path rays from every receiver (R,3) back to the start of every source in `sources` (a range or a
+        (begin, count) pair; default: all), read off the converged fields on the device (include/sweeptt.h,
+        sweeptt_trace_rays).  The default max_nodes is nx+ny+nz; when a ray is longer the call is repeated with
+        twice the capacity until none is truncated.  An explicit max_nodes is kept, and longer rays come back
+        RAY_TRUNCATED."""
+        if sources is None:
+            begin, count = 0, self.nsrc
+        elif isinstance(sources, range):
+            if sources.step != 1:
+                raise SweepError("trace_rays: sources must be a contiguous range")
+            begin, count = sources.start, len(sources)
+        else:
+            begin, count = (int(x) for x in sources)
+        rec = _make_starts(receivers)
+        nrec = len(rec)
+        grow = max_nodes is None
+        cap = int(max_nodes) if max_nodes is not None else (sum(self.dims) if self.dims else 1)
+        while True:
+            tt = np.empty((count, nrec), np.float32)
+            status = np.empty((count, nrec), np.int32)
+            length = np.empty((count, nrec), np.int32)
+            nodes = np.full((count, nrec, cap, 3), -1, np.int32)
+            s = _Stats()
+            _check(self._lib.sweeptt_trace_rays(self._h, begin, count, rec, nrec, cap, nodes.ctypes.data,
+                                                length.ctypes.data, status.ctypes.data, tt.ctypes.data, C.byref(s)),
+                   "sweeptt_trace_rays")
+            if not (grow and (status == RAY_TRUNCATED).any()):
+                return Rays(tt, status, length, nodes, SweepStats._from(s))
+            cap *= 2
+
     @property
     def relaxations_per_round(self) -> int:
         return self._lib.sweeptt_relaxations_per_round(self._h)
@@ -391,6 +442,18 @@ class SweepContext:
     @property
     def pool_bytes(self) -> int:
         return self._lib.sweeptt_pool_bytes(self._h)
+
+
+def trace_rays(slowness, star, starts, receivers, *, delta: float = 10.0, max_nodes: int | None = None,
+               device: int | None = None, kernel: int | None = None, star_used: int | None = None) -> Rays:
+    """One-shot: solve every start on one device, then trace rays from every receiver back to each start
+    (SweepContext.trace_rays).  Only the rays and receiver times leave the device, never the fields."""
+    with SweepContext(device=device, kernel=kernel, star_used=star_used) as ctx:
+        ctx.set_model(slowness)
+        ctx.set_star(star, delta)
+        ctx.set_sources(starts)
+        ctx.run()
+        return ctx.trace_rays(receivers, max_nodes=max_nodes)
 
 
 # ---- file formats -------------------------------------------------------------------------

@@ -100,6 +100,16 @@ struct StarDev {   // star as the simple kernel / verifier read it (global memor
   int guarded;
 };
 
+struct RayPull {   // one candidate-predecessor offset of the ray tracer (16 bytes, one LDS.128)
+  short i, j, k;         // kernel-axis offset m - n
+  unsigned short rank;   // bits 0-14: position of the offset in caller-axis lexicographic order (the tie rule:
+                         // for in-bounds m it orders the FLOATBOX index of m); bit 15: guarded (invalid at m == start)
+  int off;               // padded-box offset of m - n
+  float hd;
+};
+constexpr unsigned RAY_GUARD_BIT = 0x8000u;
+constexpr int RAY_MAX_PULLS = 1 << 15;
+
 constexpr int MAX_PARTS = 16;    // devices (or contexts sharing devices) that one grid can be spread over
 
 constexpr int MAX_COLUMNS = 320;

@@ -27,12 +27,16 @@
 //                     verification path and the fallback for stars wider than the halo.
 //   count_violations  the fixed-point invariant (testconvergence,
 //                     old/wavefront-openmp/wave-multistart.c:300-347) on the device.
+//   trace_rays        shortest-path rays from receivers back to the start, read off a converged field
+//                     (one warp per ray, exact-match predecessor with a fixed tie rule).
 //   fill/pad/unpad/init_sources/min_slowness  the device float-box pool's utilities
 //                     (boxsetall/boxput, include/floatbox.h:176-199).
 // One grid over several devices (solver.cu, sweeptt_solve_slabs) runs relax_tiled unchanged on a travel-time box
 // whose pages live block-cyclically on the devices: halo planes arrive over NVLink through the same TMA loads,
 // neighbours on other devices are woken through their owner's key array (RelaxArgs::part_key, tx_owner).
 #include "kernels.h"
+
+#include "../../include/sweeptt.h"
 
 #include <cuda_runtime.h>
 #include <math_constants.h>
@@ -1178,6 +1182,124 @@ __global__ void __launch_bounds__(128) count_violations_kernel(const RelaxArgs a
 }
 
 // ---------------------------------------------------------------------------------------
+// ray tracer (include/sweeptt.h, sweeptt_trace_rays)
+// ---------------------------------------------------------------------------------------
+// One warp per ray, a grid-stride loop over the (source, receiver) pairs in source-major order, so the rays in
+// flight read one source's padded box, which stays in L2.  The pull table is staged once per CTA in shared memory
+// (not __constant__: the 32 lanes read 32 different entries).  Per step lane q evaluates entries q, q+32, ... with
+// the sweep's exact candidate expression; a warp min-reduction over the key (tt[m] in total order, caller-axis rank)
+// of the exact matches picks the predecessor.
+constexpr int TRACE_THREADS = 256;
+constexpr int RAY_BATCH = 4;  // table entries per lane whose gathers are in flight together
+
+// float -> unsigned with the same order (-0 before +0; no NaN ever reaches a key: cand == tt[n] excludes it)
+__device__ __forceinline__ unsigned ordered_bits(float f) {
+  const unsigned u = __float_as_uint(f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+__global__ void __launch_bounds__(TRACE_THREADS) trace_rays_kernel(const TraceArgs t) {
+  extern __shared__ int4 s_pull_raw[];
+  const RayPull* s_pull = reinterpret_cast<const RayPull*>(s_pull_raw);
+#ifdef SWEEPTT_DEBUG_BOUNDS
+  unsigned dyn_smem;
+  asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn_smem));
+  DBG_BOUNDS(t.npull >= 1 && t.npull < RAY_MAX_PULLS && (size_t)t.npull * sizeof(RayPull) <= dyn_smem);
+#endif
+  for (int e = threadIdx.x; e < t.npull; e += blockDim.x) s_pull_raw[e] = reinterpret_cast<const int4*>(t.pull)[e];
+  __syncthreads();
+  const unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+  unsigned long long evals = 0;
+  for (long long q = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); q < t.nrays; q += warps) {
+    const int sr = (int)(q / t.nrec), r = (int)(q % t.nrec);
+    const int s = t.source_begin + sr;
+    const int px = t.src_xyz[3 * s], py = t.src_xyz[3 * s + 1], pz = t.src_xyz[3 * s + 2];
+    const float* tt = t.tt + (size_t)s * t.g.vol;
+    int x = t.rec_xyz[3 * r], y = t.rec_xyz[3 * r + 1], z = t.rec_xyz[3 * r + 2];
+    DBG_BOUNDS((unsigned)x < (unsigned)t.g.nx && (unsigned)y < (unsigned)t.g.ny && (unsigned)z < (unsigned)t.g.nz);
+    long long n = ((long long)(x + AX) * t.g.py + (y + AY)) * t.g.pz + (z + AZ);
+    int* nodes = t.nodes ? t.nodes + (size_t)q * t.max_nodes * 3 : nullptr;
+    auto put = [&](int len, int kx, int ky, int kz) {  // node `len` of the ray, written in caller axes
+      if (nodes && lane == 0) {
+        DBG_BOUNDS(len >= 0 && len < t.max_nodes);
+        for (int a = 0; a < 3; ++a)  // caller axis a is kernel axis q with perm[q] == a
+          nodes[3 * len + a] = t.g.perm[0] == a ? kx : t.g.perm[1] == a ? ky : kz;
+      }
+    };
+    const float t_rec = tt[n];
+    float tn = t_rec;
+    int len = 1, status;
+    put(0, x, y, z);
+    if (tn == CUDART_INF_F) {
+      status = SWEEPTT_RAY_UNREACHED;
+    } else {
+      for (;;) {
+        if (x == px && y == py && z == pz) { status = SWEEPTT_RAY_OK; break; }
+        const float vn = t.slow[n];
+        bool below = false;
+        unsigned long long best = ~0ull;  // (ordered tt[m] << 32) | rank of the best exact match so far
+        int be = 0;                       // ... and its table entry
+        // batches of RAY_BATCH entries per lane: the gathers of a batch are issued together (predicated, from n
+        // itself for pulls that do not count), then evaluated
+        for (int e0 = lane; e0 < t.npull; e0 += 32 * RAY_BATCH) {
+          RayPull o[RAY_BATCH];
+          bool ok[RAY_BATCH];
+          float tm[RAY_BATCH], vm[RAY_BATCH];
+#pragma unroll
+          for (int u = 0; u < RAY_BATCH; ++u) {
+            const int e = e0 + 32 * u;
+            o[u] = s_pull[min(e, t.npull - 1)];
+            const int xo = x + o[u].i, yo = y + o[u].j, zo = z + o[u].k;
+            ok[u] = e < t.npull && (unsigned)xo < (unsigned)t.g.nx && (unsigned)yo < (unsigned)t.g.ny &&
+                    (unsigned)zo < (unsigned)t.g.nz && !((o[u].rank & RAY_GUARD_BIT) && xo == px && yo == py && zo == pz);
+            const long long m = n + (ok[u] ? o[u].off : 0);
+            DBG_BOUNDS(m >= 0 && m < t.g.vol);
+            tm[u] = tt[m];
+            vm[u] = t.slow[m];
+          }
+#pragma unroll
+          for (int u = 0; u < RAY_BATCH; ++u) {
+            const float cand = __fadd_rn(__fmul_rn(o[u].hd, __fadd_rn(vn, vm[u])), tm[u]);
+            evals += ok[u];
+            below |= ok[u] && cand < tn;
+            const unsigned long long key = ((unsigned long long)ordered_bits(tm[u]) << 32) | (o[u].rank & (RAY_GUARD_BIT - 1u));
+            if (ok[u] && cand == tn && key < best) { best = key; be = e0 + 32 * u; }
+          }
+        }
+        if (__any_sync(FULL, below)) { status = SWEEPTT_RAY_NOT_FIXED_POINT; break; }
+        // keys are below ~0 (ordered +INF is 0xff800000), so ~0 means no exact match
+        const unsigned mt = __reduce_min_sync(FULL, (unsigned)(best >> 32));
+        if (mt == ~0u) { status = SWEEPTT_RAY_NO_PREDECESSOR; break; }
+        const unsigned mr = __reduce_min_sync(FULL, (unsigned)(best >> 32) == mt ? (unsigned)best : ~0u);
+        const int w = __ffs(__ballot_sync(FULL, best == (((unsigned long long)mt << 32) | mr))) - 1;
+        DBG_BOUNDS(w >= 0 && w < 32);
+        const int eb = __shfl_sync(FULL, be, w);
+        DBG_BOUNDS(eb >= 0 && eb < t.npull);
+        const RayPull o = s_pull[eb];
+        x += o.i; y += o.j; z += o.k;
+        n += o.off;
+        const float tm = tt[n];
+        if (!(tm < tn)) { status = SWEEPTT_RAY_STALLED; break; }
+        if (len == t.max_nodes) { status = SWEEPTT_RAY_TRUNCATED; break; }
+        put(len, x, y, z);
+        ++len;
+        tn = tm;
+      }
+    }
+    if (lane == 0) {
+      DBG_BOUNDS(q >= 0 && q < t.nrays && len >= 1 && len <= t.max_nodes);
+      t.length[q] = len;
+      t.status[q] = status;
+      t.tt_rec[q] = t_rec;
+    }
+  }
+  for (int o = 16; o; o >>= 1) evals += __shfl_xor_sync(FULL, evals, o);
+  if (lane == 0 && evals) atomicAdd(t.evals, evals);
+}
+
+// ---------------------------------------------------------------------------------------
 // float-box utilities
 // ---------------------------------------------------------------------------------------
 __global__ void fill_kernel(float4* p, long long n4, float value) {
@@ -1525,6 +1647,25 @@ cudaError_t launch_count_violations(const RelaxArgs& a, int source, const StarDe
                                     unsigned long long* out, cudaStream_t stream) {
   dim3 grid(a.g.nx * a.g.ny, (a.g.nz + 127) / 128, 1);
   count_violations_kernel<<<grid, 128, 0, stream>>>(a, source, star, nstar, out);
+  return cudaGetLastError();
+}
+
+size_t trace_rays_smem_bytes(int npull) { return (size_t)npull * sizeof(RayPull); }
+
+cudaError_t launch_trace_rays(const TraceArgs& t, int device, cudaStream_t stream) {
+  static_assert(sizeof(RayPull) == 16, "one LDS.128 per pull entry");
+  const size_t smem = trace_rays_smem_bytes(t.npull);
+  cudaError_t e = cudaFuncSetAttribute(trace_rays_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  int sms = 0, per_sm = 0;
+  e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+  if (e != cudaSuccess) return e;
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trace_rays_kernel, TRACE_THREADS, smem);
+  if (e != cudaSuccess) return e;
+  if (per_sm < 1) return cudaErrorInvalidConfiguration;
+  const long long need = (t.nrays + TRACE_THREADS / 32 - 1) / (TRACE_THREADS / 32);
+  const int grid = (int)std::max(1LL, std::min<long long>(need, (long long)sms * per_sm));
+  trace_rays_kernel<<<grid, TRACE_THREADS, smem, stream>>>(t);
   return cudaGetLastError();
 }
 

@@ -102,6 +102,27 @@ cudaError_t launch_init_sources(const RelaxArgs& a, cudaStream_t stream);
 cudaError_t launch_count_violations(const RelaxArgs& a, int source, const StarDev* star, int nstar,
                                     unsigned long long* out, cudaStream_t stream);
 
+// Ray tracer (include/sweeptt.h, sweeptt_trace_rays): one warp per (source, receiver) pair, source-major.
+struct TraceArgs {
+  BoxGeom g;
+  const float* slow;           // padded slowness box
+  const float* tt;             // padded travel-time boxes of the context
+  const int* src_xyz;          // 3 ints per source (kernel axes)
+  const int* rec_xyz;          // 3 ints per receiver (kernel axes)
+  const RayPull* pull;         // npull entries, sorted by kernel-axis (i,j,k)
+  int npull;
+  int source_begin, nrec;
+  long long nrays;             // source_count * nrec
+  int max_nodes;
+  int* nodes;                  // [nrays * max_nodes * 3] caller-axis node coordinates, or nullptr
+  int* length;                 // [nrays]
+  int* status;                 // [nrays]
+  float* tt_rec;               // [nrays]
+  unsigned long long* evals;   // candidate evaluations executed (one counter)
+};
+size_t trace_rays_smem_bytes(int npull);
+cudaError_t launch_trace_rays(const TraceArgs& t, int device, cudaStream_t stream);
+
 // Box utilities (device float-box pool).
 cudaError_t launch_fill(float* p, long long n, float value, cudaStream_t stream);
 cudaError_t launch_pad_box(const float* dense, float* padded, BoxGeom g, cudaStream_t stream);

@@ -11,6 +11,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -25,6 +26,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "../../include/sweeptt.h"
@@ -156,6 +158,16 @@ struct sweeptt_ctx {
   int pulls_sig[7] = {0, 0, 0, 0, 0, 0, -1};  // geometry + star generation d_tile_pulls was built for
   int star_gen = 0;                           // bumped by every sweeptt_set_star
   unsigned long long* d_viol = nullptr;
+  // ray tracer (sweeptt_trace_rays): pull table, receivers and a grow-only output buffer
+  std::vector<RayPull> ray_pull;
+  RayPull* d_ray_pull = nullptr;
+  size_t ray_pull_cap = 0;
+  int ray_sig[6] = {-1, -1, -1, -1, -1, -1};  // star generation, axis permutation and padded pitches of the table
+  std::vector<int> rec_xyz;
+  int* d_rec = nullptr;
+  size_t rec_cap = 0;
+  unsigned char* d_ray_out = nullptr;
+  size_t ray_out_cap = 0;
   float* d_stage = nullptr;  // dense staging box for pad/unpad
   size_t stage_floats = 0;
   size_t pool_bytes = 0;
@@ -358,6 +370,7 @@ extern "C" void sweeptt_destroy(sweeptt_ctx* c) {
   cudaFree(c->d_src); cudaFree(c->d_state);
   cudaFree(c->d_worklist); cudaFree(c->d_key); cudaFree(c->d_tmax); cudaFree(c->d_busy); cudaFree(c->d_keysnap); cudaFree(c->d_tile_pulls); cudaFree(c->d_viol);
   cudaFree(c->d_stage); cudaFree(c->d_star);
+  cudaFree(c->d_ray_pull); cudaFree(c->d_rec); cudaFree(c->d_ray_out);
   if (c->h_state) cudaFreeHost(c->h_state);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
@@ -1470,6 +1483,153 @@ extern "C" int sweeptt_count_violations(sweeptt_ctx* c, int s, long long* violat
   CK(cudaMemcpyAsync(&v, c->d_viol, 8, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   *violations = (long long)v;
+  return 1;
+}
+
+// Grow-only device buffer counted in pool_bytes.
+template <typename T>
+static int ensure_dev(sweeptt_ctx* c, T** p, size_t* cap_bytes, size_t bytes) {
+  if (*cap_bytes >= bytes) return 1;
+  dev_free(c, *p, *cap_bytes);
+  *p = nullptr; *cap_bytes = 0;
+  if (!dev_alloc(c, (void**)p, bytes)) return 0;
+  *cap_bytes = bytes;
+  return 1;
+}
+
+// Pull table of the ray tracer: the context's pull star (kernel axes) with each entry's padded-box offset and its
+// rank in caller-axis lexicographic order, sorted by kernel-axis (i,j,k) so that the lanes of one step read
+// neighbouring z addresses.  Rebuilt when the star, the axis permutation or the padded geometry changes.
+static int build_ray_pulls(sweeptt_ctx* c) {
+  const BoxGeom& g = c->g;
+  const int sig[6] = {c->star_gen, g.perm[0], g.perm[1], g.perm[2], g.py, g.pz};
+  if (c->d_ray_pull && std::memcmp(sig, c->ray_sig, sizeof sig) == 0) return 1;
+  const std::vector<PullOffset>& all = c->star.all;
+  const int n = (int)all.size();
+  if (n >= RAY_MAX_PULLS) return fail("sweeptt_trace_rays: %d pull offsets, the tracer holds fewer than %d", n, RAY_MAX_PULLS);
+  std::vector<std::array<int, 3>> caller(n);
+  for (int l = 0; l < n; ++l) {
+    const int k[3] = {all[l].i, all[l].j, all[l].k};
+    for (int q = 0; q < 3; ++q) caller[l][g.perm[q]] = k[q];
+  }
+  std::vector<int> by_caller(n);
+  for (int l = 0; l < n; ++l) by_caller[l] = l;
+  std::sort(by_caller.begin(), by_caller.end(), [&](int a, int b) { return caller[a] < caller[b]; });
+  std::vector<int> rank(n);
+  for (int p = 0, r = 0; p < n; ++p) {  // equal offsets (same m) share a rank
+    if (p > 0 && caller[by_caller[p]] != caller[by_caller[p - 1]]) ++r;
+    rank[by_caller[p]] = r;
+  }
+  std::vector<int> by_kernel(n);
+  for (int l = 0; l < n; ++l) by_kernel[l] = l;
+  std::stable_sort(by_kernel.begin(), by_kernel.end(), [&](int a, int b) {
+    return std::tie(all[a].i, all[a].j, all[a].k) < std::tie(all[b].i, all[b].j, all[b].k);
+  });
+  c->ray_pull.resize(n);
+  for (int p = 0; p < n; ++p) {
+    const PullOffset& o = all[by_kernel[p]];
+    if (std::abs(o.i) > 32767 || std::abs(o.j) > 32767 || std::abs(o.k) > 32767)
+      return fail("sweeptt_trace_rays: star offset (%d,%d,%d) is wider than the tracer's 16-bit offsets", o.i, o.j, o.k);
+    const long long off = (long long)o.i * g.sx + (long long)o.j * g.pz + o.k;
+    if (off > INT32_MAX || off < INT32_MIN) return fail("sweeptt_trace_rays: star offset (%d,%d,%d) too wide for this box", o.i, o.j, o.k);
+    c->ray_pull[p] = RayPull{(short)o.i, (short)o.j, (short)o.k,
+                             (unsigned short)(rank[by_kernel[p]] | (o.guarded ? RAY_GUARD_BIT : 0u)), (int)off, o.hd};
+  }
+  if (!ensure_dev(c, &c->d_ray_pull, &c->ray_pull_cap, (size_t)n * sizeof(RayPull))) return 0;
+  CK(cudaMemcpyAsync(c->d_ray_pull, c->ray_pull.data(), (size_t)n * sizeof(RayPull), cudaMemcpyHostToDevice, c->stream));
+  std::memcpy(c->ray_sig, sig, sizeof sig);
+  return 1;
+}
+
+extern "C" int sweeptt_trace_rays(sweeptt_ctx* c, int source_begin, int source_count, const struct START* receivers,
+                                  int nrec, int max_nodes, struct START* nodes_out, int32_t* length_out,
+                                  int32_t* status_out, float* tt_out, sweeptt_stats* stats) {
+  ConstLease lease;
+  if (!ready(c, &lease)) return 0;
+  if (stats) std::memset(stats, 0, sizeof *stats);
+  if (!receivers || nrec < 1) return fail("sweeptt_trace_rays: need at least one receiver");
+  if (source_count < 1 || source_begin < 0 || source_begin > c->nsrc - source_count)
+    return fail("sweeptt_trace_rays: sources [%d, %d) are not within the context's %d sources", source_begin,
+                source_begin + source_count, c->nsrc);
+  if (max_nodes < 1) return fail("sweeptt_trace_rays: max_nodes must be >= 1 (got %d)", max_nodes);
+  const BoxGeom& g = c->g;
+  int on[3];  // caller-order dims
+  on[g.perm[0]] = g.nx; on[g.perm[1]] = g.ny; on[g.perm[2]] = g.nz;
+  c->rec_xyz.resize(3 * (size_t)nrec);
+  for (int r = 0; r < nrec; ++r) {
+    const int o[3] = {receivers[r].i, receivers[r].j, receivers[r].k};
+    if (o[0] < 0 || o[0] >= on[0] || o[1] < 0 || o[1] >= on[1] || o[2] < 0 || o[2] >= on[2])
+      return fail("receiver %d (%d,%d,%d) is outside the %d x %d x %d model", r, o[0], o[1], o[2], on[0], on[1], on[2]);
+    for (int q = 0; q < 3; ++q) c->rec_xyz[3 * (size_t)r + q] = o[g.perm[q]];
+  }
+  const long long nrays = (long long)source_count * nrec;
+  if (nodes_out && (unsigned long long)nrays > (1ull << 60) / (12ull * (unsigned long long)max_nodes))
+    return fail("sweeptt_trace_rays: %lld rays of up to %d nodes do not fit one call", nrays, max_nodes);
+  if (!build_ray_pulls(c)) return 0;
+  if (!ensure_dev(c, &c->d_rec, &c->rec_cap, 3 * sizeof(int) * (size_t)nrec)) return 0;
+  CK(cudaMemcpyAsync(c->d_rec, c->rec_xyz.data(), 3 * sizeof(int) * (size_t)nrec, cudaMemcpyHostToDevice, c->stream));
+  // output buffer: [evaluation counter | length | status | tt | nodes], every part 16-byte aligned
+  auto up16 = [](size_t b) { return (b + 15) / 16 * 16; };
+  const size_t per_ray = up16(4 * (size_t)nrays);
+  const size_t node_bytes = nodes_out ? (size_t)nrays * max_nodes * sizeof(START) : 0;
+  if (!ensure_dev(c, &c->d_ray_out, &c->ray_out_cap, 16 + 3 * per_ray + node_bytes)) return 0;
+  TraceArgs t{};
+  t.g = g;
+  t.slow = c->d_slow;
+  t.tt = c->d_tt;
+  t.src_xyz = c->d_src;
+  t.rec_xyz = c->d_rec;
+  t.pull = c->d_ray_pull;
+  t.npull = (int)c->ray_pull.size();
+  t.source_begin = source_begin;
+  t.nrec = nrec;
+  t.nrays = nrays;
+  t.max_nodes = max_nodes;
+  t.evals = reinterpret_cast<unsigned long long*>(c->d_ray_out);
+  t.length = reinterpret_cast<int*>(c->d_ray_out + 16);
+  t.status = reinterpret_cast<int*>(c->d_ray_out + 16 + per_ray);
+  t.tt_rec = reinterpret_cast<float*>(c->d_ray_out + 16 + 2 * per_ray);
+  t.nodes = nodes_out ? reinterpret_cast<int*>(c->d_ray_out + 16 + 3 * per_ray) : nullptr;
+  CK(cudaMemsetAsync(t.evals, 0, 8, c->stream));
+  if (t.nodes) CK(cudaMemsetAsync(t.nodes, 0xff, node_bytes, c->stream));  // (-1,-1,-1) past every ray's length
+  CK(cudaEventRecord(c->ev0, c->stream));
+  CK(launch_trace_rays(t, c->device, c->stream));
+  CK(cudaEventRecord(c->ev1, c->stream));
+  CK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+
+  const auto t_copy = std::chrono::steady_clock::now();
+  std::vector<int32_t> len_tmp;
+  int32_t* len_host = length_out;
+  if (!len_host && nodes_out) { len_tmp.resize(nrays); len_host = len_tmp.data(); }
+  unsigned long long evals = 0;
+  long long bytes = 8;
+  CK(cudaMemcpyAsync(&evals, t.evals, 8, cudaMemcpyDeviceToHost, c->stream));
+  if (len_host) { CK(cudaMemcpyAsync(len_host, t.length, 4 * nrays, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * nrays; }
+  if (status_out) { CK(cudaMemcpyAsync(status_out, t.status, 4 * nrays, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * nrays; }
+  if (tt_out) { CK(cudaMemcpyAsync(tt_out, t.tt_rec, 4 * nrays, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * nrays; }
+  CK(cudaStreamSynchronize(c->stream));
+  if (nodes_out) {
+    // only the first max(length) nodes of every ray's slot travel; the rest of nodes_out is left untouched
+    const int lmax = *std::max_element(len_host, len_host + nrays);
+    const size_t pitch = (size_t)max_nodes * sizeof(START), width = (size_t)lmax * sizeof(START);
+    if (lmax == max_nodes)
+      CK(cudaMemcpyAsync(nodes_out, t.nodes, node_bytes, cudaMemcpyDeviceToHost, c->stream));
+    else
+      CK(cudaMemcpy2DAsync(nodes_out, pitch, t.nodes, pitch, width, (size_t)nrays, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    bytes += (long long)(width * nrays);
+  }
+  if (stats) {
+    stats->struct_size = (int)sizeof *stats;
+    stats->solve_ms = ms;
+    stats->relaxations = (long long)evals;
+    stats->kernel_launches = 1;
+    stats->devices_used = 1;
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes = bytes;
+  }
   return 1;
 }
 
