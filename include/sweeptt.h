@@ -248,6 +248,42 @@ int sweeptt_trace_rays(sweeptt_ctx *ctx, int source_begin, int source_count,
                        int32_t *length_out, int32_t *status_out, float *tt_out, /* [source_count*nrec] */
                        sweeptt_stats *stats);
 
+/* ---- tomography: the linear operators of a travel-time inversion over the rays -------- */
+
+/* Both calls trace exactly the rays of sweeptt_trace_rays (same predecessor rule, statuses and max_nodes
+ * truncation; ray q = (s - source_begin)*nrec + r) and use only the rays with status SWEEPTT_RAY_OK.  The edges of
+ * a ray are its consecutive node pairs (n, m), n nearer the receiver, each with hd = 0.5f*d of its star offset (the
+ * sweep's hd).  Nothing but the results leaves the device.  Argument checks, the stream, the synchronisation at the
+ * end and stats (solve_ms = device time, relaxations = candidate evaluations, kernel_launches, d2h_ms / d2h_bytes)
+ * are those of sweeptt_trace_rays.
+ *
+ * Projection (G*d): proj_out[q] is the perturbation summed along ray q with the sweep's own expression, from the
+ * start point towards the receiver: acc = +0; for each edge from the start end, acc = fl(fl(hd*fl(d_n + d_m)) + acc).
+ * A ray of one node gives +0, a ray that is not OK a quiet NaN.  So the projection of the slowness itself equals
+ * tt[receiver] bit for bit for every OK ray of a converged field.  Perturbation values are not validated (they
+ * propagate per IEEE).  perturbation: nx*ny*nz floats, FLOATBOX order, caller axes.  Outputs may be NULL. */
+int sweeptt_ray_project(sweeptt_ctx *ctx, int source_begin, int source_count,
+                        const struct START *receivers, int nrec, int max_nodes,
+                        const float *perturbation,          /* nx*ny*nz, FLOATBOX, caller axes */
+                        float *proj_out, int32_t *status_out, int32_t *length_out, /* [source_count*nrec], may be NULL */
+                        sweeptt_stats *stats);
+
+/* Back-projection (G^T*w): grad[j] = sum over OK rays q, over the edges e of q that touch node j, of w_q*hd_e (an
+ * interior node of a ray gets the hd of its two edges, the receiver and the start one each; w = 1 gives the ray
+ * coverage).  Exact and deterministic: with hd_max the largest hd of the used star entries, W = max|w_q| and
+ * N = source_count*nrec, E is the smallest integer with 2*hd_max*W*N <= 2^(E+62); every contribution
+ * c = rint_even(w_q*hd_e*2^-E) (an int64; w*hd is exact in double) is added to both ends of its edge in int64, and
+ * grad[j] = S_j*2^E is rounded once to float32 (nearest, ties to even, subnormals included).  A ray visits a node
+ * at most once (travel time strictly decreases along it), so no sum overflows.  *quantum_exp_out = E.  W = 0 (or a
+ * star whose hd are all 0) gives all +0 and E = 0.  weights: [source_count*nrec], finite, required; grad_out:
+ * nx*ny*nz floats, FLOATBOX order, caller axes, required; quantum_exp_out and status_out may be NULL. */
+int sweeptt_ray_backproject(sweeptt_ctx *ctx, int source_begin, int source_count,
+                            const struct START *receivers, int nrec, int max_nodes,
+                            const float *weights,               /* [source_count*nrec], finite */
+                            float *grad_out,                    /* nx*ny*nz, FLOATBOX, caller axes */
+                            int *quantum_exp_out, int32_t *status_out, /* may be NULL */
+                            sweeptt_stats *stats);
+
 /* In-bounds pull evaluations of one full round of one source (analytic). */
 long long sweeptt_relaxations_per_round(sweeptt_ctx *ctx);
 /* Bytes of device memory currently held by the context's pool. */

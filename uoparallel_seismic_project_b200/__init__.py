@@ -8,6 +8,9 @@ raises ``SweepError`` when the extension or a CUDA device is missing.
 """
 from .api import (  # noqa: F401
     FS,
+    Backprojection,
+    MisfitGradient,
+    RayProjection,
     Rays,
     START,
     SweepContext,
@@ -24,6 +27,7 @@ from .api import (  # noqa: F401
     star_load,
     starts_load,
     text_load,
+    misfit_gradient,
     trace_rays,
     vbox_load,
     vbox_load_subset,

@@ -91,7 +91,7 @@ _EXPORTS = [
     "sweeptt_host_alloc", "sweeptt_host_free",
     "sweeptt_create", "sweeptt_destroy", "sweeptt_set_stream", "sweeptt_set_model", "sweeptt_set_star",
     "sweeptt_set_sources", "sweeptt_run", "sweeptt_step", "sweeptt_reset", "sweeptt_get_tt", "sweeptt_put_tt",
-    "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_solve_slabs",
+    "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
     "sweeptt_vbox_load", "sweeptt_vbox_store", "sweeptt_vbox_load_subset", "sweeptt_text_load",
     "sweeptt_star_load", "sweeptt_starts_load", "sweeptt_write_output_tt", "sweeptt_free",
@@ -138,6 +138,10 @@ def load_library() -> C.CDLL:
     lib.sweeptt_count_violations.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_longlong)]
     lib.sweeptt_trace_rays.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(START), C.c_int, C.c_int, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
+    lib.sweeptt_ray_project.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(START), C.c_int, C.c_int, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
+    lib.sweeptt_ray_backproject.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(START), C.c_int, C.c_int,
+                                            C.c_void_p, C.c_void_p, C.POINTER(C.c_int), C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_relaxations_per_round.argtypes = [C.c_void_p]
     lib.sweeptt_relaxations_per_round.restype = C.c_longlong
     lib.sweeptt_pool_bytes.argtypes = [C.c_void_p]
@@ -326,6 +330,39 @@ class Rays:
         return self.nodes[s, r, : self.length[s, r]]
 
 
+@dataclass
+class RayProjection:
+    """G*d over the rays of sources [S] x receivers [R] (SweepContext.ray_project): values[s, r] is the perturbation
+    summed along the ray with the sweep's expression from the start towards the receiver (NaN unless status is
+    RAY_OK); the projection of the slowness itself is the receiver's travel time, bit for bit."""
+    values: np.ndarray    # float32[S, R]
+    status: np.ndarray    # int32[S, R]
+    length: np.ndarray    # int32[S, R]
+    stats: SweepStats
+
+
+@dataclass
+class Backprojection:
+    """G^T*w (SweepContext.ray_backproject): grad[nx, ny, nz] = sum over the OK rays of w times the half edge length
+    of every ray edge touching the node, accumulated exactly in integer quanta of 2^quantum_exp and rounded once."""
+    grad: np.ndarray      # float32[nx, ny, nz]
+    quantum_exp: int
+    status: np.ndarray    # int32[S, R]
+    stats: SweepStats
+
+
+@dataclass
+class MisfitGradient:
+    """misfit_gradient: misfit = 1/2 sum residual^2 (float64) over the OK rays with a pick; residual[s, r] =
+    float32(tt_receiver - observed), NaN where the ray is not OK or has no pick; gradient = G^T*residual over those
+    rays (ray_backproject, quantum 2^quantum_exp)."""
+    misfit: float
+    gradient: np.ndarray  # float32[nx, ny, nz]
+    residual: np.ndarray  # float32[S, R]
+    status: np.ndarray    # int32[S, R]
+    quantum_exp: int
+
+
 class SweepContext:
     """Device-resident context: padded slowness box + pool of travel-time boxes on one GPU."""
 
@@ -400,25 +437,38 @@ class SweepContext:
         _check(self._lib.sweeptt_count_violations(self._h, source, C.byref(n)), "sweeptt_count_violations")
         return n.value
 
+    def _source_range(self, sources, who):
+        if sources is None:
+            return 0, self.nsrc
+        if isinstance(sources, range):
+            if sources.step != 1:
+                raise SweepError(f"{who}: sources must be a contiguous range")
+            return sources.start, len(sources)
+        begin, count = (int(x) for x in sources)
+        return begin, count
+
+    def _ray_calls(self, max_nodes, call):
+        """The max_nodes policy of the ray calls: call(cap) -> (result, status), repeated with twice the capacity
+        (from nx+ny+nz) while a ray is RAY_TRUNCATED, unless max_nodes is given."""
+        grow = max_nodes is None
+        cap = int(max_nodes) if max_nodes is not None else (sum(self.dims) if self.dims else 1)
+        while True:
+            out, status = call(cap)
+            if not (grow and (status == RAY_TRUNCATED).any()):
+                return out
+            cap *= 2
+
     def trace_rays(self, receivers, sources=None, max_nodes: int | None = None) -> Rays:
         """Shortest-path rays from every receiver (R,3) back to the start of every source in `sources` (a range or a
         (begin, count) pair; default: all), read off the converged fields on the device (include/sweeptt.h,
         sweeptt_trace_rays).  The default max_nodes is nx+ny+nz; when a ray is longer the call is repeated with
         twice the capacity until none is truncated.  An explicit max_nodes is kept, and longer rays come back
         RAY_TRUNCATED."""
-        if sources is None:
-            begin, count = 0, self.nsrc
-        elif isinstance(sources, range):
-            if sources.step != 1:
-                raise SweepError("trace_rays: sources must be a contiguous range")
-            begin, count = sources.start, len(sources)
-        else:
-            begin, count = (int(x) for x in sources)
+        begin, count = self._source_range(sources, "trace_rays")
         rec = _make_starts(receivers)
         nrec = len(rec)
-        grow = max_nodes is None
-        cap = int(max_nodes) if max_nodes is not None else (sum(self.dims) if self.dims else 1)
-        while True:
+
+        def call(cap):
             tt = np.empty((count, nrec), np.float32)
             status = np.empty((count, nrec), np.int32)
             length = np.empty((count, nrec), np.int32)
@@ -427,9 +477,54 @@ class SweepContext:
             _check(self._lib.sweeptt_trace_rays(self._h, begin, count, rec, nrec, cap, nodes.ctypes.data,
                                                 length.ctypes.data, status.ctypes.data, tt.ctypes.data, C.byref(s)),
                    "sweeptt_trace_rays")
-            if not (grow and (status == RAY_TRUNCATED).any()):
-                return Rays(tt, status, length, nodes, SweepStats._from(s))
-            cap *= 2
+            return Rays(tt, status, length, nodes, SweepStats._from(s)), status
+
+        return self._ray_calls(max_nodes, call)
+
+    def ray_project(self, perturbation, receivers, sources=None, max_nodes: int | None = None) -> RayProjection:
+        """G*d: the perturbation (nx, ny, nz) summed along the ray of every (source, receiver) pair, on the device
+        (include/sweeptt.h, sweeptt_ray_project).  Sources and max_nodes as in trace_rays."""
+        begin, count = self._source_range(sources, "ray_project")
+        d = np.ascontiguousarray(perturbation, dtype=np.float32)
+        if self.dims is None or d.shape != tuple(self.dims):
+            raise SweepError(f"ray_project: perturbation of shape {d.shape}, the model is {self.dims}")
+        rec = _make_starts(receivers)
+        nrec = len(rec)
+
+        def call(cap):
+            values = np.empty((count, nrec), np.float32)
+            status = np.empty((count, nrec), np.int32)
+            length = np.empty((count, nrec), np.int32)
+            s = _Stats()
+            _check(self._lib.sweeptt_ray_project(self._h, begin, count, rec, nrec, cap, d.ctypes.data,
+                                                 values.ctypes.data, status.ctypes.data, length.ctypes.data,
+                                                 C.byref(s)), "sweeptt_ray_project")
+            return RayProjection(values, status, length, SweepStats._from(s)), status
+
+        return self._ray_calls(max_nodes, call)
+
+    def ray_backproject(self, weights, receivers, sources=None, max_nodes: int | None = None) -> Backprojection:
+        """G^T*w: the weights [S, R] (finite; usually travel-time residuals) back-projected onto the grid along the
+        rays, exactly and deterministically (include/sweeptt.h, sweeptt_ray_backproject).  w = 1 gives the ray
+        coverage.  Sources and max_nodes as in trace_rays."""
+        begin, count = self._source_range(sources, "ray_backproject")
+        rec = _make_starts(receivers)
+        nrec = len(rec)
+        w = np.ascontiguousarray(weights, dtype=np.float32)
+        if w.shape != (count, nrec):
+            raise SweepError(f"ray_backproject: weights of shape {w.shape}, expected {(count, nrec)}")
+
+        def call(cap):
+            grad = np.empty(self.dims, np.float32)
+            status = np.empty((count, nrec), np.int32)
+            e = C.c_int(0)
+            s = _Stats()
+            _check(self._lib.sweeptt_ray_backproject(self._h, begin, count, rec, nrec, cap, w.ctypes.data,
+                                                     grad.ctypes.data, C.byref(e), status.ctypes.data, C.byref(s)),
+                   "sweeptt_ray_backproject")
+            return Backprojection(grad, e.value, status, SweepStats._from(s)), status
+
+        return self._ray_calls(max_nodes, call)
 
     @property
     def relaxations_per_round(self) -> int:
@@ -454,6 +549,43 @@ def trace_rays(slowness, star, starts, receivers, *, delta: float = 10.0, max_no
         ctx.set_sources(starts)
         ctx.run()
         return ctx.trace_rays(receivers, max_nodes=max_nodes)
+
+
+def misfit_gradient(slowness, star, starts, receivers, observed, *, delta: float = 10.0, device: int | None = None,
+                    kernel: int | None = None, star_used: int | None = None) -> MisfitGradient:
+    """One-shot gradient of the ray-linearised travel-time misfit 1/2 sum (t - observed)^2 with respect to slowness.
+
+    Solves every start, reads the receiver times (trace_rays with max_nodes=1: one step per ray), forms
+    residual = float32(t - observed) (a NaN in observed [S, R] means no pick: weight 0) and back-projects the residuals
+    of the OK rays (SweepContext.ray_backproject).  The misfit is summed in float64 over the OK rays with a pick; every
+    other residual is NaN, and the gradient equals ray_backproject of the residuals with those NaN set to 0.
+
+    The gradient is that of the misfit with the rays held fixed.  The discrete travel time is a minimum over paths of
+    sums linear in the slowness, so it is concave: the row of G of a ray is a supergradient of that ray's travel time
+    (T(v + h) <= T(v) + G h up to rounding), and its exact derivative wherever the predecessor of every node on the ray
+    is unique."""
+    obs = np.asarray(observed, dtype=np.float32)
+    with SweepContext(device=device, kernel=kernel, star_used=star_used) as ctx:
+        ctx.set_model(slowness)
+        ctx.set_star(star, delta)
+        ctx.set_sources(starts)
+        ctx.run()
+        rec = _make_starts(receivers)
+        if obs.shape != (ctx.nsrc, len(rec)):
+            raise SweepError(f"misfit_gradient: observed of shape {obs.shape}, expected {(ctx.nsrc, len(rec))}")
+        t = ctx.trace_rays(receivers, max_nodes=1).tt
+        with np.errstate(invalid="ignore", over="ignore"):
+            residual = (t - obs).astype(np.float32)
+        use = np.isfinite(residual)   # a pick, and a reached receiver
+        while True:
+            bp = ctx.ray_backproject(np.where(use, residual, np.float32(0)), receivers)
+            ok = use & (bp.status == RAY_OK)
+            if (ok == use).all():
+                break
+            use = ok   # a ray with a weight turned out not OK: drop it, so the quantum depends on the used rays only
+    residual = np.where(use, residual, np.float32(np.nan)).astype(np.float32)
+    misfit = 0.5 * float(np.sum(residual[use].astype(np.float64) ** 2))
+    return MisfitGradient(misfit, bp.grad, residual, bp.status, bp.quantum_exp)
 
 
 # ---- file formats -------------------------------------------------------------------------

@@ -29,6 +29,8 @@
 //                     old/wavefront-openmp/wave-multistart.c:300-347) on the device.
 //   trace_rays        shortest-path rays from receivers back to the start, read off a converged field
 //                     (one warp per ray, exact-match predecessor with a fixed tie rule).
+//   ray_project / ray_backproject  the travel-time tomography operators G*d and G^T*w over those rays (the tracer's
+//                     predecessor step, then a walk of the recorded path; exact int64 accumulation for G^T*w).
 //   fill/pad/unpad/init_sources/min_slowness  the device float-box pool's utilities
 //                     (boxsetall/boxput, include/floatbox.h:176-199).
 // One grid over several devices (solver.cu, sweeptt_solve_slabs) runs relax_tiled unchanged on a travel-time box
@@ -1198,16 +1200,80 @@ __device__ __forceinline__ unsigned ordered_bits(float f) {
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 
+// Stages the pull table in shared memory (once per CTA).
+__device__ __forceinline__ const RayPull* stage_ray_pulls(const TraceArgs& t, int4* s_pull_raw) {
+  for (int e = threadIdx.x; e < t.npull; e += blockDim.x) s_pull_raw[e] = reinterpret_cast<const int4*>(t.pull)[e];
+  __syncthreads();
+  return reinterpret_cast<const RayPull*>(s_pull_raw);
+}
+
+// One predecessor step of the warp's ray from node n (kernel axes x,y,z; padded index n; tn = tt[n]; n is not the
+// start p): every lane evaluates its share of the pull table, the exact-match key reduction picks pred(n).  Returns
+// the status that ends the ray (NOT_FIXED_POINT, NO_PREDECESSOR, STALLED), or -1 after moving (x,y,z,n,tn) to pred(n);
+// *eb_out is the table entry of the step, the same on every lane.
+__device__ __forceinline__ int ray_pred_step(const TraceArgs& t, const RayPull* s_pull, const float* tt, int px,
+                                             int py, int pz, int& x, int& y, int& z, long long& n, float& tn,
+                                             int* eb_out, unsigned long long& evals) {
+  const unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  const float vn = t.slow[n];
+  bool below = false;
+  unsigned long long best = ~0ull;  // (ordered tt[m] << 32) | rank of the best exact match so far
+  int be = 0;                       // ... and its table entry
+  // batches of RAY_BATCH entries per lane: the gathers of a batch are issued together (predicated, from n
+  // itself for pulls that do not count), then evaluated
+  for (int e0 = lane; e0 < t.npull; e0 += 32 * RAY_BATCH) {
+    RayPull o[RAY_BATCH];
+    bool ok[RAY_BATCH];
+    float tm[RAY_BATCH], vm[RAY_BATCH];
+#pragma unroll
+    for (int u = 0; u < RAY_BATCH; ++u) {
+      const int e = e0 + 32 * u;
+      o[u] = s_pull[min(e, t.npull - 1)];
+      const int xo = x + o[u].i, yo = y + o[u].j, zo = z + o[u].k;
+      ok[u] = e < t.npull && (unsigned)xo < (unsigned)t.g.nx && (unsigned)yo < (unsigned)t.g.ny &&
+              (unsigned)zo < (unsigned)t.g.nz && !((o[u].rank & RAY_GUARD_BIT) && xo == px && yo == py && zo == pz);
+      const long long m = n + (ok[u] ? o[u].off : 0);
+      DBG_BOUNDS(m >= 0 && m < t.g.vol);
+      tm[u] = tt[m];
+      vm[u] = t.slow[m];
+    }
+#pragma unroll
+    for (int u = 0; u < RAY_BATCH; ++u) {
+      const float cand = __fadd_rn(__fmul_rn(o[u].hd, __fadd_rn(vn, vm[u])), tm[u]);
+      evals += ok[u];
+      below |= ok[u] && cand < tn;
+      const unsigned long long key = ((unsigned long long)ordered_bits(tm[u]) << 32) | (o[u].rank & (RAY_GUARD_BIT - 1u));
+      if (ok[u] && cand == tn && key < best) { best = key; be = e0 + 32 * u; }
+    }
+  }
+  if (__any_sync(FULL, below)) return SWEEPTT_RAY_NOT_FIXED_POINT;
+  // keys are below ~0 (ordered +INF is 0xff800000), so ~0 means no exact match
+  const unsigned mt = __reduce_min_sync(FULL, (unsigned)(best >> 32));
+  if (mt == ~0u) return SWEEPTT_RAY_NO_PREDECESSOR;
+  const unsigned mr = __reduce_min_sync(FULL, (unsigned)(best >> 32) == mt ? (unsigned)best : ~0u);
+  const int w = __ffs(__ballot_sync(FULL, best == (((unsigned long long)mt << 32) | mr))) - 1;
+  DBG_BOUNDS(w >= 0 && w < 32);
+  const int eb = __shfl_sync(FULL, be, w);
+  DBG_BOUNDS(eb >= 0 && eb < t.npull);
+  const RayPull o = s_pull[eb];
+  x += o.i; y += o.j; z += o.k;
+  n += o.off;
+  const float tm = tt[n];
+  if (!(tm < tn)) return SWEEPTT_RAY_STALLED;
+  tn = tm;
+  *eb_out = eb;
+  return -1;
+}
+
 __global__ void __launch_bounds__(TRACE_THREADS) trace_rays_kernel(const TraceArgs t) {
   extern __shared__ int4 s_pull_raw[];
-  const RayPull* s_pull = reinterpret_cast<const RayPull*>(s_pull_raw);
 #ifdef SWEEPTT_DEBUG_BOUNDS
   unsigned dyn_smem;
   asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn_smem));
   DBG_BOUNDS(t.npull >= 1 && t.npull < RAY_MAX_PULLS && (size_t)t.npull * sizeof(RayPull) <= dyn_smem);
 #endif
-  for (int e = threadIdx.x; e < t.npull; e += blockDim.x) s_pull_raw[e] = reinterpret_cast<const int4*>(t.pull)[e];
-  __syncthreads();
+  const RayPull* s_pull = stage_ray_pulls(t, s_pull_raw);
   const unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31;
   const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
@@ -1237,55 +1303,12 @@ __global__ void __launch_bounds__(TRACE_THREADS) trace_rays_kernel(const TraceAr
     } else {
       for (;;) {
         if (x == px && y == py && z == pz) { status = SWEEPTT_RAY_OK; break; }
-        const float vn = t.slow[n];
-        bool below = false;
-        unsigned long long best = ~0ull;  // (ordered tt[m] << 32) | rank of the best exact match so far
-        int be = 0;                       // ... and its table entry
-        // batches of RAY_BATCH entries per lane: the gathers of a batch are issued together (predicated, from n
-        // itself for pulls that do not count), then evaluated
-        for (int e0 = lane; e0 < t.npull; e0 += 32 * RAY_BATCH) {
-          RayPull o[RAY_BATCH];
-          bool ok[RAY_BATCH];
-          float tm[RAY_BATCH], vm[RAY_BATCH];
-#pragma unroll
-          for (int u = 0; u < RAY_BATCH; ++u) {
-            const int e = e0 + 32 * u;
-            o[u] = s_pull[min(e, t.npull - 1)];
-            const int xo = x + o[u].i, yo = y + o[u].j, zo = z + o[u].k;
-            ok[u] = e < t.npull && (unsigned)xo < (unsigned)t.g.nx && (unsigned)yo < (unsigned)t.g.ny &&
-                    (unsigned)zo < (unsigned)t.g.nz && !((o[u].rank & RAY_GUARD_BIT) && xo == px && yo == py && zo == pz);
-            const long long m = n + (ok[u] ? o[u].off : 0);
-            DBG_BOUNDS(m >= 0 && m < t.g.vol);
-            tm[u] = tt[m];
-            vm[u] = t.slow[m];
-          }
-#pragma unroll
-          for (int u = 0; u < RAY_BATCH; ++u) {
-            const float cand = __fadd_rn(__fmul_rn(o[u].hd, __fadd_rn(vn, vm[u])), tm[u]);
-            evals += ok[u];
-            below |= ok[u] && cand < tn;
-            const unsigned long long key = ((unsigned long long)ordered_bits(tm[u]) << 32) | (o[u].rank & (RAY_GUARD_BIT - 1u));
-            if (ok[u] && cand == tn && key < best) { best = key; be = e0 + 32 * u; }
-          }
-        }
-        if (__any_sync(FULL, below)) { status = SWEEPTT_RAY_NOT_FIXED_POINT; break; }
-        // keys are below ~0 (ordered +INF is 0xff800000), so ~0 means no exact match
-        const unsigned mt = __reduce_min_sync(FULL, (unsigned)(best >> 32));
-        if (mt == ~0u) { status = SWEEPTT_RAY_NO_PREDECESSOR; break; }
-        const unsigned mr = __reduce_min_sync(FULL, (unsigned)(best >> 32) == mt ? (unsigned)best : ~0u);
-        const int w = __ffs(__ballot_sync(FULL, best == (((unsigned long long)mt << 32) | mr))) - 1;
-        DBG_BOUNDS(w >= 0 && w < 32);
-        const int eb = __shfl_sync(FULL, be, w);
-        DBG_BOUNDS(eb >= 0 && eb < t.npull);
-        const RayPull o = s_pull[eb];
-        x += o.i; y += o.j; z += o.k;
-        n += o.off;
-        const float tm = tt[n];
-        if (!(tm < tn)) { status = SWEEPTT_RAY_STALLED; break; }
+        int eb;
+        status = ray_pred_step(t, s_pull, tt, px, py, pz, x, y, z, n, tn, &eb, evals);
+        if (status >= 0) break;
         if (len == t.max_nodes) { status = SWEEPTT_RAY_TRUNCATED; break; }
         put(len, x, y, z);
         ++len;
-        tn = tm;
       }
     }
     if (lane == 0) {
@@ -1297,6 +1320,209 @@ __global__ void __launch_bounds__(TRACE_THREADS) trace_rays_kernel(const TraceAr
   }
   for (int o = 16; o; o >>= 1) evals += __shfl_xor_sync(FULL, evals, o);
   if (lane == 0 && evals) atomicAdd(t.evals, evals);
+}
+
+// ---------------------------------------------------------------------------------------
+// tomography operators (include/sweeptt.h, sweeptt_ray_project / sweeptt_ray_backproject)
+// ---------------------------------------------------------------------------------------
+// The same warp-per-ray traversal and predecessor step as trace_rays_kernel, but instead of writing nodes the warp
+// records the ray's steps as pull-table entries (16 bits: RAY_MAX_PULLS = 2^15) in a per-warp scratch of max_nodes
+// entries, in shared memory behind the pull table when that costs no occupancy, else in a global slot per resident
+// warp.  Only once the ray is known to be OK is the record walked, 32 edges per round with every lane on one edge,
+// from the start end:
+//   projection       acc = fl(fl(hd*fl(d_n + d_m)) + acc) from acc = +0, the sweep's own sum in the sweep's order
+//                    (sequential: one shuffle + add per edge; the gathers of the chunk are lane-parallel);
+//   back-projection  every node of the ray gets rint_even(w*hd*2^-E) of each of its (one or two) edges, added as
+//                    int64 atomics into a padded accumulator box: integer sums do not depend on the order, so the
+//                    result is deterministic.
+// Every ray ends at its start node, so the atomics there contend; they are not aggregated per warp or CTA because the
+// back-projection measured no slower than the projection (DESIGN §4d).
+
+// Walks the recorded path of the warp's OK ray from the start end.  Round c gives lane j edge k = nedge-1-(32c+j)
+// (live when k >= 0): its table entry e, and the padded indices of its ends n_k (nearer the receiver) and n_{k+1}.
+template <class F>
+__device__ __forceinline__ void walk_ray_path(const unsigned short* path, int nedge, long long n_start,
+                                              const RayPull* s_pull, int npull, F&& f) {
+  const unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  long long cur = n_start;  // n_{k+1} of lane 0's edge
+  for (int base = 0; base < nedge; base += 32) {
+    const int k = nedge - 1 - (base + lane);
+    const bool live = k >= 0;
+    const int e = live ? path[k] : 0;
+    DBG_BOUNDS(e >= 0 && e < npull);
+    const long long o = live ? s_pull[e].off : 0;
+    long long sum = o;  // inclusive prefix sum of the offsets over the lanes: n_k = cur - sum
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const long long v = __shfl_up_sync(FULL, sum, d);
+      if (lane >= d) sum += v;
+    }
+    f(live, k, e, cur - sum, cur - sum + o);
+    cur -= __shfl_sync(FULL, sum, 31);
+  }
+}
+
+__device__ __forceinline__ float project_ray(const TomoArgs& a, const RayPull* s_pull, const unsigned short* path,
+                                             int nedge, long long n_start) {
+  const unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  float acc = 0.f;
+  float d_far = a.pert[n_start];  // perturbation at n_{k+1} of lane 0's edge
+  walk_ray_path(path, nedge, n_start, s_pull, a.t.npull, [&](bool live, int k, int e, long long n, long long m) {
+    DBG_BOUNDS(!live || (n >= 0 && n < a.t.g.vol && m >= 0 && m < a.t.g.vol));
+    const float dn = live ? a.pert[n] : 0.f;
+    float dm = __shfl_up_sync(FULL, dn, 1);
+    if (lane == 0) dm = d_far;
+    const float term = live ? __fmul_rn(s_pull[e].hd, __fadd_rn(dn, dm)) : 0.f;
+    const int nlive = min(32, k + lane + 1);  // lanes of this round with an edge (k + lane = nedge-1-base)
+    for (int j = 0; j < nlive; ++j) acc = __fadd_rn(__shfl_sync(FULL, term, j), acc);
+    d_far = __shfl_sync(FULL, dn, 31);
+  });
+  return acc;
+}
+
+__device__ __forceinline__ long long backproject_quantum(float w, float hd, double scale) {
+  // w*hd is exact in double (24 x 24 bits), the power-of-two scale is exact unless the product underflows, which
+  // happens only far below 1/2 (rounds to 0 either way)
+  return __double2ll_rn(__dmul_rn(__dmul_rn((double)w, (double)hd), scale));
+}
+
+__device__ __forceinline__ void backproject_ray(const TomoArgs& a, const RayPull* s_pull, const unsigned short* path,
+                                                int nedge, long long n_start, float w) {
+  const int lane = threadIdx.x & 31;
+  if (lane == 0 && nedge > 0) {  // the start node: its one in-edge
+    DBG_BOUNDS(path[nedge - 1] < a.t.npull && n_start >= 0 && n_start < a.t.g.vol);
+    const long long c = backproject_quantum(w, s_pull[path[nedge - 1]].hd, a.scale);
+    if (c) atomicAdd(reinterpret_cast<unsigned long long*>(a.acc + n_start), (unsigned long long)c);
+  }
+  walk_ray_path(path, nedge, n_start, s_pull, a.t.npull, [&](bool live, int k, int e, long long n, long long) {
+    if (!live) return;
+    // node n_k gets edge k and, unless it is the receiver, edge k-1
+    long long c = backproject_quantum(w, s_pull[e].hd, a.scale);
+    if (k > 0) {
+      DBG_BOUNDS(path[k - 1] < a.t.npull);
+      c += backproject_quantum(w, s_pull[path[k - 1]].hd, a.scale);
+    }
+    DBG_BOUNDS(n >= 0 && n < a.t.g.vol);
+    if (c) atomicAdd(reinterpret_cast<unsigned long long*>(a.acc + n), (unsigned long long)c);
+  });
+}
+
+template <bool BACK>
+__device__ __forceinline__ void ray_walk_body(const TomoArgs& a, int4* smem) {
+  const TraceArgs& t = a.t;
+#ifdef SWEEPTT_DEBUG_BOUNDS
+  unsigned dyn_smem;
+  asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn_smem));
+  DBG_BOUNDS(t.npull >= 1 && t.npull < RAY_MAX_PULLS && t.max_nodes >= 1 &&
+             (size_t)t.npull * sizeof(RayPull) + (a.path_global ? 0 : (size_t)(TRACE_THREADS / 32) * t.max_nodes * 2) <= dyn_smem);
+#endif
+  const RayPull* s_pull = stage_ray_pulls(t, smem);
+  const int lane = threadIdx.x & 31;
+  const int warp = threadIdx.x >> 5;
+  const long long slot = (long long)blockIdx.x * (blockDim.x >> 5) + warp;
+  DBG_BOUNDS(!a.path_global || (slot + 1) * t.max_nodes <= a.path_entries);
+  unsigned short* path = a.path_global ? a.path_global + slot * t.max_nodes
+                                       : reinterpret_cast<unsigned short*>(smem + t.npull) + (size_t)warp * t.max_nodes;
+  const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+  unsigned long long evals = 0;
+  for (long long q = slot; q < t.nrays; q += warps) {
+    const int sr = (int)(q / t.nrec), r = (int)(q % t.nrec);
+    const int s = t.source_begin + sr;
+    const int px = t.src_xyz[3 * s], py = t.src_xyz[3 * s + 1], pz = t.src_xyz[3 * s + 2];
+    const float* tt = t.tt + (size_t)s * t.g.vol;
+    int x = t.rec_xyz[3 * r], y = t.rec_xyz[3 * r + 1], z = t.rec_xyz[3 * r + 2];
+    DBG_BOUNDS((unsigned)x < (unsigned)t.g.nx && (unsigned)y < (unsigned)t.g.ny && (unsigned)z < (unsigned)t.g.nz);
+    long long n = ((long long)(x + AX) * t.g.py + (y + AY)) * t.g.pz + (z + AZ);
+    const float w = BACK ? a.weights[q] : 0.f;
+    float tn = tt[n];
+    int len = 1, status;
+    __syncwarp();  // the previous ray's walk has read its record
+    if (tn == CUDART_INF_F) {
+      status = SWEEPTT_RAY_UNREACHED;
+    } else {
+      for (;;) {
+        if (x == px && y == py && z == pz) { status = SWEEPTT_RAY_OK; break; }
+        int eb;
+        status = ray_pred_step(t, s_pull, tt, px, py, pz, x, y, z, n, tn, &eb, evals);
+        if (status >= 0) break;
+        if (len == t.max_nodes) { status = SWEEPTT_RAY_TRUNCATED; break; }
+        if (lane == 0) {
+          DBG_BOUNDS(len - 1 >= 0 && len - 1 < t.max_nodes);
+          path[len - 1] = (unsigned short)eb;
+        }
+        ++len;
+      }
+    }
+    __syncwarp();  // the record is visible to every lane
+    if (BACK) {
+      if (status == SWEEPTT_RAY_OK && w != 0.f) backproject_ray(a, s_pull, path, len - 1, n, w);
+    } else {
+      const float v = status == SWEEPTT_RAY_OK ? project_ray(a, s_pull, path, len - 1, n) : CUDART_NAN_F;
+      if (lane == 0) {
+        DBG_BOUNDS(q >= 0 && q < t.nrays);
+        a.proj[q] = v;
+      }
+    }
+    if (lane == 0) {
+      DBG_BOUNDS(q >= 0 && q < t.nrays && len >= 1 && len <= t.max_nodes);
+      t.length[q] = len;
+      t.status[q] = status;
+    }
+  }
+  for (int o = 16; o; o >>= 1) evals += __shfl_xor_sync(0xffffffffu, evals, o);
+  if (lane == 0 && evals) atomicAdd(t.evals, evals);
+}
+
+__global__ void __launch_bounds__(TRACE_THREADS) ray_project_kernel(const TomoArgs a) {
+  extern __shared__ int4 s_tomo_raw[];
+  ray_walk_body<false>(a, s_tomo_raw);
+}
+
+__global__ void __launch_bounds__(TRACE_THREADS) ray_backproject_kernel(const TomoArgs a) {
+  extern __shared__ int4 s_tomo_raw[];
+  ray_walk_body<true>(a, s_tomo_raw);
+}
+
+// grad (dense, caller axes) := S * 2^E rounded once to float32 (nearest, ties to even), S the int64 accumulator
+// (padded kernel layout).  Normal results: __ll2float_rn is the one rounding (to 24 bits) and the power-of-two
+// scaling after it is exact or overflows exactly when the rounded value does.  Results below 2^-126: the quantum
+// is 2^-149, so S is shifted to that quantum with one round-half-even on the integer and stored as the subnormal
+// (or smallest normal) it encodes.
+__device__ __forceinline__ float round_scaled(long long S, int E) {
+  if (S == 0) return 0.f;
+  const unsigned sign = S < 0 ? 0x80000000u : 0u;
+  const unsigned long long u = S < 0 ? 0ull - (unsigned long long)S : (unsigned long long)S;
+  const int lim = -126 - E;  // |S| * 2^E < 2^-126  <=>  |S| < 2^lim
+  if (lim > 0 && (lim >= 64 || u < (1ull << lim))) {
+    const int sh = -(E + 149);  // S * 2^E = S * 2^-sh quanta of 2^-149
+    unsigned long long qv;
+    if (sh <= 0) {
+      qv = u << -sh;  // < 2^23: exact
+    } else if (sh >= 64) {
+      qv = 0;         // u < 2^63 <= half a quantum
+    } else {
+      qv = u >> sh;
+      const unsigned long long rem = u & ((1ull << sh) - 1), half = 1ull << (sh - 1);
+      if (rem > half || (rem == half && (qv & 1))) ++qv;
+    }
+    return __uint_as_float(sign | (unsigned)qv);  // qv <= 2^23: subnormal, zero or 2^-126
+  }
+  return scalbnf(__ll2float_rn(S), E);
+}
+
+__global__ void grad_finish_kernel(const long long* __restrict__ acc, float* __restrict__ dense, BoxGeom g, int E) {
+  const long long vol = (long long)g.nx * g.ny * g.nz;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < vol; i += (long long)gridDim.x * blockDim.x) {
+    const int z = (int)(i % g.nz);
+    const long long r = i / g.nz;
+    const int y = (int)(r % g.ny), x = (int)(r / g.ny);
+    const long long p = ((long long)(x + AX) * g.py + (y + AY)) * g.pz + (z + AZ);
+    const long long d = x * g.dstride[0] + y * g.dstride[1] + z * g.dstride[2];
+    DBG_BOUNDS(p >= 0 && p < g.vol && d >= 0 && d < vol);
+    dense[d] = round_scaled(acc[p], E);
+  }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1666,6 +1892,47 @@ cudaError_t launch_trace_rays(const TraceArgs& t, int device, cudaStream_t strea
   const long long need = (t.nrays + TRACE_THREADS / 32 - 1) / (TRACE_THREADS / 32);
   const int grid = (int)std::max(1LL, std::min<long long>(need, (long long)sms * per_sm));
   trace_rays_kernel<<<grid, TRACE_THREADS, smem, stream>>>(t);
+  return cudaGetLastError();
+}
+
+cudaError_t ray_walk_prepare(bool backproject, int npull, int max_nodes, long long nrays, int device, RayWalkLaunch* out) {
+  const void* fn = backproject ? (const void*)ray_backproject_kernel : (const void*)ray_project_kernel;
+  const size_t table = (size_t)npull * sizeof(RayPull);
+  const size_t with_path = table + (size_t)(TRACE_THREADS / 32) * max_nodes * sizeof(unsigned short);
+  int sms = 0, optin = 0, per_sm_table = 0, per_sm_path = 0;
+  cudaError_t e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+  if (e != cudaSuccess) return e;
+  e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+  if (e != cudaSuccess) return e;
+  const bool fits = with_path <= (size_t)optin;
+  e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(fits ? with_path : table));
+  if (e != cudaSuccess) return e;
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_table, fn, TRACE_THREADS, table);
+  if (e != cudaSuccess) return e;
+  if (fits) {
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_path, fn, TRACE_THREADS, with_path);
+    if (e != cudaSuccess) return e;
+  }
+  out->path_in_smem = fits && per_sm_path == per_sm_table;
+  const int per_sm = out->path_in_smem ? per_sm_path : per_sm_table;
+  if (per_sm < 1) return cudaErrorInvalidConfiguration;
+  out->smem = out->path_in_smem ? with_path : table;
+  const long long need = (nrays + TRACE_THREADS / 32 - 1) / (TRACE_THREADS / 32);
+  out->grid = (int)std::max(1LL, std::min<long long>(need, (long long)sms * per_sm));
+  out->path_entries = out->path_in_smem ? 0 : (long long)out->grid * (TRACE_THREADS / 32) * max_nodes;
+  return cudaSuccess;
+}
+
+cudaError_t launch_ray_walk(bool backproject, const RayWalkLaunch& l, const TomoArgs& a, cudaStream_t stream) {
+  if (backproject)
+    ray_backproject_kernel<<<l.grid, TRACE_THREADS, l.smem, stream>>>(a);
+  else
+    ray_project_kernel<<<l.grid, TRACE_THREADS, l.smem, stream>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_grad_finish(const long long* acc, float* dense, BoxGeom g, int E, cudaStream_t stream) {
+  grad_finish_kernel<<<1184, 256, 0, stream>>>(acc, dense, g, E);
   return cudaGetLastError();
 }
 

@@ -123,6 +123,31 @@ struct TraceArgs {
 size_t trace_rays_smem_bytes(int npull);
 cudaError_t launch_trace_rays(const TraceArgs& t, int device, cudaStream_t stream);
 
+// Tomography operators over the same rays (include/sweeptt.h, sweeptt_ray_project / sweeptt_ray_backproject).
+// t.nodes and t.tt_rec are unused.
+struct TomoArgs {
+  TraceArgs t;
+  const float* pert;           // projection: padded perturbation box
+  float* proj;                 // projection: [nrays] results
+  const float* weights;        // back-projection: [nrays] weights
+  long long* acc;              // back-projection: padded int64 accumulator box (zeroed by the caller)
+  double scale;                // back-projection: 2^-E
+  unsigned short* path_global; // per-warp path records in global memory (path_entries entries), or nullptr: in smem
+  long long path_entries;
+};
+// Launch shape of a projection or back-projection: persistent grid, dynamic shared memory and where the path
+// records live (shared memory when that costs no occupancy; else path_global needs grid * warps * max_nodes entries).
+struct RayWalkLaunch {
+  int grid;
+  size_t smem;
+  bool path_in_smem;
+  long long path_entries;      // global path entries needed (0 when in smem)
+};
+cudaError_t ray_walk_prepare(bool backproject, int npull, int max_nodes, long long nrays, int device, RayWalkLaunch* out);
+cudaError_t launch_ray_walk(bool backproject, const RayWalkLaunch& l, const TomoArgs& a, cudaStream_t stream);
+// grad (dense, caller axes) := acc * 2^E rounded once to float32.
+cudaError_t launch_grad_finish(const long long* acc, float* dense, BoxGeom g, int E, cudaStream_t stream);
+
 // Box utilities (device float-box pool).
 cudaError_t launch_fill(float* p, long long n, float value, cudaStream_t stream);
 cudaError_t launch_pad_box(const float* dense, float* padded, BoxGeom g, cudaStream_t stream);

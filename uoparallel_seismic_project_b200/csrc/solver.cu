@@ -168,6 +168,14 @@ struct sweeptt_ctx {
   size_t rec_cap = 0;
   unsigned char* d_ray_out = nullptr;
   size_t ray_out_cap = 0;
+  // tomography operators (sweeptt_ray_project / sweeptt_ray_backproject): grow-only padded perturbation box, int64
+  // accumulator box and per-warp path records
+  float* d_pert = nullptr;
+  size_t pert_cap = 0;
+  long long* d_acc = nullptr;
+  size_t acc_cap = 0;
+  unsigned short* d_path = nullptr;
+  size_t path_cap = 0;
   float* d_stage = nullptr;  // dense staging box for pad/unpad
   size_t stage_floats = 0;
   size_t pool_bytes = 0;
@@ -371,6 +379,7 @@ extern "C" void sweeptt_destroy(sweeptt_ctx* c) {
   cudaFree(c->d_worklist); cudaFree(c->d_key); cudaFree(c->d_tmax); cudaFree(c->d_busy); cudaFree(c->d_keysnap); cudaFree(c->d_tile_pulls); cudaFree(c->d_viol);
   cudaFree(c->d_stage); cudaFree(c->d_star);
   cudaFree(c->d_ray_pull); cudaFree(c->d_rec); cudaFree(c->d_ray_out);
+  cudaFree(c->d_pert); cudaFree(c->d_acc); cudaFree(c->d_path);
   if (c->h_state) cudaFreeHost(c->h_state);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
@@ -1541,17 +1550,17 @@ static int build_ray_pulls(sweeptt_ctx* c) {
   return 1;
 }
 
-extern "C" int sweeptt_trace_rays(sweeptt_ctx* c, int source_begin, int source_count, const struct START* receivers,
-                                  int nrec, int max_nodes, struct START* nodes_out, int32_t* length_out,
-                                  int32_t* status_out, float* tt_out, sweeptt_stats* stats) {
-  ConstLease lease;
-  if (!ready(c, &lease)) return 0;
+// Argument checks shared by the ray calls (sweeptt_trace_rays, sweeptt_ray_project, sweeptt_ray_backproject), then
+// the receivers range-checked and permuted to kernel axes into c->rec_xyz.
+static int check_ray_call(sweeptt_ctx* c, ConstLease* lease, const char* who, int source_begin, int source_count,
+                          const struct START* receivers, int nrec, int max_nodes, sweeptt_stats* stats) {
+  if (!ready(c, lease)) return 0;
   if (stats) std::memset(stats, 0, sizeof *stats);
-  if (!receivers || nrec < 1) return fail("sweeptt_trace_rays: need at least one receiver");
+  if (!receivers || nrec < 1) return fail("%s: need at least one receiver", who);
   if (source_count < 1 || source_begin < 0 || source_begin > c->nsrc - source_count)
-    return fail("sweeptt_trace_rays: sources [%d, %d) are not within the context's %d sources", source_begin,
+    return fail("%s: sources [%d, %d) are not within the context's %d sources", who, source_begin,
                 source_begin + source_count, c->nsrc);
-  if (max_nodes < 1) return fail("sweeptt_trace_rays: max_nodes must be >= 1 (got %d)", max_nodes);
+  if (max_nodes < 1) return fail("%s: max_nodes must be >= 1 (got %d)", who, max_nodes);
   const BoxGeom& g = c->g;
   int on[3];  // caller-order dims
   on[g.perm[0]] = g.nx; on[g.perm[1]] = g.ny; on[g.perm[2]] = g.nz;
@@ -1562,19 +1571,20 @@ extern "C" int sweeptt_trace_rays(sweeptt_ctx* c, int source_begin, int source_c
       return fail("receiver %d (%d,%d,%d) is outside the %d x %d x %d model", r, o[0], o[1], o[2], on[0], on[1], on[2]);
     for (int q = 0; q < 3; ++q) c->rec_xyz[3 * (size_t)r + q] = o[g.perm[q]];
   }
-  const long long nrays = (long long)source_count * nrec;
-  if (nodes_out && (unsigned long long)nrays > (1ull << 60) / (12ull * (unsigned long long)max_nodes))
-    return fail("sweeptt_trace_rays: %lld rays of up to %d nodes do not fit one call", nrays, max_nodes);
+  return 1;
+}
+
+// Pull table and the checked receivers on the device.
+static int upload_ray_tables(sweeptt_ctx* c, int nrec) {
   if (!build_ray_pulls(c)) return 0;
   if (!ensure_dev(c, &c->d_rec, &c->rec_cap, 3 * sizeof(int) * (size_t)nrec)) return 0;
   CK(cudaMemcpyAsync(c->d_rec, c->rec_xyz.data(), 3 * sizeof(int) * (size_t)nrec, cudaMemcpyHostToDevice, c->stream));
-  // output buffer: [evaluation counter | length | status | tt | nodes], every part 16-byte aligned
-  auto up16 = [](size_t b) { return (b + 15) / 16 * 16; };
-  const size_t per_ray = up16(4 * (size_t)nrays);
-  const size_t node_bytes = nodes_out ? (size_t)nrays * max_nodes * sizeof(START) : 0;
-  if (!ensure_dev(c, &c->d_ray_out, &c->ray_out_cap, 16 + 3 * per_ray + node_bytes)) return 0;
+  return 1;
+}
+
+static TraceArgs ray_trace_args(sweeptt_ctx* c, int source_begin, int nrec, long long nrays, int max_nodes) {
   TraceArgs t{};
-  t.g = g;
+  t.g = c->g;
   t.slow = c->d_slow;
   t.tt = c->d_tt;
   t.src_xyz = c->d_src;
@@ -1585,6 +1595,25 @@ extern "C" int sweeptt_trace_rays(sweeptt_ctx* c, int source_begin, int source_c
   t.nrec = nrec;
   t.nrays = nrays;
   t.max_nodes = max_nodes;
+  return t;
+}
+
+extern "C" int sweeptt_trace_rays(sweeptt_ctx* c, int source_begin, int source_count, const struct START* receivers,
+                                  int nrec, int max_nodes, struct START* nodes_out, int32_t* length_out,
+                                  int32_t* status_out, float* tt_out, sweeptt_stats* stats) {
+  ConstLease lease;
+  if (!check_ray_call(c, &lease, "sweeptt_trace_rays", source_begin, source_count, receivers, nrec, max_nodes, stats))
+    return 0;
+  const long long nrays = (long long)source_count * nrec;
+  if (nodes_out && (unsigned long long)nrays > (1ull << 60) / (12ull * (unsigned long long)max_nodes))
+    return fail("sweeptt_trace_rays: %lld rays of up to %d nodes do not fit one call", nrays, max_nodes);
+  if (!upload_ray_tables(c, nrec)) return 0;
+  // output buffer: [evaluation counter | length | status | tt | nodes], every part 16-byte aligned
+  auto up16 = [](size_t b) { return (b + 15) / 16 * 16; };
+  const size_t per_ray = up16(4 * (size_t)nrays);
+  const size_t node_bytes = nodes_out ? (size_t)nrays * max_nodes * sizeof(START) : 0;
+  if (!ensure_dev(c, &c->d_ray_out, &c->ray_out_cap, 16 + 3 * per_ray + node_bytes)) return 0;
+  TraceArgs t = ray_trace_args(c, source_begin, nrec, nrays, max_nodes);
   t.evals = reinterpret_cast<unsigned long long*>(c->d_ray_out);
   t.length = reinterpret_cast<int*>(c->d_ray_out + 16);
   t.status = reinterpret_cast<int*>(c->d_ray_out + 16 + per_ray);
@@ -1630,6 +1659,145 @@ extern "C" int sweeptt_trace_rays(sweeptt_ctx* c, int source_begin, int source_c
     stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
     stats->d2h_bytes = bytes;
   }
+  return 1;
+}
+
+// Smallest E with 2*hd_max*W*N <= 2^(E+62), in exact arithmetic (hd_max, W > 0 finite).  With hd_max = Mh*2^(eh-24)
+// and W = Mw*2^(ew-24) (Mh, Mw the 24-bit integer significands), the condition is X = Mh*Mw*N <= 2^(E+109-eh-ew).
+static int quantum_exponent(float hd_max, float W, long long N) {
+  int eh = 0, ew = 0;
+  const unsigned long long Mh = (unsigned long long)std::ldexp(std::frexp((double)hd_max, &eh), 24);
+  const unsigned long long Mw = (unsigned long long)std::ldexp(std::frexp((double)W, &ew), 24);
+  const unsigned __int128 X = (unsigned __int128)(Mh * Mw) * (unsigned long long)N;
+  int b = 0;  // bit length: 2^(b-1) <= X < 2^b
+  while ((X >> b) != 0) ++b;
+  const int k = (X & (X - 1)) == 0 ? b - 1 : b;  // smallest k with X <= 2^k
+  return k - 109 + eh + ew;
+}
+
+// Shared part of sweeptt_ray_project / sweeptt_ray_backproject after the inputs are on the device: the walk kernel
+// (and, for the back-projection, the rounding kernel into c->d_stage), timed with events; then the evaluation
+// counter, statuses and lengths copied back.
+static int run_ray_walk(sweeptt_ctx* c, bool back, TomoArgs& a, int E, int kernels_before,
+                        int32_t* status_out, int32_t* length_out, float* proj_out, sweeptt_stats* stats) {
+  const long long nrays = a.t.nrays;
+  RayWalkLaunch l{};
+  CK(ray_walk_prepare(back, a.t.npull, a.t.max_nodes, nrays, c->device, &l));
+  if (!l.path_in_smem) {
+    if (!ensure_dev(c, &c->d_path, &c->path_cap, (size_t)l.path_entries * sizeof(unsigned short))) return 0;
+    a.path_global = c->d_path;
+    a.path_entries = l.path_entries;
+  }
+  CK(launch_ray_walk(back, l, a, c->stream));
+  if (back) CK(launch_grad_finish(a.acc, c->d_stage, c->g, E, c->stream));
+  CK(cudaEventRecord(c->ev1, c->stream));
+  CK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+
+  const auto t_copy = std::chrono::steady_clock::now();
+  unsigned long long evals = 0;
+  long long bytes = 8;
+  CK(cudaMemcpyAsync(&evals, a.t.evals, 8, cudaMemcpyDeviceToHost, c->stream));
+  if (length_out) { CK(cudaMemcpyAsync(length_out, a.t.length, 4 * nrays, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * nrays; }
+  if (status_out) { CK(cudaMemcpyAsync(status_out, a.t.status, 4 * nrays, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * nrays; }
+  if (proj_out) { CK(cudaMemcpyAsync(proj_out, a.proj, 4 * nrays, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * nrays; }
+  CK(cudaStreamSynchronize(c->stream));
+  if (stats) {
+    stats->struct_size = (int)sizeof *stats;
+    stats->solve_ms = ms;
+    stats->relaxations = (long long)evals;
+    stats->kernel_launches = kernels_before + 1 + (back ? 1 : 0);
+    stats->devices_used = 1;
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes += bytes;
+  }
+  return 1;
+}
+
+// Output buffer of the tomography calls: [evaluation counter | length | status | projection or weights], every part
+// 16-byte aligned.
+static int tomo_args(sweeptt_ctx* c, int source_begin, int nrec, long long nrays, int max_nodes, TomoArgs* a,
+                     size_t* per_ray) {
+  *per_ray = ((size_t)4 * nrays + 15) / 16 * 16;
+  if (!ensure_dev(c, &c->d_ray_out, &c->ray_out_cap, 16 + 3 * *per_ray)) return 0;
+  *a = TomoArgs{};
+  a->t = ray_trace_args(c, source_begin, nrec, nrays, max_nodes);
+  a->t.evals = reinterpret_cast<unsigned long long*>(c->d_ray_out);
+  a->t.length = reinterpret_cast<int*>(c->d_ray_out + 16);
+  a->t.status = reinterpret_cast<int*>(c->d_ray_out + 16 + *per_ray);
+  CK(cudaMemsetAsync(a->t.evals, 0, 8, c->stream));
+  return 1;
+}
+
+extern "C" int sweeptt_ray_project(sweeptt_ctx* c, int source_begin, int source_count, const struct START* receivers,
+                                   int nrec, int max_nodes, const float* perturbation, float* proj_out,
+                                   int32_t* status_out, int32_t* length_out, sweeptt_stats* stats) {
+  ConstLease lease;
+  if (!check_ray_call(c, &lease, "sweeptt_ray_project", source_begin, source_count, receivers, nrec, max_nodes, stats))
+    return 0;
+  if (!perturbation) return fail("sweeptt_ray_project: null perturbation");
+  const long long nrays = (long long)source_count * nrec;
+  if (!upload_ray_tables(c, nrec)) return 0;
+  const BoxGeom& g = c->g;
+  const size_t dense = (size_t)g.nx * g.ny * g.nz;
+  if (!ensure_stage(c, dense)) return 0;
+  if (!ensure_dev(c, &c->d_pert, &c->pert_cap, (size_t)g.vol * 4)) return 0;
+  TomoArgs a;
+  size_t per_ray;
+  if (!tomo_args(c, source_begin, nrec, nrays, max_nodes, &a, &per_ray)) return 0;
+  a.pert = c->d_pert;
+  a.proj = reinterpret_cast<float*>(c->d_ray_out + 16 + 2 * per_ray);
+  // only nodes on a ray are read, and those are in the box: the apron of d_pert is never looked at
+  CK(cudaMemcpyAsync(c->d_stage, perturbation, dense * 4, cudaMemcpyHostToDevice, c->stream));
+  CK(cudaEventRecord(c->ev0, c->stream));
+  CK(launch_pad_box(c->d_stage, c->d_pert, g, c->stream));
+  return run_ray_walk(c, false, a, 0, 1, status_out, length_out, proj_out, stats);
+}
+
+extern "C" int sweeptt_ray_backproject(sweeptt_ctx* c, int source_begin, int source_count,
+                                       const struct START* receivers, int nrec, int max_nodes, const float* weights,
+                                       float* grad_out, int* quantum_exp_out, int32_t* status_out,
+                                       sweeptt_stats* stats) {
+  ConstLease lease;
+  if (!check_ray_call(c, &lease, "sweeptt_ray_backproject", source_begin, source_count, receivers, nrec, max_nodes,
+                      stats))
+    return 0;
+  if (!weights || !grad_out) return fail("sweeptt_ray_backproject: weights and grad_out are required");
+  const long long nrays = (long long)source_count * nrec;
+  float W = 0.f;
+  for (long long q = 0; q < nrays; ++q) {
+    if (!std::isfinite(weights[q])) return fail("sweeptt_ray_backproject: weight %lld is not finite", q);
+    W = std::max(W, std::fabs(weights[q]));
+  }
+  if (!upload_ray_tables(c, nrec)) return 0;
+  float hd_max = 0.f;
+  for (const RayPull& p : c->ray_pull) hd_max = std::max(hd_max, p.hd);
+  if (!std::isfinite(hd_max)) return fail("sweeptt_ray_backproject: the star's edge lengths are not finite");
+  const int E = (W > 0.f && hd_max > 0.f) ? quantum_exponent(hd_max, W, nrays) : 0;
+  const BoxGeom& g = c->g;
+  const size_t dense = (size_t)g.nx * g.ny * g.nz;
+  if (!ensure_stage(c, dense)) return 0;
+  if (!ensure_dev(c, &c->d_acc, &c->acc_cap, (size_t)g.vol * 8)) return 0;
+  TomoArgs a;
+  size_t per_ray;
+  if (!tomo_args(c, source_begin, nrec, nrays, max_nodes, &a, &per_ray)) return 0;
+  float* d_w = reinterpret_cast<float*>(c->d_ray_out + 16 + 2 * per_ray);
+  a.weights = d_w;
+  a.acc = c->d_acc;
+  a.scale = std::ldexp(1.0, -E);
+  CK(cudaMemcpyAsync(d_w, weights, 4 * nrays, cudaMemcpyHostToDevice, c->stream));
+  CK(cudaEventRecord(c->ev0, c->stream));
+  CK(cudaMemsetAsync(c->d_acc, 0, (size_t)g.vol * 8, c->stream));
+  if (!run_ray_walk(c, true, a, E, 0, status_out, nullptr, nullptr, stats)) return 0;
+  const auto t_copy = std::chrono::steady_clock::now();
+  CK(cudaMemcpyAsync(grad_out, c->d_stage, dense * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  if (stats) {
+    stats->d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes += (long long)(dense * 4);
+  }
+  if (quantum_exp_out) *quantum_exp_out = E;
   return 1;
 }
 
