@@ -284,6 +284,60 @@ int sweeptt_ray_backproject(sweeptt_ctx *ctx, int source_begin, int source_count
                             int *quantum_exp_out, int32_t *status_out, /* may be NULL */
                             sweeptt_stats *stats);
 
+/* ---- ray sets: rays traced once, kept on the device, applied as often as needed -------------- */
+
+/* A linearised inversion step holds the rays fixed and applies G and G^T tens of times; a ray set traces them once.
+ *
+ * sweeptt_rayset_freeze traces exactly the rays of sweeptt_trace_rays (same predecessor rule, statuses, max_nodes
+ * truncation and numbering q = (s - source_begin)*nrec + r; argument checks, stream and synchronisation as there) and
+ * keeps, for every OK ray, its steps as pull-table entries (2 bytes each), ray-major in q order.  A ray that is not OK
+ * keeps only its status, length and receiver time.  Returns NULL (sweeptt_last_error() set) on any failure, out of
+ * device memory included, and then holds nothing.  stats (may be NULL): solve_ms = device time of the trace and the
+ * packing, relaxations = candidate evaluations, kernel_launches, d2h_ms / d2h_bytes.
+ *
+ * Contract: sweeptt_rayset_project and sweeptt_rayset_backproject return bit for bit what sweeptt_ray_project and
+ * sweeptt_ray_backproject return for the context state, source range, receivers and max_nodes of the freeze: NaN for
+ * a ray that is not OK, +0 for a ray of one node, and the same quantum exponent E (N in its formula is
+ * source_count*nrec of the set, rays that are not OK included).
+ *
+ * The set is a snapshot: it owns copies of the pull table, the geometry and axis permutation, the padded start
+ * indices, and its own padded-perturbation, int64-accumulator and staging buffers.  Later set_model, set_star,
+ * set_sources, run, step, reset or put_tt calls on the context leave it valid and unchanged.  It borrows only the
+ * context's device and stream; its calls run on that stream and synchronise it.  Threading is the context's: use a set
+ * from the thread that uses its context, and destroy every set before its context.  The operators read no
+ * __constant__ table, so they never wait for another context's star.
+ *
+ * Device memory (sweeptt_rayset_bytes, not counted in sweeptt_pool_bytes): with N rays, P entries in all, a pull table
+ * of npull entries, S = source_count and a padded box of V floats (nx*ny*nz = D nodes),
+ *   2*P + 16*N + 8 + 16*npull + 8*S + 12*V + 4*D
+ * (entries, offsets int64[N+1], status and one per-ray in/out float, pull table, start indices, perturbation and
+ * accumulator boxes, dense staging).  The buffers that freezing needs for a while (the receivers, a chunk of padded
+ * records) are the context's grow-only buffers, counted in sweeptt_pool_bytes like those of the other ray calls. */
+typedef struct sweeptt_rayset sweeptt_rayset;
+
+sweeptt_rayset *sweeptt_rayset_freeze(sweeptt_ctx *ctx, int source_begin, int source_count,
+                                      const struct START *receivers, int nrec, int max_nodes,
+                                      sweeptt_stats *stats);
+void sweeptt_rayset_destroy(sweeptt_rayset *set);
+size_t sweeptt_rayset_bytes(const sweeptt_rayset *set);
+
+/* The per-ray table [source_count*nrec], the values sweeptt_trace_rays returns.  Any output may be NULL. */
+int sweeptt_rayset_table(const sweeptt_rayset *set, int32_t *length_out, int32_t *status_out, float *tt_out);
+
+/* Compact node export, decoded on the host from the set's pull table: ray q has the nodes
+ * nodes_out[offsets_out[q] .. offsets_out[q+1]) in caller axes, receiver first; only OK rays have nodes (length_q of
+ * them), every other ray none.  offsets_out: int64[N+1]; nodes_out: START[offsets_out[N]].  Either may be NULL. */
+int sweeptt_rayset_paths(const sweeptt_rayset *set, int64_t *offsets_out, struct START *nodes_out);
+
+/* G*d over every ray of the set (see sweeptt_ray_project).  perturbation: nx*ny*nz floats, FLOATBOX, caller axes of
+ * the freeze; proj_out [N] may be NULL.  stats: solve_ms = device time (pad + walk), kernel_launches, d2h. */
+int sweeptt_rayset_project(sweeptt_rayset *set, const float *perturbation, float *proj_out, sweeptt_stats *stats);
+
+/* G^T*w over every ray of the set (see sweeptt_ray_backproject).  weights [N] finite, required; grad_out nx*ny*nz
+ * floats, required; quantum_exp_out may be NULL.  stats: solve_ms = device time (zeroing, walk, rounding). */
+int sweeptt_rayset_backproject(sweeptt_rayset *set, const float *weights, float *grad_out, int *quantum_exp_out,
+                               sweeptt_stats *stats);
+
 /* In-bounds pull evaluations of one full round of one source (analytic). */
 long long sweeptt_relaxations_per_round(sweeptt_ctx *ctx);
 /* Bytes of device memory currently held by the context's pool. */

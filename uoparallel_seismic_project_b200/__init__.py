@@ -9,8 +9,10 @@ raises ``SweepError`` when the extension or a CUDA device is missing.
 from .api import (  # noqa: F401
     FS,
     Backprojection,
+    LinearizedUpdate,
     MisfitGradient,
     RayProjection,
+    RaySet,
     Rays,
     START,
     SweepContext,
@@ -20,6 +22,7 @@ from .api import (  # noqa: F401
     device_count,
     lib_path,
     load_library,
+    linearized_update,
     make_star,
     solve,
     solve_slabs,

@@ -12,6 +12,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import pathlib
+import weakref
 from dataclasses import dataclass
 
 import numpy as np
@@ -91,7 +92,9 @@ _EXPORTS = [
     "sweeptt_host_alloc", "sweeptt_host_free",
     "sweeptt_create", "sweeptt_destroy", "sweeptt_set_stream", "sweeptt_set_model", "sweeptt_set_star",
     "sweeptt_set_sources", "sweeptt_run", "sweeptt_step", "sweeptt_reset", "sweeptt_get_tt", "sweeptt_put_tt",
-    "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_solve_slabs",
+    "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject",
+    "sweeptt_rayset_freeze", "sweeptt_rayset_destroy", "sweeptt_rayset_bytes", "sweeptt_rayset_table",
+    "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
     "sweeptt_vbox_load", "sweeptt_vbox_store", "sweeptt_vbox_load_subset", "sweeptt_text_load",
     "sweeptt_star_load", "sweeptt_starts_load", "sweeptt_write_output_tt", "sweeptt_free",
@@ -142,6 +145,18 @@ def load_library() -> C.CDLL:
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_ray_backproject.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(START), C.c_int, C.c_int,
                                             C.c_void_p, C.c_void_p, C.POINTER(C.c_int), C.c_void_p, C.POINTER(_Stats)]
+    lib.sweeptt_rayset_freeze.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(START), C.c_int, C.c_int,
+                                          C.POINTER(_Stats)]
+    lib.sweeptt_rayset_freeze.restype = C.c_void_p
+    lib.sweeptt_rayset_destroy.argtypes = [C.c_void_p]
+    lib.sweeptt_rayset_destroy.restype = None
+    lib.sweeptt_rayset_bytes.argtypes = [C.c_void_p]
+    lib.sweeptt_rayset_bytes.restype = C.c_size_t
+    lib.sweeptt_rayset_table.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.sweeptt_rayset_paths.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.sweeptt_rayset_project.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
+    lib.sweeptt_rayset_backproject.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int),
+                                               C.POINTER(_Stats)]
     lib.sweeptt_relaxations_per_round.argtypes = [C.c_void_p]
     lib.sweeptt_relaxations_per_round.restype = C.c_longlong
     lib.sweeptt_pool_bytes.argtypes = [C.c_void_p]
@@ -363,6 +378,21 @@ class MisfitGradient:
     quantum_exp: int
 
 
+@dataclass
+class LinearizedUpdate:
+    """linearized_update: delta (float32[nx, ny, nz]) is the damped least-squares slowness perturbation of one
+    linearised step (LSQR over the frozen rays); residual[s, r] = float32(observed - t), NaN where the ray is not OK
+    or has no pick; misfit = 1/2 sum residual^2 (float64) before the step; istop, iterations and residual_norm
+    (||r - G delta||, LSQR's r1norm) as scipy.sparse.linalg.lsqr reports them."""
+    delta: np.ndarray     # float32[nx, ny, nz]
+    residual: np.ndarray  # float32[S, R]
+    status: np.ndarray    # int32[S, R]
+    misfit: float
+    istop: int
+    iterations: int
+    residual_norm: float
+
+
 class SweepContext:
     """Device-resident context: padded slowness box + pool of travel-time boxes on one GPU."""
 
@@ -377,9 +407,13 @@ class SweepContext:
             raise SweepError(f"sweeptt_create: {self._lib.sweeptt_last_error().decode()}")
         self.dims = None
         self.nsrc = 0
+        self._sets = weakref.WeakSet()
 
     def close(self):
+        """Closes every ray set frozen from this context that is still open, then the context."""
         if getattr(self, "_h", None):
+            for rs in list(self._sets):
+                rs.close()
             self._lib.sweeptt_destroy(self._h)
             self._h = None
 
@@ -526,6 +560,30 @@ class SweepContext:
 
         return self._ray_calls(max_nodes, call)
 
+    def freeze_rays(self, receivers, sources=None, max_nodes: int | None = None) -> "RaySet":
+        """Traces the rays of trace_rays once and keeps them on the device as a RaySet (include/sweeptt.h,
+        sweeptt_rayset_freeze), whose project / backproject equal ray_project / ray_backproject of this context as it
+        is now, bit for bit, however the context changes later.  Sources and max_nodes as in trace_rays: with the
+        default the freeze is repeated at twice the capacity while a ray is RAY_TRUNCATED."""
+        begin, count = self._source_range(sources, "freeze_rays")
+        rec = _make_starts(receivers)
+        nrec = len(rec)
+
+        def call(cap):
+            s = _Stats()
+            h = self._lib.sweeptt_rayset_freeze(self._h, begin, count, rec, nrec, cap, C.byref(s))
+            if not h:
+                raise SweepError(f"sweeptt_rayset_freeze: {self._lib.sweeptt_last_error().decode()}")
+            rs = RaySet(self, h, (count, nrec), tuple(self.dims), SweepStats._from(s))
+            if grow and (rs.status == RAY_TRUNCATED).any():
+                rs.close()
+            return rs, rs.status
+
+        grow = max_nodes is None
+        rs = self._ray_calls(max_nodes, call)
+        self._sets.add(rs)
+        return rs
+
     @property
     def relaxations_per_round(self) -> int:
         return self._lib.sweeptt_relaxations_per_round(self._h)
@@ -537,6 +595,107 @@ class SweepContext:
     @property
     def pool_bytes(self) -> int:
         return self._lib.sweeptt_pool_bytes(self._h)
+
+
+class RaySet:
+    """Rays of sources [S] x receivers [R] traced once and kept on the device (SweepContext.freeze_rays): G*d and G^T*w
+    from the stored rays, bit for bit what ray_project / ray_backproject gave at the freeze.  A snapshot: later changes
+    of the context (model, star, fields) leave it unchanged.  Close it (or its context) to release nbytes of device
+    memory; a closed set raises."""
+
+    def __init__(self, ctx: SweepContext, handle, shape, dims, stats: SweepStats):
+        self._lib = ctx._lib
+        self._ctx = ctx              # the context outlives its sets
+        self._h = handle
+        self.shape = shape           # (S, R)
+        self.dims = dims             # (nx, ny, nz) of the model at the freeze
+        self.stats = stats           # of the freeze
+        self.length = np.empty(shape, np.int32)
+        self.status = np.empty(shape, np.int32)
+        self.tt = np.empty(shape, np.float32)
+        _check(self._lib.sweeptt_rayset_table(self._h, self.length.ctypes.data, self.status.ctypes.data,
+                                              self.tt.ctypes.data), "sweeptt_rayset_table")
+
+    def _handle(self):
+        if not self._h:
+            raise SweepError("ray set is closed")
+        return self._h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.sweeptt_rayset_destroy(self._h)
+            self._h = None
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    @property
+    def nbytes(self) -> int:
+        """Device memory the set holds (include/sweeptt.h, sweeptt_rayset_bytes)."""
+        return self._lib.sweeptt_rayset_bytes(self._handle())
+
+    def project(self, perturbation) -> RayProjection:
+        """G*d over every ray of the set (values NaN unless status is RAY_OK)."""
+        d = np.ascontiguousarray(perturbation, dtype=np.float32)
+        if d.shape != self.dims:
+            raise SweepError(f"RaySet.project: perturbation of shape {d.shape}, the rays are on {self.dims}")
+        values = np.empty(self.shape, np.float32)
+        s = _Stats()
+        _check(self._lib.sweeptt_rayset_project(self._handle(), d.ctypes.data, values.ctypes.data, C.byref(s)),
+               "sweeptt_rayset_project")
+        return RayProjection(values, self.status, self.length, SweepStats._from(s))
+
+    def backproject(self, weights) -> Backprojection:
+        """G^T*w over every ray of the set; weights [S, R] finite (only the OK rays contribute)."""
+        w = np.ascontiguousarray(weights, dtype=np.float32)
+        if w.shape != self.shape:
+            raise SweepError(f"RaySet.backproject: weights of shape {w.shape}, expected {self.shape}")
+        grad = np.empty(self.dims, np.float32)
+        e = C.c_int(0)
+        s = _Stats()
+        _check(self._lib.sweeptt_rayset_backproject(self._handle(), w.ctypes.data, grad.ctypes.data, C.byref(e),
+                                                    C.byref(s)), "sweeptt_rayset_backproject")
+        return Backprojection(grad, e.value, self.status, SweepStats._from(s))
+
+    def paths(self):
+        """(offsets int64[S*R+1], nodes int32[offsets[-1], 3]): ray q = s*R + r has the nodes
+        nodes[offsets[q]:offsets[q+1]] (caller axes, receiver first); rays that are not OK have none."""
+        h = self._handle()
+        offsets = np.empty(self.status.size + 1, np.int64)
+        _check(self._lib.sweeptt_rayset_paths(h, offsets.ctypes.data, None), "sweeptt_rayset_paths")
+        nodes = np.empty((int(offsets[-1]), 3), np.int32)
+        _check(self._lib.sweeptt_rayset_paths(h, None, nodes.ctypes.data), "sweeptt_rayset_paths")
+        return offsets, nodes
+
+    def as_linear_operator(self, rows=None):
+        """G as a scipy.sparse.linalg.LinearOperator (float64) over the rays selected by rows (bool [S, R]; default:
+        the OK rays) and every node of the box (raveled FLOATBOX order).  The conversions are part of the definition:
+          matvec(x)  = float64(project(float32(x)).values[rows])
+          rmatvec(y) = float64(backproject(W).grad).ravel(), W = float32(y) scattered into [S, R], 0 outside rows.
+        Both run on the device; only the vectors cross PCIe."""
+        from scipy.sparse.linalg import LinearOperator
+        rows = self.status == RAY_OK if rows is None else np.asarray(rows, bool)
+        if rows.shape != self.shape:
+            raise SweepError(f"RaySet.as_linear_operator: rows of shape {rows.shape}, expected {self.shape}")
+        if not (self.status[rows] == RAY_OK).all():
+            raise SweepError("RaySet.as_linear_operator: rows selects a ray that is not OK")
+        n = int(np.prod(self.dims))
+
+        def matvec(x):
+            d = np.asarray(x, np.float32).reshape(self.dims)
+            return self.project(d).values[rows].astype(np.float64)
+
+        def rmatvec(y):
+            w = np.zeros(self.shape, np.float32)
+            w[rows] = np.asarray(y, np.float32).ravel()
+            return self.backproject(w).grad.astype(np.float64).ravel()
+
+        return LinearOperator((int(rows.sum()), n), matvec=matvec, rmatvec=rmatvec, dtype=np.float64)
 
 
 def trace_rays(slowness, star, starts, receivers, *, delta: float = 10.0, max_nodes: int | None = None,
@@ -586,6 +745,43 @@ def misfit_gradient(slowness, star, starts, receivers, observed, *, delta: float
     residual = np.where(use, residual, np.float32(np.nan)).astype(np.float32)
     misfit = 0.5 * float(np.sum(residual[use].astype(np.float64) ** 2))
     return MisfitGradient(misfit, bp.grad, residual, bp.status, bp.quantum_exp)
+
+
+def linearized_update(slowness, star, starts, receivers, observed, *, damp: float, iter_lim: int,
+                      atol: float = 1e-6, btol: float = 1e-6, delta: float = 10.0, device: int | None = None,
+                      kernel: int | None = None, star_used: int | None = None) -> LinearizedUpdate:
+    """One damped linearised inversion step: the slowness perturbation that minimises ||G d - r||^2 + damp^2 ||d||^2
+    with the rays held fixed.  The companion of misfit_gradient, with its pick rule.
+
+    Solves every start, freezes the rays (SweepContext.freeze_rays), forms r = float32(observed - t) over the OK rays
+    with a pick (a NaN in observed [S, R] means no pick) and runs scipy.sparse.linalg.lsqr(G, r, damp, atol, btol,
+    iter_lim) on RaySet.as_linear_operator of those rays, every operator applied on the device from the frozen rays.
+    The update is returned, not applied: clamping the slowness and re-solving are the caller's policy.
+
+    G holds the rays fixed.  The discrete travel time is a minimum over paths of sums linear in the slowness, so it is
+    concave: the row of G of a ray is a supergradient of that ray's travel time (T(v + h) <= T(v) + G h up to
+    rounding), and its exact derivative wherever the predecessor of every node on the ray is unique."""
+    from scipy.sparse.linalg import lsqr
+    obs = np.asarray(observed, dtype=np.float32)
+    with SweepContext(device=device, kernel=kernel, star_used=star_used) as ctx:
+        ctx.set_model(slowness)
+        ctx.set_star(star, delta)
+        ctx.set_sources(starts)
+        ctx.run()
+        nrec = len(_make_starts(receivers))
+        if obs.shape != (ctx.nsrc, nrec):
+            raise SweepError(f"linearized_update: observed of shape {obs.shape}, expected {(ctx.nsrc, nrec)}")
+        with ctx.freeze_rays(receivers) as rs:
+            with np.errstate(invalid="ignore", over="ignore"):
+                residual = (obs - rs.tt).astype(np.float32)
+            use = np.isfinite(residual) & (rs.status == RAY_OK)
+            residual = np.where(use, residual, np.float32(np.nan)).astype(np.float32)
+            out = lsqr(rs.as_linear_operator(use), residual[use].astype(np.float64), damp=damp, atol=atol, btol=btol,
+                       iter_lim=iter_lim)
+            status = rs.status
+    misfit = 0.5 * float(np.sum(residual[use].astype(np.float64) ** 2))
+    return LinearizedUpdate(out[0].astype(np.float32).reshape(np.shape(slowness)), residual, status, misfit,
+                            int(out[1]), int(out[2]), float(out[3]))
 
 
 # ---- file formats -------------------------------------------------------------------------

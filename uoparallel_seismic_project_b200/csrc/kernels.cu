@@ -31,6 +31,8 @@
 //                     (one warp per ray, exact-match predecessor with a fixed tie rule).
 //   ray_project / ray_backproject  the travel-time tomography operators G*d and G^T*w over those rays (the tracer's
 //                     predecessor step, then a walk of the recorded path; exact int64 accumulation for G^T*w).
+//   rayset_record / rayset_compact / rayset_project / rayset_backproject  ray sets: the same rays traced once and
+//                     kept on the device as pull-table entries, then the same walks of the stored records.
 //   fill/pad/unpad/init_sources/min_slowness  the device float-box pool's utilities
 //                     (boxsetall/boxput, include/floatbox.h:176-199).
 // One grid over several devices (solver.cu, sweeptt_solve_slabs) runs relax_tiled unchanged on a travel-time box
@@ -1409,7 +1411,13 @@ __device__ __forceinline__ void backproject_ray(const TomoArgs& a, const RayPull
   });
 }
 
-template <bool BACK>
+// What the walk body does with a traced ray: the two operators, or (ray sets) keep its record.
+enum { WALK_PROJECT = 0, WALK_BACKPROJECT = 1, WALK_RECORD = 2 };
+
+// WALK_RECORD (sweeptt_rayset_freeze): the launch covers rays a.q_begin .. a.q_begin + t.nrays - 1 of the call; ray
+// q_begin + q leaves its record in staging slot q (a.path_global + q * max_nodes), its length, status and receiver
+// time at index q, and nothing is walked.
+template <int MODE>
 __device__ __forceinline__ void ray_walk_body(const TomoArgs& a, int4* smem) {
   const TraceArgs& t = a.t;
 #ifdef SWEEPTT_DEBUG_BOUNDS
@@ -1422,21 +1430,28 @@ __device__ __forceinline__ void ray_walk_body(const TomoArgs& a, int4* smem) {
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   const long long slot = (long long)blockIdx.x * (blockDim.x >> 5) + warp;
-  DBG_BOUNDS(!a.path_global || (slot + 1) * t.max_nodes <= a.path_entries);
-  unsigned short* path = a.path_global ? a.path_global + slot * t.max_nodes
-                                       : reinterpret_cast<unsigned short*>(smem + t.npull) + (size_t)warp * t.max_nodes;
+  DBG_BOUNDS(MODE == WALK_RECORD || !a.path_global || (slot + 1) * t.max_nodes <= a.path_entries);
+  unsigned short* path = MODE == WALK_RECORD ? nullptr
+                        : a.path_global      ? a.path_global + slot * t.max_nodes
+                                             : reinterpret_cast<unsigned short*>(smem + t.npull) + (size_t)warp * t.max_nodes;
   const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
   unsigned long long evals = 0;
   for (long long q = slot; q < t.nrays; q += warps) {
-    const int sr = (int)(q / t.nrec), r = (int)(q % t.nrec);
+    const long long qr = MODE == WALK_RECORD ? a.q_begin + q : q;  // the ray's number in the call
+    const int sr = (int)(qr / t.nrec), r = (int)(qr % t.nrec);
     const int s = t.source_begin + sr;
     const int px = t.src_xyz[3 * s], py = t.src_xyz[3 * s + 1], pz = t.src_xyz[3 * s + 2];
     const float* tt = t.tt + (size_t)s * t.g.vol;
     int x = t.rec_xyz[3 * r], y = t.rec_xyz[3 * r + 1], z = t.rec_xyz[3 * r + 2];
     DBG_BOUNDS((unsigned)x < (unsigned)t.g.nx && (unsigned)y < (unsigned)t.g.ny && (unsigned)z < (unsigned)t.g.nz);
     long long n = ((long long)(x + AX) * t.g.py + (y + AY)) * t.g.pz + (z + AZ);
-    const float w = BACK ? a.weights[q] : 0.f;
-    float tn = tt[n];
+    if (MODE == WALK_RECORD) {
+      DBG_BOUNDS(a.path_global && (q + 1) * t.max_nodes <= a.path_entries);
+      path = a.path_global + q * t.max_nodes;
+    }
+    const float w = MODE == WALK_BACKPROJECT ? a.weights[q] : 0.f;
+    const float t_rec = tt[n];
+    float tn = t_rec;
     int len = 1, status;
     __syncwarp();  // the previous ray's walk has read its record
     if (tn == CUDART_INF_F) {
@@ -1456,9 +1471,9 @@ __device__ __forceinline__ void ray_walk_body(const TomoArgs& a, int4* smem) {
       }
     }
     __syncwarp();  // the record is visible to every lane
-    if (BACK) {
+    if (MODE == WALK_BACKPROJECT) {
       if (status == SWEEPTT_RAY_OK && w != 0.f) backproject_ray(a, s_pull, path, len - 1, n, w);
-    } else {
+    } else if (MODE == WALK_PROJECT) {
       const float v = status == SWEEPTT_RAY_OK ? project_ray(a, s_pull, path, len - 1, n) : CUDART_NAN_F;
       if (lane == 0) {
         DBG_BOUNDS(q >= 0 && q < t.nrays);
@@ -1469,6 +1484,7 @@ __device__ __forceinline__ void ray_walk_body(const TomoArgs& a, int4* smem) {
       DBG_BOUNDS(q >= 0 && q < t.nrays && len >= 1 && len <= t.max_nodes);
       t.length[q] = len;
       t.status[q] = status;
+      if (MODE == WALK_RECORD) t.tt_rec[q] = t_rec;
     }
   }
   for (int o = 16; o; o >>= 1) evals += __shfl_xor_sync(0xffffffffu, evals, o);
@@ -1477,12 +1493,79 @@ __device__ __forceinline__ void ray_walk_body(const TomoArgs& a, int4* smem) {
 
 __global__ void __launch_bounds__(TRACE_THREADS) ray_project_kernel(const TomoArgs a) {
   extern __shared__ int4 s_tomo_raw[];
-  ray_walk_body<false>(a, s_tomo_raw);
+  ray_walk_body<WALK_PROJECT>(a, s_tomo_raw);
 }
 
 __global__ void __launch_bounds__(TRACE_THREADS) ray_backproject_kernel(const TomoArgs a) {
   extern __shared__ int4 s_tomo_raw[];
-  ray_walk_body<true>(a, s_tomo_raw);
+  ray_walk_body<WALK_BACKPROJECT>(a, s_tomo_raw);
+}
+
+// ---------------------------------------------------------------------------------------
+// ray sets (include/sweeptt.h, sweeptt_rayset_*)
+// ---------------------------------------------------------------------------------------
+// Freezing traces a bounded chunk of rays at a time with the walk body in record mode (every ray's record in a staging
+// slot of max_nodes entries), then rayset_compact_kernel packs the records of the chunk's OK rays ray-major in q order.
+// Applying the set walks the stored records with the operators' own project_ray / backproject_ray: no predecessor is
+// picked again, and no __constant__ table is read.
+// (4 CTAs per SM, as the tracer has: with no minimum ptxas settles on 48 registers and spills 8 bytes)
+__global__ void __launch_bounds__(TRACE_THREADS, 4) rayset_record_kernel(const TomoArgs a) {
+  extern __shared__ int4 s_tomo_raw[];
+  ray_walk_body<WALK_RECORD>(a, s_tomo_raw);
+}
+
+// One warp per ray of the chunk: the nedge = off[q+1] - off[q] leading entries of staging slot q go to dst + off[q].
+__global__ void __launch_bounds__(TRACE_THREADS) rayset_compact_kernel(const unsigned short* __restrict__ staging,
+                                                                      int max_nodes, const long long* __restrict__ off,
+                                                                      long long nrays, unsigned short* __restrict__ dst) {
+  const int lane = threadIdx.x & 31;
+  const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+  for (long long q = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); q < nrays; q += warps) {
+    const long long b = off[q], nedge = off[q + 1] - b;
+    DBG_BOUNDS(b >= 0 && nedge >= 0 && nedge < max_nodes && b + nedge <= off[nrays]);
+    for (long long j = lane; j < nedge; j += 32) dst[b + j] = staging[q * max_nodes + j];
+  }
+}
+
+template <bool BACK>
+__device__ __forceinline__ void rayset_walk_body(const RaySetArgs& s, int4* smem) {
+  const TomoArgs& a = s.a;
+  const TraceArgs& t = a.t;
+#ifdef SWEEPTT_DEBUG_BOUNDS
+  unsigned dyn_smem;
+  asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn_smem));
+  DBG_BOUNDS(t.npull >= 1 && t.npull < RAY_MAX_PULLS && (size_t)t.npull * sizeof(RayPull) <= dyn_smem);
+#endif
+  const RayPull* s_pull = stage_ray_pulls(t, smem);
+  const int lane = threadIdx.x & 31;
+  const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+  for (long long q = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); q < t.nrays; q += warps) {
+    const bool ok = t.status[q] == SWEEPTT_RAY_OK;
+    const long long b = s.offsets[q];
+    const int nedge = (int)(s.offsets[q + 1] - b);
+    const int sr = (int)(q / t.nrec);
+    const long long n_start = s.start_idx[sr];
+    DBG_BOUNDS(b >= 0 && nedge >= 0 && b + nedge <= s.entries_n && (ok || nedge == 0));
+    DBG_BOUNDS(sr >= 0 && (long long)sr * t.nrec < t.nrays && n_start >= 0 && n_start < t.g.vol);
+    const unsigned short* path = s.entries + b;
+    if (BACK) {
+      const float w = a.weights[q];
+      if (ok && w != 0.f) backproject_ray(a, s_pull, path, nedge, n_start, w);
+    } else {
+      const float v = ok ? project_ray(a, s_pull, path, nedge, n_start) : CUDART_NAN_F;
+      if (lane == 0) a.proj[q] = v;
+    }
+  }
+}
+
+__global__ void __launch_bounds__(TRACE_THREADS) rayset_project_kernel(const RaySetArgs s) {
+  extern __shared__ int4 s_tomo_raw[];
+  rayset_walk_body<false>(s, s_tomo_raw);
+}
+
+__global__ void __launch_bounds__(TRACE_THREADS) rayset_backproject_kernel(const RaySetArgs s) {
+  extern __shared__ int4 s_tomo_raw[];
+  rayset_walk_body<true>(s, s_tomo_raw);
 }
 
 // grad (dense, caller axes) := S * 2^E rounded once to float32 (nearest, ties to even), S the int64 accumulator
@@ -1928,6 +2011,52 @@ cudaError_t launch_ray_walk(bool backproject, const RayWalkLaunch& l, const Tomo
     ray_backproject_kernel<<<l.grid, TRACE_THREADS, l.smem, stream>>>(a);
   else
     ray_project_kernel<<<l.grid, TRACE_THREADS, l.smem, stream>>>(a);
+  return cudaGetLastError();
+}
+
+// Persistent warp-per-ray grid with the pull table in shared memory (the ray-set kernels).
+static cudaError_t rayset_grid(const void* fn, int npull, long long nrays, int device, int* grid, size_t* smem) {
+  *smem = (size_t)npull * sizeof(RayPull);
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)*smem);
+  if (e != cudaSuccess) return e;
+  int sms = 0, per_sm = 0;
+  e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+  if (e != cudaSuccess) return e;
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, TRACE_THREADS, *smem);
+  if (e != cudaSuccess) return e;
+  if (per_sm < 1) return cudaErrorInvalidConfiguration;
+  const long long need = (nrays + TRACE_THREADS / 32 - 1) / (TRACE_THREADS / 32);
+  *grid = (int)std::max(1LL, std::min<long long>(need, (long long)sms * per_sm));
+  return cudaSuccess;
+}
+
+cudaError_t launch_rayset_record(const TomoArgs& a, int device, cudaStream_t stream) {
+  int grid;
+  size_t smem;
+  cudaError_t e = rayset_grid((const void*)rayset_record_kernel, a.t.npull, a.t.nrays, device, &grid, &smem);
+  if (e != cudaSuccess) return e;
+  rayset_record_kernel<<<grid, TRACE_THREADS, smem, stream>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rayset_compact(const unsigned short* staging, int max_nodes, const long long* off, long long nrays,
+                                  unsigned short* dst, cudaStream_t stream) {
+  const long long need = (nrays + TRACE_THREADS / 32 - 1) / (TRACE_THREADS / 32);
+  rayset_compact_kernel<<<(unsigned)std::min<long long>(need, 4096), TRACE_THREADS, 0, stream>>>(staging, max_nodes, off,
+                                                                                                 nrays, dst);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rayset_walk(bool backproject, const RaySetArgs& s, int device, cudaStream_t stream) {
+  const void* fn = backproject ? (const void*)rayset_backproject_kernel : (const void*)rayset_project_kernel;
+  int grid;
+  size_t smem;
+  cudaError_t e = rayset_grid(fn, s.a.t.npull, s.a.t.nrays, device, &grid, &smem);
+  if (e != cudaSuccess) return e;
+  if (backproject)
+    rayset_backproject_kernel<<<grid, TRACE_THREADS, smem, stream>>>(s);
+  else
+    rayset_project_kernel<<<grid, TRACE_THREADS, smem, stream>>>(s);
   return cudaGetLastError();
 }
 

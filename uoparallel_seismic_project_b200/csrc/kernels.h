@@ -133,7 +133,9 @@ struct TomoArgs {
   long long* acc;              // back-projection: padded int64 accumulator box (zeroed by the caller)
   double scale;                // back-projection: 2^-E
   unsigned short* path_global; // per-warp path records in global memory (path_entries entries), or nullptr: in smem
+                               // (ray-set record mode: one staging slot of max_nodes entries per ray of the launch)
   long long path_entries;
+  long long q_begin;           // ray-set record mode: number of the launch's first ray in the call (t.nrays rays)
 };
 // Launch shape of a projection or back-projection: persistent grid, dynamic shared memory and where the path
 // records live (shared memory when that costs no occupancy; else path_global needs grid * warps * max_nodes entries).
@@ -145,6 +147,23 @@ struct RayWalkLaunch {
 };
 cudaError_t ray_walk_prepare(bool backproject, int npull, int max_nodes, long long nrays, int device, RayWalkLaunch* out);
 cudaError_t launch_ray_walk(bool backproject, const RayWalkLaunch& l, const TomoArgs& a, cudaStream_t stream);
+// Ray sets (include/sweeptt.h, sweeptt_rayset_*).  Record: rays q_begin .. q_begin + t.nrays - 1 traced as by
+// the operators, each ray's pull-table entries left in its staging slot a.path_global + q * max_nodes, its length,
+// status and receiver time in t.length / t.status / t.tt_rec at q.  Compact: the off[q+1] - off[q] leading entries
+// of slot q to dst + off[q].
+cudaError_t launch_rayset_record(const TomoArgs& a, int device, cudaStream_t stream);
+cudaError_t launch_rayset_compact(const unsigned short* staging, int max_nodes, const long long* off, long long nrays,
+                                  unsigned short* dst, cudaStream_t stream);
+// G*d or G^T*w over the stored records: a.t supplies g, pull, npull, nrec, nrays and status (the set's); a.pert /
+// a.proj or a.weights / a.acc / a.scale as for the operators.
+struct RaySetArgs {
+  TomoArgs a;
+  const long long* offsets;       // [nrays + 1] ray q's entries are entries[offsets[q] .. offsets[q+1])
+  const unsigned short* entries;  // pull-table entries of the OK rays, receiver end first (entries_n of them)
+  long long entries_n;
+  const long long* start_idx;     // [source_count] padded index of every source's start point
+};
+cudaError_t launch_rayset_walk(bool backproject, const RaySetArgs& s, int device, cudaStream_t stream);
 // grad (dense, caller axes) := acc * 2^E rounded once to float32.
 cudaError_t launch_grad_finish(const long long* acc, float* dense, BoxGeom g, int E, cudaStream_t stream);
 

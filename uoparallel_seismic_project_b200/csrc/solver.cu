@@ -1801,6 +1801,334 @@ extern "C" int sweeptt_ray_backproject(sweeptt_ctx* c, int source_begin, int sou
   return 1;
 }
 
+// ---------------------------------------------------------------------------------------
+// ray sets (include/sweeptt.h, sweeptt_rayset_*)
+// ---------------------------------------------------------------------------------------
+// A snapshot of traced rays: the records of the OK rays as pull-table entries, ray-major in q order (CSR), with the
+// pull table, geometry and start indices they are decoded with, and the buffers the two operators need.  Only the
+// context's device and stream are borrowed.
+struct sweeptt_rayset {
+  sweeptt_ctx* ctx = nullptr;
+  int device = 0;
+  BoxGeom g{};
+  int source_count = 0, nrec = 0;
+  long long nrays = 0, nentries = 0;
+  float hd_max = 0.f;
+  std::vector<RayPull> pull;          // the pull table at the freeze
+  std::vector<int> rec;               // receivers, caller axes
+  std::vector<int64_t> offsets;       // [nrays + 1] over the entries
+  std::vector<int32_t> length, status;
+  std::vector<float> tt;
+  RayPull* d_pull = nullptr;
+  long long* d_offsets = nullptr;
+  unsigned short* d_entries = nullptr;
+  int* d_status = nullptr;
+  long long* d_start = nullptr;
+  float* d_pert = nullptr;            // padded perturbation box
+  long long* d_acc = nullptr;         // padded int64 accumulator box
+  float* d_stage = nullptr;           // dense staging box
+  float* d_io = nullptr;              // [nrays] projections or weights
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  size_t bytes = 0;
+};
+
+static void rayset_free(sweeptt_rayset* r) {
+  void* bufs[] = {r->d_pull, r->d_offsets, r->d_entries, r->d_status, r->d_start, r->d_pert, r->d_acc, r->d_stage, r->d_io};
+  for (void* b : bufs) cudaFree(b);
+  if (r->ev0) cudaEventDestroy(r->ev0);
+  if (r->ev1) cudaEventDestroy(r->ev1);
+  delete r;
+}
+
+static int rayset_alloc(sweeptt_rayset* r, void** p, size_t bytes) {
+  if (bytes == 0) return 1;
+  CK(cudaMalloc(p, bytes));
+  r->bytes += bytes;
+  return 1;
+}
+
+// Staging of one freeze chunk: at most this many bytes of padded records (the chunk is at least one ray).
+static constexpr size_t RAYSET_STAGING_BYTES = size_t(256) << 20;
+
+static int rayset_freeze(sweeptt_ctx* c, int source_begin, int source_count, const struct START* receivers, int nrec,
+                         int max_nodes, sweeptt_stats* stats, sweeptt_rayset* r) {
+  ConstLease lease;
+  if (!check_ray_call(c, &lease, "sweeptt_rayset_freeze", source_begin, source_count, receivers, nrec, max_nodes, stats))
+    return 0;
+  if (!upload_ray_tables(c, nrec)) return 0;
+  const long long nrays = (long long)source_count * nrec;
+  const long long chunk = std::max(1LL, std::min<long long>(nrays, (long long)(RAYSET_STAGING_BYTES / (2 * (size_t)max_nodes))));
+  if (!ensure_dev(c, &c->d_path, &c->path_cap, (size_t)chunk * max_nodes * sizeof(unsigned short))) return 0;
+  // [evaluation counter | length | status | tt | chunk offsets], every part 16-byte aligned
+  const size_t per_ray = ((size_t)4 * chunk + 15) / 16 * 16;
+  if (!ensure_dev(c, &c->d_ray_out, &c->ray_out_cap, 16 + 3 * per_ray + 8 * (size_t)(chunk + 1))) return 0;
+  r->ctx = c;
+  r->device = c->device;
+  r->g = c->g;
+  r->source_count = source_count;
+  r->nrec = nrec;
+  r->nrays = nrays;
+  r->pull = c->ray_pull;
+  for (const RayPull& p : r->pull) r->hd_max = std::max(r->hd_max, p.hd);
+  r->rec.resize(3 * (size_t)nrec);
+  for (int q = 0; q < nrec; ++q) { r->rec[3 * q] = receivers[q].i; r->rec[3 * q + 1] = receivers[q].j; r->rec[3 * q + 2] = receivers[q].k; }
+  r->length.resize(nrays); r->status.resize(nrays); r->tt.resize(nrays); r->offsets.assign(nrays + 1, 0);
+  CK(cudaEventCreate(&r->ev0));
+  CK(cudaEventCreate(&r->ev1));
+
+  TomoArgs a{};
+  a.t = ray_trace_args(c, source_begin, nrec, 0, max_nodes);
+  a.t.evals = reinterpret_cast<unsigned long long*>(c->d_ray_out);
+  a.t.length = reinterpret_cast<int*>(c->d_ray_out + 16);
+  a.t.status = reinterpret_cast<int*>(c->d_ray_out + 16 + per_ray);
+  a.t.tt_rec = reinterpret_cast<float*>(c->d_ray_out + 16 + 2 * per_ray);
+  long long* d_off = reinterpret_cast<long long*>(c->d_ray_out + 16 + 3 * per_ray);
+  a.path_global = c->d_path;
+  CK(cudaMemsetAsync(a.t.evals, 0, 8, c->stream));
+  // each chunk's OK records are packed into a piece of their own; the pieces are joined once the total is known
+  struct Pieces {
+    std::vector<std::pair<unsigned short*, long long>> v;
+    ~Pieces() { for (auto& p : v) cudaFree(p.first); }
+  } pieces;
+  std::vector<int64_t> rel(chunk + 1);
+  double ms_total = 0, d2h_ms = 0;
+  long long launches = 0, d2h_bytes = 8;
+  for (long long q0 = 0; q0 < nrays; q0 += chunk) {
+    const long long nc = std::min(chunk, nrays - q0);
+    a.t.nrays = nc;
+    a.q_begin = q0;
+    a.path_entries = nc * max_nodes;
+    CK(cudaEventRecord(r->ev0, c->stream));
+    CK(launch_rayset_record(a, c->device, c->stream));
+    CK(cudaEventRecord(r->ev1, c->stream));
+    const auto t_copy = std::chrono::steady_clock::now();
+    CK(cudaMemcpyAsync(r->length.data() + q0, a.t.length, 4 * nc, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(r->status.data() + q0, a.t.status, 4 * nc, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(r->tt.data() + q0, a.t.tt_rec, 4 * nc, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    d2h_bytes += 12 * nc;
+    float ms = 0;
+    CK(cudaEventElapsedTime(&ms, r->ev0, r->ev1));
+    ms_total += ms;
+    ++launches;
+    rel[0] = 0;
+    for (long long q = 0; q < nc; ++q)
+      rel[q + 1] = rel[q] + (r->status[q0 + q] == SWEEPTT_RAY_OK ? r->length[q0 + q] - 1 : 0);
+    for (long long q = 0; q < nc; ++q) r->offsets[q0 + q + 1] = r->offsets[q0] + rel[q + 1];
+    if (rel[nc] == 0) continue;
+    unsigned short* piece = nullptr;
+    CK(cudaMalloc(&piece, (size_t)rel[nc] * sizeof(unsigned short)));
+    pieces.v.emplace_back(piece, rel[nc]);
+    CK(cudaMemcpyAsync(d_off, rel.data(), 8 * (size_t)(nc + 1), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaEventRecord(r->ev0, c->stream));
+    CK(launch_rayset_compact(c->d_path, max_nodes, d_off, nc, piece, c->stream));
+    CK(cudaEventRecord(r->ev1, c->stream));
+    CK(cudaEventSynchronize(r->ev1));  // before d_off and the staging slots are reused
+    CK(cudaEventElapsedTime(&ms, r->ev0, r->ev1));
+    ms_total += ms;
+    ++launches;
+  }
+  r->nentries = r->offsets[nrays];
+  unsigned long long evals = 0;
+  CK(cudaMemcpyAsync(&evals, a.t.evals, 8, cudaMemcpyDeviceToHost, c->stream));
+
+  const BoxGeom& g = r->g;
+  const size_t dense = (size_t)g.nx * g.ny * g.nz;
+  if (!rayset_alloc(r, (void**)&r->d_entries, (size_t)r->nentries * sizeof(unsigned short)) ||
+      !rayset_alloc(r, (void**)&r->d_offsets, 8 * (size_t)(nrays + 1)) ||
+      !rayset_alloc(r, (void**)&r->d_status, 4 * (size_t)nrays) ||
+      !rayset_alloc(r, (void**)&r->d_io, 4 * (size_t)nrays) ||
+      !rayset_alloc(r, (void**)&r->d_pull, r->pull.size() * sizeof(RayPull)) ||
+      !rayset_alloc(r, (void**)&r->d_start, 8 * (size_t)source_count) ||
+      !rayset_alloc(r, (void**)&r->d_pert, 4 * (size_t)g.vol) ||
+      !rayset_alloc(r, (void**)&r->d_acc, 8 * (size_t)g.vol) ||
+      !rayset_alloc(r, (void**)&r->d_stage, 4 * dense))
+    return 0;
+  long long at = 0;
+  for (auto& p : pieces.v) {
+    CK(cudaMemcpyAsync(r->d_entries + at, p.first, (size_t)p.second * sizeof(unsigned short), cudaMemcpyDeviceToDevice, c->stream));
+    at += p.second;
+  }
+  std::vector<long long> start(source_count);
+  for (int s = 0; s < source_count; ++s) {
+    const int* p = &c->src_xyz[3 * (size_t)(source_begin + s)];
+    start[s] = ((long long)(p[0] + AX) * g.py + (p[1] + AY)) * g.pz + (p[2] + AZ);
+  }
+  CK(cudaMemcpyAsync(r->d_offsets, r->offsets.data(), 8 * (size_t)(nrays + 1), cudaMemcpyHostToDevice, c->stream));
+  CK(cudaMemcpyAsync(r->d_status, r->status.data(), 4 * (size_t)nrays, cudaMemcpyHostToDevice, c->stream));
+  CK(cudaMemcpyAsync(r->d_pull, r->pull.data(), r->pull.size() * sizeof(RayPull), cudaMemcpyHostToDevice, c->stream));
+  CK(cudaMemcpyAsync(r->d_start, start.data(), 8 * (size_t)source_count, cudaMemcpyHostToDevice, c->stream));
+  CK(cudaStreamSynchronize(c->stream));  // the pieces and the host vectors above are released after this
+  if (stats) {
+    stats->struct_size = (int)sizeof *stats;
+    stats->solve_ms = ms_total;
+    stats->relaxations = (long long)evals;
+    stats->kernel_launches = launches;
+    stats->devices_used = 1;
+    stats->d2h_ms = d2h_ms;
+    stats->d2h_bytes = d2h_bytes;
+  }
+  return 1;
+}
+
+extern "C" sweeptt_rayset* sweeptt_rayset_freeze(sweeptt_ctx* c, int source_begin, int source_count,
+                                                 const struct START* receivers, int nrec, int max_nodes,
+                                                 sweeptt_stats* stats) {
+  auto* r = new sweeptt_rayset();
+  if (!rayset_freeze(c, source_begin, source_count, receivers, nrec, max_nodes, stats, r)) {
+    if (c) cudaSetDevice(c->device);
+    rayset_free(r);
+    return nullptr;
+  }
+  return r;
+}
+
+extern "C" void sweeptt_rayset_destroy(sweeptt_rayset* r) {
+  if (!r) return;
+  cudaSetDevice(r->device);
+  cudaStreamSynchronize(r->ctx->stream);
+  rayset_free(r);
+}
+
+extern "C" size_t sweeptt_rayset_bytes(const sweeptt_rayset* r) { return r ? r->bytes : 0; }
+
+extern "C" int sweeptt_rayset_table(const sweeptt_rayset* r, int32_t* length_out, int32_t* status_out, float* tt_out) {
+  if (!r) return fail("null ray set");
+  const size_t n = (size_t)r->nrays;
+  if (length_out) std::memcpy(length_out, r->length.data(), 4 * n);
+  if (status_out) std::memcpy(status_out, r->status.data(), 4 * n);
+  if (tt_out) std::memcpy(tt_out, r->tt.data(), 4 * n);
+  return 1;
+}
+
+extern "C" int sweeptt_rayset_paths(const sweeptt_rayset* r, int64_t* offsets_out, struct START* nodes_out) {
+  if (!r) return fail("null ray set");
+  if (offsets_out) {
+    offsets_out[0] = 0;
+    for (long long q = 0; q < r->nrays; ++q)
+      offsets_out[q + 1] = offsets_out[q] + (r->status[q] == SWEEPTT_RAY_OK ? r->length[q] : 0);
+  }
+  if (!nodes_out) return 1;
+  std::vector<unsigned short> e((size_t)r->nentries);
+  CK(cudaSetDevice(r->device));
+  if (r->nentries) {
+    CK(cudaMemcpyAsync(e.data(), r->d_entries, e.size() * sizeof(unsigned short), cudaMemcpyDeviceToHost, r->ctx->stream));
+    CK(cudaStreamSynchronize(r->ctx->stream));
+  }
+  const int* perm = r->g.perm;
+  START* out = nodes_out;
+  for (long long q = 0; q < r->nrays; ++q) {
+    if (r->status[q] != SWEEPTT_RAY_OK) continue;
+    int p[3];  // caller axes
+    std::memcpy(p, &r->rec[3 * (size_t)(q % r->nrec)], sizeof p);
+    *out++ = START{p[0], p[1], p[2]};
+    for (int64_t k = r->offsets[q]; k < r->offsets[q + 1]; ++k) {
+      const RayPull& o = r->pull[e[(size_t)k]];
+      p[perm[0]] += o.i; p[perm[1]] += o.j; p[perm[2]] += o.k;  // kernel axis q is caller axis perm[q]
+      *out++ = START{p[0], p[1], p[2]};
+    }
+  }
+  return 1;
+}
+
+// Shared part of the two operators once the inputs are on the device: the walk (and the rounding into d_stage),
+// timed with events, the stream synchronised.
+static int rayset_walk(sweeptt_rayset* r, bool back, RaySetArgs& s, int E, sweeptt_stats* stats) {
+  cudaStream_t st = r->ctx->stream;
+  CK(launch_rayset_walk(back, s, r->device, st));
+  if (back) CK(launch_grad_finish(r->d_acc, r->d_stage, r->g, E, st));
+  CK(cudaEventRecord(r->ev1, st));
+  CK(cudaEventSynchronize(r->ev1));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, r->ev0, r->ev1));
+  if (stats) {
+    stats->struct_size = (int)sizeof *stats;
+    stats->solve_ms = ms;
+    stats->kernel_launches = 2;
+    stats->devices_used = 1;
+  }
+  return 1;
+}
+
+static RaySetArgs rayset_args(const sweeptt_rayset* r) {
+  RaySetArgs s{};
+  s.a.t.g = r->g;
+  s.a.t.pull = r->d_pull;
+  s.a.t.npull = (int)r->pull.size();
+  s.a.t.nrec = r->nrec;
+  s.a.t.nrays = r->nrays;
+  s.a.t.status = r->d_status;
+  s.offsets = r->d_offsets;
+  s.entries = r->d_entries;
+  s.entries_n = r->nentries;
+  s.start_idx = r->d_start;
+  return s;
+}
+
+extern "C" int sweeptt_rayset_project(sweeptt_rayset* r, const float* perturbation, float* proj_out,
+                                      sweeptt_stats* stats) {
+  if (!r) return fail("null ray set");
+  if (stats) std::memset(stats, 0, sizeof *stats);
+  if (!perturbation) return fail("sweeptt_rayset_project: null perturbation");
+  CK(cudaSetDevice(r->device));
+  cudaStream_t st = r->ctx->stream;
+  const size_t dense = (size_t)r->g.nx * r->g.ny * r->g.nz;
+  RaySetArgs s = rayset_args(r);
+  s.a.pert = r->d_pert;
+  s.a.proj = r->d_io;
+  // only nodes on a ray are read, and those are in the box: the apron of d_pert is never looked at
+  CK(cudaMemcpyAsync(r->d_stage, perturbation, dense * 4, cudaMemcpyHostToDevice, st));
+  CK(cudaEventRecord(r->ev0, st));
+  CK(launch_pad_box(r->d_stage, r->d_pert, r->g, st));
+  if (!rayset_walk(r, false, s, 0, stats)) return 0;
+  const auto t_copy = std::chrono::steady_clock::now();
+  if (proj_out) {
+    CK(cudaMemcpyAsync(proj_out, r->d_io, 4 * (size_t)r->nrays, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+  }
+  if (stats) {
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes = proj_out ? 4 * r->nrays : 0;
+  }
+  return 1;
+}
+
+extern "C" int sweeptt_rayset_backproject(sweeptt_rayset* r, const float* weights, float* grad_out,
+                                          int* quantum_exp_out, sweeptt_stats* stats) {
+  if (!r) return fail("null ray set");
+  if (stats) std::memset(stats, 0, sizeof *stats);
+  if (!weights || !grad_out) return fail("sweeptt_rayset_backproject: weights and grad_out are required");
+  float W = 0.f;
+  for (long long q = 0; q < r->nrays; ++q) {
+    if (!std::isfinite(weights[q])) return fail("sweeptt_rayset_backproject: weight %lld is not finite", q);
+    W = std::max(W, std::fabs(weights[q]));
+  }
+  if (!std::isfinite(r->hd_max)) return fail("sweeptt_rayset_backproject: the star's edge lengths are not finite");
+  const int E = (W > 0.f && r->hd_max > 0.f) ? quantum_exponent(r->hd_max, W, r->nrays) : 0;
+  CK(cudaSetDevice(r->device));
+  cudaStream_t st = r->ctx->stream;
+  const BoxGeom& g = r->g;
+  const size_t dense = (size_t)g.nx * g.ny * g.nz;
+  RaySetArgs s = rayset_args(r);
+  s.a.weights = r->d_io;
+  s.a.acc = r->d_acc;
+  s.a.scale = std::ldexp(1.0, -E);
+  CK(cudaMemcpyAsync(r->d_io, weights, 4 * (size_t)r->nrays, cudaMemcpyHostToDevice, st));
+  CK(cudaEventRecord(r->ev0, st));
+  CK(cudaMemsetAsync(r->d_acc, 0, (size_t)g.vol * 8, st));
+  if (!rayset_walk(r, true, s, E, stats)) return 0;
+  const auto t_copy = std::chrono::steady_clock::now();
+  CK(cudaMemcpyAsync(grad_out, r->d_stage, dense * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  if (stats) {
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes = (long long)(dense * 4);
+  }
+  if (quantum_exp_out) *quantum_exp_out = E;
+  return 1;
+}
+
 extern "C" long long sweeptt_relaxations_per_round(sweeptt_ctx* c) { return c ? c->pulls_per_round : 0; }
 extern "C" size_t sweeptt_pool_bytes(sweeptt_ctx* c) { return c ? c->pool_bytes : 0; }
 extern "C" long long sweeptt_tiles_per_source(sweeptt_ctx* c) {
