@@ -94,7 +94,7 @@ _EXPORTS = [
     "sweeptt_set_sources", "sweeptt_run", "sweeptt_step", "sweeptt_reset", "sweeptt_get_tt", "sweeptt_put_tt",
     "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject",
     "sweeptt_rayset_freeze", "sweeptt_rayset_destroy", "sweeptt_rayset_bytes", "sweeptt_rayset_table",
-    "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_solve_slabs",
+    "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_debug_model_stats", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
     "sweeptt_vbox_load", "sweeptt_vbox_store", "sweeptt_vbox_load_subset", "sweeptt_text_load",
     "sweeptt_star_load", "sweeptt_starts_load", "sweeptt_write_output_tt", "sweeptt_free",
@@ -163,6 +163,7 @@ def load_library() -> C.CDLL:
     lib.sweeptt_pool_bytes.restype = C.c_size_t
     lib.sweeptt_tiles_per_source.argtypes = [C.c_void_p]
     lib.sweeptt_tiles_per_source.restype = C.c_longlong
+    lib.sweeptt_debug_model_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.sweeptt_solve_slabs.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(FS), C.c_int, START,
                                         C.c_void_p, C.POINTER(_Opts), C.POINTER(_Stats)]
     lib.sweeptt_solve_slabs_vbox.argtypes = [C.c_char_p, C.POINTER(FS), C.c_int, START, C.c_void_p, C.POINTER(_Opts),
@@ -430,8 +431,8 @@ class SweepContext:
 
     def set_model(self, slowness):
         v = np.ascontiguousarray(slowness, dtype=np.float32)
-        self.dims = v.shape
         _check(self._lib.sweeptt_set_model(self._h, v.ctypes.data, *v.shape), "sweeptt_set_model")
+        self.dims = v.shape  # (a refused model leaves the previous one, and its dimensions)
 
     def set_star(self, star, delta: float = 10.0):
         fs = _as_star(star, delta)
@@ -439,8 +440,8 @@ class SweepContext:
 
     def set_sources(self, starts):
         st = _make_starts(starts)
-        self.nsrc = len(st)
         _check(self._lib.sweeptt_set_sources(self._h, st, len(st)), "sweeptt_set_sources")
+        self.nsrc = len(st)
 
     def run(self) -> SweepStats:
         s = _Stats()
@@ -595,6 +596,13 @@ class SweepContext:
     @property
     def pool_bytes(self) -> int:
         return self._lib.sweeptt_pool_bytes(self._h)
+
+    def model_stats(self):
+        """Test hook: (vmin, vmax, vpos) the context keeps of its model (include/sweeptt.h)."""
+        out = np.zeros(3, np.float32)
+        _check(self._lib.sweeptt_debug_model_stats(self._h, out[0:].ctypes.data, out[1:].ctypes.data,
+                                                   out[2:].ctypes.data), "sweeptt_debug_model_stats")
+        return tuple(out)
 
 
 class RaySet:

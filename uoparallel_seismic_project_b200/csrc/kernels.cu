@@ -3,7 +3,7 @@
 // What is computed (arithmetic contract, SURVEY.md §8a): for every node n != start
 //     tt[n] = min(tt[n], min over pull offsets o of  fl(fl(hd_o * fl(v_n + v_{n+o})) + tt[n+o]))
 // which is the pull form of the reference's two-sided relaxation
-// (serial_new/sweep-tt-multistart.c:216,222-249) with hd_o = d_o/2 (exact halving) and NO
+// (serial_new/sweep-tt-multistart.c:216,222-249) with hd_o = d_o/2 (exact inside the domain of DESIGN §1) and NO
 // fused multiply-add anywhere (__fmul_rn/__fadd_rn never contract; the file is also built
 // with -fmad=false).  Any fair relaxation order reaches the same fixed point bit-for-bit,
 // because fl(a+c) is monotone in a and travel times only ever decrease.
@@ -1642,18 +1642,29 @@ __global__ void unpad_kernel(const float* __restrict__ padded, float* __restrict
 }
 // Statistics of the model in one pass over the dense staged box: out[0] = float bits of the smallest slowness,
 // out[1] != 0 when a value is negative or NaN (switches the downwind filter off), then (8-byte aligned) the sum
-// (double) and the count (unsigned long long) of the finite values -- the mean only scales the activation bucket.
+// (double) and the count (unsigned long long) of the finite values -- the mean only scales the activation bucket --
+// then out[6] = bits of the largest finite slowness and out[7] = bits of the smallest positive one (+INF if none).
+// The bits of non-negative floats order like the floats; -0.0 counts as +0.0 (its bits would order above +INF).
 __global__ void min_slowness_kernel(const float* __restrict__ dense, long long n, unsigned* out) {
-  unsigned m = 0x7f800000u, bad = 0u;
+  unsigned m = 0x7f800000u, bad = 0u, mx = 0u, pos = 0x7f800000u;
   double sum = 0.0;
   unsigned long long cnt = 0ull;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const float v = dense[i];
-    if (v >= 0.f) m = min(m, __float_as_uint(v)); else bad = 1u;
+    if (v >= 0.f) {
+      const unsigned b = __float_as_uint(v) & 0x7fffffffu;
+      m = min(m, b);
+      if (b != 0x7f800000u) mx = max(mx, b);
+      if (b != 0u) pos = min(pos, b);
+    } else {
+      bad = 1u;
+    }
     if (v == v && fabsf(v) != CUDART_INF_F) { sum += (double)v; ++cnt; }
   }
   m = __reduce_min_sync(0xffffffffu, m);
   bad = __reduce_or_sync(0xffffffffu, bad);
+  mx = __reduce_max_sync(0xffffffffu, mx);
+  pos = __reduce_min_sync(0xffffffffu, pos);
   for (int o = 16; o; o >>= 1) {
     sum += __shfl_xor_sync(0xffffffffu, sum, o);
     cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
@@ -1663,15 +1674,15 @@ __global__ void min_slowness_kernel(const float* __restrict__ dense, long long n
     if (bad) atomicOr(&out[1], 1u);
     atomicAdd(reinterpret_cast<double*>(out + 2), sum);
     atomicAdd(reinterpret_cast<unsigned long long*>(out + 4), cnt);
+    atomicMax(&out[6], mx);
+    atomicMin(&out[7], pos);
   }
 }
-cudaError_t launch_min_slowness(const float* dense, long long n, unsigned* out6, cudaStream_t stream) {
-  cudaError_t e = cudaMemsetAsync(out6, 0, 24, stream);
+cudaError_t launch_min_slowness(const float* dense, long long n, unsigned* out8, cudaStream_t stream) {
+  static const unsigned init[8] = {0x7f800000u, 0u, 0u, 0u, 0u, 0u, 0u, 0x7f800000u};
+  cudaError_t e = cudaMemcpyAsync(out8, init, sizeof init, cudaMemcpyHostToDevice, stream);  // (pageable source: staged at call time)
   if (e != cudaSuccess) return e;
-  const unsigned inf_bits = 0x7f800000u;
-  e = cudaMemcpyAsync(out6, &inf_bits, 4, cudaMemcpyHostToDevice, stream);  // (pageable 4-byte source: staged at call time)
-  if (e != cudaSuccess) return e;
-  min_slowness_kernel<<<1184, 256, 0, stream>>>(dense, n, out6);
+  min_slowness_kernel<<<1184, 256, 0, stream>>>(dense, n, out8);
   return cudaGetLastError();
 }
 

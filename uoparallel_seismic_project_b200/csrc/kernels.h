@@ -173,9 +173,11 @@ cudaError_t launch_pad_box(const float* dense, float* padded, BoxGeom g, cudaStr
 cudaError_t launch_unpad_box(const float* padded, float* dense, BoxGeom g, cudaStream_t stream);
 // tt := INF everywhere, 0 at each start; state, flags and the first work list reset.
 cudaError_t launch_reset(const RelaxArgs& a, int max_rounds, cudaStream_t stream);
-// Model statistics, 24 bytes (8-byte aligned): out6[0] = float bits of the smallest slowness of the dense staged
-// model, out6[1] != 0 if any value is negative/NaN, then sum (double) and count (u64) of the finite values
-cudaError_t launch_min_slowness(const float* dense, long long n, unsigned* out6, cudaStream_t stream);
+// Model statistics, 32 bytes (8-byte aligned): out8[0] = float bits of the smallest slowness of the dense staged
+// model (-0.0 counted as +0.0), out8[1] != 0 if any value is negative/NaN, then sum (double) and count (u64) of the
+// finite values, out8[6] = bits of the largest finite slowness (0 if none), out8[7] = bits of the smallest positive
+// slowness (+INF if none)
+cudaError_t launch_min_slowness(const float* dense, long long n, unsigned* out8, cudaStream_t stream);
 // tmax[] := INF (call whenever travel times were overwritten from outside, e.g. sweeptt_put_tt)
 cudaError_t launch_fill_tmax(const RelaxArgs& a, cudaStream_t stream);
 cudaError_t launch_reset_state_only(SolveState* st, int max_rounds, cudaStream_t stream);

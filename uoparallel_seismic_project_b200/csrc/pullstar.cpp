@@ -37,6 +37,12 @@ PullStar build_pull_star(const FS* fs, int starsize, int star_used) {
   for (int l = 0; l < star_used; ++l) {
     const FS& e = fs[l];
     if (e.i == 0 && e.j == 0 && e.k == 0) continue;  // self edge: can never change anything
+    if (!(e.d >= 0.f) || std::isinf(e.d)) {  // negative or NaN, or infinite
+      if (ps.bad_d < 0) ps.bad_d = l;
+    } else {
+      ps.dmax = std::max(ps.dmax, e.d);
+      if (e.d > 0.f) ps.dpos = std::min(ps.dpos, e.d);
+    }
     have[Key{e.i, e.j, e.k, bits_of(e.d)}] |= 1;
     have[Key{-e.i, -e.j, -e.k, bits_of(e.d)}] |= 2;
   }

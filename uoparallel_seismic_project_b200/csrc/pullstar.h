@@ -7,6 +7,7 @@
 // equivalent PULL form: for node n, which neighbours m = n+o may lower tt[n], with which
 // half-distance, and which of those pulls are invalid when m is the start point.
 #pragma once
+#include <cmath>
 #include <cstdint>
 #include <vector>
 
@@ -16,7 +17,7 @@ namespace sweeptt {
 
 struct PullOffset {
   int i, j, k;   // m = n + (i,j,k)
-  float hd;      // 0.5f * d   (halving is exact, so hd*(v_n+v_m) == d*(v_n+v_m)/2.0)
+  float hd;      // 0.5f * d   (hd*(v_n+v_m) == d*(v_n+v_m)/2.0 inside the domain of DESIGN §1)
   int guarded;   // 1: only supplied by "centre m relaxes neighbour n" => invalid when m == start
 };
 
@@ -37,6 +38,9 @@ struct PullStar {
   std::vector<float> col_hd;         // hd of the column-grouped pulls
   std::vector<PullOffset> extra;     // pulls handled one at a time (guarded or duplicates)
   int rx = 0, ry = 0, rz = 0;        // max |i|, |j|, |k| over all pulls
+  float dmax = 0.f;                  // largest d of the star's edges (0 if none)
+  float dpos = HUGE_VALF;            // smallest positive d of the star's edges (+INF if none)
+  int bad_d = -1;                    // first used entry whose d is negative, NaN or infinite (-1: none)
   bool fits_tiled() const { return rx <= RXY_MAX && ry <= RXY_MAX && rz <= KHALO; }
 };
 

@@ -151,6 +151,8 @@ struct sweeptt_ctx {
   unsigned* d_busy = nullptr;  // per-tile "on a list / being relaxed" flags (single-launch scheduling)
   unsigned* d_keysnap = nullptr;  // key snapshot of the device-side list builder
   float min_slowness = 0.f;    // exact minimum of the model (device reduction); < 0: negative/NaN values present
+  float max_slowness = 0.f;    // largest finite slowness of the model (domain guard, ready())
+  float pos_slowness = std::numeric_limits<float>::infinity();  // smallest positive slowness (+INF: none)
   float bucket = -1.f;         // bucket width in travel-time units (<0: relax every dirty tile each round)
   double mean_slowness = 0;
   size_t tiles_cap = 0;  // nsrc*ntiles the lists/flags were sized for
@@ -462,6 +464,67 @@ static int compute_geometry(sweeptt_ctx* c, int nx, int ny, int nz, BoxGeom* out
   return 1;
 }
 
+// Halo variant of the tiled kernel that holds the star (0: the star does not fit the tiled kernel).
+static int tiled_rxy(const PullStar& s) {
+  const bool fits = s.fits_tiled() && (int)s.columns.size() + MAX_PATTERNS + 2 <= MAX_COLUMNS &&
+                    (int)s.col_hd.size() <= MAX_COL_HD && (int)s.extra.size() <= MAX_EXTRA;
+  return fits ? tiled_variant_for_radius(std::max(s.rx, s.ry)) : 0;
+}
+
+// A star built in kernel axis order and checked, not yet part of the context: every refusal of a star happens in
+// build_star, before set_star or set_model changes anything.
+struct StarBuild {
+  std::vector<FS> fs;  // the caller's entries, caller axis order
+  PullStar ps;         // the pull star in kernel axis order
+};
+
+static int build_star(const sweeptt_ctx* c, const FS* fs, int starsize, const int* perm, const char* who, StarBuild* out) {
+  out->fs.assign(fs, fs + starsize);  // (fs may alias c->fs)
+  std::vector<FS> pf(out->fs);
+  if (perm)
+    for (auto& e : pf) {
+      const int o[3] = {e.i, e.j, e.k};
+      e.i = o[perm[0]]; e.j = o[perm[1]]; e.k = o[perm[2]];
+    }
+  const PullStar& ps = out->ps = build_pull_star(pf.data(), starsize, c->opts.star_used);
+  if (ps.bad_d >= 0) {
+    const FS& e = out->fs[ps.bad_d];
+    return fail("%s: entry %d (%d,%d,%d) has distance d = %g; every used entry needs a finite d >= 0 (a negative d "
+                "gives travel times that are not bounded below)", who, ps.bad_d, e.i, e.j, e.k, (double)e.d);
+  }
+  if (ps.all.empty()) return fail("%s: the star has no usable offsets", who);
+  if (c->opts.kernel == SWEEPTT_KERNEL_TILED && tiled_rxy(ps) == 0)
+    return fail("%s: the tiled kernel holds |i|,|j| <= %d, |k| <= %d and <= %d guarded offsets; this star needs "
+                "(%d,%d,%d) / %d in kernel axis order", who, RXY_MAX, KHALO, MAX_EXTRA, ps.rx, ps.ry, ps.rz,
+                (int)ps.extra.size());
+  return 1;
+}
+
+// Makes a built star the context's star (fails only on a CUDA error).
+static int commit_star(sweeptt_ctx* c, StarBuild& b) {
+  std::vector<StarDev> sd(b.ps.all.size());
+  for (size_t l = 0; l < sd.size(); ++l) {
+    const PullOffset& p = b.ps.all[l];
+    sd[l] = StarDev{p.i, p.j, p.k, p.hd, p.guarded};
+  }
+  CK(cudaStreamSynchronize(c->stream));
+  cudaFree(c->d_star);
+  c->d_star = nullptr;
+  c->have_star = false;
+  CK(cudaMalloc(&c->d_star, sd.size() * sizeof(StarDev)));
+  CK(cudaMemcpy(c->d_star, sd.data(), sd.size() * sizeof(StarDev), cudaMemcpyHostToDevice));
+  c->fs.swap(b.fs);
+  c->star = std::move(b.ps);
+  c->nstar = (int)sd.size();
+  c->have_star = true;
+  c->star_gen += 1;
+  c->consts_rxy = -1;
+  invalidate_graph(c);
+  if (!choose_kernel(c)) return 0;
+  if (c->have_model && !build_tile_pulls(c)) return 0;
+  return 1;
+}
+
 extern "C" int sweeptt_set_model(sweeptt_ctx* c, const float* slowness, int nx, int ny, int nz) {
   if (!c || !slowness) return fail("sweeptt_set_model: null argument");
   if (nx <= 0 || ny <= 0 || nz <= 0) return fail("sweeptt_set_model: bad dimensions %d x %d x %d", nx, ny, nz);
@@ -471,36 +534,45 @@ extern "C" int sweeptt_set_model(sweeptt_ctx* c, const float* slowness, int nx, 
   nx = g.nx; ny = g.ny; nz = g.nz;  // from here on: kernel axis order
   const bool same = c->have_model && c->g.px == g.px && c->g.py == g.py && c->g.pz == g.pz;
   const bool perm_changed = !c->have_model || std::memcmp(c->g.perm, g.perm, sizeof g.perm) != 0;
-  if (!same) {
+  // check the model, and the star in the model's kernel axis order (the star tables are kept in that order), before
+  // anything of the context changes: a refused model leaves the previous model, star and sources
+  const bool rebuild_star = c->have_star && perm_changed;
+  StarBuild sb;
+  if (rebuild_star && !build_star(c, c->fs.data(), (int)c->fs.size(), g.perm, "sweeptt_set_model", &sb)) return 0;
+  const size_t dense = (size_t)nx * ny * nz;
+  if (!ensure_stage(c, dense)) return 0;
+  unsigned r[8];
+  {
+    // exact minimum of the model: lower bound of every edge delay for the downwind filter; the largest finite and
+    // the smallest positive value bound the domain (ready()); the mean of the finite values only scales the
+    // activation bucket (scheduling, never the arithmetic).  One device pass instead of a host loop.
+    CK(cudaMemcpyAsync(c->d_stage, slowness, dense * 4, cudaMemcpyHostToDevice, c->stream));
+    CK(launch_min_slowness(c->d_stage, (long long)dense, reinterpret_cast<unsigned*>(c->d_viol), c->stream));
+    CK(cudaMemcpyAsync(r, c->d_viol, sizeof r, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
+    if (r[1])
+      return fail("sweeptt_set_model: the model holds negative or NaN slowness values (travel times would not be "
+                  "bounded below; the reference itself never converges on such input)");
+  }
+  if (!same) {
     dev_free(c, c->d_slow, (size_t)c->g.vol * 4);
     c->d_slow = nullptr;
     dev_free(c, c->d_tt, (size_t)c->g.vol * 4 * c->tt_cap);
     c->d_tt = nullptr; c->tt_cap = 0; c->have_sources = false;
-    if (!dev_alloc(c, (void**)&c->d_slow, (size_t)g.vol * 4)) return 0;
+    c->have_model = false;
     c->maps_valid = false;
     invalidate_graph(c);
+    if (!dev_alloc(c, (void**)&c->d_slow, (size_t)g.vol * 4)) return 0;
   }
   c->g = g;
-  const size_t dense = (size_t)nx * ny * nz;
-  if (!ensure_stage(c, dense)) return 0;
   CK(launch_fill(c->d_slow, g.vol, std::numeric_limits<float>::infinity(), c->stream));
-  CK(cudaMemcpyAsync(c->d_stage, slowness, dense * 4, cudaMemcpyHostToDevice, c->stream));
   CK(launch_pad_box(c->d_stage, c->d_slow, g, c->stream));
   {
-    // exact minimum of the model: lower bound of every edge delay for the downwind filter
-    // ... and the mean of the finite values, which only scales the activation bucket (scheduling, never the
-    // arithmetic); one device pass instead of a host loop over the caller's array
-    unsigned r[6] = {0, 1, 0, 0, 0, 0};
-    CK(launch_min_slowness(c->d_stage, (long long)dense, reinterpret_cast<unsigned*>(c->d_viol), c->stream));
-    CK(cudaMemcpyAsync(r, c->d_viol, sizeof r, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
     float vmin;
     std::memcpy(&vmin, &r[0], 4);
-    if (r[1])
-      return fail("sweeptt_set_model: the model holds negative or NaN slowness values (travel times would not be "
-                  "bounded below; the reference itself never converges on such input)");
     c->min_slowness = !std::isfinite(vmin) ? -1.f : vmin;
+    std::memcpy(&c->max_slowness, &r[6], 4);
+    std::memcpy(&c->pos_slowness, &r[7], 4);
     double sum;
     unsigned long long cnt;
     std::memcpy(&sum, &r[2], 8);
@@ -509,15 +581,9 @@ extern "C" int sweeptt_set_model(sweeptt_ctx* c, const float* slowness, int nx, 
     invalidate_graph(c);
   }
   c->have_model = true;
-  if (c->have_star) {
-    if (perm_changed) {  // the star tables are kept in kernel axis order
-      std::vector<FS> fs = c->fs;
-      if (!sweeptt_set_star(c, fs.data(), (int)fs.size())) return 0;
-    } else if (!build_tile_pulls(c)) {
-      return 0;
-    }
-  }
   if (perm_changed) c->have_sources = false;
+  if (rebuild_star) return commit_star(c, sb);
+  if (c->have_star && !build_tile_pulls(c)) return 0;
   return 1;
 }
 
@@ -577,53 +643,19 @@ extern "C" int sweeptt_set_star(sweeptt_ctx* c, const struct FS* fs, int starsiz
   if (!c || !fs) return fail("sweeptt_set_star: null argument");
   if (starsize < 2) return fail("sweeptt_set_star: a forward star needs at least 2 entries (the last one is unused)");
   CK(cudaSetDevice(c->device));
-  {
-    std::vector<FS> keep(fs, fs + starsize);  // (fs may alias c->fs)
-    c->fs.swap(keep);
-  }
-  {
-    // kernel axis order (identity until a model has been set; set_model re-runs this)
-    std::vector<FS> pf(c->fs);
-    if (c->have_model)
-      for (auto& e : pf) {
-        const int o[3] = {e.i, e.j, e.k};
-        e.i = o[c->g.perm[0]]; e.j = o[c->g.perm[1]]; e.k = o[c->g.perm[2]];
-      }
-    c->star = build_pull_star(pf.data(), starsize, c->opts.star_used);
-  }
-  if (c->star.all.empty()) return fail("sweeptt_set_star: the star has no usable offsets");
-  std::vector<StarDev> sd(c->star.all.size());
-  for (size_t l = 0; l < sd.size(); ++l) {
-    const PullOffset& p = c->star.all[l];
-    sd[l] = StarDev{p.i, p.j, p.k, p.hd, p.guarded};
-  }
-  CK(cudaStreamSynchronize(c->stream));
-  cudaFree(c->d_star);
-  c->d_star = nullptr;
-  CK(cudaMalloc(&c->d_star, sd.size() * sizeof(StarDev)));
-  CK(cudaMemcpy(c->d_star, sd.data(), sd.size() * sizeof(StarDev), cudaMemcpyHostToDevice));
-  c->nstar = (int)sd.size();
-  c->have_star = true;
-  c->star_gen += 1;
-  c->consts_rxy = -1;
-  invalidate_graph(c);
-  if (!choose_kernel(c)) return 0;
-  if (c->have_model && !build_tile_pulls(c)) return 0;
-  return 1;
+  // kernel axis order: identity until a model has been set (set_model re-builds the star when the order changes)
+  StarBuild b;
+  if (!build_star(c, fs, starsize, c->have_model ? c->g.perm : nullptr, "sweeptt_set_star", &b)) return 0;
+  return commit_star(c, b);
 }
 
 static int choose_kernel(sweeptt_ctx* c) {
   const int want = c->opts.kernel;
-  int rxy = 0;
-  const bool fits = c->star.fits_tiled() && (int)c->star.columns.size() + MAX_PATTERNS + 2 <= MAX_COLUMNS && (int)c->star.col_hd.size() <= MAX_COL_HD && (int)c->star.extra.size() <= MAX_EXTRA;
-  if (fits) rxy = tiled_variant_for_radius(std::max(c->star.rx, c->star.ry));
+  int rxy = tiled_rxy(c->star);
   if (want == SWEEPTT_KERNEL_SIMPLE || (want == SWEEPTT_KERNEL_AUTO && rxy == 0)) {
     c->kernel_used = SWEEPTT_KERNEL_SIMPLE;
     return 1;
   }
-  if (rxy == 0)
-    return fail("the tiled kernel holds |i|,|j| <= %d, |k| <= %d and <= %d guarded offsets; this star needs (%d,%d,%d) / %d",
-                RXY_MAX, KHALO, MAX_EXTRA, c->star.rx, c->star.ry, c->star.rz, (int)c->star.extra.size());
   // group the columns by k-pattern (ascending mask): the stock-star kernels run one unrolled
   // code block per pattern over a contiguous column range
   std::stable_sort(c->star.columns.begin(), c->star.columns.end(),
@@ -958,9 +990,35 @@ static RelaxArgs make_args(sweeptt_ctx* c) {
   return a;
 }
 
+// The kernels evaluate an edge delay as fl(hd * fl(v_n + v_m)) with hd = fl(0.5f * d), the reference as
+// fl(fl(d * fl(v_n + v_m)) / 2.0).  The two agree for every edge of the model and star when (DESIGN §1)
+//   fl(dmax * fl(vmax + vmax)) is finite    (else the reference's product overflows where the kernels' does not),
+//   every positive d is >= 2^-125            (else hd = 0.5f * d rounds),
+//   fl(dpos * vpos) >= 2^-125                (else the reference's halving rounds a second time, in the subnormals),
+// with dmax / dpos the largest / smallest positive d of the star's edges and vmax / vpos the largest finite /
+// smallest positive slowness (every fl(v_n + v_m) that is not 0 is >= vpos).  A model and star outside are refused.
+static int check_domain(const sweeptt_ctx* c) {
+  const float lo = std::ldexp(1.f, -125);
+  const PullStar& s = c->star;
+  if (s.dpos < lo)
+    return fail("star distance d = %g is below 2^-125: 0.5f * d would round, the kernels' delays would differ from "
+                "the reference's d * (v_n + v_m) / 2.0", (double)s.dpos);
+  const float two_v = c->max_slowness + c->max_slowness;
+  if (std::isinf(s.dmax * two_v))
+    return fail("slowness %g with star distance %g: d * (v + v) = inf overflows float (the largest slowness must keep "
+                "dmax * 2 vmax <= FLT_MAX), the kernels' delays would differ from the reference's d * (v_n + v_m) / 2.0",
+                (double)c->max_slowness, (double)s.dmax);
+  if (s.dpos * c->pos_slowness < lo)
+    return fail("slowness %g with star distance %g: d * v = %g is below 2^-125 (the smallest positive slowness must keep "
+                "dpos * vpos >= 2^-125), the kernels' delays would differ from the reference's d * (v_n + v_m) / 2.0",
+                (double)c->pos_slowness, (double)s.dpos, (double)(s.dpos * c->pos_slowness));
+  return 1;
+}
+
 static int ready(sweeptt_ctx* c, ConstLease* lease) {
   if (!c) return fail("null context");
   if (!c->have_model || !c->have_star || !c->have_sources) return fail("context needs a model, a star and start points first");
+  if (!check_domain(c)) return 0;
   CK(cudaSetDevice(c->device));
   if (c->kernel_used == SWEEPTT_KERNEL_TILED) {
     if (!build_maps(c)) return 0;
@@ -2131,6 +2189,13 @@ extern "C" int sweeptt_rayset_backproject(sweeptt_rayset* r, const float* weight
 
 extern "C" long long sweeptt_relaxations_per_round(sweeptt_ctx* c) { return c ? c->pulls_per_round : 0; }
 extern "C" size_t sweeptt_pool_bytes(sweeptt_ctx* c) { return c ? c->pool_bytes : 0; }
+extern "C" int sweeptt_debug_model_stats(sweeptt_ctx* c, float* vmin, float* vmax, float* vpos) {
+  if (!c || !c->have_model) return fail("sweeptt_debug_model_stats: no model");
+  if (vmin) *vmin = c->min_slowness;
+  if (vmax) *vmax = c->max_slowness;
+  if (vpos) *vpos = c->pos_slowness;
+  return 1;
+}
 extern "C" long long sweeptt_tiles_per_source(sweeptt_ctx* c) {
   return (c && c->have_model) ? (long long)c->g.ntx * c->g.nty * c->g.ntz : 0;
 }
@@ -2501,6 +2566,7 @@ struct Part {
   int ok = 1;
   std::string err;
   double min_slow = std::numeric_limits<double>::infinity(), sum_slow = 0;
+  float max_slow = 0.f, pos_slow = std::numeric_limits<float>::infinity();  // domain guard (check_domain)
   unsigned long long cnt_slow = 0;
   bool bad_slow = false;
 };
@@ -2694,14 +2760,17 @@ static int solve_slabs_impl(const std::function<int(const int*, const int*, floa
         // local plane of logical plane x of this block: lb * PB + (x - b.first) + 7  (= padded plane x + AX of the
         // global box, shifted to the block's origin); launch_pad_box writes relative plane r at r + AX
         PCK(launch_pad_box(c->d_stage, c->d_slow + ((long long)lb * PB + (e.first - b.first) + RXY_MAX - AX) * g.sx, gs, c->stream));
-        unsigned r[6] = {0, 0, 0, 0, 0, 0};
+        unsigned r[8] = {0, 0, 0, 0, 0, 0, 0, 0};
         PCK(launch_min_slowness(c->d_stage, (long long)cnt, reinterpret_cast<unsigned*>(c->d_viol), c->stream));
         PCK(cudaMemcpyAsync(r, c->d_viol, sizeof r, cudaMemcpyDeviceToHost, c->stream));
         PCK(cudaStreamSynchronize(c->stream));
-        float vmin; double sum; unsigned long long cn;
+        float vmin, vmax, vpos; double sum; unsigned long long cn;
         std::memcpy(&vmin, &r[0], 4); std::memcpy(&sum, &r[2], 8); std::memcpy(&cn, &r[4], 8);
+        std::memcpy(&vmax, &r[6], 4); std::memcpy(&vpos, &r[7], 4);
         if (r[1]) pt.bad_slow = true;
         pt.min_slow = std::min(pt.min_slow, (double)vmin);
+        pt.max_slow = std::max(pt.max_slow, vmax);
+        pt.pos_slow = std::min(pt.pos_slow, vpos);
         pt.sum_slow += sum; pt.cnt_slow += cn;
       }
       if (h_stage) cudaFreeHost(h_stage);
@@ -2710,11 +2779,17 @@ static int solve_slabs_impl(const std::function<int(const int*, const int*, floa
     // phase 3: model statistics are global; star, start point, per-part scheduling arrays
     if (pt.ok && !setup_failed) {
       double mn = std::numeric_limits<double>::infinity(), sum = 0;
+      float mx = 0.f, pos = INF;
       unsigned long long cn = 0;
       bool bad = false;
-      for (auto& q : parts) { mn = std::min(mn, q.min_slow); sum += q.sum_slow; cn += q.cnt_slow; bad = bad || q.bad_slow; }
+      for (auto& q : parts) {
+        mn = std::min(mn, q.min_slow); mx = std::max(mx, q.max_slow); pos = std::min(pos, q.pos_slow);
+        sum += q.sum_slow; cn += q.cnt_slow; bad = bad || q.bad_slow;
+      }
       if (bad) { fail("the model holds negative or NaN slowness values"); bail("model"); }
       c->min_slowness = std::isfinite(mn) ? (float)mn : -1.f;
+      c->max_slowness = mx;
+      c->pos_slowness = pos;
       c->mean_slowness = cn ? sum / (double)cn : 0.0;
       c->allow_outside_sources = false;
       if (pt.ok && (!sweeptt_set_star(c, fs, starsize) || !sweeptt_set_sources(c, &start, 1))) bail("star / start point");
