@@ -204,7 +204,7 @@ int sweeptt_set_sources(sweeptt_ctx *ctx, const struct START *starts, int numsta
  *   fl(dmax * fl(vmax + vmax)) is finite,  every positive d >= 2^-125,  fl(dpos * vpos) >= 2^-125.
  * Outside it this call refuses, with a message naming the bound, and so do sweeptt_step,
  * sweeptt_reset, sweeptt_put_tt, sweeptt_count_violations, the ray and tomography calls,
- * sweeptt_rayset_freeze, sweeptt_solve and sweeptt_solve_slabs. */
+ * sweeptt_rayset_freeze, the event-location calls, sweeptt_solve and sweeptt_solve_slabs. */
 int sweeptt_run(sweeptt_ctx *ctx, sweeptt_stats *stats);
 
 /* Exactly `rounds` relaxation rounds without re-initialising (rounds >= 1); *changed
@@ -352,6 +352,56 @@ int sweeptt_rayset_project(sweeptt_rayset *set, const float *perturbation, float
  * floats, required; quantum_exp_out may be NULL.  stats: solve_ms = device time (zeroing, walk, rounding). */
 int sweeptt_rayset_backproject(sweeptt_rayset *set, const float *weights, float *grad_out, int *quantum_exp_out,
                                sweeptt_stats *stats);
+
+/* ---- event location: grid search over the stations' travel-time fields ----------------------- */
+
+/* The context's sources [source_begin, source_begin+source_count) are the STATIONS: a field started at a station s
+ * gives, by reciprocity, the time from every node n to s.  An event e has source_count picks obs[e][s] (float32, in the
+ * units of the fields); NaN means "no pick", every other value must be finite.  P_e = the picked stations in increasing
+ * s, k_e = |P_e|.  For every node n (caller axes; j(n) its FLOATBOX index), in IEEE float64, round to nearest, no
+ * fused multiply-add, in exactly this order:
+ *
+ *   if tt_s(n) == +INF for some s in P_e:  misfit = +INF, the node is EXCLUDED
+ *   else:
+ *     r_s = (double)obs[e][s] - (double)tt_s(n)                 for s in P_e
+ *     acc = +0;  for s in P_e ascending: acc = acc + r_s
+ *     t0  = acc / (double)k_e
+ *     m   = +0;  for s in P_e ascending: u = r_s - t0;  m = m + u*u
+ *     misfit = (float)m                                         (one rounding to float32, nearest even)
+ *
+ * This is least squares with the origin time t0 eliminated.  The two passes keep the misfit >= 0 (the argmin relies
+ * on it) and give exactly 0 when all residuals are equal.
+ *
+ * Best node of e: the node of smallest float32 misfit, ties to the smallest j(n); a node that is not excluded but
+ * whose misfit overflows float32 to +INF ranks before every excluded node.  Its origin time is that node's t0.
+ * Status (data, never an error return): SWEEPTT_LOC_OK; SWEEPTT_LOC_NO_PICKS when k_e = 0; SWEEPTT_LOC_UNREACHED when
+ * every node is excluded.  When the status is not OK: node (-1,-1,-1), misfit +INF, origin NaN; npicks = k_e always.
+ *
+ * Reciprocity is approximate.  The method uses the station fields as they are.  tt_s(n) can differ slightly from the
+ * time of a field started at n: the edge set is not symmetric, because the guarded pull of DESIGN §1 removes the edge
+ * {p - o_{L-1}, p} next to each field's own start p.  The contract is the formula above; it claims no exact symmetry.
+ *
+ * Both calls read only the fields (d_tt) and the geometry, no __constant__ table, so they work after any solve,
+ * sweeptt_step or sweeptt_put_tt.  They run on the context's stream and synchronise it.  They refuse, and leave the
+ * context as it was, when: the context is not ready (sweeptt_run's checks, the domain guard included); the source
+ * range is not within the context's sources; a required output or the picks are NULL; nev < 0; a pick is +INF or
+ * -INF; nx*ny*nz > 2^32 (the argmin key holds j(n) in 32 bits); or (sweeptt_locate_events only) source_count exceeds
+ * the stations whose times at 32 nodes (8 bytes each) fit the device's shared memory next to the kernel's 1 KB of
+ * node tables (904 on a B200).  stats (may be NULL): solve_ms = device time, kernel_launches, h2d_ms / h2d_bytes, d2h_ms / d2h_bytes. */
+enum { SWEEPTT_LOC_OK = 0, SWEEPTT_LOC_NO_PICKS = 1, SWEEPTT_LOC_UNREACHED = 2 };
+
+/* picks [nev*source_count], event-major.  best_out (caller-axis node) and status_out are required; misfit_out,
+ * origin_out and npicks_out (each [nev]) may be NULL.  The environment variable SWEEPTT_LOCATE_CHUNK (events per
+ * launch, default 4096) splits a large nev into several launches; the result does not depend on it. */
+int sweeptt_locate_events(sweeptt_ctx *ctx, int source_begin, int source_count, const float *picks, int nev,
+                          struct START *best_out, float *misfit_out, double *origin_out,
+                          int32_t *npicks_out, int32_t *status_out, sweeptt_stats *stats);
+
+/* The misfit of one event at every node: nx*ny*nz float32 values, FLOATBOX order, caller axes, +INF where excluded
+ * (with no pick at all, every node is +0: the formula has no term).  A best node from sweeptt_locate_events is the
+ * argmin of this box (ties to the lowest index). */
+int sweeptt_misfit_box(sweeptt_ctx *ctx, int source_begin, int source_count, const float *picks /*[source_count]*/,
+                       float *misfit_out, sweeptt_stats *stats);
 
 /* In-bounds pull evaluations of one full round of one source (analytic). */
 long long sweeptt_relaxations_per_round(sweeptt_ctx *ctx);

@@ -9,7 +9,11 @@ raises ``SweepError`` when the extension or a CUDA device is missing.
 from .api import (  # noqa: F401
     FS,
     Backprojection,
+    LOC_NO_PICKS,
+    LOC_OK,
+    LOC_UNREACHED,
     LinearizedUpdate,
+    Locations,
     MisfitGradient,
     RayProjection,
     RaySet,
@@ -23,6 +27,7 @@ from .api import (  # noqa: F401
     lib_path,
     load_library,
     linearized_update,
+    locate_events,
     make_star,
     solve,
     solve_slabs,

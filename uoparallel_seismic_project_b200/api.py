@@ -24,6 +24,8 @@ KERNEL_AUTO, KERNEL_SIMPLE, KERNEL_TILED = 0, 1, 2
 LOOP_AUTO, LOOP_BATCHED, LOOP_GRAPH = 0, 1, 2
 # status of a traced ray (SWEEPTT_RAY_*, include/sweeptt.h)
 RAY_OK, RAY_UNREACHED, RAY_NOT_FIXED_POINT, RAY_NO_PREDECESSOR, RAY_STALLED, RAY_TRUNCATED = range(6)
+# status of a located event (SWEEPTT_LOC_*, include/sweeptt.h)
+LOC_OK, LOC_NO_PICKS, LOC_UNREACHED = range(3)
 
 
 class SweepError(RuntimeError):
@@ -94,7 +96,8 @@ _EXPORTS = [
     "sweeptt_set_sources", "sweeptt_run", "sweeptt_step", "sweeptt_reset", "sweeptt_get_tt", "sweeptt_put_tt",
     "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject",
     "sweeptt_rayset_freeze", "sweeptt_rayset_destroy", "sweeptt_rayset_bytes", "sweeptt_rayset_table",
-    "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_debug_model_stats", "sweeptt_solve_slabs",
+    "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_locate_events",
+    "sweeptt_misfit_box", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_debug_model_stats", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
     "sweeptt_vbox_load", "sweeptt_vbox_store", "sweeptt_vbox_load_subset", "sweeptt_text_load",
     "sweeptt_star_load", "sweeptt_starts_load", "sweeptt_write_output_tt", "sweeptt_free",
@@ -157,6 +160,9 @@ def load_library() -> C.CDLL:
     lib.sweeptt_rayset_project.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_rayset_backproject.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int),
                                                C.POINTER(_Stats)]
+    lib.sweeptt_locate_events.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
+    lib.sweeptt_misfit_box.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_relaxations_per_round.argtypes = [C.c_void_p]
     lib.sweeptt_relaxations_per_round.restype = C.c_longlong
     lib.sweeptt_pool_bytes.argtypes = [C.c_void_p]
@@ -394,6 +400,21 @@ class LinearizedUpdate:
     residual_norm: float
 
 
+@dataclass
+class Locations:
+    """Events located by grid search (SweepContext.locate_events): for event e, node[e] (caller axes) minimises the
+    float64 least-squares misfit of its picks with the origin time eliminated, ties to the smallest FLOATBOX index;
+    misfit[e] is that minimum rounded to float32 and origin_time[e] the origin time there.  status[e] is LOC_OK,
+    LOC_NO_PICKS (npicks[e] = 0) or LOC_UNREACHED (every node has an infinite time at a picked station); then node is
+    (-1, -1, -1), misfit +inf and origin_time NaN."""
+    node: np.ndarray         # int32[E, 3]
+    misfit: np.ndarray       # float32[E]
+    origin_time: np.ndarray  # float64[E]
+    npicks: np.ndarray       # int32[E]
+    status: np.ndarray       # int32[E]
+    stats: SweepStats
+
+
 class SweepContext:
     """Device-resident context: padded slowness box + pool of travel-time boxes on one GPU."""
 
@@ -584,6 +605,41 @@ class SweepContext:
         rs = self._ray_calls(max_nodes, call)
         self._sets.add(rs)
         return rs
+
+    def locate_events(self, picks, sources=None) -> Locations:
+        """Locates every event of picks [E, S] (float32, NaN = no pick) by grid search over the fields of the sources
+        in `sources` (the stations; a range or a (begin, count) pair; default: all), on the device (include/sweeptt.h,
+        sweeptt_locate_events).  The misfit is computed in float64 exactly as the header states it."""
+        begin, count = self._source_range(sources, "locate_events")
+        p = np.ascontiguousarray(picks, dtype=np.float32)
+        if p.ndim != 2 or p.shape[1] != count:
+            raise SweepError(f"locate_events: picks of shape {p.shape}, expected (events, {count})")
+        nev = p.shape[0]
+        node = np.empty((nev, 3), np.int32)
+        misfit = np.empty(nev, np.float32)
+        origin = np.empty(nev, np.float64)
+        npicks = np.empty(nev, np.int32)
+        status = np.empty(nev, np.int32)
+        s = _Stats()
+        _check(self._lib.sweeptt_locate_events(self._h, begin, count, p.ctypes.data, nev, node.ctypes.data,
+                                               misfit.ctypes.data, origin.ctypes.data, npicks.ctypes.data,
+                                               status.ctypes.data, C.byref(s)), "sweeptt_locate_events")
+        return Locations(node, misfit, origin, npicks, status, SweepStats._from(s))
+
+    def misfit_box(self, picks, sources=None) -> np.ndarray:
+        """The misfit of one event (picks [S], NaN = no pick) at every node: float32[nx, ny, nz], +inf where a picked
+        station's time is infinite (include/sweeptt.h, sweeptt_misfit_box).  locate_events returns its argmin."""
+        begin, count = self._source_range(sources, "misfit_box")
+        p = np.ascontiguousarray(picks, dtype=np.float32)
+        if p.shape != (count,):
+            raise SweepError(f"misfit_box: picks of shape {p.shape}, expected ({count},)")
+        if self.dims is None:
+            raise SweepError("misfit_box: the context needs a model first")
+        out = np.empty(self.dims, np.float32)
+        s = _Stats()
+        _check(self._lib.sweeptt_misfit_box(self._h, begin, count, p.ctypes.data, out.ctypes.data, C.byref(s)),
+               "sweeptt_misfit_box")
+        return out
 
     @property
     def relaxations_per_round(self) -> int:
@@ -790,6 +846,19 @@ def linearized_update(slowness, star, starts, receivers, observed, *, damp: floa
     misfit = 0.5 * float(np.sum(residual[use].astype(np.float64) ** 2))
     return LinearizedUpdate(out[0].astype(np.float32).reshape(np.shape(slowness)), residual, status, misfit,
                             int(out[1]), int(out[2]), float(out[3]))
+
+
+def locate_events(slowness, star, stations, picks, *, delta: float = 10.0, device: int | None = None,
+                  kernel: int | None = None) -> Locations:
+    """One-shot event location: solve one field per station (stations (S, 3) as start points; by reciprocity the
+    field of station s holds the time from every node to s), then locate every event of picks [E, S]
+    (SweepContext.locate_events).  Only the locations leave the device, never the fields."""
+    with SweepContext(device=device, kernel=kernel) as ctx:
+        ctx.set_model(slowness)
+        ctx.set_star(star, delta)
+        ctx.set_sources(stations)
+        ctx.run()
+        return ctx.locate_events(picks)
 
 
 # ---- file formats -------------------------------------------------------------------------

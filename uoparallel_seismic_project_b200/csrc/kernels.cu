@@ -33,6 +33,8 @@
 //                     predecessor step, then a walk of the recorded path; exact int64 accumulation for G^T*w).
 //   rayset_record / rayset_compact / rayset_project / rayset_backproject  ray sets: the same rays traced once and
 //                     kept on the device as pull-table entries, then the same walks of the stored records.
+//   locate / locate_finish / misfit_box  event location: the float64 origin-free least-squares misfit of every
+//                     event at every node from the stations' fields, its argmin and the misfit box of one event.
 //   fill/pad/unpad/init_sources/min_slowness  the device float-box pool's utilities
 //                     (boxsetall/boxput, include/floatbox.h:176-199).
 // One grid over several devices (solver.cu, sweeptt_solve_slabs) runs relax_tiled unchanged on a travel-time box
@@ -1609,6 +1611,191 @@ __global__ void grad_finish_kernel(const long long* __restrict__ acc, float* __r
 }
 
 // ---------------------------------------------------------------------------------------
+// event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box; DESIGN §3.10)
+// ---------------------------------------------------------------------------------------
+constexpr int LOC_THREADS = 512;
+constexpr unsigned LOC_EXCLUDED = 0x7f800001u;  // key bits of an excluded node: after every float32 misfit, +INF too
+
+// RN(a / k) for a finite double a and an integer 1 <= k < 2^26, with DMUL / DADD only: ptxas expands div.rn.f64 into
+// a DFMA sequence, and these kernels keep no fused multiply-add.  q = RN(a * rk), rk = RN(1/k), is within two ulps of
+// a/k.  The remainder a - q*k is exact: q splits (Veltkamp, 2^27 + 1) into a 26-bit qh and a 27-bit ql, so qh*k and
+// ql*k are exact, a - qh*k is exact by Sterbenz's lemma, and the last difference is a multiple of ulp(q) below
+// 2^53 ulp(q).  Its sign tells on which side of q the quotient lies; q steps to that neighbour while the neighbour is
+// nearer.  a/k is never halfway between two doubles (an odd multiple of a 54-bit odd significand needs more than 53
+// bits), so the nearer of two neighbours is RN(a/k).
+__device__ __forceinline__ double loc_remainder(double a, double q, double k) {
+  const double c = __dmul_rn(134217729.0, q);
+  const double qh = __dsub_rn(c, __dsub_rn(c, q));
+  const double ql = __dsub_rn(q, qh);
+  return __dsub_rn(__dsub_rn(a, __dmul_rn(qh, k)), __dmul_rn(ql, k));
+}
+__device__ __forceinline__ double loc_div(double a, int k, double rk) {
+  if (k == 0) return __longlong_as_double(0x7ff8000000000000ll);  // 0 / 0
+  const double kd = (double)k;
+  double q = __dmul_rn(a, rk);
+  double r = loc_remainder(a, q, kd);
+  for (int it = 0; it < 4 && r != 0.0; ++it) {
+    // the neighbour of q towards a/k: a larger magnitude when r has q's sign
+    const long long step = ((r > 0.0) == (q > 0.0)) ? 1 : -1;
+    const double qn = __longlong_as_double(__double_as_longlong(q) + step);
+    const double rn = loc_remainder(a, qn, kd);
+    if (!(fabs(rn) < fabs(r))) break;
+    q = qn;
+    r = rn;
+  }
+  return q;
+}
+
+// The per-node formula of include/sweeptt.h, at NB nodes of one event: the ONE implementation, shared by locate_kernel,
+// misfit_box_kernel and locate_finish_kernel.  tt(s, q) is station s's travel time at node q as a double; ps / po are
+// the event's k picks, ascending.  bits[q] = float bits of the misfit, or LOC_EXCLUDED; t0[q] = the origin time.
+template <int NB, class TT>
+__device__ __forceinline__ void event_misfit(const int* __restrict__ ps, const double* __restrict__ po, int k, double rk,
+                                             const TT& tt, unsigned (&bits)[NB], double (&t0)[NB]) {
+  double acc[NB], m[NB];
+#pragma unroll
+  for (int q = 0; q < NB; ++q) acc[q] = 0.0, m[q] = 0.0;
+#pragma unroll 4
+  for (int j = 0; j < k; ++j) {
+    const int s = ps[j];
+    const double o = po[j];
+#pragma unroll
+    for (int q = 0; q < NB; ++q) acc[q] = __dadd_rn(acc[q], __dsub_rn(o, tt(s, q)));
+  }
+#pragma unroll
+  for (int q = 0; q < NB; ++q) t0[q] = loc_div(acc[q], k, rk);
+#pragma unroll 4
+  for (int j = 0; j < k; ++j) {
+    const int s = ps[j];
+    const double o = po[j];
+#pragma unroll
+    for (int q = 0; q < NB; ++q) {
+      const double u = __dsub_rn(__dsub_rn(o, tt(s, q)), t0[q]);
+      m[q] = __dadd_rn(m[q], __dmul_rn(u, u));
+    }
+  }
+#pragma unroll
+  for (int q = 0; q < NB; ++q) {
+    // picks are finite, so a +INF time makes acc -INF or NaN; a finite acc rules every +INF out
+    bool excluded = false;
+    if (!isfinite(acc[q]))
+      for (int j = 0; j < k; ++j) excluded |= tt(ps[j], q) == CUDART_INF;
+    bits[q] = excluded ? LOC_EXCLUDED : __float_as_uint(__double2float_rn(m[q]));
+  }
+}
+
+struct LocSmemTT {  // the CTA's staged times: station s, node q of this lane at base[s * B + 32 * q]
+  const double* base;
+  int B;
+  __device__ __forceinline__ double operator()(int s, int q) const { return base[s * B + 32 * q]; }
+};
+struct LocBoxTT {   // the padded boxes in global memory, at one node
+  const float* tt;
+  long long vol, p;
+  __device__ __forceinline__ double operator()(int s, int) const { return (double)__ldg(tt + s * vol + p); }
+};
+
+// Caller FLOATBOX index and padded index of kernel-order node i = (x*ny + y)*nz + z.
+__device__ __forceinline__ void loc_node(const BoxGeom& g, long long i, long long* p, long long* d) {
+  const int z = (int)(i % g.nz);
+  const long long r = i / g.nz;
+  const int y = (int)(r % g.ny), x = (int)(r / g.ny);
+  *p = ((long long)(x + AX) * g.py + (y + AY)) * g.pz + (z + AZ);
+  *d = x * g.dstride[0] + y * g.dstride[1] + z * g.dstride[2];
+}
+
+// A CTA owns B = 32*NB consecutive nodes in kernel order (a run along kernel z: coalesced reads), stages the times of
+// every station there once (doubles, [nsta][B]), then its warps take the launch's events in turn: lane l evaluates
+// nodes l, l+32, ... of the run for the warp's event, whose picks are warp-uniform loads.  The warp's smallest key goes
+// to the event with one 64-bit atomicMin (integer min: the result does not depend on the schedule).
+template <int NB>
+__global__ void __launch_bounds__(LOC_THREADS, 1) locate_kernel(const LocateArgs a) {
+  constexpr int B = 32 * NB;
+  extern __shared__ double s_tt[];
+  __shared__ long long s_p[B];
+  __shared__ unsigned s_j[B];
+  const long long D = (long long)a.g.nx * a.g.ny * a.g.nz;
+  const long long n0 = (long long)blockIdx.x * B;
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    long long p = -1, d = 0;
+    if (n0 + b < D) loc_node(a.g, n0 + b, &p, &d);
+    s_p[b] = p;
+    s_j[b] = (unsigned)d;
+  }
+  __syncthreads();
+  for (int idx = threadIdx.x; idx < a.nsta * B; idx += blockDim.x) {
+    const int s = idx / B, b = idx % B;
+    const long long p = s_p[b];
+    s_tt[idx] = p >= 0 ? (double)__ldg(a.tt + s * a.g.vol + p) : CUDART_INF;
+  }
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  bool live[NB];
+  unsigned jn[NB];
+#pragma unroll
+  for (int q = 0; q < NB; ++q) live[q] = s_p[32 * q + lane] >= 0, jn[q] = s_j[32 * q + lane];
+  const LocSmemTT tt{s_tt + lane, B};
+  for (int e = a.e_begin + warp; e < a.e_begin + a.e_count; e += LOC_THREADS / 32) {
+    const int off = a.pick_off[e], k = a.pick_off[e + 1] - off;
+    if (k == 0) continue;
+    unsigned bits[NB];
+    double t0[NB];
+    event_misfit<NB>(a.pick_sta + off, a.pick_obs + off, k, a.pick_rk[e], tt, bits, t0);
+    unsigned long long best = ~0ull;
+#pragma unroll
+    for (int q = 0; q < NB; ++q)
+      if (live[q]) best = min(best, ((unsigned long long)bits[q] << 32) | jn[q]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
+    if (lane == 0 && best != ~0ull) atomicMin(a.key + e, best);
+  }
+}
+
+__global__ void locate_finish_kernel(const LocateArgs a, int nev) {
+  const BoxGeom& g = a.g;
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < nev; e += gridDim.x * blockDim.x) {
+    const int off = a.pick_off[e], k = a.pick_off[e + 1] - off;
+    const unsigned long long key = a.key[e];
+    a.npicks[e] = k;
+    if (k == 0 || (unsigned)(key >> 32) == LOC_EXCLUDED || key == ~0ull) {
+      a.node[3 * e] = a.node[3 * e + 1] = a.node[3 * e + 2] = -1;
+      a.misfit[e] = CUDART_INF_F;
+      a.origin[e] = __longlong_as_double(0x7ff8000000000000ll);
+      a.status[e] = k == 0 ? SWEEPTT_LOC_NO_PICKS : SWEEPTT_LOC_UNREACHED;
+      continue;
+    }
+    // caller coordinates of j = (c0*n1 + c1)*n2 + c2, then kernel axes (kernel axis q = caller axis perm[q])
+    int n[3], c[3];
+    n[g.perm[0]] = g.nx; n[g.perm[1]] = g.ny; n[g.perm[2]] = g.nz;
+    const unsigned long long j = key & 0xffffffffull;
+    c[2] = (int)(j % n[2]);
+    c[1] = (int)(j / n[2] % n[1]);
+    c[0] = (int)(j / n[2] / n[1]);
+    const long long p = ((long long)(c[g.perm[0]] + AX) * g.py + (c[g.perm[1]] + AY)) * g.pz + (c[g.perm[2]] + AZ);
+    unsigned bits[1];
+    double t0[1];
+    event_misfit<1>(a.pick_sta + off, a.pick_obs + off, k, a.pick_rk[e], LocBoxTT{a.tt, g.vol, p}, bits, t0);
+    a.node[3 * e] = c[0]; a.node[3 * e + 1] = c[1]; a.node[3 * e + 2] = c[2];
+    a.misfit[e] = __uint_as_float(bits[0]);
+    a.origin[e] = t0[0];
+    a.status[e] = SWEEPTT_LOC_OK;
+  }
+}
+
+__global__ void __launch_bounds__(256) misfit_box_kernel(const LocateArgs a, float* __restrict__ dense) {
+  const long long D = (long long)a.g.nx * a.g.ny * a.g.nz;
+  const int k = a.pick_off[1] - a.pick_off[0];
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < D; i += (long long)gridDim.x * blockDim.x) {
+    long long p, d;
+    loc_node(a.g, i, &p, &d);
+    unsigned bits[1];
+    double t0[1];
+    event_misfit<1>(a.pick_sta, a.pick_obs, k, a.pick_rk[0], LocBoxTT{a.tt, a.g.vol, p}, bits, t0);
+    dense[d] = bits[0] == LOC_EXCLUDED ? CUDART_INF_F : __uint_as_float(bits[0]);
+  }
+}
+
+// ---------------------------------------------------------------------------------------
 // float-box utilities
 // ---------------------------------------------------------------------------------------
 __global__ void fill_kernel(float4* p, long long n4, float value) {
@@ -2073,6 +2260,51 @@ cudaError_t launch_rayset_walk(bool backproject, const RaySetArgs& s, int device
 
 cudaError_t launch_grad_finish(const long long* acc, float* dense, BoxGeom g, int E, cudaStream_t stream) {
   grad_finish_kernel<<<1184, 256, 0, stream>>>(acc, dense, g, E);
+  return cudaGetLastError();
+}
+
+template <int NB>
+static size_t locate_smem(int nsta) { return (size_t)nsta * 32 * NB * sizeof(double); }
+
+template <int NB>
+static bool locate_fits(int nsta, int optin) {
+  cudaFuncAttributes fa{};  // the static node tables take their share besides the staged times
+  return cudaFuncGetAttributes(&fa, locate_kernel<NB>) == cudaSuccess &&
+         locate_smem<NB>(nsta) + fa.sharedSizeBytes <= (size_t)optin;
+}
+
+int locate_nodes_per_thread(int nsta, int device) {
+  int optin = 0;
+  if (cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device) != cudaSuccess) return 0;
+  return locate_fits<4>(nsta, optin) ? 4 : locate_fits<2>(nsta, optin) ? 2 : locate_fits<1>(nsta, optin) ? 1 : 0;
+}
+
+template <int NB>
+static cudaError_t launch_locate_nb(const LocateArgs& a, cudaStream_t stream) {
+  const size_t smem = locate_smem<NB>(a.nsta);
+  cudaError_t e = cudaFuncSetAttribute(locate_kernel<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  const long long D = (long long)a.g.nx * a.g.ny * a.g.nz;
+  locate_kernel<NB><<<(unsigned)((D + 32 * NB - 1) / (32 * NB)), LOC_THREADS, smem, stream>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_locate(const LocateArgs& a, int nodes_per_thread, cudaStream_t stream) {
+  switch (nodes_per_thread) {
+    case 4: return launch_locate_nb<4>(a, stream);
+    case 2: return launch_locate_nb<2>(a, stream);
+    case 1: return launch_locate_nb<1>(a, stream);
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+cudaError_t launch_locate_finish(const LocateArgs& a, int nev, cudaStream_t stream) {
+  locate_finish_kernel<<<(nev + 127) / 128, 128, 0, stream>>>(a, nev);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_misfit_box(const LocateArgs& a, float* dense, cudaStream_t stream) {
+  misfit_box_kernel<<<1184, 256, 0, stream>>>(a, dense);
   return cudaGetLastError();
 }
 

@@ -167,6 +167,33 @@ cudaError_t launch_rayset_walk(bool backproject, const RaySetArgs& s, int device
 // grad (dense, caller axes) := acc * 2^E rounded once to float32.
 cudaError_t launch_grad_finish(const long long* acc, float* dense, BoxGeom g, int E, cudaStream_t stream);
 
+// Event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box).  Event e's picks are entries
+// pick_off[e] .. pick_off[e+1] of pick_sta / pick_obs, in increasing station order (NaN picks left out).
+struct LocateArgs {
+  BoxGeom g;
+  const float* tt;             // padded travel-time box of the call's first station; station s at tt + s * g.vol
+  int nsta;                    // stations (source_count)
+  const int* pick_off;         // [nev + 1]
+  const int* pick_sta;         // station of every pick, relative to the first
+  const double* pick_obs;      // the pick as a double (exact)
+  const double* pick_rk;       // [nev] RN(1.0 / k_e): first guess of the division t0 = acc / k_e (0 when k_e = 0)
+  unsigned long long* key;     // [nev] argmin keys (misfit bits << 32 | caller FLOATBOX index), set to ~0 first
+  int e_begin, e_count;        // events of one location launch
+  int* node;                   // finisher outputs [nev]: caller-axis node (3 ints), misfit, origin time, k_e, status
+  float* misfit;
+  double* origin;
+  int* npicks;
+  int* status;
+};
+// Nodes per thread of the location kernel (4, 2 or 1: a CTA stages the times of nsta stations at 32 * that many
+// nodes in shared memory), or 0 when not even 32 nodes fit.
+int locate_nodes_per_thread(int nsta, int device);
+cudaError_t launch_locate(const LocateArgs& a, int nodes_per_thread, cudaStream_t stream);
+// Decodes every key: best node, and its misfit and t0 recomputed with the location kernel's formula.
+cudaError_t launch_locate_finish(const LocateArgs& a, int nev, cudaStream_t stream);
+// Event 0's misfit at every node into the dense caller-axis box.
+cudaError_t launch_misfit_box(const LocateArgs& a, float* dense, cudaStream_t stream);
+
 // Box utilities (device float-box pool).
 cudaError_t launch_fill(float* p, long long n, float value, cudaStream_t stream);
 cudaError_t launch_pad_box(const float* dense, float* padded, BoxGeom g, cudaStream_t stream);

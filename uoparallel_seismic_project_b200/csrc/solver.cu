@@ -180,6 +180,9 @@ struct sweeptt_ctx {
   size_t path_cap = 0;
   float* d_stage = nullptr;  // dense staging box for pad/unpad
   size_t stage_floats = 0;
+  // event location (sweeptt_locate_events / sweeptt_misfit_box): grow-only buffer of the picks, keys and results
+  unsigned char* d_loc = nullptr;
+  size_t loc_cap = 0;
   size_t pool_bytes = 0;
 
   std::vector<FS> fs;
@@ -382,6 +385,7 @@ extern "C" void sweeptt_destroy(sweeptt_ctx* c) {
   cudaFree(c->d_stage); cudaFree(c->d_star);
   cudaFree(c->d_ray_pull); cudaFree(c->d_rec); cudaFree(c->d_ray_out);
   cudaFree(c->d_pert); cudaFree(c->d_acc); cudaFree(c->d_path);
+  cudaFree(c->d_loc);
   if (c->h_state) cudaFreeHost(c->h_state);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
@@ -1608,6 +1612,14 @@ static int build_ray_pulls(sweeptt_ctx* c) {
   return 1;
 }
 
+// The source range of a call that reads the context's fields (ray, tomography and location calls).
+static int check_source_range(const sweeptt_ctx* c, const char* who, int source_begin, int source_count) {
+  if (source_count < 1 || source_begin < 0 || source_begin > c->nsrc - source_count)
+    return fail("%s: sources [%d, %d) are not within the context's %d sources", who, source_begin,
+                source_begin + source_count, c->nsrc);
+  return 1;
+}
+
 // Argument checks shared by the ray calls (sweeptt_trace_rays, sweeptt_ray_project, sweeptt_ray_backproject), then
 // the receivers range-checked and permuted to kernel axes into c->rec_xyz.
 static int check_ray_call(sweeptt_ctx* c, ConstLease* lease, const char* who, int source_begin, int source_count,
@@ -1615,9 +1627,7 @@ static int check_ray_call(sweeptt_ctx* c, ConstLease* lease, const char* who, in
   if (!ready(c, lease)) return 0;
   if (stats) std::memset(stats, 0, sizeof *stats);
   if (!receivers || nrec < 1) return fail("%s: need at least one receiver", who);
-  if (source_count < 1 || source_begin < 0 || source_begin > c->nsrc - source_count)
-    return fail("%s: sources [%d, %d) are not within the context's %d sources", who, source_begin,
-                source_begin + source_count, c->nsrc);
+  if (!check_source_range(c, who, source_begin, source_count)) return 0;
   if (max_nodes < 1) return fail("%s: max_nodes must be >= 1 (got %d)", who, max_nodes);
   const BoxGeom& g = c->g;
   int on[3];  // caller-order dims
@@ -2184,6 +2194,162 @@ extern "C" int sweeptt_rayset_backproject(sweeptt_rayset* r, const float* weight
     stats->d2h_bytes = (long long)(dense * 4);
   }
   if (quantum_exp_out) *quantum_exp_out = E;
+  return 1;
+}
+
+// ---------------------------------------------------------------------------------------
+// event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box)
+// ---------------------------------------------------------------------------------------
+
+// Checks shared by both location calls; then the picks of nev events (NaN left out) go to the device as a CSR with
+// RN(1/k) per event, and *a describes them, the fields of the call's stations and the result slots.  Every refusal
+// comes before the first allocation.  nodes_per_thread (may be NULL): the location kernel's shape for these stations.
+static int locate_prepare(sweeptt_ctx* c, ConstLease* lease, const char* who, int source_begin, int source_count,
+                          const float* picks, int nev, LocateArgs* a, int* nodes_per_thread, sweeptt_stats* stats) {
+  if (!ready(c, lease)) return 0;
+  if (stats) std::memset(stats, 0, sizeof *stats);
+  if (!check_source_range(c, who, source_begin, source_count)) return 0;
+  if (nodes_per_thread && (*nodes_per_thread = locate_nodes_per_thread(source_count, c->device)) == 0)
+    return fail("%s: %d stations do not fit the location kernel's shared memory (8 bytes per station and node, 32 nodes)",
+                who, source_count);
+  if (nev < 0) return fail("%s: nev = %d is negative", who, nev);
+  if (nev > 0 && !picks) return fail("%s: null picks", who);
+  const BoxGeom& g = c->g;
+  if ((unsigned long long)g.nx * g.ny * g.nz > (1ull << 32))
+    return fail("%s: %d x %d x %d nodes exceed 2^32, the argmin key holds a node index in 32 bits", who, g.nx, g.ny, g.nz);
+  std::vector<int> off(1, 0), sta;
+  std::vector<double> obs, rk;
+  off.reserve((size_t)nev + 1);
+  rk.reserve(nev);
+  for (int e = 0; e < nev; ++e) {
+    for (int s = 0; s < source_count; ++s) {
+      const float v = picks[(size_t)e * source_count + s];
+      if (std::isnan(v)) continue;
+      if (std::isinf(v)) return fail("%s: pick of event %d at station %d is %cINF (a pick is finite, or NaN for none)",
+                                     who, e, s, v > 0 ? '+' : '-');
+      sta.push_back(s);
+      obs.push_back((double)v);
+    }
+    if (sta.size() > (size_t)INT32_MAX) return fail("%s: more than 2^31 picks in one call", who);
+    const int k = (int)sta.size() - off.back();
+    off.push_back((int)sta.size());
+    rk.push_back(k ? 1.0 / k : 0.0);
+  }
+  const size_t np = sta.size(), n = (size_t)nev;
+  auto up16 = [](size_t b) { return (b + 15) / 16 * 16; };
+  const size_t part[10] = {up16(4 * (n + 1)), up16(4 * np), up16(8 * np), up16(8 * n), up16(8 * n),
+                           up16(12 * n),      up16(4 * n),  up16(8 * n),  up16(4 * n), up16(4 * n)};
+  size_t at[11] = {0};
+  for (int i = 0; i < 10; ++i) at[i + 1] = at[i] + part[i];
+  if (!ensure_dev(c, &c->d_loc, &c->loc_cap, at[10])) return 0;
+  unsigned char* b = c->d_loc;
+  *a = LocateArgs{};
+  a->g = g;
+  a->tt = c->d_tt + (size_t)source_begin * g.vol;
+  a->nsta = source_count;
+  a->pick_off = reinterpret_cast<const int*>(b + at[0]);
+  a->pick_sta = reinterpret_cast<const int*>(b + at[1]);
+  a->pick_obs = reinterpret_cast<const double*>(b + at[2]);
+  a->pick_rk = reinterpret_cast<const double*>(b + at[3]);
+  a->key = reinterpret_cast<unsigned long long*>(b + at[4]);
+  a->node = reinterpret_cast<int*>(b + at[5]);
+  a->misfit = reinterpret_cast<float*>(b + at[6]);
+  a->origin = reinterpret_cast<double*>(b + at[7]);
+  a->npicks = reinterpret_cast<int*>(b + at[8]);
+  a->status = reinterpret_cast<int*>(b + at[9]);
+  const auto t0 = std::chrono::steady_clock::now();
+  CK(cudaMemcpyAsync(b + at[0], off.data(), 4 * (n + 1), cudaMemcpyHostToDevice, c->stream));
+  if (np) {
+    CK(cudaMemcpyAsync(b + at[1], sta.data(), 4 * np, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(b + at[2], obs.data(), 8 * np, cudaMemcpyHostToDevice, c->stream));
+  }
+  if (n) CK(cudaMemcpyAsync(b + at[3], rk.data(), 8 * n, cudaMemcpyHostToDevice, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  if (stats) {
+    stats->struct_size = (int)sizeof *stats;
+    stats->devices_used = 1;
+    stats->h2d_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    stats->h2d_bytes = (long long)(4 * (n + 1) + 12 * np + 8 * n);
+  }
+  return 1;
+}
+
+// Events per location launch (SWEEPTT_LOCATE_CHUNK): bounds the run time of one launch; the result does not depend on it.
+static int locate_chunk() {
+  int chunk = 4096;
+  if (const char* e = getenv("SWEEPTT_LOCATE_CHUNK")) chunk = std::max(1, atoi(e));
+  return chunk;
+}
+
+extern "C" int sweeptt_locate_events(sweeptt_ctx* c, int source_begin, int source_count, const float* picks, int nev,
+                                     struct START* best_out, float* misfit_out, double* origin_out,
+                                     int32_t* npicks_out, int32_t* status_out, sweeptt_stats* stats) {
+  static const char* who = "sweeptt_locate_events";
+  if (!best_out || !status_out) return fail("%s: best_out and status_out are required", who);
+  ConstLease lease;
+  LocateArgs a;
+  int nb = 0;
+  if (!locate_prepare(c, &lease, who, source_begin, source_count, picks, nev, &a, &nb, stats)) return 0;
+  if (nev == 0) return 1;
+  const int chunk = locate_chunk();
+  long long launches = 0;
+  CK(cudaEventRecord(c->ev0, c->stream));
+  CK(cudaMemsetAsync(a.key, 0xff, 8 * (size_t)nev, c->stream));
+  for (int e0 = 0; e0 < nev; e0 += chunk) {
+    a.e_begin = e0;
+    a.e_count = std::min(chunk, nev - e0);
+    CK(launch_locate(a, nb, c->stream));
+    ++launches;
+  }
+  CK(launch_locate_finish(a, nev, c->stream));
+  CK(cudaEventRecord(c->ev1, c->stream));
+  CK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+
+  const auto t_copy = std::chrono::steady_clock::now();
+  const size_t n = (size_t)nev;
+  long long bytes = 16 * (long long)n;
+  static_assert(sizeof(START) == 3 * sizeof(int), "START is three ints");
+  CK(cudaMemcpyAsync(best_out, a.node, 12 * n, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(status_out, a.status, 4 * n, cudaMemcpyDeviceToHost, c->stream));
+  if (misfit_out) { CK(cudaMemcpyAsync(misfit_out, a.misfit, 4 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * n; }
+  if (origin_out) { CK(cudaMemcpyAsync(origin_out, a.origin, 8 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 8 * n; }
+  if (npicks_out) { CK(cudaMemcpyAsync(npicks_out, a.npicks, 4 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * n; }
+  CK(cudaStreamSynchronize(c->stream));
+  if (stats) {
+    stats->solve_ms = ms;
+    stats->kernel_launches = launches + 1;
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes = bytes;
+  }
+  return 1;
+}
+
+extern "C" int sweeptt_misfit_box(sweeptt_ctx* c, int source_begin, int source_count, const float* picks,
+                                  float* misfit_out, sweeptt_stats* stats) {
+  static const char* who = "sweeptt_misfit_box";
+  if (!picks || !misfit_out) return fail("%s: picks and misfit_out are required", who);
+  ConstLease lease;
+  LocateArgs a;
+  if (!locate_prepare(c, &lease, who, source_begin, source_count, picks, 1, &a, nullptr, stats)) return 0;
+  const size_t dense = (size_t)c->g.nx * c->g.ny * c->g.nz;
+  if (!ensure_stage(c, dense)) return 0;
+  CK(cudaEventRecord(c->ev0, c->stream));
+  CK(launch_misfit_box(a, c->d_stage, c->stream));
+  CK(cudaEventRecord(c->ev1, c->stream));
+  CK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+  const auto t_copy = std::chrono::steady_clock::now();
+  CK(cudaMemcpyAsync(misfit_out, c->d_stage, dense * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  if (stats) {
+    stats->solve_ms = ms;
+    stats->kernel_launches = 1;
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes = (long long)dense * 4;
+  }
   return 1;
 }
 
