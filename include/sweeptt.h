@@ -214,7 +214,11 @@ int sweeptt_reset(sweeptt_ctx *ctx); /* INF / 0-at-start re-initialisation only 
 
 /* D2H of one converged box, un-padded into FLOATBOX order (cuda/...cu:393-397). */
 int sweeptt_get_tt(sweeptt_ctx *ctx, int source, float *tt_out);
-/* H2D of a caller-provided state for source `source` (tests: arbitrary valid upper bounds). */
+/* H2D of a caller-provided state for source `source` (tests: arbitrary valid upper bounds).  Every value must be
+ * +0, positive or +INF: a box holding a NaN, a negative value, -INF or -0.0 is refused with a message naming the
+ * first such FLOATBOX index, and the context is left as it was (the scheduling orders times by their bits as
+ * unsigned integers, where a set sign bit ranks after +INF; a NaN time would make a location misfit NaN).  A field
+ * read back with sweeptt_get_tt never holds -0.0, so it can always be put back. */
 int sweeptt_put_tt(sweeptt_ctx *ctx, int source, const float *tt_in);
 
 /* Device-side fixed-point verifier: counts (node, pull offset) pairs that would still
@@ -276,7 +280,8 @@ int sweeptt_trace_rays(sweeptt_ctx *ctx, int source_begin, int source_count,
  * start point towards the receiver: acc = +0; for each edge from the start end, acc = fl(fl(hd*fl(d_n + d_m)) + acc).
  * A ray of one node gives +0, a ray that is not OK a quiet NaN.  So the projection of the slowness itself equals
  * tt[receiver] bit for bit for every OK ray of a converged field.  Perturbation values are not validated (they
- * propagate per IEEE).  perturbation: nx*ny*nz floats, FLOATBOX order, caller axes.  Outputs may be NULL. */
+ * propagate per IEEE: -0 sums to +0, d_n + d_m may overflow to INF, INF - INF is NaN).  A NaN result is a quiet NaN
+ * with no promised payload or sign.  perturbation: nx*ny*nz floats, FLOATBOX order, caller axes.  Outputs may be NULL. */
 int sweeptt_ray_project(sweeptt_ctx *ctx, int source_begin, int source_count,
                         const struct START *receivers, int nrec, int max_nodes,
                         const float *perturbation,          /* nx*ny*nz, FLOATBOX, caller axes */
@@ -288,7 +293,8 @@ int sweeptt_ray_project(sweeptt_ctx *ctx, int source_begin, int source_count,
  * coverage).  Exact and deterministic: with hd_max the largest hd of the used star entries, W = max|w_q| and
  * N = source_count*nrec, E is the smallest integer with 2*hd_max*W*N <= 2^(E+62); every contribution
  * c = rint_even(w_q*hd_e*2^-E) (an int64; w*hd is exact in double) is added to both ends of its edge in int64, and
- * grad[j] = S_j*2^E is rounded once to float32 (nearest, ties to even, subnormals included).  A ray visits a node
+ * grad[j] = S_j*2^E is rounded once to float32 (nearest, ties to even, subnormals included; +-INF from FLT_MAX plus
+ * half an ulp on; S_j = 0, contributions that cancel exactly included, gives +0, never -0).  A ray visits a node
  * at most once (travel time strictly decreases along it), so no sum overflows.  *quantum_exp_out = E.  W = 0 (or a
  * star whose hd are all 0) gives all +0 and E = 0.  weights: [source_count*nrec], finite, required; grad_out:
  * nx*ny*nz floats, FLOATBOX order, caller axes, required; quantum_exp_out and status_out may be NULL. */
@@ -386,8 +392,9 @@ int sweeptt_rayset_backproject(sweeptt_rayset *set, const float *weights, float 
  * context as it was, when: the context is not ready (sweeptt_run's checks, the domain guard included); the source
  * range is not within the context's sources; a required output or the picks are NULL; nev < 0; a pick is +INF or
  * -INF; nx*ny*nz > 2^32 (the argmin key holds j(n) in 32 bits); or (sweeptt_locate_events only) source_count exceeds
- * the stations whose times at 32 nodes (8 bytes each) fit the device's shared memory next to the kernel's 1 KB of
- * node tables (904 on a B200).  stats (may be NULL): solve_ms = device time, kernel_launches, h2d_ms / h2d_bytes, d2h_ms / d2h_bytes. */
+ * the stations whose times at 32 nodes (8 bytes each) fit the device's opt-in shared memory next to the kernel's
+ * static shared memory as cudaFuncGetAttributes reports it: 904 stations on a B200.  The times themselves are not checked here: fields from
+ * sweeptt_run / sweeptt_step are +0, positive or +INF, and sweeptt_put_tt refuses anything else.  stats (may be NULL): solve_ms = device time, kernel_launches, h2d_ms / h2d_bytes, d2h_ms / d2h_bytes. */
 enum { SWEEPTT_LOC_OK = 0, SWEEPTT_LOC_NO_PICKS = 1, SWEEPTT_LOC_UNREACHED = 2 };
 
 /* picks [nev*source_count], event-major.  best_out (caller-axis node) and status_out are required; misfit_out,

@@ -46,13 +46,14 @@ def _edges(nodes, length):
         yield live, nodes[rows, k], nodes[rows, np.minimum(k + 1, L - 1)]
 
 
-def oracle_project(d, nodes, length, status):
+def oracle_project(d, nodes, length, status, delta=10.0):
     """acc = +0; for each edge (n, m) from the start end: acc = fl(fl(hd * fl(d_n + d_m)) + acc).  NaN unless OK."""
     d = np.asarray(d, np.float32)
     acc = np.zeros(len(length), np.float32)
     for live, n, m in _edges(nodes, length):
-        term = half_distance(m - n) * (d[tuple(n.T)] + d[tuple(m.T)])
-        acc = np.where(live, term + acc, acc).astype(np.float32)
+        with np.errstate(over="ignore", invalid="ignore"):
+            term = half_distance(m - n, delta) * (d[tuple(n.T)] + d[tuple(m.T)])
+            acc = np.where(live, term + acc, acc).astype(np.float32)
     return np.where(status == OK, acc, np.float32(np.nan)).astype(np.float32)
 
 
@@ -106,7 +107,7 @@ def round_once(total, e):
     return -mag if total < 0 else mag
 
 
-def oracle_backproject(dims, rays, weights, hd_max):
+def oracle_backproject(dims, rays, weights, hd_max, delta=10.0):
     """rays: list over sources of (nodes, length, status); weights [S, R].  Returns (grad float32[dims], E)."""
     w = np.asarray(weights, np.float32)
     e = quantum_exp(hd_max, float(np.abs(w).max(initial=0)), w.size)
@@ -114,7 +115,7 @@ def oracle_backproject(dims, rays, weights, hd_max):
     for (nodes, length, status), ws in zip(rays, w):
         use = (status == OK) & (ws != 0)
         for live, n, m in _edges(nodes[use], length[use]):
-            c = _quanta(ws[use][live], half_distance(m[live] - n[live]), e)
+            c = _quanta(ws[use][live], half_distance(m[live] - n[live], delta), e)
             np.add.at(acc, np.ravel_multi_index(tuple(n[live].T), dims), c)
             np.add.at(acc, np.ravel_multi_index(tuple(m[live].T), dims), c)
     grad = np.zeros(acc.shape, np.float32)

@@ -1528,6 +1528,15 @@ extern "C" int sweeptt_put_tt(sweeptt_ctx* c, int s, const float* in) {
   if (!ready(c, &lease)) return 0;
   if (s < 0 || s >= c->nsrc) return fail("sweeptt_put_tt: source %d out of range", s);
   const size_t dense = (size_t)c->g.nx * c->g.ny * c->g.nz;
+  // A travel time is +0, positive or +INF.  The scheduling orders times by their bits as unsigned integers, where a
+  // set sign bit (-0.0, a negative time, -INF) ranks after +INF, and a NaN time would make the location's misfit NaN.
+  for (size_t i = 0; i < dense; ++i) {
+    uint32_t b;
+    std::memcpy(&b, in + i, 4);
+    if (std::isnan(in[i]) || (b >> 31))
+      return fail("sweeptt_put_tt: tt[%zu] of source %d is %s (a travel time is +0, positive or +INF)", i, s,
+                  std::isnan(in[i]) ? "NaN" : in[i] == 0.f ? "-0.0" : std::isinf(in[i]) ? "-INF" : "negative");
+  }
   if (!ensure_stage(c, dense)) return 0;
   CK(cudaMemcpyAsync(c->d_stage, in, dense * 4, cudaMemcpyHostToDevice, c->stream));
   CK(launch_pad_box(c->d_stage, c->d_tt + (size_t)s * c->g.vol, c->g, c->stream));
