@@ -359,6 +359,65 @@ int sweeptt_rayset_project(sweeptt_rayset *set, const float *perturbation, float
 int sweeptt_rayset_backproject(sweeptt_rayset *set, const float *weights, float *grad_out, int *quantum_exp_out,
                                sweeptt_stats *stats);
 
+/* ---- the damped and smoothed least-squares step of a ray set, solved on the device ---------------------------- */
+
+/* sweeptt_rayset_lsqr solves  min ||A x - [b; 0]||^2 + damp^2 ||x||^2,  A = [G_rows; smooth*D],  by LSQR on the device:
+ * only b goes to the device (once), only x and a few scalars per iteration come back.
+ *
+ * G_rows is G over the selected rays (rows[q] != 0; rows NULL = every OK ray; m of them, in q order) with the float32
+ * conversions of the set's operators written into it: G_rows x = float64(sweeptt_rayset_project(float32(x)))[rows],
+ * G_rows^T y = float64(sweeptt_rayset_backproject(W)), W = float32(y) scattered into [N] with +0 outside rows and the
+ * quantum exponent E that sweeptt_rayset_backproject chooses for that W.  Every application is bit for bit what the
+ * set's operators return for the same float32 input.
+ *
+ * D (only when smooth > 0; none at all when smooth = 0) is the first difference: for every caller axis a = 0, 1, 2 in
+ * that order and every node n whose neighbour n + e_a is in the box, in FLOATBOX order, one row with the value
+ * fl(smooth * fl(x[n+e_a] - x[n])).  Component j of its transpose product is acc = +0; for a = 0, 1, 2: if j - e_a is in
+ * the box acc = fl(acc + y_a[j - e_a]), then if j + e_a is in the box acc = fl(acc - y_a[j]); the result is
+ * fl(smooth * acc), and A^T y = fl(G part + D part).
+ *
+ * The algorithm is scipy 1.18's lsqr (scipy/sparse/linalg/_isolve/lsqr.py) statement for statement with x0 = None and
+ * calc_var = False, every square a product x*x, in IEEE float64 with no fused multiply-add, except that every
+ * np.linalg.norm(v) is sqrt(sumsq(v)) with a fixed order: square every element, pad with +0 to a multiple of 2048,
+ * sum every block of 2048 consecutive elements with the halving tree a[i] = fl(a[i] + a[i+h]), h = 1024, 512, .., 1,
+ * and apply the same tree to the vector of block sums until one value is left (sumsq of nothing is +0).  The order
+ * depends on neither the box, the device nor the grid.  istop, itn and the norms of info mean what scipy's return tuple
+ * means.  b = 0 gives x = 0 and istop = 0, as scipy does.  scipy's default iteration limit is 2*nx*ny*nz.
+ *
+ * Refused with a message before anything runs, the set left as it was: a NULL set; b, opts or x_out NULL; a
+ * struct_size of opts (or of info, when given) that is not the sizeof of its struct; rows selecting a ray that is not
+ * OK; an element of b that is not finite; damp or smooth negative or not finite; atol, btol or conlim negative or NaN;
+ * iter_lim < 0; a star whose edge lengths are not finite; and device memory the workspace cannot get.
+ *
+ * Device memory: a workspace allocated by the call and freed before it returns, with m selected rows, mD rows of D
+ * (smooth > 0: (nx-1)*ny*nz + nx*(ny-1)*nz + nx*ny*(nz-1), else 0) and D = nx*ny*nz nodes,
+ *   8*(m + mD) + 24*D + 8*m + 8*(ceil(max(m + mD, D) / 2048) + 1)  bytes
+ * (u; x, v and w; the row index int64[m]; the block sums and max|W|), plus 32 bytes of page-locked host memory.
+ * The solve uses the set's own perturbation, accumulator, staging and per-ray buffers as scratch, so the set's
+ * operators are unchanged afterwards.  It runs on the context's stream and synchronises it; it reads no __constant__
+ * table.  stats (may be NULL): solve_ms = elapsed device time of the whole solve (CUDA events; it includes the waits
+ * for the host's scalar steps), kernel_launches, h2d_ms / h2d_bytes (b and the row index), d2h_ms / d2h_bytes (the
+ * per-iteration scalars and x). */
+typedef struct {
+  int struct_size;                    /* = sizeof(sweeptt_lsqr_opts)                                         */
+  double damp, smooth;                /* finite, >= 0                                                        */
+  double atol, btol, conlim;          /* >= 0 (scipy's defaults: 1e-6, 1e-6, 1e8; conlim = 0: no limit)       */
+  int iter_lim;                       /* >= 0                                                                */
+} sweeptt_lsqr_opts;
+
+typedef struct {
+  int struct_size;                    /* = sizeof(sweeptt_lsqr_info)                                         */
+  int istop, itn;
+  double r1norm, r2norm, anorm, acond, arnorm, xnorm;
+} sweeptt_lsqr_info;
+
+int sweeptt_rayset_lsqr(sweeptt_rayset *set, const uint8_t *rows, /* [N] or NULL = the OK rays                  */
+                        const double *b,                          /* [number of selected rows], finite           */
+                        const sweeptt_lsqr_opts *opts,
+                        double *x_out,                            /* nx*ny*nz, FLOATBOX, caller axes of the freeze */
+                        sweeptt_lsqr_info *info,                  /* may be NULL                                 */
+                        sweeptt_stats *stats);
+
 /* ---- event location: grid search over the stations' travel-time fields ----------------------- */
 
 /* The context's sources [source_begin, source_begin+source_count) are the STATIONS: a field started at a station s

@@ -14,6 +14,7 @@ from .api import (  # noqa: F401
     LOC_UNREACHED,
     LinearizedUpdate,
     Locations,
+    LsqrSolution,
     MisfitGradient,
     RayProjection,
     RaySet,

@@ -58,6 +58,17 @@ class _Stats(C.Structure):
     ]
 
 
+class _LsqrOpts(C.Structure):
+    _fields_ = [("struct_size", C.c_int), ("damp", C.c_double), ("smooth", C.c_double), ("atol", C.c_double),
+                ("btol", C.c_double), ("conlim", C.c_double), ("iter_lim", C.c_int)]
+
+
+class _LsqrInfo(C.Structure):
+    _fields_ = [("struct_size", C.c_int), ("istop", C.c_int), ("itn", C.c_int), ("r1norm", C.c_double),
+                ("r2norm", C.c_double), ("anorm", C.c_double), ("acond", C.c_double), ("arnorm", C.c_double),
+                ("xnorm", C.c_double)]
+
+
 @dataclass
 class SweepStats:
     rounds: int = 0
@@ -96,7 +107,8 @@ _EXPORTS = [
     "sweeptt_set_sources", "sweeptt_run", "sweeptt_step", "sweeptt_reset", "sweeptt_get_tt", "sweeptt_put_tt",
     "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject",
     "sweeptt_rayset_freeze", "sweeptt_rayset_destroy", "sweeptt_rayset_bytes", "sweeptt_rayset_table",
-    "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_locate_events",
+    "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_rayset_lsqr",
+    "sweeptt_locate_events",
     "sweeptt_misfit_box", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_debug_model_stats", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
     "sweeptt_vbox_load", "sweeptt_vbox_store", "sweeptt_vbox_load_subset", "sweeptt_text_load",
@@ -160,6 +172,8 @@ def load_library() -> C.CDLL:
     lib.sweeptt_rayset_project.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_rayset_backproject.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int),
                                                C.POINTER(_Stats)]
+    lib.sweeptt_rayset_lsqr.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_LsqrOpts), C.c_void_p,
+                                        C.POINTER(_LsqrInfo), C.POINTER(_Stats)]
     lib.sweeptt_locate_events.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_misfit_box.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
@@ -398,6 +412,22 @@ class LinearizedUpdate:
     istop: int
     iterations: int
     residual_norm: float
+
+
+@dataclass
+class LsqrSolution:
+    """RaySet.lsqr: x (float64[nx, ny, nz]) minimises ||G_rows x - b||^2 + smooth^2 ||D x||^2 + damp^2 ||x||^2; istop,
+    itn and the six norms mean what scipy.sparse.linalg.lsqr's return tuple means."""
+    x: np.ndarray         # float64[nx, ny, nz]
+    istop: int
+    itn: int
+    r1norm: float
+    r2norm: float
+    anorm: float
+    acond: float
+    arnorm: float
+    xnorm: float
+    stats: SweepStats
 
 
 @dataclass
@@ -760,6 +790,30 @@ class RaySet:
             return self.backproject(w).grad.astype(np.float64).ravel()
 
         return LinearOperator((int(rows.sum()), n), matvec=matvec, rmatvec=rmatvec, dtype=np.float64)
+
+    def lsqr(self, b, rows=None, *, damp: float = 0.0, smooth: float = 0.0, atol: float = 1e-6, btol: float = 1e-6,
+             conlim: float = 1e8, iter_lim: int | None = None) -> LsqrSolution:
+        """scipy.sparse.linalg.lsqr on the device (include/sweeptt.h, sweeptt_rayset_lsqr): minimises
+        ||A x - [b; 0]||^2 + damp^2 ||x||^2 with A = [G_rows; smooth D], G_rows = as_linear_operator(rows) (rows: bool
+        [S, R], default the OK rays; b: float64 over the selected rays in q order) and D the first difference along
+        every axis.  Only b goes to the device and only x and a few scalars per iteration come back.  iter_lim None is
+        scipy's 2 nx ny nz."""
+        rows = self.status == RAY_OK if rows is None else np.asarray(rows, bool)
+        if rows.shape != self.shape:
+            raise SweepError(f"RaySet.lsqr: rows of shape {rows.shape}, expected {self.shape}")
+        bb = np.ascontiguousarray(b, dtype=np.float64).ravel()
+        if bb.size != int(rows.sum()):
+            raise SweepError(f"RaySet.lsqr: b has {bb.size} values, rows selects {int(rows.sum())} rays")
+        sel = np.ascontiguousarray(rows, dtype=np.uint8)
+        n = int(np.prod(self.dims))
+        opts = _LsqrOpts(C.sizeof(_LsqrOpts), damp, smooth, atol, btol, conlim, 2 * n if iter_lim is None else iter_lim)
+        info = _LsqrInfo(C.sizeof(_LsqrInfo))
+        x = np.empty(self.dims, np.float64)
+        s = _Stats()
+        _check(self._lib.sweeptt_rayset_lsqr(self._handle(), sel.ctypes.data, bb.ctypes.data, C.byref(opts),
+                                             x.ctypes.data, C.byref(info), C.byref(s)), "sweeptt_rayset_lsqr")
+        return LsqrSolution(x, info.istop, info.itn, info.r1norm, info.r2norm, info.anorm, info.acond, info.arnorm,
+                            info.xnorm, SweepStats._from(s))
 
 
 def trace_rays(slowness, star, starts, receivers, *, delta: float = 10.0, max_nodes: int | None = None,

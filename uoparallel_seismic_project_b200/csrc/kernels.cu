@@ -33,6 +33,8 @@
 //                     predecessor step, then a walk of the recorded path; exact int64 accumulation for G^T*w).
 //   rayset_record / rayset_compact / rayset_project / rayset_backproject  ray sets: the same rays traced once and
 //                     kept on the device as pull-table entries, then the same walks of the stored records.
+//   lsqr_*            the float64 vector passes of a ray set's LSQR solve (conversions, the smoothing stencil, fused
+//                     updates) with fixed-order sums of squares.
 //   locate / locate_finish / misfit_box  event location: the float64 origin-free least-squares misfit of every
 //                     event at every node from the stations' fields, its argmin and the misfit box of one event.
 //   fill/pad/unpad/init_sources/min_slowness  the device float-box pool's utilities
@@ -1611,6 +1613,181 @@ __global__ void grad_finish_kernel(const long long* __restrict__ acc, float* __r
 }
 
 // ---------------------------------------------------------------------------------------
+// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr; DESIGN §3.11)
+// ---------------------------------------------------------------------------------------
+// The vector passes of one LSQR iteration, every one float64 with DADD / DMUL only (no division or square root: the
+// host forms the reciprocals and roots).  A pass that needs a norm squares its outputs and sums every block of
+// LSQR_BLOCK consecutive squares with the halving tree a[i] = a[i] + a[i+h], h = 1024 .. 1 (elements past the end are
+// +0); lsqr_reduce_kernel applies the same tree to the block sums until one value is left.  Which CTA takes which block
+// changes nothing, so the sums are deterministic and independent of the grid.
+constexpr int LSQR_THREADS = 256;
+constexpr long long LSQR_BLOCK = 2048;
+
+// Tree sum of block [base, base + 2048) of val(0 .. n-1); val(i) is called exactly once for every i < n of the block.
+// s: 1024 doubles of shared memory.  Thread 0 returns the sum.
+template <class F>
+__device__ __forceinline__ double lsqr_block_sum(double* s, long long base, long long n, F&& val) {
+  const int t = threadIdx.x;
+#pragma unroll
+  for (int k = 0; k < 1024 / LSQR_THREADS; ++k) {
+    const int i = t + k * LSQR_THREADS;
+    const double lo = base + i < n ? val(base + i) : 0.0;
+    const double hi = base + i + 1024 < n ? val(base + i + 1024) : 0.0;
+    s[i] = __dadd_rn(lo, hi);
+  }
+  __syncthreads();
+  for (int h = 512; h >= 32; h >>= 1) {
+    for (int i = t; i < h; i += LSQR_THREADS) s[i] = __dadd_rn(s[i], s[i + h]);
+    __syncthreads();
+  }
+  double r = 0.0;
+  if (t < 32) {
+    r = s[t];
+    for (int h = 16; h; h >>= 1) r = __dadd_rn(r, __shfl_down_sync(0xffffffffu, r, h));
+  }
+  __syncthreads();  // s is reused by the next block
+  return r;
+}
+
+// First level: part[b] = tree sum of block b of val(0 .. n-1), the blocks shared out over the grid.
+template <class F>
+__device__ __forceinline__ void lsqr_blocks(long long n, double* part, F&& val) {
+  __shared__ double s[1024];
+  const long long nb = (n + LSQR_BLOCK - 1) / LSQR_BLOCK;
+  for (long long b = blockIdx.x; b < nb; b += gridDim.x) {
+    const double r = lsqr_block_sum(s, b * LSQR_BLOCK, n, val);
+    if (threadIdx.x == 0) part[b] = r;
+  }
+}
+
+// One CTA: the n block sums in part[] are summed level by level, in place (block b of a level is read before its sum
+// goes to part[b], and b < LSQR_BLOCK * b' for every later block b'), until part[0] holds the total.
+__global__ void __launch_bounds__(LSQR_THREADS) lsqr_reduce_kernel(double* part, long long n) {
+  __shared__ double s[1024];
+  while (n > 1) {
+    const long long nb = (n + LSQR_BLOCK - 1) / LSQR_BLOCK;
+    for (long long b = 0; b < nb; ++b) {
+      const double r = lsqr_block_sum(s, b * LSQR_BLOCK, n, [&](long long i) { return part[i]; });
+      if (threadIdx.x == 0) part[b] = r;
+      __syncthreads();
+    }
+    n = nb;
+  }
+}
+
+__device__ __forceinline__ double lsqr_sq(double a) { return __dmul_rn(a, a); }
+
+// Row k of D (k < mD): fl(smooth * fl(v[n + e_a] - v[n])), the rows of axis 0, then 1, then 2, each in FLOATBOX order
+// of the nodes n whose neighbour n + e_a is in the box.
+__device__ __forceinline__ double lsqr_d_row(const LsqrArgs& a, long long k) {
+  const long long nx = a.nx, ny = a.ny, nz = a.nz;
+  const long long s0 = (nx - 1) * ny * nz, s1 = nx * (ny - 1) * nz;
+  long long n, step;
+  if (k < s0) {
+    n = k;
+    step = ny * nz;
+  } else if ((k -= s0) < s1) {
+    const long long z = k % nz, r = k / nz, y = r % (ny - 1), x = r / (ny - 1);
+    n = (x * ny + y) * nz + z;
+    step = nz;
+  } else {
+    k -= s1;
+    n = k / (nz - 1) * nz + k % (nz - 1);
+    step = 1;
+  }
+  DBG_BOUNDS(n >= 0 && n + step < nx * ny * nz);
+  return __dmul_rn(a.smooth, __dsub_rn(a.v[n + step], a.v[n]));
+}
+
+// Component j of D^T y (y = the D rows of u): acc = +0; for a = 0, 1, 2: + y_a[j - e_a] if that node is in the box,
+// then - y_a[j] if j + e_a is; fl(smooth * acc).
+__device__ __forceinline__ double lsqr_dt(const LsqrArgs& a, long long j) {
+  const long long nx = a.nx, ny = a.ny, nz = a.nz;
+  const long long z = j % nz, r = j / nz, y = r % ny, x = r / ny;
+  const double* u0 = a.u + a.m;
+  const double* u1 = u0 + (nx - 1) * ny * nz;
+  const double* u2 = u1 + nx * (ny - 1) * nz;
+  double acc = 0.0;
+  if (x > 0) acc = __dadd_rn(acc, u0[j - ny * nz]);
+  if (x < nx - 1) acc = __dsub_rn(acc, u0[j]);
+  const long long i1 = (x * (ny - 1) + y) * nz + z;  // row of node j along axis 1
+  if (y > 0) acc = __dadd_rn(acc, u1[i1 - nz]);
+  if (y < ny - 1) acc = __dsub_rn(acc, u1[i1]);
+  const long long i2 = (x * ny + y) * (nz - 1) + z;  // ... along axis 2
+  if (z > 0) acc = __dadd_rn(acc, u2[i2 - 1]);
+  if (z < nz - 1) acc = __dsub_rn(acc, u2[i2]);
+  return __dmul_rn(a.smooth, acc);
+}
+
+// Partials of sumsq(p[0 .. n)).
+__global__ void __launch_bounds__(LSQR_THREADS) lsqr_sumsq_kernel(const double* __restrict__ p, long long n,
+                                                                  double* __restrict__ part) {
+  lsqr_blocks(n, part, [&](long long i) { return lsqr_sq(p[i]); });
+}
+
+// Pass A (first half): stage = float32(v), dense caller axes; launch_pad_box then pads it into the set's box.
+__global__ void lsqr_to_f32_kernel(const double* __restrict__ v, float* __restrict__ stage, long long n) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    stage[i] = __double2float_rn(v[i]);
+}
+
+// Pass C: u = A v - alpha u, A v = [float64(io[row[i]]); D v], and the partials of sumsq(u).
+__global__ void __launch_bounds__(LSQR_THREADS) lsqr_u_kernel(const LsqrArgs a, double alpha) {
+  lsqr_blocks(a.m + a.mD, a.part, [&](long long i) {
+    const double av = i < a.m ? (double)a.io[a.row[i]] : lsqr_d_row(a, i - a.m);
+    const double u = __dsub_rn(av, __dmul_rn(alpha, a.u[i]));
+    a.u[i] = u;
+    return lsqr_sq(u);
+  });
+}
+
+// Pass D: u = inv_beta * u; the G rows, as float32 weights W, go to io[row[i]] (zeroed by the caller), and the bits of
+// max |W| to *wmax (non-negative floats order like their bits).
+__global__ void __launch_bounds__(LSQR_THREADS) lsqr_scale_u_kernel(const LsqrArgs a, double inv_beta) {
+  unsigned mx = 0;
+  const long long n = a.m + a.mD;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const double u = __dmul_rn(inv_beta, a.u[i]);
+    a.u[i] = u;
+    if (i < a.m) {
+      const float W = __double2float_rn(u);
+      a.io[a.row[i]] = W;
+      mx = max(mx, __float_as_uint(W) & 0x7fffffffu);
+    }
+  }
+  for (int o = 16; o; o >>= 1) mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if ((threadIdx.x & 31) == 0 && mx) atomicMax(a.wmax, mx);
+}
+
+// Pass F: v = A^T u - beta v, A^T u = fl(float64(grad) + D^T u_D) (the D term only with smoothing; grad = the set's
+// rounded back-projection in stage), and the partials of sumsq(v).
+__global__ void __launch_bounds__(LSQR_THREADS) lsqr_v_kernel(const LsqrArgs a, double beta) {
+  lsqr_blocks((long long)a.nx * a.ny * a.nz, a.part, [&](long long j) {
+    double g = (double)a.stage[j];
+    if (a.smooth > 0.0) g = __dadd_rn(g, lsqr_dt(a, j));
+    const double v = __dsub_rn(g, __dmul_rn(beta, a.v[j]));
+    a.v[j] = v;
+    return lsqr_sq(v);
+  });
+}
+
+__global__ void lsqr_scale_kernel(double* __restrict__ p, long long n, double s) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    p[i] = __dmul_rn(s, p[i]);
+}
+
+// Step 7: dk = inv_rho * w (only its sumsq partials are kept), x = x + t1 w, w = v + t2 w.
+__global__ void __launch_bounds__(LSQR_THREADS) lsqr_xw_kernel(const LsqrArgs a, double t1, double t2, double inv_rho) {
+  lsqr_blocks((long long)a.nx * a.ny * a.nz, a.part, [&](long long j) {
+    const double w = a.w[j];
+    const double dk = __dmul_rn(inv_rho, w);
+    a.x[j] = __dadd_rn(a.x[j], __dmul_rn(t1, w));
+    a.w[j] = __dadd_rn(a.v[j], __dmul_rn(t2, w));
+    return lsqr_sq(dk);
+  });
+}
+
+// ---------------------------------------------------------------------------------------
 // event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box; DESIGN §3.10)
 // ---------------------------------------------------------------------------------------
 constexpr int LOC_THREADS = 512;
@@ -2261,6 +2438,61 @@ cudaError_t launch_rayset_walk(bool backproject, const RaySetArgs& s, int device
 cudaError_t launch_grad_finish(const long long* acc, float* dense, BoxGeom g, int E, cudaStream_t stream) {
   grad_finish_kernel<<<1184, 256, 0, stream>>>(acc, dense, g, E);
   return cudaGetLastError();
+}
+
+// CTAs of a first-level reduction over n elements: one per block, at most `ctas`.
+static unsigned lsqr_grid(long long n, int ctas) {
+  return (unsigned)std::max(1LL, std::min<long long>((n + LSQR_BLOCK - 1) / LSQR_BLOCK, ctas));
+}
+
+// After the first-level launch over n elements (none when n = 0: the sum of nothing is +0).
+static cudaError_t lsqr_finish(double* part, long long n, cudaStream_t stream, int* launches) {
+  if (n == 0) return cudaMemsetAsync(part, 0, sizeof(double), stream);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  ++*launches;
+  if (n <= LSQR_BLOCK) return cudaSuccess;
+  lsqr_reduce_kernel<<<1, LSQR_THREADS, 0, stream>>>(part, (n + LSQR_BLOCK - 1) / LSQR_BLOCK);
+  ++*launches;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_lsqr_sumsq(const double* p, long long n, double* part, int ctas, cudaStream_t stream, int* launches) {
+  if (n > 0) lsqr_sumsq_kernel<<<lsqr_grid(n, ctas), LSQR_THREADS, 0, stream>>>(p, n, part);
+  return lsqr_finish(part, n, stream, launches);
+}
+
+cudaError_t launch_lsqr_to_f32(const double* v, float* stage, long long n, cudaStream_t stream) {
+  lsqr_to_f32_kernel<<<1184, 256, 0, stream>>>(v, stage, n);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_lsqr_u(const LsqrArgs& a, double alpha, cudaStream_t stream, int* launches) {
+  const long long n = a.m + a.mD;
+  if (n > 0) lsqr_u_kernel<<<lsqr_grid(n, a.ctas), LSQR_THREADS, 0, stream>>>(a, alpha);
+  return lsqr_finish(a.part, n, stream, launches);
+}
+
+cudaError_t launch_lsqr_scale_u(const LsqrArgs& a, double inv_beta, cudaStream_t stream) {
+  lsqr_scale_u_kernel<<<1184, LSQR_THREADS, 0, stream>>>(a, inv_beta);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_lsqr_v(const LsqrArgs& a, double beta, cudaStream_t stream, int* launches) {
+  const long long n = (long long)a.nx * a.ny * a.nz;
+  lsqr_v_kernel<<<lsqr_grid(n, a.ctas), LSQR_THREADS, 0, stream>>>(a, beta);
+  return lsqr_finish(a.part, n, stream, launches);
+}
+
+cudaError_t launch_lsqr_scale(double* p, long long n, double s, cudaStream_t stream) {
+  lsqr_scale_kernel<<<1184, 256, 0, stream>>>(p, n, s);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_lsqr_xw(const LsqrArgs& a, double t1, double t2, double inv_rho, cudaStream_t stream, int* launches) {
+  const long long n = (long long)a.nx * a.ny * a.nz;
+  lsqr_xw_kernel<<<lsqr_grid(n, a.ctas), LSQR_THREADS, 0, stream>>>(a, t1, t2, inv_rho);
+  return lsqr_finish(a.part, n, stream, launches);
 }
 
 template <int NB>

@@ -167,6 +167,33 @@ cudaError_t launch_rayset_walk(bool backproject, const RaySetArgs& s, int device
 // grad (dense, caller axes) := acc * 2^E rounded once to float32.
 cudaError_t launch_grad_finish(const long long* acc, float* dense, BoxGeom g, int E, cudaStream_t stream);
 
+// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr).  float64 vectors: u over the m selected rows of G then
+// the mD rows of the smoothing operator D, x / v / w over the dense caller-FLOATBOX box.  A launcher whose pass ends
+// in a norm leaves sumsq of the pass's outputs in part[0] (the fixed-order block tree, kernels.cu) and adds its
+// launches to *launches; the others are one launch each.
+struct LsqrArgs {
+  long long m, mD;             // rows of G selected, rows of D (0 without smoothing)
+  int nx, ny, nz;              // caller axes
+  double smooth;
+  const long long* row;        // [m] ray of every selected row
+  double* u;                   // [m + mD]
+  double* x;                   // [D]
+  double* v;                   // [D]
+  double* w;                   // [D]
+  float* io;                   // the set's per-ray floats (projections in, weights out)
+  float* stage;                // the set's dense float32 box
+  double* part;                // block sums: ceil(max(m + mD, D) / 2048) doubles
+  unsigned* wmax;              // bits of max |W| of pass D (zeroed by the caller)
+  int ctas;                    // CTAs that share the blocks of a first-level reduction (the result does not depend on it)
+};
+cudaError_t launch_lsqr_sumsq(const double* p, long long n, double* part, int ctas, cudaStream_t stream, int* launches);
+cudaError_t launch_lsqr_to_f32(const double* v, float* stage, long long n, cudaStream_t stream);
+cudaError_t launch_lsqr_u(const LsqrArgs& a, double alpha, cudaStream_t stream, int* launches);
+cudaError_t launch_lsqr_scale_u(const LsqrArgs& a, double inv_beta, cudaStream_t stream);
+cudaError_t launch_lsqr_v(const LsqrArgs& a, double beta, cudaStream_t stream, int* launches);
+cudaError_t launch_lsqr_scale(double* p, long long n, double s, cudaStream_t stream);
+cudaError_t launch_lsqr_xw(const LsqrArgs& a, double t1, double t2, double inv_rho, cudaStream_t stream, int* launches);
+
 // Event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box).  Event e's picks are entries
 // pick_off[e] .. pick_off[e+1] of pick_sta / pick_obs, in increasing station order (NaN picks left out).
 struct LocateArgs {

@@ -2207,6 +2207,339 @@ extern "C" int sweeptt_rayset_backproject(sweeptt_rayset* r, const float* weight
 }
 
 // ---------------------------------------------------------------------------------------
+// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr; DESIGN §3.11)
+// ---------------------------------------------------------------------------------------
+// The vectors stay on the device; the host runs scipy's scalar recurrences (this file is built with
+// -ffp-contract=off, so they round exactly as numpy's scalars do) and reads four scalars per iteration.
+
+// CTAs that share the blocks of a first-level reduction (SWEEPTT_LSQR_CTAS; the result does not depend on it).
+static int lsqr_ctas() {
+  int ctas = 1184;
+  if (const char* e = getenv("SWEEPTT_LSQR_CTAS")) ctas = std::max(1, atoi(e));
+  return ctas;
+}
+
+namespace {
+
+struct LsqrSolve {
+  sweeptt_rayset* r = nullptr;
+  cudaStream_t st = nullptr;
+  LsqrArgs a{};
+  void* dev = nullptr;      // the whole float64 workspace, one allocation
+  double* host = nullptr;   // page-locked: [0] a sum of squares, [1] the bits of max |W|
+  long long D = 0;
+  int launches = 0;
+  double d2h_ms = 0;
+  long long d2h_bytes = 0;
+
+  ~LsqrSolve() {
+    if (dev) cudaFree(dev);
+    if (host) cudaFreeHost(host);
+  }
+
+  // sqrt of the sum of squares the last pass left in part[0]
+  int read_norm(double* out) {
+    const auto t0 = std::chrono::steady_clock::now();
+    CK(cudaMemcpyAsync(host, a.part, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    d2h_bytes += 8;
+    *out = std::sqrt(host[0]);
+    return 1;
+  }
+
+  // G x: pass A (v to float32, padded into the set's box) and pass B (the set's projection into io)
+  int project() {
+    CK(launch_lsqr_to_f32(a.v, r->d_stage, D, st));
+    CK(launch_pad_box(r->d_stage, r->d_pert, r->g, st));
+    RaySetArgs s = rayset_args(r);
+    s.a.pert = r->d_pert;
+    s.a.proj = r->d_io;
+    CK(launch_rayset_walk(false, s, r->device, st));
+    launches += 3;
+    return 1;
+  }
+
+  // Pass D (u = inv_beta u; W into io; max |W|) and pass E (the set's back-projection of W into stage with the E
+  // that sweeptt_rayset_backproject chooses)
+  int backproject(double inv_beta) {
+    CK(cudaMemsetAsync(r->d_io, 0, 4 * (size_t)r->nrays, st));
+    CK(cudaMemsetAsync(a.wmax, 0, 4, st));
+    CK(launch_lsqr_scale_u(a, inv_beta, st));
+    const auto t0 = std::chrono::steady_clock::now();
+    CK(cudaMemcpyAsync(host + 1, a.wmax, 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    d2h_bytes += 4;
+    unsigned bits;
+    std::memcpy(&bits, host + 1, 4);
+    float W;
+    std::memcpy(&W, &bits, 4);
+    const int E = (W > 0.f && r->hd_max > 0.f) ? quantum_exponent(r->hd_max, W, r->nrays) : 0;
+    RaySetArgs s = rayset_args(r);
+    s.a.weights = r->d_io;
+    s.a.acc = r->d_acc;
+    s.a.scale = std::ldexp(1.0, -E);
+    CK(cudaMemsetAsync(r->d_acc, 0, (size_t)r->g.vol * 8, st));
+    CK(launch_rayset_walk(true, s, r->device, st));
+    CK(launch_grad_finish(r->d_acc, r->d_stage, r->g, E, st));
+    launches += 3;
+    return 1;
+  }
+};
+
+// scipy's _sym_ortho
+void sym_ortho(double a, double b, double* c, double* s, double* rr) {
+  auto sign = [](double t) { return t > 0 ? 1.0 : t < 0 ? -1.0 : t; };
+  if (b == 0) {
+    *c = sign(a); *s = 0; *rr = std::fabs(a);
+  } else if (a == 0) {
+    *c = 0; *s = sign(b); *rr = std::fabs(b);
+  } else if (std::fabs(b) > std::fabs(a)) {
+    const double tau = a / b;
+    *s = sign(b) / std::sqrt(1 + tau * tau);
+    *c = *s * tau;
+    *rr = b / *s;
+  } else {
+    const double tau = b / a;
+    *c = sign(a) / std::sqrt(1 + tau * tau);
+    *s = *c * tau;
+    *rr = a / *c;
+  }
+}
+
+}  // namespace
+
+extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const double* b,
+                                   const sweeptt_lsqr_opts* opts, double* x_out, sweeptt_lsqr_info* info,
+                                   sweeptt_stats* stats) {
+  if (!r) return fail("null ray set");
+  if (stats) std::memset(stats, 0, sizeof *stats);
+  if (!b || !opts || !x_out) return fail("sweeptt_rayset_lsqr: b, opts and x_out are required");
+  if (opts->struct_size != (int)sizeof *opts)
+    return fail("sweeptt_rayset_lsqr: opts->struct_size is %d, expected %d", opts->struct_size, (int)sizeof *opts);
+  if (info && info->struct_size != (int)sizeof *info)
+    return fail("sweeptt_rayset_lsqr: info->struct_size is %d, expected %d", info->struct_size, (int)sizeof *info);
+  const double damp = opts->damp, smooth = opts->smooth;
+  if (!std::isfinite(damp) || damp < 0) return fail("sweeptt_rayset_lsqr: damp must be finite and >= 0");
+  if (!std::isfinite(smooth) || smooth < 0) return fail("sweeptt_rayset_lsqr: smooth must be finite and >= 0");
+  if (!(opts->atol >= 0) || !(opts->btol >= 0) || !(opts->conlim >= 0))
+    return fail("sweeptt_rayset_lsqr: atol, btol and conlim must be >= 0");
+  if (opts->iter_lim < 0) return fail("sweeptt_rayset_lsqr: iter_lim must be >= 0");
+  if (!std::isfinite(r->hd_max)) return fail("sweeptt_rayset_lsqr: the star's edge lengths are not finite");
+  std::vector<long long> row;
+  for (long long q = 0; q < r->nrays; ++q) {
+    const bool sel = rows ? rows[q] != 0 : r->status[q] == SWEEPTT_RAY_OK;
+    if (!sel) continue;
+    if (r->status[q] != SWEEPTT_RAY_OK) return fail("sweeptt_rayset_lsqr: rows selects ray %lld, which is not OK", q);
+    row.push_back(q);
+  }
+  const long long m = (long long)row.size();
+  for (long long i = 0; i < m; ++i)
+    if (!std::isfinite(b[i])) return fail("sweeptt_rayset_lsqr: b[%lld] is not finite", i);
+
+  const BoxGeom& g = r->g;
+  const long long nx = g.nx, ny = g.ny, nz = g.nz;  // kernel axes: the caller's through perm
+  long long cd[3];
+  for (int k = 0; k < 3; ++k) cd[g.perm[k]] = k == 0 ? nx : k == 1 ? ny : nz;
+  LsqrSolve S;
+  S.r = r;
+  S.st = r->ctx->stream;
+  S.D = cd[0] * cd[1] * cd[2];
+  const long long D = S.D;
+  const long long mD = smooth > 0 ? (cd[0] - 1) * cd[1] * cd[2] + cd[0] * (cd[1] - 1) * cd[2] + cd[0] * cd[1] * (cd[2] - 1) : 0;
+  const long long mu = m + mD;
+  const long long nblk = (std::max({mu, D, 1LL}) + 2047) / 2048;
+  CK(cudaSetDevice(r->device));
+  cudaStream_t st = S.st;
+  {
+    const size_t bytes = 8 * (size_t)mu + 24 * (size_t)D + 8 * (size_t)m + 8 * (size_t)(nblk + 1);
+    const cudaError_t e = cudaMalloc(&S.dev, bytes);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      S.dev = nullptr;
+      return fail("sweeptt_rayset_lsqr: no device memory for the %.3f GB workspace (%s)", bytes / 1e9, cudaGetErrorString(e));
+    }
+    const cudaError_t eh = cudaMallocHost(&S.host, 32);
+    if (eh != cudaSuccess) {
+      cudaGetLastError();
+      S.host = nullptr;
+      return fail("sweeptt_rayset_lsqr: no page-locked host memory (%s)", cudaGetErrorString(eh));
+    }
+  }
+  LsqrArgs& a = S.a;
+  double* p = static_cast<double*>(S.dev);
+  a.u = p; p += mu;
+  a.x = p; p += D;
+  a.v = p; p += D;
+  a.w = p; p += D;
+  a.row = reinterpret_cast<long long*>(p); p += m;
+  a.part = p; p += nblk;
+  a.wmax = reinterpret_cast<unsigned*>(p);
+  a.m = m;
+  a.mD = mD;
+  a.nx = (int)cd[0]; a.ny = (int)cd[1]; a.nz = (int)cd[2];
+  a.smooth = smooth;
+  a.io = r->d_io;
+  a.stage = r->d_stage;
+  a.ctas = lsqr_ctas();
+
+  CK(cudaEventRecord(r->ev0, st));
+  const auto t_h2d = std::chrono::steady_clock::now();
+  if (m) {
+    CK(cudaMemcpyAsync(a.u, b, 8 * (size_t)m, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(const_cast<long long*>(a.row), row.data(), 8 * (size_t)m, cudaMemcpyHostToDevice, st));
+  }
+  CK(cudaStreamSynchronize(st));  // pageable sources: the copies are complete
+  const double h2d_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_h2d).count();
+  if (mD) CK(cudaMemsetAsync(a.u + m, 0, 8 * (size_t)mD, st));
+  CK(cudaMemsetAsync(a.x, 0, 8 * (size_t)D, st));
+
+  // scipy's lsqr, x0 = None, calc_var = False
+  const double eps = std::numeric_limits<double>::epsilon();
+  const double atol = opts->atol, btol = opts->btol, conlim = opts->conlim;
+  const int iter_lim = opts->iter_lim;
+  int itn = 0, istop = 0;
+  double ctol = 0;
+  if (conlim > 0) ctol = 1 / conlim;
+  double anorm = 0, acond = 0, dampsq = damp * damp, ddnorm = 0, res2 = 0, xnorm = 0, xxnorm = 0, z = 0, cs2 = -1,
+         sn2 = 0;
+  double bnorm, alfa = 0, beta;
+  CK(launch_lsqr_sumsq(a.u, m, a.part, a.ctas, st, &S.launches));
+  if (!S.read_norm(&bnorm)) return 0;
+  beta = bnorm;
+  if (beta > 0) {
+    if (!S.backproject(1 / beta)) return 0;
+    CK(cudaMemsetAsync(a.v, 0, 8 * (size_t)D, st));
+    CK(launch_lsqr_v(a, 0.0, st, &S.launches));  // v = A^T u (- 0 * 0)
+    if (!S.read_norm(&alfa)) return 0;
+  } else {
+    CK(cudaMemsetAsync(a.v, 0, 8 * (size_t)D, st));
+  }
+  if (alfa > 0) {
+    CK(launch_lsqr_scale(a.v, D, 1 / alfa, st));
+    ++S.launches;
+  }
+  CK(cudaMemcpyAsync(a.w, a.v, 8 * (size_t)D, cudaMemcpyDeviceToDevice, st));
+  double rhobar = alfa, phibar = beta, rnorm = beta, r1norm = rnorm, r2norm = rnorm, arnorm = alfa * beta;
+
+  const bool solved = arnorm == 0;  // scipy returns x = 0 before its loop
+  while (!solved && itn < iter_lim) {
+    itn = itn + 1;
+    if (!S.project()) return 0;
+    CK(launch_lsqr_u(a, alfa, st, &S.launches));
+    if (!S.read_norm(&beta)) return 0;
+    if (beta > 0) {
+      if (!S.backproject(1 / beta)) return 0;
+      anorm = std::sqrt(anorm * anorm + alfa * alfa + beta * beta + dampsq);
+      CK(launch_lsqr_v(a, beta, st, &S.launches));
+      if (!S.read_norm(&alfa)) return 0;
+      if (alfa > 0) {
+        CK(launch_lsqr_scale(a.v, D, 1 / alfa, st));
+        ++S.launches;
+      }
+    }
+    double rhobar1, psi;
+    if (damp > 0) {
+      rhobar1 = std::sqrt(rhobar * rhobar + dampsq);
+      const double cs1 = rhobar / rhobar1;
+      const double sn1 = damp / rhobar1;
+      psi = sn1 * phibar;
+      phibar = cs1 * phibar;
+    } else {
+      rhobar1 = rhobar;
+      psi = 0.;
+    }
+    double cs, sn, rho;
+    sym_ortho(rhobar1, beta, &cs, &sn, &rho);
+    const double theta = sn * alfa;
+    rhobar = -cs * alfa;
+    const double phi = cs * phibar;
+    phibar = sn * phibar;
+    const double tau = sn * phi;
+    double t1 = phi / rho;
+    const double t2 = -theta / rho;
+    CK(launch_lsqr_xw(a, t1, t2, 1 / rho, st, &S.launches));  // x += t1 w; sumsq of dk = (1/rho) w; w = v + t2 w
+    double dknorm;
+    if (!S.read_norm(&dknorm)) return 0;
+    ddnorm = ddnorm + dknorm * dknorm;
+
+    const double delta = sn2 * rho;
+    const double gambar = -cs2 * rho;
+    const double rhs = phi - delta * z;
+    const double zbar = rhs / gambar;
+    xnorm = std::sqrt(xxnorm + zbar * zbar);
+    const double gamma = std::sqrt(gambar * gambar + theta * theta);
+    cs2 = gambar / gamma;
+    sn2 = theta / gamma;
+    z = rhs / gamma;
+    xxnorm = xxnorm + z * z;
+
+    acond = anorm * std::sqrt(ddnorm);
+    const double res1 = phibar * phibar;
+    res2 = res2 + psi * psi;
+    rnorm = std::sqrt(res1 + res2);
+    arnorm = alfa * std::fabs(tau);
+
+    if (damp > 0) {
+      const double r1sq = rnorm * rnorm - dampsq * xxnorm;
+      r1norm = std::sqrt(std::fabs(r1sq));
+      if (r1sq < 0) r1norm = -r1norm;
+    } else {
+      r1norm = rnorm;
+    }
+    r2norm = rnorm;
+
+    const double test1 = rnorm / bnorm;
+    const double test2 = arnorm / (anorm * rnorm + eps);
+    const double test3 = 1 / (acond + eps);
+    t1 = test1 / (1 + anorm * xnorm / bnorm);
+    const double rtol = btol + atol * anorm * xnorm / bnorm;
+
+    if (itn >= iter_lim) istop = 7;
+    if (1 + test3 <= 1) istop = 6;
+    if (1 + test2 <= 1) istop = 5;
+    if (1 + t1 <= 1) istop = 4;
+
+    if (test3 <= ctol) istop = 3;
+    if (test2 <= atol) istop = 2;
+    if (test1 <= rtol) istop = 1;
+
+    if (istop != 0) break;
+  }
+
+  CK(cudaEventRecord(r->ev1, st));
+  const auto t_x = std::chrono::steady_clock::now();
+  CK(cudaMemcpyAsync(x_out, a.x, 8 * (size_t)D, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  S.d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_x).count();
+  S.d2h_bytes += 8 * D;
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, r->ev0, r->ev1));
+  if (info) {
+    info->istop = istop;
+    info->itn = itn;
+    info->r1norm = r1norm;
+    info->r2norm = r2norm;
+    info->anorm = anorm;
+    info->acond = acond;
+    info->arnorm = arnorm;
+    info->xnorm = xnorm;
+  }
+  if (stats) {
+    stats->struct_size = (int)sizeof *stats;
+    stats->solve_ms = ms;
+    stats->kernel_launches = S.launches;
+    stats->devices_used = 1;
+    stats->h2d_ms = h2d_ms;
+    stats->h2d_bytes = 16 * m;
+    stats->d2h_ms = S.d2h_ms;
+    stats->d2h_bytes = S.d2h_bytes;
+  }
+  return 1;
+}
+
+// ---------------------------------------------------------------------------------------
 // event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box)
 // ---------------------------------------------------------------------------------------
 
