@@ -469,6 +469,31 @@ int sweeptt_locate_events(sweeptt_ctx *ctx, int source_begin, int source_count, 
 int sweeptt_misfit_box(sweeptt_ctx *ctx, int source_begin, int source_count, const float *picks /*[source_count]*/,
                        float *misfit_out, sweeptt_stats *stats);
 
+/* The uncertainty of located events: for every event e, the region R_e = { n : misfit_e(n) <= levels[e] } (float32
+ * comparison; misfit_e as above), summarised exactly on the device, so that a few dozen numbers per event leave it
+ * instead of a misfit box.  Stations, picks [nev*source_count], the per-node formula, the exclusion rule, the
+ * refusals, the station limit (the same rule for the call's own kernel: 904 stations on a B200) and the stats are
+ * those of sweeptt_locate_events.
+ *   - Excluded nodes, and nodes whose misfit overflows float32 to +INF, are never in R_e: for every accepted level R_e
+ *     is exactly { n : box[n] <= levels[e] } of the event's sweeptt_misfit_box.  An event with no pick has an empty
+ *     region (its misfit box is +0 everywhere: the one exception), and so has a NaN level.
+ *   - levels [nev]: NaN, or finite and >= 0.  -0.0 is +0.  +INF, -INF and negative levels are refused, with the
+ *     event's index in the message.
+ *   - count_out [nev]: |R_e|.  bbox_out [nev*6]: lo0 lo1 lo2 hi0 hi1 hi2, inclusive, caller axes.  moments_out [nev*9]:
+ *     S0 S1 S2 S00 S11 S22 S01 S02 S12, the sums over R_e of c_a and c_a*c_b for the caller-axis node coordinates c.
+ *     origin_range_out [nev*2]: the smallest and largest origin time t0 over R_e, the formula's t0.  status_out [nev]:
+ *     SWEEPTT_LOC_* exactly as sweeptt_locate_events gives it.  An empty region has bbox -1s, moments 0 and origin
+ *     range NaN, NaN.  count_out and status_out are required; the others may be NULL.
+ *   - Exactness: every output is an integer sum, an integer min / max or a min / max of doubles (compared through the
+ *     order-preserving map of their bits to uint64; t0 is never -0, since its sum starts at +0 and a nonzero sum of
+ *     float32 differences, at least 2^-149, divided by k <= 2^31 does not underflow).  So every output is bit-identical
+ *     for any schedule, chunking (SWEEPTT_LOCATE_CHUNK), kernel that produced the fields or axis permutation.
+ *   - A further refusal: a box whose second moments could overflow int64, D * max_a (n_a - 1)^2 > 2^63 - 1 with
+ *     D = nx*ny*nz (a line of 2^21 + 1 nodes; 2401 x 2401 x 501 gives 1.7e16), before any allocation. */
+int sweeptt_misfit_regions(sweeptt_ctx *ctx, int source_begin, int source_count, const float *picks, int nev,
+                           const float *levels, int64_t *count_out, int32_t *bbox_out, int64_t *moments_out,
+                           double *origin_range_out, int32_t *status_out, sweeptt_stats *stats);
+
 /* In-bounds pull evaluations of one full round of one source (analytic). */
 long long sweeptt_relaxations_per_round(sweeptt_ctx *ctx);
 /* Bytes of device memory currently held by the context's pool. */

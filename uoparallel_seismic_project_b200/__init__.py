@@ -16,6 +16,7 @@ from .api import (  # noqa: F401
     Locations,
     LsqrSolution,
     MisfitGradient,
+    MisfitRegions,
     RayProjection,
     RaySet,
     Rays,
@@ -29,6 +30,7 @@ from .api import (  # noqa: F401
     load_library,
     linearized_update,
     locate_events,
+    location_uncertainty,
     make_star,
     solve,
     solve_slabs,
@@ -38,6 +40,7 @@ from .api import (  # noqa: F401
     text_load,
     misfit_gradient,
     trace_rays,
+    uncertainty_levels,
     vbox_load,
     vbox_load_subset,
     vbox_store,

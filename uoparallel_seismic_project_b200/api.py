@@ -108,7 +108,7 @@ _EXPORTS = [
     "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject",
     "sweeptt_rayset_freeze", "sweeptt_rayset_destroy", "sweeptt_rayset_bytes", "sweeptt_rayset_table",
     "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_rayset_lsqr",
-    "sweeptt_locate_events",
+    "sweeptt_locate_events", "sweeptt_misfit_regions",
     "sweeptt_misfit_box", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_debug_model_stats", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
     "sweeptt_vbox_load", "sweeptt_vbox_store", "sweeptt_vbox_load_subset", "sweeptt_text_load",
@@ -176,6 +176,8 @@ def load_library() -> C.CDLL:
                                         C.POINTER(_LsqrInfo), C.POINTER(_Stats)]
     lib.sweeptt_locate_events.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
+    lib.sweeptt_misfit_regions.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_misfit_box.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_relaxations_per_round.argtypes = [C.c_void_p]
     lib.sweeptt_relaxations_per_round.restype = C.c_longlong
@@ -445,6 +447,48 @@ class Locations:
     stats: SweepStats
 
 
+@dataclass
+class MisfitRegions:
+    """The region R_e = {n : misfit_e(n) <= level_e} of every event, summarised exactly on the device
+    (SweepContext.misfit_regions, include/sweeptt.h sweeptt_misfit_regions).  count[e] = |R_e|; lo[e] / hi[e] the
+    inclusive caller-axis bounding box (-1 when empty); moments[e] = S0 S1 S2 S00 S11 S22 S01 S02 S12, the integer sums
+    of c_a and c_a*c_b over the node coordinates c in R_e; origin_min / origin_max the extremes of the origin time over
+    R_e (NaN when empty); npicks and status as in Locations."""
+    count: np.ndarray        # int64[E]
+    lo: np.ndarray           # int32[E, 3]
+    hi: np.ndarray           # int32[E, 3]
+    moments: np.ndarray      # int64[E, 9]
+    origin_min: np.ndarray   # float64[E]
+    origin_max: np.ndarray   # float64[E]
+    npicks: np.ndarray       # int32[E]
+    status: np.ndarray       # int32[E]
+    stats: SweepStats
+
+    def mean(self) -> np.ndarray:
+        """float64 [E, 3]: the mean node coordinate of each region, each value the exact quotient rounded once; NaN
+        where the region is empty."""
+        from fractions import Fraction
+        out = np.full((len(self.count), 3), np.nan)
+        for e, n in enumerate(self.count.tolist()):
+            if n:
+                for a in range(3):
+                    out[e, a] = float(Fraction(int(self.moments[e, a]), n))
+        return out
+
+    def covariance(self) -> np.ndarray:
+        """float64 [E, 3, 3]: the population covariance of each region's node coordinates (node units),
+        (n*S_ab - S_a*S_b) / n^2 computed exactly and rounded once; NaN where the region is empty."""
+        from fractions import Fraction
+        out = np.full((len(self.count), 3, 3), np.nan)
+        second = {(0, 0): 3, (1, 1): 4, (2, 2): 5, (0, 1): 6, (0, 2): 7, (1, 2): 8}
+        for e, n in enumerate(self.count.tolist()):
+            if n:
+                m = [int(x) for x in self.moments[e]]
+                for (a, b), i in second.items():
+                    out[e, a, b] = out[e, b, a] = float(Fraction(n * m[i] - m[a] * m[b], n * n))
+        return out
+
+
 class SweepContext:
     """Device-resident context: padded slowness box + pool of travel-time boxes on one GPU."""
 
@@ -655,6 +699,32 @@ class SweepContext:
                                                misfit.ctypes.data, origin.ctypes.data, npicks.ctypes.data,
                                                status.ctypes.data, C.byref(s)), "sweeptt_locate_events")
         return Locations(node, misfit, origin, npicks, status, SweepStats._from(s))
+
+    def misfit_regions(self, picks, levels, sources=None) -> MisfitRegions:
+        """The nodes of every event of picks [E, S] whose misfit is at most levels[e] (float32 [E]; finite and >= 0, or
+        NaN for no region), summarised exactly on the device: count, bounding box, integer moments and origin-time range
+        (include/sweeptt.h, sweeptt_misfit_regions).  The region is exactly misfit_box(picks[e]) <= levels[e]; an event
+        without a pick has an empty one.  Sources as in locate_events."""
+        begin, count = self._source_range(sources, "misfit_regions")
+        p = np.ascontiguousarray(picks, dtype=np.float32)
+        if p.ndim != 2 or p.shape[1] != count:
+            raise SweepError(f"misfit_regions: picks of shape {p.shape}, expected (events, {count})")
+        nev = p.shape[0]
+        lv = np.ascontiguousarray(levels, dtype=np.float32)
+        if lv.shape != (nev,):
+            raise SweepError(f"misfit_regions: levels of shape {lv.shape}, expected ({nev},)")
+        n = np.empty(nev, np.int64)
+        bbox = np.empty((nev, 6), np.int32)
+        moments = np.empty((nev, 9), np.int64)
+        origin = np.empty((nev, 2), np.float64)
+        status = np.empty(nev, np.int32)
+        s = _Stats()
+        _check(self._lib.sweeptt_misfit_regions(self._h, begin, count, p.ctypes.data, nev, lv.ctypes.data, n.ctypes.data,
+                                                bbox.ctypes.data, moments.ctypes.data, origin.ctypes.data,
+                                                status.ctypes.data, C.byref(s)), "sweeptt_misfit_regions")
+        npicks = (~np.isnan(p)).sum(1).astype(np.int32)
+        return MisfitRegions(n, bbox[:, :3].copy(), bbox[:, 3:].copy(), moments, origin[:, 0].copy(),
+                             origin[:, 1].copy(), npicks, status, SweepStats._from(s))
 
     def misfit_box(self, picks, sources=None) -> np.ndarray:
         """The misfit of one event (picks [S], NaN = no pick) at every node: float32[nx, ny, nz], +inf where a picked
@@ -913,6 +983,47 @@ def locate_events(slowness, star, stations, picks, *, delta: float = 10.0, devic
         ctx.set_sources(stations)
         ctx.run()
         return ctx.locate_events(picks)
+
+
+def uncertainty_levels(locations: Locations, sigma, confidence: float = 0.95) -> np.ndarray:
+    """The levels of location_uncertainty: float32(float64(misfit) + sigma^2 * chi2.ppf(confidence, 3)) for the
+    events located OK, NaN for the others and where the best misfit overflowed to +inf; a sum beyond float32 becomes
+    its largest finite value (every node with a finite misfit is then inside)."""
+    from scipy.stats import chi2
+    misfit = np.asarray(locations.misfit, np.float32)
+    sig = np.broadcast_to(np.asarray(sigma, np.float64), misfit.shape)
+    if not (np.isfinite(sig).all() and (sig > 0).all()):
+        raise SweepError("location_uncertainty: sigma must be finite and > 0")
+    if not 0.0 < confidence < 1.0:
+        raise SweepError(f"location_uncertainty: confidence {confidence} is not in (0, 1)")
+    ok = (np.asarray(locations.status) == LOC_OK) & np.isfinite(misfit)
+    with np.errstate(over="ignore"):
+        lv = (misfit.astype(np.float64) + sig * sig * float(chi2.ppf(confidence, 3))).astype(np.float32)
+    lv = np.where(np.isinf(lv), np.finfo(np.float32).max, lv)
+    return np.where(ok, lv, np.float32(np.nan)).astype(np.float32)
+
+
+def location_uncertainty(slowness, star, stations, picks, *, sigma, confidence: float = 0.95, delta: float = 10.0,
+                         device: int | None = None, kernel: int | None = None):
+    """One-shot location with uncertainty: on one context, solve one field per station, locate every event of picks
+    [E, S] (SweepContext.locate_events), then summarise each event's confidence region (SweepContext.misfit_regions)
+    at the level misfit_best + sigma^2 * chi2.ppf(confidence, 3) (uncertainty_levels).  Returns (Locations,
+    MisfitRegions).
+
+    The statistical assumption: the picks are the fields' times at the true node plus a common origin time plus
+    independent Gaussian errors of standard deviation sigma (a scalar or one value per event, finite and > 0, in the
+    fields' units).  Then the misfit, with the origin time profiled out, exceeds its minimum by sigma^2 times a
+    chi-square variable of 3 degrees of freedom (the three coordinates) at the true node, in the linearised limit, and
+    the region is the usual delta-chi-square confidence region at that confidence.  The discretisation of the grid is
+    not part of it: the region is a set of nodes, and a region of one node says the grid is too coarse to resolve
+    the uncertainty, not that there is none."""
+    with SweepContext(device=device, kernel=kernel) as ctx:
+        ctx.set_model(slowness)
+        ctx.set_star(star, delta)
+        ctx.set_sources(stations)
+        ctx.run()
+        loc = ctx.locate_events(picks)
+        return loc, ctx.misfit_regions(picks, uncertainty_levels(loc, sigma, confidence))
 
 
 # ---- file formats -------------------------------------------------------------------------

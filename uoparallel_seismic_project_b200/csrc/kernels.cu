@@ -37,6 +37,7 @@
 //                     updates) with fixed-order sums of squares.
 //   locate / locate_finish / misfit_box  event location: the float64 origin-free least-squares misfit of every
 //                     event at every node from the stations' fields, its argmin and the misfit box of one event.
+//   region            the nodes of every event under a misfit level, summarised by integer sums and extremes.
 //   fill/pad/unpad/init_sources/min_slowness  the device float-box pool's utilities
 //                     (boxsetall/boxput, include/floatbox.h:176-199).
 // One grid over several devices (solver.cu, sweeptt_solve_slabs) runs relax_tiled unchanged on a travel-time box
@@ -1788,7 +1789,8 @@ __global__ void __launch_bounds__(LSQR_THREADS) lsqr_xw_kernel(const LsqrArgs a,
 }
 
 // ---------------------------------------------------------------------------------------
-// event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box; DESIGN §3.10)
+// event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box / sweeptt_misfit_regions;
+// DESIGN §3.10, §3.12)
 // ---------------------------------------------------------------------------------------
 constexpr int LOC_THREADS = 512;
 constexpr unsigned LOC_EXCLUDED = 0x7f800001u;  // key bits of an excluded node: after every float32 misfit, +INF too
@@ -1824,7 +1826,7 @@ __device__ __forceinline__ double loc_div(double a, int k, double rk) {
 }
 
 // The per-node formula of include/sweeptt.h, at NB nodes of one event: the ONE implementation, shared by locate_kernel,
-// misfit_box_kernel and locate_finish_kernel.  tt(s, q) is station s's travel time at node q as a double; ps / po are
+// region_kernel, misfit_box_kernel and locate_finish_kernel.  tt(s, q) is station s's travel time at node q as a double; ps / po are
 // the event's k picks, ascending.  bits[q] = float bits of the misfit, or LOC_EXCLUDED; t0[q] = the origin time.
 template <int NB, class TT>
 __device__ __forceinline__ void event_misfit(const int* __restrict__ ps, const double* __restrict__ po, int k, double rk,
@@ -1881,16 +1883,12 @@ __device__ __forceinline__ void loc_node(const BoxGeom& g, long long i, long lon
   *d = x * g.dstride[0] + y * g.dstride[1] + z * g.dstride[2];
 }
 
-// A CTA owns B = 32*NB consecutive nodes in kernel order (a run along kernel z: coalesced reads), stages the times of
-// every station there once (doubles, [nsta][B]), then its warps take the launch's events in turn: lane l evaluates
-// nodes l, l+32, ... of the run for the warp's event, whose picks are warp-uniform loads.  The warp's smallest key goes
-// to the event with one 64-bit atomicMin (integer min: the result does not depend on the schedule).
+// The staging both grid-search kernels share: a CTA owns B = 32*NB consecutive nodes in kernel order (a run along kernel
+// z: coalesced reads) and stages the times of every station there once (doubles, s_tt [nsta][B]), with each node's
+// padded index (s_p, -1 past the box) and caller FLOATBOX index j(n) (s_j).
 template <int NB>
-__global__ void __launch_bounds__(LOC_THREADS, 1) locate_kernel(const LocateArgs a) {
+__device__ __forceinline__ void loc_stage(const LocateArgs& a, double* s_tt, long long* s_p, unsigned* s_j) {
   constexpr int B = 32 * NB;
-  extern __shared__ double s_tt[];
-  __shared__ long long s_p[B];
-  __shared__ unsigned s_j[B];
   const long long D = (long long)a.g.nx * a.g.ny * a.g.nz;
   const long long n0 = (long long)blockIdx.x * B;
   for (int b = threadIdx.x; b < B; b += blockDim.x) {
@@ -1906,6 +1904,18 @@ __global__ void __launch_bounds__(LOC_THREADS, 1) locate_kernel(const LocateArgs
     s_tt[idx] = p >= 0 ? (double)__ldg(a.tt + s * a.g.vol + p) : CUDART_INF;
   }
   __syncthreads();
+}
+
+// After the staging, the CTA's warps take the launch's events in turn: lane l evaluates nodes l, l+32, ... of the run
+// for the warp's event, whose picks are warp-uniform loads.  The warp's smallest key goes to the event with one 64-bit
+// atomicMin (integer min: the result does not depend on the schedule).
+template <int NB>
+__global__ void __launch_bounds__(LOC_THREADS, 1) locate_kernel(const LocateArgs a) {
+  constexpr int B = 32 * NB;
+  extern __shared__ double s_tt[];
+  __shared__ long long s_p[B];
+  __shared__ unsigned s_j[B];
+  loc_stage<NB>(a, s_tt, s_p, s_j);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   bool live[NB];
   unsigned jn[NB];
@@ -1925,6 +1935,90 @@ __global__ void __launch_bounds__(LOC_THREADS, 1) locate_kernel(const LocateArgs
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
     if (lane == 0 && best != ~0ull) atomicMin(a.key + e, best);
+  }
+}
+
+// Order-preserving map of a double's bits to an unsigned integer (negative values reversed below the positive ones).
+__device__ __forceinline__ unsigned long long loc_order_key(double x) {
+  const unsigned long long b = (unsigned long long)__double_as_longlong(x);
+  return (b >> 63) ? ~b : b | 0x8000000000000000ull;
+}
+
+// The region {n : misfit(n) <= level} of every event of the launch (sweeptt_misfit_regions), summarised exactly: the
+// staging and the formula of locate_kernel, then per event the integer sums, integer extremes and ordered t0 keys of
+// the nodes inside.  A live node is inside when its misfit bits are below r.lim[e] = (level bits) + 1, or never
+// (0) for a NaN level: misfits and levels are >= 0, so their bits order like their values, and LOC_EXCLUDED and +INF
+// rank above every finite level.  Only nodes inside pay for the decoding of j(n) into caller coordinates.  Every
+// result is an integer sum, min or max, so it does not depend on the schedule or the chunking.  Layout per event e:
+// r.sum[10e ..] = count, S0 S1 S2 S00 S11 S22 S01 S02 S12; r.box[6e ..] = min c0, c1, c2, then min ~c0, ~c1, ~c2
+// (unsigned: the maxima reversed, so that one fill of ones is every identity); r.t0[2e ..] = min key, min ~key of
+// loc_order_key(t0); r.reached[e] != 0 when some node is not excluded.
+template <int NB>
+__global__ void __launch_bounds__(LOC_THREADS, 1) region_kernel(const LocateArgs a, const RegionArgs r) {
+  constexpr int B = 32 * NB;
+  extern __shared__ double s_tt[];
+  __shared__ long long s_p[B];
+  __shared__ unsigned s_j[B];
+  loc_stage<NB>(a, s_tt, s_p, s_j);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  bool live[NB];
+  unsigned jn[NB];
+#pragma unroll
+  for (int q = 0; q < NB; ++q) live[q] = s_p[32 * q + lane] >= 0, jn[q] = s_j[32 * q + lane];
+  // caller dimensions: j = (c0*n1 + c1)*n2 + c2, and kernel axis q is caller axis perm[q]
+  int n[3];
+  n[a.g.perm[0]] = a.g.nx; n[a.g.perm[1]] = a.g.ny; n[a.g.perm[2]] = a.g.nz;
+  const unsigned n1 = (unsigned)n[1], n2 = (unsigned)n[2];
+  const LocSmemTT tt{s_tt + lane, B};
+  for (int e = a.e_begin + warp; e < a.e_begin + a.e_count; e += LOC_THREADS / 32) {
+    const int off = a.pick_off[e], k = a.pick_off[e + 1] - off;
+    if (k == 0) continue;
+    unsigned bits[NB];
+    double t0[NB];
+    event_misfit<NB>(a.pick_sta + off, a.pick_obs + off, k, a.pick_rk[e], tt, bits, t0);
+    const unsigned lim = r.lim[e];
+    bool reached = false;
+    long long m[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    unsigned box[6] = {~0u, ~0u, ~0u, ~0u, ~0u, ~0u};
+    unsigned long long tk[2] = {~0ull, ~0ull};
+#pragma unroll
+    for (int q = 0; q < NB; ++q) {
+      if (!live[q]) continue;
+      reached |= bits[q] != LOC_EXCLUDED;
+      if (bits[q] >= lim) continue;
+      const unsigned j = jn[q], row = j / n2;
+      const unsigned c[3] = {row / n1, row % n1, j % n2};
+      const long long c0 = c[0], c1 = c[1], c2 = c[2];
+      m[0] += 1;
+      m[1] += c0; m[2] += c1; m[3] += c2;
+      m[4] += c0 * c0; m[5] += c1 * c1; m[6] += c2 * c2;
+      m[7] += c0 * c1; m[8] += c0 * c2; m[9] += c1 * c2;
+#pragma unroll
+      for (int i = 0; i < 3; ++i) box[i] = min(box[i], c[i]), box[3 + i] = min(box[3 + i], ~c[i]);
+      const unsigned long long key = loc_order_key(t0[q]);
+      tk[0] = min(tk[0], key);
+      tk[1] = min(tk[1], ~key);
+    }
+    if (__any_sync(0xffffffffu, reached) && lane == 0) atomicOr(r.reached + e, 1u);
+    if (!__any_sync(0xffffffffu, m[0] != 0)) continue;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+      for (int i = 0; i < 10; ++i) m[i] += __shfl_xor_sync(0xffffffffu, m[i], o);
+#pragma unroll
+      for (int i = 0; i < 6; ++i) box[i] = min(box[i], __shfl_xor_sync(0xffffffffu, box[i], o));
+#pragma unroll
+      for (int i = 0; i < 2; ++i) tk[i] = min(tk[i], __shfl_xor_sync(0xffffffffu, tk[i], o));
+    }
+    if (lane == 0) {
+      unsigned long long* sum = r.sum + 10 * (size_t)e;
+#pragma unroll
+      for (int i = 0; i < 10; ++i) atomicAdd(sum + i, (unsigned long long)m[i]);
+#pragma unroll
+      for (int i = 0; i < 6; ++i) atomicMin(r.box + 6 * (size_t)e + i, box[i]);
+#pragma unroll
+      for (int i = 0; i < 2; ++i) atomicMin(r.t0 + 2 * (size_t)e + i, tk[i]);
+    }
   }
 }
 
@@ -2499,16 +2593,24 @@ template <int NB>
 static size_t locate_smem(int nsta) { return (size_t)nsta * 32 * NB * sizeof(double); }
 
 template <int NB>
-static bool locate_fits(int nsta, int optin) {
+static bool locate_fits(const void* kernel, int nsta, int optin) {
   cudaFuncAttributes fa{};  // the static node tables take their share besides the staged times
-  return cudaFuncGetAttributes(&fa, locate_kernel<NB>) == cudaSuccess &&
-         locate_smem<NB>(nsta) + fa.sharedSizeBytes <= (size_t)optin;
+  return cudaFuncGetAttributes(&fa, kernel) == cudaSuccess && locate_smem<NB>(nsta) + fa.sharedSizeBytes <= (size_t)optin;
 }
 
 int locate_nodes_per_thread(int nsta, int device) {
   int optin = 0;
   if (cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device) != cudaSuccess) return 0;
-  return locate_fits<4>(nsta, optin) ? 4 : locate_fits<2>(nsta, optin) ? 2 : locate_fits<1>(nsta, optin) ? 1 : 0;
+  return locate_fits<4>((const void*)locate_kernel<4>, nsta, optin)   ? 4
+         : locate_fits<2>((const void*)locate_kernel<2>, nsta, optin) ? 2
+         : locate_fits<1>((const void*)locate_kernel<1>, nsta, optin) ? 1 : 0;
+}
+int region_nodes_per_thread(int nsta, int device) {
+  int optin = 0;
+  if (cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device) != cudaSuccess) return 0;
+  return locate_fits<4>((const void*)region_kernel<4>, nsta, optin)   ? 4
+         : locate_fits<2>((const void*)region_kernel<2>, nsta, optin) ? 2
+         : locate_fits<1>((const void*)region_kernel<1>, nsta, optin) ? 1 : 0;
 }
 
 template <int NB>
@@ -2526,6 +2628,25 @@ cudaError_t launch_locate(const LocateArgs& a, int nodes_per_thread, cudaStream_
     case 4: return launch_locate_nb<4>(a, stream);
     case 2: return launch_locate_nb<2>(a, stream);
     case 1: return launch_locate_nb<1>(a, stream);
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+template <int NB>
+static cudaError_t launch_regions_nb(const LocateArgs& a, const RegionArgs& r, cudaStream_t stream) {
+  const size_t smem = locate_smem<NB>(a.nsta);
+  cudaError_t e = cudaFuncSetAttribute(region_kernel<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  const long long D = (long long)a.g.nx * a.g.ny * a.g.nz;
+  region_kernel<NB><<<(unsigned)((D + 32 * NB - 1) / (32 * NB)), LOC_THREADS, smem, stream>>>(a, r);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_regions(const LocateArgs& a, const RegionArgs& r, int nodes_per_thread, cudaStream_t stream) {
+  switch (nodes_per_thread) {
+    case 4: return launch_regions_nb<4>(a, r, stream);
+    case 2: return launch_regions_nb<2>(a, r, stream);
+    case 1: return launch_regions_nb<1>(a, r, stream);
     default: return cudaErrorInvalidValue;
   }
 }

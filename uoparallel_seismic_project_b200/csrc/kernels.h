@@ -194,7 +194,7 @@ cudaError_t launch_lsqr_v(const LsqrArgs& a, double beta, cudaStream_t stream, i
 cudaError_t launch_lsqr_scale(double* p, long long n, double s, cudaStream_t stream);
 cudaError_t launch_lsqr_xw(const LsqrArgs& a, double t1, double t2, double inv_rho, cudaStream_t stream, int* launches);
 
-// Event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box).  Event e's picks are entries
+// Event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box / sweeptt_misfit_regions).  Event e's picks are entries
 // pick_off[e] .. pick_off[e+1] of pick_sta / pick_obs, in increasing station order (NaN picks left out).
 struct LocateArgs {
   BoxGeom g;
@@ -212,10 +212,21 @@ struct LocateArgs {
   int* npicks;
   int* status;
 };
+// The region slots of sweeptt_misfit_regions (region_kernel, layout in kernels.cu), per event e at [e] or [e * width]:
+struct RegionArgs {
+  const unsigned* lim;             // level bits + 1 (0: NaN level, no node)
+  unsigned long long* sum;         // [10]: count and the 9 moments, zeroed first
+  unsigned* box;                   // [6]: min c, min ~c, filled with ones first
+  unsigned long long* t0;          // [2]: min key, min ~key of the ordered t0, filled with ones first
+  unsigned* reached;               // some node not excluded, zeroed first
+};
 // Nodes per thread of the location kernel (4, 2 or 1: a CTA stages the times of nsta stations at 32 * that many
-// nodes in shared memory), or 0 when not even 32 nodes fit.
+// nodes in shared memory), or 0 when not even 32 nodes fit; the same for the region kernel, by its own attributes.
 int locate_nodes_per_thread(int nsta, int device);
+int region_nodes_per_thread(int nsta, int device);
 cudaError_t launch_locate(const LocateArgs& a, int nodes_per_thread, cudaStream_t stream);
+// Events [e_begin, e_begin + e_count): the region summaries of sweeptt_misfit_regions.
+cudaError_t launch_regions(const LocateArgs& a, const RegionArgs& r, int nodes_per_thread, cudaStream_t stream);
 // Decodes every key: best node, and its misfit and t0 recomputed with the location kernel's formula.
 cudaError_t launch_locate_finish(const LocateArgs& a, int nev, cudaStream_t stream);
 // Event 0's misfit at every node into the dense caller-axis box.

@@ -2543,15 +2543,19 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
 // event location (include/sweeptt.h, sweeptt_locate_events / sweeptt_misfit_box)
 // ---------------------------------------------------------------------------------------
 
-// Checks shared by both location calls; then the picks of nev events (NaN left out) go to the device as a CSR with
-// RN(1/k) per event, and *a describes them, the fields of the call's stations and the result slots.  Every refusal
-// comes before the first allocation.  nodes_per_thread (may be NULL): the location kernel's shape for these stations.
+// Checks shared by the location calls; then the picks of nev events (NaN left out) go to the device as a CSR with
+// RN(1/k) per event, and *a describes them, the fields of the call's stations and the result slots.  With levels
+// and r (sweeptt_misfit_regions), also the levels' and the moment bound's checks, the region kernel's shape, and the
+// region slots after the location slots, initialised.  Every refusal comes before the first allocation.
+// nodes_per_thread (may be NULL): the grid-search kernel's shape for these stations.
 static int locate_prepare(sweeptt_ctx* c, ConstLease* lease, const char* who, int source_begin, int source_count,
-                          const float* picks, int nev, LocateArgs* a, int* nodes_per_thread, sweeptt_stats* stats) {
+                          const float* picks, int nev, LocateArgs* a, int* nodes_per_thread, sweeptt_stats* stats,
+                          const float* levels = nullptr, RegionArgs* r = nullptr) {
   if (!ready(c, lease)) return 0;
   if (stats) std::memset(stats, 0, sizeof *stats);
   if (!check_source_range(c, who, source_begin, source_count)) return 0;
-  if (nodes_per_thread && (*nodes_per_thread = locate_nodes_per_thread(source_count, c->device)) == 0)
+  if (nodes_per_thread &&
+      (*nodes_per_thread = (levels ? region_nodes_per_thread : locate_nodes_per_thread)(source_count, c->device)) == 0)
     return fail("%s: %d stations do not fit the location kernel's shared memory (8 bytes per station and node, 32 nodes)",
                 who, source_count);
   if (nev < 0) return fail("%s: nev = %d is negative", who, nev);
@@ -2559,6 +2563,25 @@ static int locate_prepare(sweeptt_ctx* c, ConstLease* lease, const char* who, in
   const BoxGeom& g = c->g;
   if ((unsigned long long)g.nx * g.ny * g.nz > (1ull << 32))
     return fail("%s: %d x %d x %d nodes exceed 2^32, the argmin key holds a node index in 32 bits", who, g.nx, g.ny, g.nz);
+  std::vector<unsigned> lim;
+  if (levels) {
+    // every second moment is at most D * max_a (n_a - 1)^2; it must fit int64
+    const unsigned long long D = (unsigned long long)g.nx * g.ny * g.nz;
+    const unsigned long long m = (unsigned long long)std::max({g.nx, g.ny, g.nz}) - 1;
+    if (m * m > (unsigned long long)INT64_MAX / D)
+      return fail("%s: %d x %d x %d nodes: the region moments (up to D * (n - 1)^2 for the longest axis n) overflow "
+                  "int64", who, g.nx, g.ny, g.nz);
+    lim.resize((size_t)nev);
+    for (int e = 0; e < nev; ++e) {
+      const float v = levels[e];
+      if (std::isnan(v)) { lim[e] = 0; continue; }   // no region
+      if (!(v >= 0.f) || std::isinf(v))
+        return fail("%s: level of event %d is %g (a level is finite and >= 0, or NaN for no region)", who, e, (double)v);
+      const float pos = v == 0.f ? 0.f : v;          // -0.0 is +0: its bits would let every node in
+      std::memcpy(&lim[e], &pos, 4);
+      lim[e] += 1;
+    }
+  }
   std::vector<int> off(1, 0), sta;
   std::vector<double> obs, rk;
   off.reserve((size_t)nev + 1);
@@ -2579,11 +2602,14 @@ static int locate_prepare(sweeptt_ctx* c, ConstLease* lease, const char* who, in
   }
   const size_t np = sta.size(), n = (size_t)nev;
   auto up16 = [](size_t b) { return (b + 15) / 16 * 16; };
-  const size_t part[10] = {up16(4 * (n + 1)), up16(4 * np), up16(8 * np), up16(8 * n), up16(8 * n),
-                           up16(12 * n),      up16(4 * n),  up16(8 * n),  up16(4 * n), up16(4 * n)};
-  size_t at[11] = {0};
-  for (int i = 0; i < 10; ++i) at[i + 1] = at[i] + part[i];
-  if (!ensure_dev(c, &c->d_loc, &c->loc_cap, at[10])) return 0;
+  // location slots, then (levels only) lim, sum, reached (zeroed), t0, box (ones) of RegionArgs
+  const size_t part[15] = {up16(4 * (n + 1)), up16(4 * np), up16(8 * np), up16(8 * n), up16(8 * n),
+                           up16(12 * n),      up16(4 * n),  up16(8 * n),  up16(4 * n), up16(4 * n),
+                           up16(4 * n),       up16(80 * n), up16(4 * n),  up16(16 * n), up16(24 * n)};
+  const int nparts = levels ? 15 : 10;
+  size_t at[16] = {0};
+  for (int i = 0; i < nparts; ++i) at[i + 1] = at[i] + part[i];
+  if (!ensure_dev(c, &c->d_loc, &c->loc_cap, at[nparts])) return 0;
   unsigned char* b = c->d_loc;
   *a = LocateArgs{};
   a->g = g;
@@ -2606,12 +2632,24 @@ static int locate_prepare(sweeptt_ctx* c, ConstLease* lease, const char* who, in
     CK(cudaMemcpyAsync(b + at[2], obs.data(), 8 * np, cudaMemcpyHostToDevice, c->stream));
   }
   if (n) CK(cudaMemcpyAsync(b + at[3], rk.data(), 8 * n, cudaMemcpyHostToDevice, c->stream));
+  if (levels) {
+    r->lim = reinterpret_cast<const unsigned*>(b + at[10]);
+    r->sum = reinterpret_cast<unsigned long long*>(b + at[11]);
+    r->reached = reinterpret_cast<unsigned*>(b + at[12]);
+    r->t0 = reinterpret_cast<unsigned long long*>(b + at[13]);
+    r->box = reinterpret_cast<unsigned*>(b + at[14]);
+    if (n) {
+      CK(cudaMemcpyAsync(b + at[10], lim.data(), 4 * n, cudaMemcpyHostToDevice, c->stream));
+      CK(cudaMemsetAsync(b + at[11], 0, at[13] - at[11], c->stream));
+      CK(cudaMemsetAsync(b + at[13], 0xff, at[15] - at[13], c->stream));
+    }
+  }
   CK(cudaStreamSynchronize(c->stream));
   if (stats) {
     stats->struct_size = (int)sizeof *stats;
     stats->devices_used = 1;
     stats->h2d_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    stats->h2d_bytes = (long long)(4 * (n + 1) + 12 * np + 8 * n);
+    stats->h2d_bytes = (long long)(4 * (n + 1) + 12 * np + 8 * n + (levels ? 4 * n : 0));
   }
   return 1;
 }
@@ -2691,6 +2729,79 @@ extern "C" int sweeptt_misfit_box(sweeptt_ctx* c, int source_begin, int source_c
     stats->kernel_launches = 1;
     stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
     stats->d2h_bytes = (long long)dense * 4;
+  }
+  return 1;
+}
+
+extern "C" int sweeptt_misfit_regions(sweeptt_ctx* c, int source_begin, int source_count, const float* picks, int nev,
+                                      const float* levels, int64_t* count_out, int32_t* bbox_out, int64_t* moments_out,
+                                      double* origin_range_out, int32_t* status_out, sweeptt_stats* stats) {
+  static const char* who = "sweeptt_misfit_regions";
+  if (!count_out || !status_out) return fail("%s: count_out and status_out are required", who);
+  if (nev > 0 && !levels) return fail("%s: null levels", who);
+  ConstLease lease;
+  LocateArgs a;
+  RegionArgs r{};
+  int nb = 0;
+  static const float no_levels[1] = {0.f};   // nev = 0 reads no level, but still takes the region checks
+  if (!locate_prepare(c, &lease, who, source_begin, source_count, picks, nev, &a, &nb, stats, levels ? levels : no_levels,
+                      &r))
+    return 0;
+  if (nev == 0) return 1;
+  const int chunk = locate_chunk();
+  long long launches = 0;
+  CK(cudaEventRecord(c->ev0, c->stream));
+  for (int e0 = 0; e0 < nev; e0 += chunk) {
+    a.e_begin = e0;
+    a.e_count = std::min(chunk, nev - e0);
+    CK(launch_regions(a, r, nb, c->stream));
+    ++launches;
+  }
+  CK(cudaEventRecord(c->ev1, c->stream));
+  CK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+
+  const auto t_copy = std::chrono::steady_clock::now();
+  const size_t n = (size_t)nev;
+  std::vector<unsigned long long> sum(10 * n), tk(2 * n);
+  std::vector<unsigned> box(6 * n), reached(n);
+  CK(cudaMemcpyAsync(sum.data(), r.sum, 80 * n, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(reached.data(), r.reached, 4 * n, cudaMemcpyDeviceToHost, c->stream));
+  long long bytes = 84 * (long long)n;
+  if (bbox_out) { CK(cudaMemcpyAsync(box.data(), r.box, 24 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 24 * n; }
+  if (origin_range_out) { CK(cudaMemcpyAsync(tk.data(), r.t0, 16 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 16 * n; }
+  CK(cudaStreamSynchronize(c->stream));
+  const double nan = std::numeric_limits<double>::quiet_NaN();
+  auto from_key = [](unsigned long long k) {   // inverse of kernels.cu's loc_order_key
+    const unsigned long long b = (k >> 63) ? k & ~0x8000000000000000ull : ~k;
+    double x;
+    std::memcpy(&x, &b, 8);
+    return x;
+  };
+  for (size_t e = 0; e < n; ++e) {
+    int k = 0;
+    for (int s = 0; s < source_count; ++s) k += !std::isnan(picks[e * source_count + s]);
+    status_out[e] = k == 0 ? SWEEPTT_LOC_NO_PICKS : reached[e] ? SWEEPTT_LOC_OK : SWEEPTT_LOC_UNREACHED;
+    const unsigned long long cnt = sum[10 * e];
+    count_out[e] = (int64_t)cnt;
+    if (moments_out)
+      for (int i = 0; i < 9; ++i) moments_out[9 * e + i] = (int64_t)sum[10 * e + 1 + i];
+    if (bbox_out)
+      for (int i = 0; i < 3; ++i) {
+        bbox_out[6 * e + i] = cnt ? (int32_t)box[6 * e + i] : -1;
+        bbox_out[6 * e + 3 + i] = cnt ? (int32_t)~box[6 * e + 3 + i] : -1;
+      }
+    if (origin_range_out) {
+      origin_range_out[2 * e] = cnt ? from_key(tk[2 * e]) : nan;
+      origin_range_out[2 * e + 1] = cnt ? from_key(~tk[2 * e + 1]) : nan;
+    }
+  }
+  if (stats) {
+    stats->solve_ms = ms;
+    stats->kernel_launches = launches;
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes = bytes;
   }
   return 1;
 }
