@@ -183,7 +183,9 @@ int sweeptt_set_stream(sweeptt_ctx *ctx, void *cuda_stream);
  * with a negative or NaN value (-0.0 is zero), and a model whose kernel axis order the context's
  * star cannot follow (SWEEPTT_KERNEL_TILED: the star, re-ordered, exceeds the tiled kernel's
  * halo); a refused model leaves the context as it was: model, dimensions, star, sources and
- * travel-time boxes. */
+ * travel-time boxes.  An accepted model keeps the start points only when its padded size and
+ * kernel axis order are the previous model's and every start point lies inside it; otherwise
+ * sweeptt_set_sources must be called again before sweeptt_run. */
 int sweeptt_set_model(sweeptt_ctx *ctx, const float *slowness, int nx, int ny, int nz);
 /* Star tables into __constant__ memory (cuda/...cu:74,285).  Refuses a star in which a used
  * entry (l < starsize-1, or < star_used; the self offset (0,0,0) excepted) has a negative, NaN

@@ -586,6 +586,12 @@ extern "C" int sweeptt_set_model(sweeptt_ctx* c, const float* slowness, int nx, 
   }
   c->have_model = true;
   if (perm_changed) c->have_sources = false;
+  // start points kept from the previous model (same axis order) must lie inside this one: a box that shrinks within
+  // the same padded size would otherwise leave a start in the +INF padding and every travel time infinite
+  for (int s = 0; c->have_sources && !c->allow_outside_sources && s < c->nsrc; ++s) {
+    const int* p = &c->src_xyz[3 * s];
+    if (p[0] >= g.nx || p[1] >= g.ny || p[2] >= g.nz) c->have_sources = false;
+  }
   if (rebuild_star) return commit_star(c, sb);
   if (c->have_star && !build_tile_pulls(c)) return 0;
   return 1;
