@@ -496,6 +496,57 @@ int sweeptt_misfit_regions(sweeptt_ctx *ctx, int source_begin, int source_count,
                            const float *levels, int64_t *count_out, int32_t *bbox_out, int64_t *moments_out,
                            double *origin_range_out, int32_t *status_out, sweeptt_stats *stats);
 
+/* ---- sub-node refinement: trilinear station times on a lattice around each located node ---------------------------
+ *
+ * Lattice.  subdiv = f, 1 <= f <= 64.  A lattice point is an integer triple u in caller axes at position u / f in node
+ * units, inside the box: 0 <= u_a <= f*(n_a - 1).  Event e has a centre node c_e (caller axes, inside the box); its
+ * CUBE is every lattice point with |u_a - f*c_a| <= f on each axis, clipped to the box: at most (2f+1)^3 points, the
+ * eight cells around the node.  With f = 1 the cube is the up-to-27 nodes around c_e.
+ *
+ * Time at a lattice point, for station s: per axis a, i_a = u_a div f, r_a = u_a mod f, w_a = W[r_a] with
+ * W[r] = RN((double)r / (double)f) computed on the host.  t(b) = (double) of station s's float32 time at node i + b,
+ * b in {0,1}^3; a corner with b_a = 1 is read only when r_a != 0, so no node outside the box is read and an axis of one
+ * node works.  Interpolate along caller axis 2 first, then axis 1, then axis 0; on each axis with r_a != 0,
+ * lerp(p, q, w) = fl(p + fl(w * fl(q - p))) in IEEE float64, no fused multiply-add; an axis with r_a = 0 keeps its
+ * b_a = 0 value.  If any corner read is +INF, the time is +INF.  The result does not depend on the axis permutation,
+ * the kernel or the schedule, and a lattice point that is a node (r = 0) gets that node's time exactly.
+ *
+ * Misfit, best point, status: the per-node formula of sweeptt_locate_events with tt_s(n) replaced by the time above
+ * (same picks, exclusion, float64 two-pass t0 and misfit, rounding to float32).  The best point of e is the smallest
+ * misfit in its cube, ties to the lexicographically smallest u; a point whose misfit overflows to +INF ranks before
+ * every excluded point.  Status as sweeptt_locate_events, over the cube: SWEEPTT_LOC_OK, NO_PICKS when k_e = 0,
+ * UNREACHED when every point of the cube is excluded; when not OK: point (-1,-1,-1), misfit +INF, origin NaN.
+ * Two facts follow:
+ *   - a point's misfit depends only on the point, never on which cube contains it;
+ *   - when c_e is the node from sweeptt_locate_events, the refined misfit is <= the node's misfit (the node is in the
+ *     cube, with the same bits).  With f = 1 the result is that node, its misfit and its origin time, bit for bit.
+ *
+ * Stations, picks, stats, SWEEPTT_LOCATE_CHUNK and the refusals are those of sweeptt_locate_events, except the 2^32-node
+ * limit, which neither call has (a key holds a cube-local index).  Further refusals, each before anything runs and
+ * leaving the context as it was: centres NULL with nev > 0; a centre outside the box (with the event's index); subdiv
+ * outside [1, 64].  The station limit is the location call's (904 on a B200): the refinement kernels stage 27 nodes of
+ * every station as doubles (195,264 bytes at 904 stations), which fits next to their static shared memory; a count
+ * the location call accepts that did not fit would be refused with "shared memory".  Scratch is the location calls'
+ * grow-only buffer.  SWEEPTT_REFINE_POINTS (lattice points of a cube per CTA, default 1024) splits each cube over
+ * CTAs; the result does not depend on it. */
+
+/* point_out [nev*3] (u, caller axes) and status_out [nev] are required; misfit_out, origin_out, npicks_out [nev] may
+ * be NULL. */
+int sweeptt_refine_events(sweeptt_ctx *ctx, int source_begin, int source_count, const float *picks, int nev,
+                          const struct START *centres, int subdiv, int64_t *point_out, float *misfit_out,
+                          double *origin_out, int32_t *npicks_out, int32_t *status_out, sweeptt_stats *stats);
+
+/* sweeptt_misfit_regions over the cube: R_e = { u in cube : misfit(u) <= levels[e] }, with that call's rules for levels
+ * (NaN: empty; -0.0 is +0; +-INF and negative levels refused with the event's index), excluded and overflowing points
+ * (never inside), and empty regions (bbox -1, moments 0, origin range NaN; -1 is never a lattice coordinate).
+ * bbox_out [nev*6]: lo u, hi u, inclusive.  moments_out [nev*9]: S0 S1 S2 S00 S11 S22 S01 S02 S12 about the centre,
+ * over t = u - f*c_e; |t_a| <= 64 and a cube holds <= 129^3 points, so they fit int64 for every box and this call has
+ * no moment bound.  origin_range_out [nev*2], status_out [nev] as there.  count_out and status_out are required. */
+int sweeptt_refine_regions(sweeptt_ctx *ctx, int source_begin, int source_count, const float *picks, int nev,
+                           const struct START *centres, int subdiv, const float *levels, int64_t *count_out,
+                           int64_t *bbox_out, int64_t *moments_out, double *origin_range_out, int32_t *status_out,
+                           sweeptt_stats *stats);
+
 /* In-bounds pull evaluations of one full round of one source (analytic). */
 long long sweeptt_relaxations_per_round(sweeptt_ctx *ctx);
 /* Bytes of device memory currently held by the context's pool. */

@@ -18,6 +18,8 @@ from .api import (  # noqa: F401
     MisfitGradient,
     MisfitRegions,
     RayProjection,
+    RefinedLocations,
+    RefinedRegions,
     RaySet,
     Rays,
     START,
@@ -32,6 +34,9 @@ from .api import (  # noqa: F401
     locate_events,
     location_uncertainty,
     make_star,
+    recentre,
+    refine_located,
+    refine_locations,
     solve,
     solve_slabs,
     solve_slabs_vbox,

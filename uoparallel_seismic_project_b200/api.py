@@ -108,7 +108,7 @@ _EXPORTS = [
     "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject",
     "sweeptt_rayset_freeze", "sweeptt_rayset_destroy", "sweeptt_rayset_bytes", "sweeptt_rayset_table",
     "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_rayset_lsqr",
-    "sweeptt_locate_events", "sweeptt_misfit_regions",
+    "sweeptt_locate_events", "sweeptt_misfit_regions", "sweeptt_refine_events", "sweeptt_refine_regions",
     "sweeptt_misfit_box", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_debug_model_stats", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
     "sweeptt_vbox_load", "sweeptt_vbox_store", "sweeptt_vbox_load_subset", "sweeptt_text_load",
@@ -178,6 +178,11 @@ def load_library() -> C.CDLL:
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_misfit_regions.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
+    lib.sweeptt_refine_events.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
+    lib.sweeptt_refine_regions.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.POINTER(_Stats)]
     lib.sweeptt_misfit_box.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_relaxations_per_round.argtypes = [C.c_void_p]
     lib.sweeptt_relaxations_per_round.restype = C.c_longlong
@@ -489,6 +494,102 @@ class MisfitRegions:
         return out
 
 
+@dataclass
+class RefinedLocations:
+    """Events refined below the grid spacing (SweepContext.refine_events, include/sweeptt.h sweeptt_refine_events):
+    point[e] is the lattice point u (caller axes, position u / subdiv in node units) of smallest misfit in the cube
+    |u - subdiv * centre[e]| <= subdiv around centre[e], the stations' times interpolated trilinearly; ties to the
+    lexicographically smallest u.  misfit, origin_time, npicks and status as in Locations, over the cube; when the
+    status is not LOC_OK, point is (-1, -1, -1).  dims is the box (caller axes); moves[e] (refine_locations only) the
+    times the event's cube was recentred."""
+    point: np.ndarray        # int64[E, 3]
+    subdiv: int
+    centre: np.ndarray       # int32[E, 3]
+    misfit: np.ndarray       # float32[E]
+    origin_time: np.ndarray  # float64[E]
+    npicks: np.ndarray       # int32[E]
+    status: np.ndarray       # int32[E]
+    stats: SweepStats
+    dims: tuple = None
+    moves: np.ndarray = None  # int32[E]
+
+    @property
+    def position(self) -> np.ndarray:
+        """float64 [E, 3]: point / subdiv, in node units; NaN where the status is not LOC_OK."""
+        pos = np.asarray(self.point, np.float64) / self.subdiv
+        pos[np.asarray(self.status) != LOC_OK] = np.nan
+        return pos
+
+    @property
+    def on_edge(self) -> np.ndarray:
+        """bool [E]: LOC_OK events whose best point lies on a face of the cube that is interior to the box
+        (|u_a - f c_a| = f and 0 < u_a < f (n_a - 1) on some axis a): the minimum may lie beyond the cube."""
+        f = self.subdiv
+        u = np.asarray(self.point, np.int64)
+        t = u - f * np.asarray(self.centre, np.int64)
+        top = f * (np.asarray(self.dims, np.int64) - 1)
+        face = (np.abs(t) == f) & (u > 0) & (u < top)
+        return face.any(1) & (np.asarray(self.status) == LOC_OK)
+
+
+@dataclass
+class RefinedRegions:
+    """The region R_e = {u in cube_e : misfit_e(u) <= level_e} of every event, over the lattice of
+    SweepContext.refine_regions (include/sweeptt.h sweeptt_refine_regions), summarised exactly.  count[e] = |R_e|;
+    lo[e] / hi[e] the inclusive bounding box in lattice coordinates u (-1 when empty); moments[e] = S0 S1 S2 S00 S11 S22
+    S01 S02 S12, the integer sums of t_a and t_a*t_b over t = u - subdiv * centre[e] in R_e; origin_min / origin_max
+    the extremes of the origin time over R_e (NaN when empty); npicks and status as in RefinedLocations."""
+    count: np.ndarray        # int64[E]
+    lo: np.ndarray           # int64[E, 3]
+    hi: np.ndarray           # int64[E, 3]
+    moments: np.ndarray      # int64[E, 9]
+    origin_min: np.ndarray   # float64[E]
+    origin_max: np.ndarray   # float64[E]
+    centre: np.ndarray       # int32[E, 3]
+    subdiv: int
+    npicks: np.ndarray       # int32[E]
+    status: np.ndarray       # int32[E]
+    stats: SweepStats = None
+    dims: tuple = None
+
+    def mean(self) -> np.ndarray:
+        """float64 [E, 3]: the mean position of each region in node units, centre + S_a / (n f), each value the exact
+        quotient rounded once; NaN where the region is empty."""
+        from fractions import Fraction
+        out = np.full((len(self.count), 3), np.nan)
+        f = int(self.subdiv)
+        for e, n in enumerate(self.count.tolist()):
+            if n:
+                for a in range(3):
+                    out[e, a] = float(int(self.centre[e, a]) + Fraction(int(self.moments[e, a]), n * f))
+        return out
+
+    def covariance(self) -> np.ndarray:
+        """float64 [E, 3, 3]: the population covariance of each region's positions in node^2 units,
+        (n*S_ab - S_a*S_b) / (n f)^2 computed exactly and rounded once; NaN where the region is empty."""
+        from fractions import Fraction
+        out = np.full((len(self.count), 3, 3), np.nan)
+        f = int(self.subdiv)
+        second = {(0, 0): 3, (1, 1): 4, (2, 2): 5, (0, 1): 6, (0, 2): 7, (1, 2): 8}
+        for e, n in enumerate(self.count.tolist()):
+            if n:
+                m = [int(x) for x in self.moments[e]]
+                for (a, b), i in second.items():
+                    out[e, a, b] = out[e, b, a] = float(Fraction(n * m[i] - m[a] * m[b], n * n * f * f))
+        return out
+
+    @property
+    def truncated(self) -> np.ndarray:
+        """bool [E]: the region reaches a face of its cube that is interior to the box, so the level set may extend
+        beyond the cube."""
+        f = self.subdiv
+        c = f * np.asarray(self.centre, np.int64)
+        top = f * (np.asarray(self.dims, np.int64) - 1)
+        lo, hi = np.asarray(self.lo, np.int64), np.asarray(self.hi, np.int64)
+        face = ((lo == c - f) & (lo > 0)) | ((hi == c + f) & (hi < top))
+        return face.any(1) & (np.asarray(self.count) > 0)
+
+
 class SweepContext:
     """Device-resident context: padded slowness box + pool of travel-time boxes on one GPU."""
 
@@ -725,6 +826,63 @@ class SweepContext:
         npicks = (~np.isnan(p)).sum(1).astype(np.int32)
         return MisfitRegions(n, bbox[:, :3].copy(), bbox[:, 3:].copy(), moments, origin[:, 0].copy(),
                              origin[:, 1].copy(), npicks, status, SweepStats._from(s))
+
+    def _refine_args(self, picks, centres, subdiv, sources, who):
+        begin, count = self._source_range(sources, who)
+        p = np.ascontiguousarray(picks, dtype=np.float32)
+        if p.ndim != 2 or p.shape[1] != count:
+            raise SweepError(f"{who}: picks of shape {p.shape}, expected (events, {count})")
+        c = np.ascontiguousarray(centres, dtype=np.int32)
+        if c.shape != (p.shape[0], 3):
+            raise SweepError(f"{who}: centres of shape {c.shape}, expected ({p.shape[0]}, 3)")
+        if self.dims is None:
+            raise SweepError(f"{who}: the context needs a model first")
+        return begin, count, p, c, int(subdiv)
+
+    def refine_events(self, picks, centres, subdiv: int, sources=None) -> RefinedLocations:
+        """Refines every event of picks [E, S] below the grid spacing, on the device (include/sweeptt.h,
+        sweeptt_refine_events): the best lattice point, at 1/subdiv of a node (1 <= subdiv <= 64), in the cube of
+        +-1 node around centres[e] (int [E, 3], caller axes, inside the box), with the stations' times interpolated
+        trilinearly.  With centres from locate_events, the refined misfit is never above the located one; with
+        subdiv = 1 the result is that node.  Sources as in locate_events."""
+        begin, count, p, c, f = self._refine_args(picks, centres, subdiv, sources, "refine_events")
+        nev = p.shape[0]
+        point = np.empty((nev, 3), np.int64)
+        misfit = np.empty(nev, np.float32)
+        origin = np.empty(nev, np.float64)
+        npicks = np.empty(nev, np.int32)
+        status = np.empty(nev, np.int32)
+        s = _Stats()
+        _check(self._lib.sweeptt_refine_events(self._h, begin, count, p.ctypes.data, nev, c.ctypes.data, f,
+                                               point.ctypes.data, misfit.ctypes.data, origin.ctypes.data,
+                                               npicks.ctypes.data, status.ctypes.data, C.byref(s)),
+               "sweeptt_refine_events")
+        return RefinedLocations(point, f, c.copy(), misfit, origin, npicks, status, SweepStats._from(s),
+                                tuple(self.dims))
+
+    def refine_regions(self, picks, centres, subdiv: int, levels, sources=None) -> RefinedRegions:
+        """The lattice points of every event's cube (as refine_events) whose misfit is at most levels[e] (float32 [E];
+        finite and >= 0, or NaN for no region), summarised exactly on the device (include/sweeptt.h,
+        sweeptt_refine_regions).  With subdiv = 1 the region is misfit_box(picks[e]) <= levels[e] restricted to the
+        27 nodes around the centre."""
+        begin, count, p, c, f = self._refine_args(picks, centres, subdiv, sources, "refine_regions")
+        nev = p.shape[0]
+        lv = np.ascontiguousarray(levels, dtype=np.float32)
+        if lv.shape != (nev,):
+            raise SweepError(f"refine_regions: levels of shape {lv.shape}, expected ({nev},)")
+        n = np.empty(nev, np.int64)
+        bbox = np.empty((nev, 6), np.int64)
+        moments = np.empty((nev, 9), np.int64)
+        origin = np.empty((nev, 2), np.float64)
+        status = np.empty(nev, np.int32)
+        s = _Stats()
+        _check(self._lib.sweeptt_refine_regions(self._h, begin, count, p.ctypes.data, nev, c.ctypes.data, f,
+                                                lv.ctypes.data, n.ctypes.data, bbox.ctypes.data, moments.ctypes.data,
+                                                origin.ctypes.data, status.ctypes.data, C.byref(s)),
+               "sweeptt_refine_regions")
+        npicks = (~np.isnan(p)).sum(1).astype(np.int32)
+        return RefinedRegions(n, bbox[:, :3].copy(), bbox[:, 3:].copy(), moments, origin[:, 0].copy(),
+                              origin[:, 1].copy(), c.copy(), f, npicks, status, SweepStats._from(s), tuple(self.dims))
 
     def misfit_box(self, picks, sources=None) -> np.ndarray:
         """The misfit of one event (picks [S], NaN = no pick) at every node: float32[nx, ny, nz], +inf where a picked
@@ -1024,6 +1182,78 @@ def location_uncertainty(slowness, star, stations, picks, *, sigma, confidence: 
         ctx.run()
         loc = ctx.locate_events(picks)
         return loc, ctx.misfit_regions(picks, uncertainty_levels(loc, sigma, confidence))
+
+
+def recentre(refined: RefinedLocations) -> np.ndarray:
+    """int32 [E, 3]: the node nearest each event's best point, c'_a = (2 u_a + f) div (2 f) clipped to the box (the
+    centre of refine_locations' next cube, which holds the old best point at |u_a - f c'_a| <= f / 2)."""
+    f = refined.subdiv
+    u = np.asarray(refined.point, np.int64)
+    c = (2 * u + f) // (2 * f)
+    return np.clip(c, 0, np.asarray(refined.dims, np.int64) - 1).astype(np.int32)
+
+
+def refine_locations(slowness, star, stations, picks, *, subdiv: int, max_moves: int = 4, sigma=None,
+                     confidence: float = 0.95, delta: float = 10.0, device: int | None = None,
+                     kernel: int | None = None):
+    """One-shot sub-node location: on one context, solve one field per station, locate every event of picks [E, S]
+    on the grid (SweepContext.locate_events), then refine the events located OK on the lattice of 1/subdiv of a node
+    in the cube around their node (SweepContext.refine_events).  While some event's best point lies on a face of its
+    cube that is interior to the box (RefinedLocations.on_edge) and fewer than max_moves moves have been made, those
+    events alone are recentred on the node nearest their best point (recentre) and refined again.
+
+    A point's misfit does not depend on the cube that contains it, and the new cube holds the old best point within
+    f/2 of its centre.  So a move either finds a point of strictly lower key (misfit, then u lexicographically) or keeps
+    the point, which then lies off the new cube's faces and the event stops: the loop terminates, and it never returns
+    a worse point than the previous cube's.
+
+    With sigma (as in location_uncertainty), also summarises each event's confidence region over its final cube
+    (SweepContext.refine_regions) at uncertainty_levels(refined, sigma, confidence).  Returns (Locations,
+    RefinedLocations[, RefinedRegions]); events not located OK keep their status, point (-1, -1, -1), misfit +inf and
+    origin time NaN, and get no region."""
+    f = int(subdiv)
+    with SweepContext(device=device, kernel=kernel) as ctx:
+        ctx.set_model(slowness)
+        ctx.set_star(star, delta)
+        ctx.set_sources(stations)
+        ctx.run()
+        p = np.ascontiguousarray(picks, dtype=np.float32)
+        loc = ctx.locate_events(p)
+        out = refine_located(ctx, p, loc, subdiv=f, max_moves=max_moves)
+        if sigma is None:
+            return loc, out
+        # events not located OK have a NaN level; any centre inside the box serves them
+        reg = ctx.refine_regions(p, out.centre, f, uncertainty_levels(out, sigma, confidence))
+        return loc, out, reg
+
+
+def refine_located(ctx: SweepContext, picks, locations: Locations, *, subdiv: int, max_moves: int = 4,
+                   sources=None) -> RefinedLocations:
+    """The refinement loop of refine_locations on a context whose fields are already there: the events of
+    `locations` (from ctx.locate_events(picks, sources)) located OK, refined around their nodes and recentred while
+    on_edge, at most max_moves times.  The others keep their status, point (-1, -1, -1), misfit +inf and NaN origin
+    time, with centre (0, 0, 0).  stats are those of the first refinement call."""
+    f = int(subdiv)
+    p = np.ascontiguousarray(picks, dtype=np.float32)
+    E = len(p)
+    idx = np.nonzero(locations.status == LOC_OK)[0]
+    ref = ctx.refine_events(p[idx], locations.node[idx], f, sources=sources)
+    out = RefinedLocations(np.full((E, 3), -1, np.int64), f, np.zeros((E, 3), np.int32), np.full(E, np.inf, np.float32),
+                           np.full(E, np.nan), locations.npicks.copy(), locations.status.copy(), ref.stats,
+                           tuple(ctx.dims), np.zeros(E, np.int32))
+
+    def store(rows, r):
+        out.point[rows], out.centre[rows], out.misfit[rows] = r.point, r.centre, r.misfit
+        out.origin_time[rows], out.status[rows] = r.origin_time, r.status
+
+    store(idx, ref)
+    for _ in range(int(max_moves)):
+        edge = np.nonzero(out.on_edge)[0]
+        if not len(edge):
+            break
+        store(edge, ctx.refine_events(p[edge], recentre(out)[edge], f, sources=sources))
+        out.moves[edge] += 1
+    return out
 
 
 # ---- file formats -------------------------------------------------------------------------

@@ -1944,6 +1944,33 @@ __device__ __forceinline__ unsigned long long loc_order_key(double x) {
   return (b >> 63) ? ~b : b | 0x8000000000000000ull;
 }
 
+// One warp's share of event e's region summary into the slots of r (layout below): reached, then the warp's sums,
+// minima and t0 keys reduced over the lanes and added with one atomic per slot.  Shared by region_kernel and
+// refine_regions_kernel; the whole warp calls it.
+__device__ __forceinline__ void region_flush(const RegionArgs& r, int e, int lane, bool reached, long long (&m)[10],
+                                             unsigned (&box)[6], unsigned long long (&tk)[2]) {
+  if (__any_sync(0xffffffffu, reached) && lane == 0) atomicOr(r.reached + e, 1u);
+  if (!__any_sync(0xffffffffu, m[0] != 0)) return;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+    for (int i = 0; i < 10; ++i) m[i] += __shfl_xor_sync(0xffffffffu, m[i], o);
+#pragma unroll
+    for (int i = 0; i < 6; ++i) box[i] = min(box[i], __shfl_xor_sync(0xffffffffu, box[i], o));
+#pragma unroll
+    for (int i = 0; i < 2; ++i) tk[i] = min(tk[i], __shfl_xor_sync(0xffffffffu, tk[i], o));
+  }
+  if (lane == 0) {
+    unsigned long long* sum = r.sum + 10 * (size_t)e;
+#pragma unroll
+    for (int i = 0; i < 10; ++i) atomicAdd(sum + i, (unsigned long long)m[i]);
+#pragma unroll
+    for (int i = 0; i < 6; ++i) atomicMin(r.box + 6 * (size_t)e + i, box[i]);
+#pragma unroll
+    for (int i = 0; i < 2; ++i) atomicMin(r.t0 + 2 * (size_t)e + i, tk[i]);
+  }
+}
+
 // The region {n : misfit(n) <= level} of every event of the launch (sweeptt_misfit_regions), summarised exactly: the
 // staging and the formula of locate_kernel, then per event the integer sums, integer extremes and ordered t0 keys of
 // the nodes inside.  A live node is inside when its misfit bits are below r.lim[e] = (level bits) + 1, or never
@@ -1999,26 +2026,7 @@ __global__ void __launch_bounds__(LOC_THREADS, 1) region_kernel(const LocateArgs
       tk[0] = min(tk[0], key);
       tk[1] = min(tk[1], ~key);
     }
-    if (__any_sync(0xffffffffu, reached) && lane == 0) atomicOr(r.reached + e, 1u);
-    if (!__any_sync(0xffffffffu, m[0] != 0)) continue;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-      for (int i = 0; i < 10; ++i) m[i] += __shfl_xor_sync(0xffffffffu, m[i], o);
-#pragma unroll
-      for (int i = 0; i < 6; ++i) box[i] = min(box[i], __shfl_xor_sync(0xffffffffu, box[i], o));
-#pragma unroll
-      for (int i = 0; i < 2; ++i) tk[i] = min(tk[i], __shfl_xor_sync(0xffffffffu, tk[i], o));
-    }
-    if (lane == 0) {
-      unsigned long long* sum = r.sum + 10 * (size_t)e;
-#pragma unroll
-      for (int i = 0; i < 10; ++i) atomicAdd(sum + i, (unsigned long long)m[i]);
-#pragma unroll
-      for (int i = 0; i < 6; ++i) atomicMin(r.box + 6 * (size_t)e + i, box[i]);
-#pragma unroll
-      for (int i = 0; i < 2; ++i) atomicMin(r.t0 + 2 * (size_t)e + i, tk[i]);
-    }
+    region_flush(r, e, lane, reached, m, box, tk);
   }
 }
 
@@ -2063,6 +2071,244 @@ __global__ void __launch_bounds__(256) misfit_box_kernel(const LocateArgs a, flo
     double t0[1];
     event_misfit<1>(a.pick_sta, a.pick_obs, k, a.pick_rk[0], LocBoxTT{a.tt, a.g.vol, p}, bits, t0);
     dense[d] = bits[0] == LOC_EXCLUDED ? CUDART_INF_F : __uint_as_float(bits[0]);
+  }
+}
+
+// ---------------------------------------------------------------------------------------
+// sub-node refinement (include/sweeptt.h, sweeptt_refine_events / sweeptt_refine_regions; DESIGN §3.13)
+// ---------------------------------------------------------------------------------------
+// Event e's cube: lattice points u = f*c + t, |t_a| <= f, clipped to the box, in the offsets s_a = t_a + f in [0, 2f]
+// (never negative, so divisions are of small non-negative ints).  Point u reads the nodes c - 1 + s_a div f (+1 where
+// s_a mod f != 0): the 27 nodes around c, staged once per CTA for every station.  Its cube-local index, the key's low
+// word, is (s0*L + s1)*L + s2 with L = 2f + 1 < 2^7: lexicographic in u.
+constexpr int REF_THREADS = 256;
+constexpr int REF_NODES = 27;
+
+// fl(p + fl(w * fl(q - p))), no fused multiply-add.  With q == p (an axis whose remainder is 0 reads its b = 0 corner
+// twice) it is p exactly: q - p = +0, w * +0 = +0 (w >= 0) and p + +0 = p for the times' p >= +0.
+__device__ __forceinline__ double loc_lerp(double p, double q, double w) {
+  return __dadd_rn(p, __dmul_rn(w, __dsub_rn(q, p)));
+}
+__device__ __forceinline__ double loc_ld(const double* p) { return *p; }
+__device__ __forceinline__ double loc_ld(const float* p) { return (double)__ldg(p); }
+
+// The trilinear time of one lattice point (the header's rule): station s's corner b is at base[s*sstride + o + b.d];
+// d[a] = 0 on an axis whose remainder is 0, so that its b_a = 1 corner is its b_a = 0 corner and no node outside the
+// box is read.  Any +INF corner gives +INF, explicitly (lerp(INF, x) is NaN, and event_misfit's exclusion compares
+// with +INF).  Interpolated along caller axis 2, then 1, then 0, whatever the kernel axes.  T = double: the CTA's staged
+// cube in shared memory; T = float: the padded boxes in global memory (the finisher).
+template <class T>
+struct LocLatticeTT {
+  const T* base;
+  long long sstride, o;
+  long long d[3];
+  double w[3];
+  __device__ __forceinline__ double operator()(int s, int) const {
+    const T* b = base + s * sstride + o;
+    double c[8];
+    bool inf = false;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      c[i] = loc_ld(b + ((i >> 2) & 1) * d[0] + ((i >> 1) & 1) * d[1] + (i & 1) * d[2]);
+      inf |= c[i] == CUDART_INF;
+    }
+    if (inf) return CUDART_INF;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) c[i] = loc_lerp(c[2 * i], c[2 * i + 1], w[2]);   // axis 2
+#pragma unroll
+    for (int i = 0; i < 2; ++i) c[i] = loc_lerp(c[2 * i], c[2 * i + 1], w[1]);   // axis 1
+    return loc_lerp(c[0], c[1], w[0]);                                          // axis 0
+  }
+};
+
+// The caller-axis dims and the padded stride of each caller axis (kernel axis q = caller axis perm[q]), and the padded
+// index of the caller-axis node c.  Selects rather than indexing through perm: the arrays stay in registers.
+__device__ __forceinline__ void loc_caller_dims(const BoxGeom& g, int (&n)[3], long long (&stride)[3]) {
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    n[a] = g.perm[0] == a ? g.nx : g.perm[1] == a ? g.ny : g.nz;
+    stride[a] = g.perm[0] == a ? g.sx : g.perm[1] == a ? (long long)g.pz : 1;
+  }
+}
+__device__ __forceinline__ long long loc_padded(const BoxGeom& g, const long long (&stride)[3], const int (&c)[3]) {
+  return (long long)AX * g.sx + (long long)AY * g.pz + AZ + c[0] * stride[0] + c[1] * stride[1] + c[2] * stride[2];
+}
+
+// The range of s_a in event e's cube: [lo_a, lo_a + ext_a).
+__device__ __forceinline__ int ref_cube(const BoxGeom& g, const RefineArgs& rf, int e, int (&c)[3], int (&lo)[3],
+                                        int (&ext)[3]) {
+  int n[3];
+  long long stride[3];
+  loc_caller_dims(g, n, stride);
+  const int f = rf.f;
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    c[i] = rf.centre[3 * e + i];
+    lo[i] = c[i] > 0 ? 0 : f;
+    ext[i] = (c[i] < n[i] - 1 ? 2 * f : f) - lo[i] + 1;
+  }
+  return ext[0] * ext[1] * ext[2];
+}
+
+// The CTA's staging for event e: the times of every station at the 27 nodes c - 1 .. c + 1 (caller axes; +INF past
+// the box, never read), s_tt[s * 27 + (l0*3 + l1)*3 + l2], and the weights W[0..f).
+__device__ __forceinline__ void ref_stage(const LocateArgs& a, const RefineArgs& rf, const int (&c)[3], double* s_tt,
+                                          double* s_w) {
+  int n[3];
+  long long stride[3];
+  loc_caller_dims(a.g, n, stride);
+  for (int r = threadIdx.x; r < rf.f; r += blockDim.x) s_w[r] = rf.w[r];
+  for (int idx = threadIdx.x; idx < a.nsta * REF_NODES; idx += blockDim.x) {
+    const int s = idx / REF_NODES, l = idx % REF_NODES;
+    const int q[3] = {c[0] + l / 9 - 1, c[1] + l / 3 % 3 - 1, c[2] + l % 3 - 1};
+    const bool in = q[0] >= 0 && q[0] < n[0] && q[1] >= 0 && q[1] < n[1] && q[2] >= 0 && q[2] < n[2];
+    s_tt[idx] = in ? (double)__ldg(a.tt + s * a.g.vol + loc_padded(a.g, stride, q)) : CUDART_INF;
+  }
+  __syncthreads();
+}
+
+// Lattice point t (0 <= t < the cube's point count, row-major over the clipped s ranges) of the staged cube: its
+// offsets s, cube-local index, and the functor of its time.
+__device__ __forceinline__ LocLatticeTT<double> ref_point(unsigned t, int f, const int (&lo)[3], const int (&ext)[3],
+                                                          const double* s_tt, const double* s_w, int (&s)[3],
+                                                          unsigned* local) {
+  s[2] = lo[2] + (int)(t % ext[2]);
+  t /= ext[2];
+  s[1] = lo[1] + (int)(t % ext[1]);
+  s[0] = lo[0] + (int)(t / ext[1]);
+  const unsigned L = 2 * f + 1;
+  *local = ((unsigned)s[0] * L + s[1]) * L + s[2];
+  LocLatticeTT<double> tt{s_tt, REF_NODES, 0, {0, 0, 0}, {0.0, 0.0, 0.0}};
+  constexpr int step[3] = {9, 3, 1};
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    const int l = s[i] / f, r = s[i] - l * f;
+    tt.o += l * step[i];
+    tt.d[i] = r ? step[i] : 0;
+    tt.w[i] = s_w[r];
+  }
+  return tt;
+}
+
+// The best lattice point of every event of the launch (sweeptt_refine_events): blockIdx.y takes events in turn, and
+// blockIdx.x is a slab of rf.points_per_cta consecutive points of the event's cube, taken by the CTA's threads in
+// turn.  The CTA's smallest key goes to the event with one 64-bit atomicMin (integer min: schedule-independent).
+__global__ void __launch_bounds__(REF_THREADS) refine_kernel(const LocateArgs a, const RefineArgs rf) {
+  extern __shared__ double s_tt[];
+  __shared__ double s_w[64];
+  __shared__ unsigned long long s_best;
+  for (int e = a.e_begin + blockIdx.y; e < a.e_begin + a.e_count; e += gridDim.y) {
+    const int off = a.pick_off[e], k = a.pick_off[e + 1] - off;
+    int c[3], lo[3], ext[3];
+    const unsigned P = (unsigned)ref_cube(a.g, rf, e, c, lo, ext);
+    const unsigned t_begin = blockIdx.x * (unsigned)rf.points_per_cta;
+    if (k == 0 || t_begin >= P) continue;   // CTA-uniform
+    const unsigned t_end = min(P, t_begin + (unsigned)rf.points_per_cta);
+    if (threadIdx.x == 0) s_best = ~0ull;
+    ref_stage(a, rf, c, s_tt, s_w);
+    unsigned long long best = ~0ull;
+    for (unsigned t = t_begin + threadIdx.x; t < t_end; t += blockDim.x) {
+      int s[3];
+      unsigned local;
+      const LocLatticeTT<double> tt = ref_point(t, rf.f, lo, ext, s_tt, s_w, s, &local);
+      unsigned bits[1];
+      double t0[1];
+      event_misfit<1>(a.pick_sta + off, a.pick_obs + off, k, a.pick_rk[e], tt, bits, t0);
+      best = min(best, ((unsigned long long)bits[0] << 32) | local);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(0xffffffffu, best, o));
+    if ((threadIdx.x & 31) == 0) atomicMin(&s_best, best);
+    __syncthreads();
+    if (threadIdx.x == 0 && s_best != ~0ull) atomicMin(a.key + e, s_best);
+    __syncthreads();   // the staging and s_best of the next event
+  }
+}
+
+// The region { u in cube : misfit(u) <= level } of every event of the launch (sweeptt_refine_regions): the shape and
+// point evaluation of refine_kernel, and the accumulation of region_kernel (region_flush) with the moments taken over
+// t = s - f (about the centre) and the box over s (unsigned, 0 .. 2f).
+__global__ void __launch_bounds__(REF_THREADS) refine_regions_kernel(const LocateArgs a, const RefineArgs rf,
+                                                                    const RegionArgs r) {
+  extern __shared__ double s_tt[];
+  __shared__ double s_w[64];
+  const int lane = threadIdx.x & 31;
+  for (int e = a.e_begin + blockIdx.y; e < a.e_begin + a.e_count; e += gridDim.y) {
+    const int off = a.pick_off[e], k = a.pick_off[e + 1] - off;
+    int c[3], lo[3], ext[3];
+    const unsigned P = (unsigned)ref_cube(a.g, rf, e, c, lo, ext);
+    const unsigned t_begin = blockIdx.x * (unsigned)rf.points_per_cta;
+    if (k == 0 || t_begin >= P) continue;   // CTA-uniform
+    const unsigned t_end = min(P, t_begin + (unsigned)rf.points_per_cta);
+    ref_stage(a, rf, c, s_tt, s_w);
+    const unsigned lim = r.lim[e];
+    bool reached = false;
+    long long m[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    unsigned box[6] = {~0u, ~0u, ~0u, ~0u, ~0u, ~0u};
+    unsigned long long tk[2] = {~0ull, ~0ull};
+    for (unsigned t = t_begin + threadIdx.x; t < t_end; t += blockDim.x) {
+      int s[3];
+      unsigned local;
+      const LocLatticeTT<double> tt = ref_point(t, rf.f, lo, ext, s_tt, s_w, s, &local);
+      unsigned bits[1];
+      double t0[1];
+      event_misfit<1>(a.pick_sta + off, a.pick_obs + off, k, a.pick_rk[e], tt, bits, t0);
+      reached |= bits[0] != LOC_EXCLUDED;
+      if (bits[0] >= lim) continue;
+      const long long v0 = s[0] - rf.f, v1 = s[1] - rf.f, v2 = s[2] - rf.f;
+      m[0] += 1;
+      m[1] += v0; m[2] += v1; m[3] += v2;
+      m[4] += v0 * v0; m[5] += v1 * v1; m[6] += v2 * v2;
+      m[7] += v0 * v1; m[8] += v0 * v2; m[9] += v1 * v2;
+#pragma unroll
+      for (int i = 0; i < 3; ++i) box[i] = min(box[i], (unsigned)s[i]), box[3 + i] = min(box[3 + i], ~(unsigned)s[i]);
+      const unsigned long long key = loc_order_key(t0[0]);
+      tk[0] = min(tk[0], key);
+      tk[1] = min(tk[1], ~key);
+    }
+    region_flush(r, e, lane, reached, m, box, tk);
+    __syncthreads();   // the staging of the next event
+  }
+}
+
+// Decodes every cube key: best lattice point u (caller axes), and its misfit and t0 recomputed through the same
+// lattice rule from the padded boxes.  Status as locate_finish_kernel.
+__global__ void refine_finish_kernel(const LocateArgs a, const RefineArgs rf, int nev) {
+  const BoxGeom& g = a.g;
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < nev; e += gridDim.x * blockDim.x) {
+    const int off = a.pick_off[e], k = a.pick_off[e + 1] - off;
+    const unsigned long long key = a.key[e];
+    a.npicks[e] = k;
+    if (k == 0 || (unsigned)(key >> 32) == LOC_EXCLUDED || key == ~0ull) {
+      rf.point[3 * e] = rf.point[3 * e + 1] = rf.point[3 * e + 2] = -1;
+      a.misfit[e] = CUDART_INF_F;
+      a.origin[e] = __longlong_as_double(0x7ff8000000000000ll);
+      a.status[e] = k == 0 ? SWEEPTT_LOC_NO_PICKS : SWEEPTT_LOC_UNREACHED;
+      continue;
+    }
+    int n[3];
+    long long stride[3];
+    loc_caller_dims(g, n, stride);
+    const int f = rf.f;
+    const unsigned L = 2 * f + 1, local = (unsigned)key;
+    const int s[3] = {(int)(local / L / L), (int)(local / L % L), (int)(local % L)};
+    int i[3];   // the b = 0 corner node
+    LocLatticeTT<float> tt{a.tt, g.vol, 0, {0, 0, 0}, {0.0, 0.0, 0.0}};
+#pragma unroll
+    for (int q = 0; q < 3; ++q) {
+      const int c = rf.centre[3 * e + q], l = s[q] / f, r = s[q] - l * f;
+      i[q] = c - 1 + l;
+      tt.d[q] = r ? stride[q] : 0;
+      tt.w[q] = rf.w[r];
+      rf.point[3 * e + q] = (long long)f * (c - 1) + s[q];
+    }
+    tt.o = loc_padded(g, stride, i);
+    unsigned bits[1];
+    double t0[1];
+    event_misfit<1>(a.pick_sta + off, a.pick_obs + off, k, a.pick_rk[e], tt, bits, t0);
+    a.misfit[e] = __uint_as_float(bits[0]);
+    a.origin[e] = t0[0];
+    a.status[e] = SWEEPTT_LOC_OK;
   }
 }
 
@@ -2653,6 +2899,44 @@ cudaError_t launch_regions(const LocateArgs& a, const RegionArgs& r, int nodes_p
 
 cudaError_t launch_locate_finish(const LocateArgs& a, int nev, cudaStream_t stream) {
   locate_finish_kernel<<<(nev + 127) / 128, 128, 0, stream>>>(a, nev);
+  return cudaGetLastError();
+}
+
+bool refine_fits(int nsta, int device) {
+  int optin = 0;
+  if (cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device) != cudaSuccess) return false;
+  const size_t smem = (size_t)nsta * REF_NODES * sizeof(double);
+  for (const void* k : {(const void*)refine_kernel, (const void*)refine_regions_kernel}) {
+    cudaFuncAttributes fa{};
+    if (cudaFuncGetAttributes(&fa, k) != cudaSuccess || smem + fa.sharedSizeBytes > (size_t)optin) return false;
+  }
+  return true;
+}
+
+// grid: x = the slabs of the largest cube, (2f + 1)^3 points; y = events (a CTA takes events e, e + gridDim.y, ...)
+static dim3 refine_grid(const LocateArgs& a, const RefineArgs& rf) {
+  const unsigned L = 2 * rf.f + 1;
+  return dim3((L * L * L + rf.points_per_cta - 1) / rf.points_per_cta, (unsigned)std::min(a.e_count, 65535));
+}
+
+cudaError_t launch_refine(const LocateArgs& a, const RefineArgs& rf, cudaStream_t stream) {
+  const size_t smem = (size_t)a.nsta * REF_NODES * sizeof(double);
+  cudaError_t e = cudaFuncSetAttribute(refine_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  refine_kernel<<<refine_grid(a, rf), REF_THREADS, smem, stream>>>(a, rf);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_refine_regions(const LocateArgs& a, const RefineArgs& rf, const RegionArgs& r, cudaStream_t stream) {
+  const size_t smem = (size_t)a.nsta * REF_NODES * sizeof(double);
+  cudaError_t e = cudaFuncSetAttribute(refine_regions_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  refine_regions_kernel<<<refine_grid(a, rf), REF_THREADS, smem, stream>>>(a, rf, r);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_refine_finish(const LocateArgs& a, const RefineArgs& rf, int nev, cudaStream_t stream) {
+  refine_finish_kernel<<<(nev + 127) / 128, 128, 0, stream>>>(a, rf, nev);
   return cudaGetLastError();
 }
 

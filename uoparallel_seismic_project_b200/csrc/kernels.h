@@ -220,6 +220,14 @@ struct RegionArgs {
   unsigned long long* t0;          // [2]: min key, min ~key of the ordered t0, filled with ones first
   unsigned* reached;               // some node not excluded, zeroed first
 };
+// The refinement of sweeptt_refine_events / sweeptt_refine_regions (refine kernels, cube layout in kernels.cu):
+struct RefineArgs {
+  const int* centre;               // [3 nev] centre node of every event, caller axes
+  const double* w;                 // [f] W[r] = RN(r / f)
+  int f;                           // subdiv, 1 .. 64
+  int points_per_cta;              // lattice points of a cube per CTA (SWEEPTT_REFINE_POINTS)
+  long long* point;                // finisher output [3 nev]: the best lattice point u, caller axes
+};
 // Nodes per thread of the location kernel (4, 2 or 1: a CTA stages the times of nsta stations at 32 * that many
 // nodes in shared memory), or 0 when not even 32 nodes fit; the same for the region kernel, by its own attributes.
 int locate_nodes_per_thread(int nsta, int device);
@@ -229,6 +237,14 @@ cudaError_t launch_locate(const LocateArgs& a, int nodes_per_thread, cudaStream_
 cudaError_t launch_regions(const LocateArgs& a, const RegionArgs& r, int nodes_per_thread, cudaStream_t stream);
 // Decodes every key: best node, and its misfit and t0 recomputed with the location kernel's formula.
 cudaError_t launch_locate_finish(const LocateArgs& a, int nev, cudaStream_t stream);
+// Whether the refinement kernels' staging of nsta stations at 27 nodes (doubles) fits next to their static shared memory.
+bool refine_fits(int nsta, int device);
+// Events [e_begin, e_begin + e_count): the cube keys of sweeptt_refine_events into a.key (set to ~0 first), or the
+// cube region summaries of sweeptt_refine_regions.
+cudaError_t launch_refine(const LocateArgs& a, const RefineArgs& rf, cudaStream_t stream);
+cudaError_t launch_refine_regions(const LocateArgs& a, const RefineArgs& rf, const RegionArgs& r, cudaStream_t stream);
+// Decodes every cube key: best lattice point, its misfit and t0 recomputed through the same lattice rule.
+cudaError_t launch_refine_finish(const LocateArgs& a, const RefineArgs& rf, int nev, cudaStream_t stream);
 // Event 0's misfit at every node into the dense caller-axis box.
 cudaError_t launch_misfit_box(const LocateArgs& a, float* dense, cudaStream_t stream);
 

@@ -2552,29 +2552,49 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
 // Checks shared by the location calls; then the picks of nev events (NaN left out) go to the device as a CSR with
 // RN(1/k) per event, and *a describes them, the fields of the call's stations and the result slots.  With levels
 // and r (sweeptt_misfit_regions), also the levels' and the moment bound's checks, the region kernel's shape, and the
-// region slots after the location slots, initialised.  Every refusal comes before the first allocation.
+// region slots after the location slots, initialised.  With centres and rf (sweeptt_refine_events / _regions), the
+// refinement: the centres' and subdiv's checks in place of the 2^32-node and moment bounds (a cube key holds a
+// cube-local index, and cube moments are small), the station limit of the location call and the refinement kernels'
+// own fit, and the centres, the weight table W[r] = RN(r / f) and the point slots after the others.  The cube keys
+// are the location keys.  Every refusal comes before the first allocation.
 // nodes_per_thread (may be NULL): the grid-search kernel's shape for these stations.
 static int locate_prepare(sweeptt_ctx* c, ConstLease* lease, const char* who, int source_begin, int source_count,
                           const float* picks, int nev, LocateArgs* a, int* nodes_per_thread, sweeptt_stats* stats,
-                          const float* levels = nullptr, RegionArgs* r = nullptr) {
+                          const float* levels = nullptr, RegionArgs* r = nullptr, const START* centres = nullptr,
+                          int subdiv = 0, RefineArgs* rf = nullptr) {
   if (!ready(c, lease)) return 0;
   if (stats) std::memset(stats, 0, sizeof *stats);
   if (!check_source_range(c, who, source_begin, source_count)) return 0;
   if (nodes_per_thread &&
-      (*nodes_per_thread = (levels ? region_nodes_per_thread : locate_nodes_per_thread)(source_count, c->device)) == 0)
+      (*nodes_per_thread = (levels && !rf ? region_nodes_per_thread : locate_nodes_per_thread)(source_count, c->device)) == 0)
     return fail("%s: %d stations do not fit the location kernel's shared memory (8 bytes per station and node, 32 nodes)",
+                who, source_count);
+  if (rf && !refine_fits(source_count, c->device))
+    return fail("%s: %d stations do not fit the refinement kernel's shared memory (8 bytes per station and node, 27 nodes)",
                 who, source_count);
   if (nev < 0) return fail("%s: nev = %d is negative", who, nev);
   if (nev > 0 && !picks) return fail("%s: null picks", who);
   const BoxGeom& g = c->g;
-  if ((unsigned long long)g.nx * g.ny * g.nz > (1ull << 32))
+  if (!rf && (unsigned long long)g.nx * g.ny * g.nz > (1ull << 32))
     return fail("%s: %d x %d x %d nodes exceed 2^32, the argmin key holds a node index in 32 bits", who, g.nx, g.ny, g.nz);
+  if (rf) {
+    if (subdiv < 1 || subdiv > 64) return fail("%s: subdiv = %d is not in [1, 64]", who, subdiv);
+    if (nev > 0 && !centres) return fail("%s: null centres", who);
+    int n[3];
+    n[g.perm[0]] = g.nx; n[g.perm[1]] = g.ny; n[g.perm[2]] = g.nz;
+    for (int e = 0; e < nev; ++e) {
+      const START& q = centres[e];
+      if (q.i < 0 || q.i >= n[0] || q.j < 0 || q.j >= n[1] || q.k < 0 || q.k >= n[2])
+        return fail("%s: centre of event %d, (%d, %d, %d), is outside the %d x %d x %d box", who, e, q.i, q.j, q.k,
+                    n[0], n[1], n[2]);
+    }
+  }
   std::vector<unsigned> lim;
   if (levels) {
     // every second moment is at most D * max_a (n_a - 1)^2; it must fit int64
     const unsigned long long D = (unsigned long long)g.nx * g.ny * g.nz;
     const unsigned long long m = (unsigned long long)std::max({g.nx, g.ny, g.nz}) - 1;
-    if (m * m > (unsigned long long)INT64_MAX / D)
+    if (!rf && m * m > (unsigned long long)INT64_MAX / D)
       return fail("%s: %d x %d x %d nodes: the region moments (up to D * (n - 1)^2 for the longest axis n) overflow "
                   "int64", who, g.nx, g.ny, g.nz);
     lim.resize((size_t)nev);
@@ -2608,12 +2628,15 @@ static int locate_prepare(sweeptt_ctx* c, ConstLease* lease, const char* who, in
   }
   const size_t np = sta.size(), n = (size_t)nev;
   auto up16 = [](size_t b) { return (b + 15) / 16 * 16; };
-  // location slots, then (levels only) lim, sum, reached (zeroed), t0, box (ones) of RegionArgs
-  const size_t part[15] = {up16(4 * (n + 1)), up16(4 * np), up16(8 * np), up16(8 * n), up16(8 * n),
+  // location slots, then (levels only) lim, sum, reached (zeroed), t0, box (ones) of RegionArgs, then (rf only)
+  // centres, W, points of RefineArgs
+  const size_t rg = levels ? 1 : 0, f = rf ? (size_t)subdiv : 0;
+  const size_t part[18] = {up16(4 * (n + 1)), up16(4 * np), up16(8 * np), up16(8 * n), up16(8 * n),
                            up16(12 * n),      up16(4 * n),  up16(8 * n),  up16(4 * n), up16(4 * n),
-                           up16(4 * n),       up16(80 * n), up16(4 * n),  up16(16 * n), up16(24 * n)};
-  const int nparts = levels ? 15 : 10;
-  size_t at[16] = {0};
+                           rg * up16(4 * n),  rg * up16(80 * n), rg * up16(4 * n),  rg * up16(16 * n), rg * up16(24 * n),
+                           f ? up16(12 * n) : 0, up16(8 * f), f ? up16(24 * n) : 0};
+  const int nparts = rf ? 18 : levels ? 15 : 10;
+  size_t at[19] = {0};
   for (int i = 0; i < nparts; ++i) at[i + 1] = at[i] + part[i];
   if (!ensure_dev(c, &c->d_loc, &c->loc_cap, at[nparts])) return 0;
   unsigned char* b = c->d_loc;
@@ -2650,12 +2673,25 @@ static int locate_prepare(sweeptt_ctx* c, ConstLease* lease, const char* who, in
       CK(cudaMemsetAsync(b + at[13], 0xff, at[15] - at[13], c->stream));
     }
   }
+  std::vector<double> w(f);
+  if (rf) {
+    for (size_t i = 0; i < f; ++i) w[i] = (double)i / (double)f;
+    rf->centre = reinterpret_cast<const int*>(b + at[15]);
+    rf->w = reinterpret_cast<const double*>(b + at[16]);
+    rf->point = reinterpret_cast<long long*>(b + at[17]);
+    rf->f = subdiv;
+    rf->points_per_cta = 1024;
+    if (const char* e = getenv("SWEEPTT_REFINE_POINTS")) rf->points_per_cta = std::max(1, atoi(e));
+    static_assert(sizeof(START) == 3 * sizeof(int), "START is three ints");
+    if (n) CK(cudaMemcpyAsync(b + at[15], centres, 12 * n, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(b + at[16], w.data(), 8 * f, cudaMemcpyHostToDevice, c->stream));
+  }
   CK(cudaStreamSynchronize(c->stream));
   if (stats) {
     stats->struct_size = (int)sizeof *stats;
     stats->devices_used = 1;
     stats->h2d_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    stats->h2d_bytes = (long long)(4 * (n + 1) + 12 * np + 8 * n + (levels ? 4 * n : 0));
+    stats->h2d_bytes = (long long)(4 * (n + 1) + 12 * np + 8 * n + (levels ? 4 * n : 0) + (rf ? 12 * n + 8 * f : 0));
   }
   return 1;
 }
@@ -2798,6 +2834,133 @@ extern "C" int sweeptt_misfit_regions(sweeptt_ctx* c, int source_begin, int sour
         bbox_out[6 * e + i] = cnt ? (int32_t)box[6 * e + i] : -1;
         bbox_out[6 * e + 3 + i] = cnt ? (int32_t)~box[6 * e + 3 + i] : -1;
       }
+    if (origin_range_out) {
+      origin_range_out[2 * e] = cnt ? from_key(tk[2 * e]) : nan;
+      origin_range_out[2 * e + 1] = cnt ? from_key(~tk[2 * e + 1]) : nan;
+    }
+  }
+  if (stats) {
+    stats->solve_ms = ms;
+    stats->kernel_launches = launches;
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes = bytes;
+  }
+  return 1;
+}
+
+extern "C" int sweeptt_refine_events(sweeptt_ctx* c, int source_begin, int source_count, const float* picks, int nev,
+                                     const struct START* centres, int subdiv, int64_t* point_out, float* misfit_out,
+                                     double* origin_out, int32_t* npicks_out, int32_t* status_out, sweeptt_stats* stats) {
+  static const char* who = "sweeptt_refine_events";
+  if (!point_out || !status_out) return fail("%s: point_out and status_out are required", who);
+  ConstLease lease;
+  LocateArgs a;
+  RefineArgs rf{};
+  int nb = 0;
+  if (!locate_prepare(c, &lease, who, source_begin, source_count, picks, nev, &a, &nb, stats, nullptr, nullptr, centres,
+                      subdiv, &rf))
+    return 0;
+  if (nev == 0) return 1;
+  const int chunk = locate_chunk();
+  long long launches = 0;
+  CK(cudaEventRecord(c->ev0, c->stream));
+  CK(cudaMemsetAsync(a.key, 0xff, 8 * (size_t)nev, c->stream));
+  for (int e0 = 0; e0 < nev; e0 += chunk) {
+    a.e_begin = e0;
+    a.e_count = std::min(chunk, nev - e0);
+    CK(launch_refine(a, rf, c->stream));
+    ++launches;
+  }
+  CK(launch_refine_finish(a, rf, nev, c->stream));
+  CK(cudaEventRecord(c->ev1, c->stream));
+  CK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+
+  const auto t_copy = std::chrono::steady_clock::now();
+  const size_t n = (size_t)nev;
+  long long bytes = 28 * (long long)n;
+  static_assert(sizeof(long long) == sizeof(int64_t), "a point coordinate is 64 bits");
+  CK(cudaMemcpyAsync(point_out, rf.point, 24 * n, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(status_out, a.status, 4 * n, cudaMemcpyDeviceToHost, c->stream));
+  if (misfit_out) { CK(cudaMemcpyAsync(misfit_out, a.misfit, 4 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * n; }
+  if (origin_out) { CK(cudaMemcpyAsync(origin_out, a.origin, 8 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 8 * n; }
+  if (npicks_out) { CK(cudaMemcpyAsync(npicks_out, a.npicks, 4 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 4 * n; }
+  CK(cudaStreamSynchronize(c->stream));
+  if (stats) {
+    stats->solve_ms = ms;
+    stats->kernel_launches = launches + 1;
+    stats->d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_copy).count();
+    stats->d2h_bytes = bytes;
+  }
+  return 1;
+}
+
+extern "C" int sweeptt_refine_regions(sweeptt_ctx* c, int source_begin, int source_count, const float* picks, int nev,
+                                      const struct START* centres, int subdiv, const float* levels, int64_t* count_out,
+                                      int64_t* bbox_out, int64_t* moments_out, double* origin_range_out,
+                                      int32_t* status_out, sweeptt_stats* stats) {
+  static const char* who = "sweeptt_refine_regions";
+  if (!count_out || !status_out) return fail("%s: count_out and status_out are required", who);
+  if (nev > 0 && !levels) return fail("%s: null levels", who);
+  ConstLease lease;
+  LocateArgs a;
+  RegionArgs r{};
+  RefineArgs rf{};
+  int nb = 0;
+  static const float no_levels[1] = {0.f};   // nev = 0 reads no level, but still takes the region checks
+  if (!locate_prepare(c, &lease, who, source_begin, source_count, picks, nev, &a, &nb, stats, levels ? levels : no_levels,
+                      &r, centres, subdiv, &rf))
+    return 0;
+  if (nev == 0) return 1;
+  const int chunk = locate_chunk();
+  long long launches = 0;
+  CK(cudaEventRecord(c->ev0, c->stream));
+  for (int e0 = 0; e0 < nev; e0 += chunk) {
+    a.e_begin = e0;
+    a.e_count = std::min(chunk, nev - e0);
+    CK(launch_refine_regions(a, rf, r, c->stream));
+    ++launches;
+  }
+  CK(cudaEventRecord(c->ev1, c->stream));
+  CK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+
+  const auto t_copy = std::chrono::steady_clock::now();
+  const size_t n = (size_t)nev;
+  std::vector<unsigned long long> sum(10 * n), tk(2 * n);
+  std::vector<unsigned> box(6 * n), reached(n);
+  CK(cudaMemcpyAsync(sum.data(), r.sum, 80 * n, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(reached.data(), r.reached, 4 * n, cudaMemcpyDeviceToHost, c->stream));
+  long long bytes = 84 * (long long)n;
+  if (bbox_out) { CK(cudaMemcpyAsync(box.data(), r.box, 24 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 24 * n; }
+  if (origin_range_out) { CK(cudaMemcpyAsync(tk.data(), r.t0, 16 * n, cudaMemcpyDeviceToHost, c->stream)); bytes += 16 * n; }
+  CK(cudaStreamSynchronize(c->stream));
+  const double nan = std::numeric_limits<double>::quiet_NaN();
+  auto from_key = [](unsigned long long k) {   // inverse of kernels.cu's loc_order_key
+    const unsigned long long b = (k >> 63) ? k & ~0x8000000000000000ull : ~k;
+    double x;
+    std::memcpy(&x, &b, 8);
+    return x;
+  };
+  const int64_t f = subdiv;
+  for (size_t e = 0; e < n; ++e) {
+    int k = 0;
+    for (int s = 0; s < source_count; ++s) k += !std::isnan(picks[e * source_count + s]);
+    status_out[e] = k == 0 ? SWEEPTT_LOC_NO_PICKS : reached[e] ? SWEEPTT_LOC_OK : SWEEPTT_LOC_UNREACHED;
+    const unsigned long long cnt = sum[10 * e];
+    count_out[e] = (int64_t)cnt;
+    if (moments_out)
+      for (int i = 0; i < 9; ++i) moments_out[9 * e + i] = (int64_t)sum[10 * e + 1 + i];
+    if (bbox_out) {
+      // the box holds the offsets s = u - f * (c - 1), 0 .. 2f
+      const int64_t base[3] = {f * (centres[e].i - 1), f * (centres[e].j - 1), f * (centres[e].k - 1)};
+      for (int i = 0; i < 3; ++i) {
+        bbox_out[6 * e + i] = cnt ? base[i] + box[6 * e + i] : -1;
+        bbox_out[6 * e + 3 + i] = cnt ? base[i] + ~box[6 * e + 3 + i] : -1;
+      }
+    }
     if (origin_range_out) {
       origin_range_out[2 * e] = cnt ? from_key(tk[2 * e]) : nan;
       origin_range_out[2 * e + 1] = cnt ? from_key(~tk[2 * e + 1]) : nan;
