@@ -384,12 +384,18 @@ int sweeptt_rayset_backproject(sweeptt_rayset *set, const float *weights, float 
  * sum every block of 2048 consecutive elements with the halving tree a[i] = fl(a[i] + a[i+h]), h = 1024, 512, .., 1,
  * and apply the same tree to the vector of block sums until one value is left (sumsq of nothing is +0).  The order
  * depends on neither the box, the device nor the grid.  istop, itn and the norms of info mean what scipy's return tuple
- * means.  b = 0 gives x = 0 and istop = 0, as scipy does.  scipy's default iteration limit is 2*nx*ny*nz.
+ * means.  b = 0 gives x = 0 and istop = 0, as scipy does; so does a b whose sum of squares underflows to +0 (every
+ * |b[i]| below about 1.5e-162).  scipy's default iteration limit is 2*nx*ny*nz.
  *
  * Refused with a message before anything runs, the set left as it was: a NULL set; b, opts or x_out NULL; a
  * struct_size of opts (or of info, when given) that is not the sizeof of its struct; rows selecting a ray that is not
  * OK; an element of b that is not finite; damp or smooth negative or not finite; atol, btol or conlim negative or NaN;
  * iter_lim < 0; a star whose edge lengths are not finite; and device memory the workspace cannot get.
+ * Refused while it runs, with x_out and info untouched, the workspace freed and the set as it was: a norm bnorm, beta
+ * or alfa that is not finite ("‖b‖² overflows" for a finite b whose sum of squares is +inf; else the norm and the
+ * iteration are named).  From there scipy's recurrences would make x all NaN and run to iter_lim.  The usual causes
+ * are a b with |b[i]| near 1e154 or above, a smooth so large that the squares of the D rows overflow, and a star
+ * distance so large that a float32 projection or back-projection overflows.
  *
  * Device memory: a workspace allocated by the call and freed before it returns, with m selected rows, mD rows of D
  * (smooth > 0: (nx-1)*ny*nz + nx*(ny-1)*nz + nx*ny*(nz-1), else 0) and D = nx*ny*nz nodes,

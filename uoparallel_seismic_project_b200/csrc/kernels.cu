@@ -2485,10 +2485,14 @@ static void launch_variant(const TiledLaunch& tl, const CUtensorMap& tm_slow, co
     relax_tiled<RXY, STAR, NW, false><<<tl.grid, dim3(32, NW, 1), tl.smem_bytes, stream>>>(tm_slow, tm_tt, a);
 }
 __global__ void compact_fused(const RelaxArgs a, unsigned long long cond);
+// the single-block compaction keeps its keys in (opt-in) dynamic shared memory; per device
+cudaError_t compact_prepare() {
+  return cudaFuncSetAttribute(compact_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, 49152 * 4);
+}
 cudaError_t tiled_prepare(int rxy, int stock_id, int device, TiledLaunch* out) {
   out->stock_id = stock_id;
-  {  // the single-block compaction keeps its keys in (opt-in) dynamic shared memory; per device
-    cudaError_t e = cudaFuncSetAttribute(compact_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, 49152 * 4);
+  {
+    cudaError_t e = compact_prepare();
     if (e != cudaSuccess) return e;
   }
 #define SWEEPTT_STOCK_STAR(id, name, r, ...) \

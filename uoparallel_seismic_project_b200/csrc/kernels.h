@@ -87,6 +87,9 @@ size_t tiled_persistent_max_keys(int rxy);
 // bucket of that minimum to the next work list (clearing its key), flip parity, advance the
 // round and (when cond != 0) set the CUDA-graph WHILE condition to "work list not empty".
 cudaError_t launch_compact(const RelaxArgs& a, unsigned long long cond, cudaStream_t stream);
+// Opts the single-block compaction into the dynamic shared memory it keeps its keys in, on the current device.
+// Every context calls it when it is created: sweeptt_put_tt compacts whatever the kernel.
+cudaError_t compact_prepare();
 
 // Simple (verification / fallback) path: one thread per node and source, global memory.
 cudaError_t launch_relax_simple(const RelaxArgs& a, const StarDev* star, int nstar,

@@ -355,6 +355,7 @@ extern "C" sweeptt_ctx* sweeptt_create(const sweeptt_opts* opts) {
        cudaMallocHost(&c->h_state, sizeof(SolveState) * STATE_SLOTS) == cudaSuccess &&
        cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) == cudaSuccess &&
        cudaMalloc(&c->d_viol, 32) == cudaSuccess;
+  ok = ok && compact_prepare() == cudaSuccess;  // put_tt compacts before any tiled kernel is prepared
   if (!ok) {
     fail("context setup failed on device %d: %s", dev, cudaGetErrorString(cudaGetLastError()));
     sweeptt_destroy(c);
@@ -2314,6 +2315,12 @@ void sym_ortho(double a, double b, double* c, double* s, double* rr) {
   }
 }
 
+// A norm that is not finite would make x NaN and every stopping test false, so the loop would run to iter_lim and
+// report NaN: the call fails instead (returning frees the workspace; x_out and the set are not touched).
+int lsqr_not_finite(const char* norm, double value, int itn) {
+  return fail("sweeptt_rayset_lsqr: %s is not finite (%g) at iteration %d", norm, value, itn);
+}
+
 }  // namespace
 
 extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const double* b,
@@ -2413,12 +2420,14 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
   double bnorm, alfa = 0, beta;
   CK(launch_lsqr_sumsq(a.u, m, a.part, a.ctas, st, &S.launches));
   if (!S.read_norm(&bnorm)) return 0;
+  if (!std::isfinite(bnorm)) return fail("sweeptt_rayset_lsqr: ‖b‖² overflows (its sum of squares is +inf)");
   beta = bnorm;
   if (beta > 0) {
     if (!S.backproject(1 / beta)) return 0;
     CK(cudaMemsetAsync(a.v, 0, 8 * (size_t)D, st));
     CK(launch_lsqr_v(a, 0.0, st, &S.launches));  // v = A^T u (- 0 * 0)
     if (!S.read_norm(&alfa)) return 0;
+    if (!std::isfinite(alfa)) return lsqr_not_finite("alfa = ‖v‖", alfa, itn);
   } else {
     CK(cudaMemsetAsync(a.v, 0, 8 * (size_t)D, st));
   }
@@ -2435,11 +2444,13 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
     if (!S.project()) return 0;
     CK(launch_lsqr_u(a, alfa, st, &S.launches));
     if (!S.read_norm(&beta)) return 0;
+    if (!std::isfinite(beta)) return lsqr_not_finite("beta = ‖u‖", beta, itn);
     if (beta > 0) {
       if (!S.backproject(1 / beta)) return 0;
       anorm = std::sqrt(anorm * anorm + alfa * alfa + beta * beta + dampsq);
       CK(launch_lsqr_v(a, beta, st, &S.launches));
       if (!S.read_norm(&alfa)) return 0;
+      if (!std::isfinite(alfa)) return lsqr_not_finite("alfa = ‖v‖", alfa, itn);
       if (alfa > 0) {
         CK(launch_lsqr_scale(a.v, D, 1 / alfa, st));
         ++S.launches;
