@@ -426,6 +426,40 @@ int sweeptt_rayset_lsqr(sweeptt_rayset *set, const uint8_t *rows, /* [N] or NULL
                         sweeptt_lsqr_info *info,                  /* may be NULL                                 */
                         sweeptt_stats *stats);
 
+/* sweeptt_rayset_lsqr_hypo is sweeptt_rayset_lsqr with 4 more columns per receiver of the set, the unknowns of
+ * local-earthquake tomography when the set was frozen with the stations as sources and the events as receivers
+ * (3 coordinates and the origin time of every event):
+ *   min ||A [x; y] - [b; 0]||^2 + damp^2 (||x||^2 + ||y||^2),  A = [G_rows H; smooth*D 0],
+ * x the D = nx*ny*nz model values, y the 4*nrec hypocentre values (column D + 4r + c).  Selected row i is ray
+ * q_i = s*nrec + r; it has h[4i + c] in column D + 4r + c, c = 0..3, and zero in every other hypocentre column.
+ *
+ * Applying A: (A [v; y])_i = fl(fl(fl(fl(g_i + fl(h[4i]*y_r0)) + fl(h[4i+1]*y_r1)) + fl(h[4i+2]*y_r2)) + fl(h[4i+3]*y_r3))
+ * for the selected rows, g_i = float64(proj[q_i]) as in sweeptt_rayset_lsqr; the D rows are unchanged.  Component
+ * D + 4r + c of A^T u is acc = +0, then acc = fl(acc + fl(h[4i+c] * u_i)) over the selected rows i of receiver r in
+ * increasing i; the model components are those of sweeptt_rayset_lsqr.  Every norm over the columns is sqrt(sumsq(.))
+ * of the concatenation [model part; hypocentre part] with the same 2048-element block tree; everything else is the
+ * algorithm of sweeptt_rayset_lsqr, statement for statement.  A receiver with no selected row keeps y = +0.
+ *
+ * With h all zero, x_out, istop, itn and the six norms are bit for bit those of sweeptt_rayset_lsqr and hypo_out is
+ * all +0: a projection is never -0 (the walk's sum starts at +0), so g + fl(0 * y) = g; the hypocentre components of
+ * v, w and x stay +0, and their +0 squares change no block sum.
+ *
+ * Refusals: those of sweeptt_rayset_lsqr (with this call's name), and h or hypo_out NULL, and an element of h that is
+ * not finite (its index is named).  Refusals while it runs leave x_out, hypo_out, info and the set untouched.
+ *
+ * Device memory: the workspace of sweeptt_rayset_lsqr with x, v and w over D + 4*nrec values, plus h, the rows of
+ * every receiver (int64[m], a CSR in increasing i) and its offsets (int64[nrec + 1]):
+ *   8*(m + mD) + 24*(D + 4*nrec) + 8*m + 8*(ceil(max(m + mD, D + 4*nrec) / 2048) + 1) + 32*m + 8*m + 8*(nrec + 1)
+ * bytes.  stats: as sweeptt_rayset_lsqr, h2d_bytes adding h and the CSR, d2h_bytes adding hypo_out. */
+int sweeptt_rayset_lsqr_hypo(sweeptt_rayset *set, const uint8_t *rows, /* [N] or NULL = the OK rays             */
+                             const double *b,                          /* [m], finite                            */
+                             const double *h,                          /* [m*4], finite, row order               */
+                             const sweeptt_lsqr_opts *opts,
+                             double *x_out,                            /* nx*ny*nz, FLOATBOX, caller axes        */
+                             double *hypo_out,                         /* [nrec*4], receiver-major               */
+                             sweeptt_lsqr_info *info,                  /* may be NULL                            */
+                             sweeptt_stats *stats);
+
 /* ---- event location: grid search over the stations' travel-time fields ----------------------- */
 
 /* The context's sources [source_begin, source_begin+source_count) are the STATIONS: a field started at a station s

@@ -9,6 +9,7 @@ raises ``SweepError`` when the extension or a CUDA device is missing.
 from .api import (  # noqa: F401
     FS,
     Backprojection,
+    JointUpdate,
     LOC_NO_PICKS,
     LOC_OK,
     LOC_UNREACHED,
@@ -28,9 +29,11 @@ from .api import (  # noqa: F401
     SweepStats,
     build_pull_star,
     device_count,
+    hypocentre_partials,
     lib_path,
     load_library,
     linearized_update,
+    joint_update,
     locate_events,
     location_uncertainty,
     make_star,

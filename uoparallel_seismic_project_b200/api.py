@@ -108,6 +108,7 @@ _EXPORTS = [
     "sweeptt_count_violations", "sweeptt_trace_rays", "sweeptt_ray_project", "sweeptt_ray_backproject",
     "sweeptt_rayset_freeze", "sweeptt_rayset_destroy", "sweeptt_rayset_bytes", "sweeptt_rayset_table",
     "sweeptt_rayset_paths", "sweeptt_rayset_project", "sweeptt_rayset_backproject", "sweeptt_rayset_lsqr",
+    "sweeptt_rayset_lsqr_hypo",
     "sweeptt_locate_events", "sweeptt_misfit_regions", "sweeptt_refine_events", "sweeptt_refine_regions",
     "sweeptt_misfit_box", "sweeptt_relaxations_per_round", "sweeptt_pool_bytes", "sweeptt_tiles_per_source", "sweeptt_debug_model_stats", "sweeptt_solve_slabs",
     "sweeptt_solve_slabs_vbox", "sweeptt_vbox_dims",
@@ -174,6 +175,8 @@ def load_library() -> C.CDLL:
                                                C.POINTER(_Stats)]
     lib.sweeptt_rayset_lsqr.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_LsqrOpts), C.c_void_p,
                                         C.POINTER(_LsqrInfo), C.POINTER(_Stats)]
+    lib.sweeptt_rayset_lsqr_hypo.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_LsqrOpts),
+                                             C.c_void_p, C.c_void_p, C.POINTER(_LsqrInfo), C.POINTER(_Stats)]
     lib.sweeptt_locate_events.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_Stats)]
     lib.sweeptt_misfit_regions.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
@@ -424,7 +427,9 @@ class LinearizedUpdate:
 @dataclass
 class LsqrSolution:
     """RaySet.lsqr: x (float64[nx, ny, nz]) minimises ||G_rows x - b||^2 + smooth^2 ||D x||^2 + damp^2 ||x||^2; istop,
-    itn and the six norms mean what scipy.sparse.linalg.lsqr's return tuple means."""
+    itn and the six norms mean what scipy.sparse.linalg.lsqr's return tuple means.  With hypocentre columns (hypo=),
+    x and hypo (float64[R, 4], one row per receiver) minimise ||G_rows x + H hypo - b||^2 + smooth^2 ||D x||^2 +
+    damp^2 (||x||^2 + ||hypo||^2); without them hypo is None."""
     x: np.ndarray         # float64[nx, ny, nz]
     istop: int
     itn: int
@@ -435,6 +440,32 @@ class LsqrSolution:
     arnorm: float
     xnorm: float
     stats: SweepStats
+    hypo: np.ndarray | None = None   # float64[R, 4]
+
+
+@dataclass
+class JointUpdate:
+    """joint_update: one damped linearised step for slowness and hypocentres together.  delta (float32[nx, ny, nz]) is
+    the slowness update; shift[e] (float64, nodes, caller axes) and origin_shift[e] (float64, time) the update of event
+    e's position and origin time; every one of them +0 for an event without a selected row.  centres [E, 3] and
+    origin_time [E] are where the step starts ((-1, -1, -1) and NaN for an event locate_events did not place);
+    rows [S, E] the rays used (a pick, an OK ray, an OK event) and
+    residual [S, E] their b = (obs - t0) - t, NaN elsewhere; istop, itn and the six norms are LSQR's."""
+    delta: np.ndarray         # float32[nx, ny, nz]
+    shift: np.ndarray         # float64[E, 3]
+    origin_shift: np.ndarray  # float64[E]
+    centres: np.ndarray       # int32[E, 3]
+    origin_time: np.ndarray   # float64[E]
+    residual: np.ndarray      # float64[S, E]
+    rows: np.ndarray          # bool[S, E]
+    istop: int
+    itn: int
+    r1norm: float
+    r2norm: float
+    anorm: float
+    acond: float
+    arnorm: float
+    xnorm: float
 
 
 @dataclass
@@ -1019,13 +1050,18 @@ class RaySet:
 
         return LinearOperator((int(rows.sum()), n), matvec=matvec, rmatvec=rmatvec, dtype=np.float64)
 
-    def lsqr(self, b, rows=None, *, damp: float = 0.0, smooth: float = 0.0, atol: float = 1e-6, btol: float = 1e-6,
-             conlim: float = 1e8, iter_lim: int | None = None) -> LsqrSolution:
+    def lsqr(self, b, rows=None, *, hypo=None, damp: float = 0.0, smooth: float = 0.0, atol: float = 1e-6,
+             btol: float = 1e-6, conlim: float = 1e8, iter_lim: int | None = None) -> LsqrSolution:
         """scipy.sparse.linalg.lsqr on the device (include/sweeptt.h, sweeptt_rayset_lsqr): minimises
         ||A x - [b; 0]||^2 + damp^2 ||x||^2 with A = [G_rows; smooth D], G_rows = as_linear_operator(rows) (rows: bool
         [S, R], default the OK rays; b: float64 over the selected rays in q order) and D the first difference along
         every axis.  Only b goes to the device and only x and a few scalars per iteration come back.  iter_lim None is
-        scipy's 2 nx ny nz."""
+        scipy's 2 nx ny nz.
+
+        hypo (float64 [m, 4], finite, one row per selected ray in q order) adds 4 columns per receiver
+        (sweeptt_rayset_lsqr_hypo): A = [G_rows H; smooth D 0], where selected row i, ray q = s R + r, has hypo[i, c]
+        in column c of receiver r.  The solution's hypo [R, 4] holds those columns' values; a receiver with no
+        selected row keeps +0.  hypo all zero gives the x, istop, itn and norms of the call without it, bit for bit."""
         rows = self.status == RAY_OK if rows is None else np.asarray(rows, bool)
         if rows.shape != self.shape:
             raise SweepError(f"RaySet.lsqr: rows of shape {rows.shape}, expected {self.shape}")
@@ -1038,10 +1074,20 @@ class RaySet:
         info = _LsqrInfo(C.sizeof(_LsqrInfo))
         x = np.empty(self.dims, np.float64)
         s = _Stats()
-        _check(self._lib.sweeptt_rayset_lsqr(self._handle(), sel.ctypes.data, bb.ctypes.data, C.byref(opts),
-                                             x.ctypes.data, C.byref(info), C.byref(s)), "sweeptt_rayset_lsqr")
+        hout = None
+        if hypo is None:
+            _check(self._lib.sweeptt_rayset_lsqr(self._handle(), sel.ctypes.data, bb.ctypes.data, C.byref(opts),
+                                                 x.ctypes.data, C.byref(info), C.byref(s)), "sweeptt_rayset_lsqr")
+        else:
+            hh = np.ascontiguousarray(hypo, dtype=np.float64)
+            if hh.shape != (bb.size, 4):
+                raise SweepError(f"RaySet.lsqr: hypo of shape {hh.shape}, expected {(bb.size, 4)}")
+            hout = np.empty((self.shape[1], 4), np.float64)
+            _check(self._lib.sweeptt_rayset_lsqr_hypo(self._handle(), sel.ctypes.data, bb.ctypes.data, hh.ctypes.data,
+                                                      C.byref(opts), x.ctypes.data, hout.ctypes.data, C.byref(info),
+                                                      C.byref(s)), "sweeptt_rayset_lsqr_hypo")
         return LsqrSolution(x, info.istop, info.itn, info.r1norm, info.r2norm, info.anorm, info.acond, info.arnorm,
-                            info.xnorm, SweepStats._from(s))
+                            info.xnorm, SweepStats._from(s), hout)
 
 
 def trace_rays(slowness, star, starts, receivers, *, delta: float = 10.0, max_nodes: int | None = None,
@@ -1128,6 +1174,89 @@ def linearized_update(slowness, star, starts, receivers, observed, *, damp: floa
     misfit = 0.5 * float(np.sum(residual[use].astype(np.float64) ** 2))
     return LinearizedUpdate(out[0].astype(np.float32).reshape(np.shape(slowness)), residual, status, misfit,
                             int(out[1]), int(out[2]), float(out[3]))
+
+
+def hypocentre_partials(ctx: SweepContext, centres, sources=None) -> np.ndarray:
+    """float64[E, S, 3]: the derivative of station s's travel time at centre e along each caller axis, in time per
+    node step, from the context's converged fields (the sources in `sources` are the stations; a range or a
+    (begin, count) pair; default: all).
+
+    The times t0 at the centre and t-, t+ at its two neighbours along each axis are read on the device with
+    SweepContext.trace_rays(max_nodes=1) (its tt, whatever the ray status) and taken to float64.  Per axis:
+      - both neighbours in the box and finite: fl(0.5 * fl(t+ - t-));
+      - only one of them: fl(t+ - t0) or fl(t0 - t-);
+      - neither (a one-node axis, an axis with both neighbours +inf): 0;
+    and NaN on every axis when t0 is +inf.  A neighbour outside the box or at +inf counts as absent."""
+    c = np.asarray(centres, np.int64).reshape(-1, 3)
+    dims = np.asarray(ctx.dims, np.int64)
+    if ((c < 0) | (c >= dims)).any():
+        raise SweepError("hypocentre_partials: a centre lies outside the box")
+    nodes, inside = [c], []
+    for a in range(3):
+        for d in (-1, 1):
+            n = c.copy()
+            n[:, a] += d
+            ok = (n[:, a] >= 0) & (n[:, a] < dims[a])
+            nodes.append(np.where(ok[:, None], n, c))
+            inside.append(ok)
+    E = len(c)
+    tt = ctx.trace_rays(np.concatenate(nodes).astype(np.int32), sources, max_nodes=1).tt.astype(np.float64)
+    t = tt.reshape(tt.shape[0], 7, E).transpose(2, 0, 1)     # [E, S, 7]: t0, then (t-, t+) for axes 0, 1, 2
+    t0 = t[..., 0]
+    out = np.zeros((E, tt.shape[0], 3))
+    with np.errstate(invalid="ignore"):
+        for a in range(3):
+            tm, tp = t[..., 1 + 2 * a], t[..., 2 + 2 * a]
+            hm = inside[2 * a][:, None] & np.isfinite(tm)
+            hp = inside[2 * a + 1][:, None] & np.isfinite(tp)
+            out[..., a] = np.where(hm & hp, 0.5 * (tp - tm),
+                                   np.where(hp, tp - t0, np.where(hm, t0 - tm, 0.0)))
+    out[np.isinf(t0)] = np.nan
+    return out
+
+
+def joint_update(slowness, star, stations, picks, *, damp: float, iter_lim: int, centres=None, smooth: float = 0.0,
+                 hypo_scale: float = 1.0, origin_scale: float = 1.0, atol: float = 1e-6, btol: float = 1e-6,
+                 delta: float = 10.0, device: int | None = None, kernel: int | None = None) -> JointUpdate:
+    """One damped linearised step for slowness and hypocentres together (local-earthquake tomography): the companion
+    of linearized_update, whose rays come from events whose positions and origin times are unknowns too.
+
+    1. Solves one field per station (stations (S, 3) as start points).
+    2. Locates the events of picks [E, S] (SweepContext.locate_events), or takes centres [E, 3] as given; the origin
+       times t0 are locate_events' either way.
+    3. Freezes the rays with the stations as sources and the event nodes as receivers (ray q = s E + e).
+    4. Uses the rays with a pick, an OK ray and an OK event (LOC_OK).
+    5. b = fl(fl(obs - t0_e) - t_s(c_e)), obs = float64(picks[e, s]).
+    6. h = [hypo_scale * dT/dx_a (hypocentre_partials), a = 0, 1, 2; origin_scale] per row.
+    7. RaySet.lsqr(b, rows, hypo=h, damp, smooth, atol, btol, iter_lim).
+    shift = hypo_scale * hypo[:, :3] (nodes) and origin_shift = origin_scale * hypo[:, 3]; hypo_scale and
+    origin_scale weigh the hypocentre columns against the slowness columns under the one damping.  Nothing is applied:
+    moving the events, clamping the slowness and re-solving are the caller's policy."""
+    p = np.asarray(picks, dtype=np.float32)
+    with SweepContext(device=device, kernel=kernel) as ctx:
+        ctx.set_model(slowness)
+        ctx.set_star(star, delta)
+        ctx.set_sources(stations)
+        ctx.run()
+        loc = ctx.locate_events(p)
+        ok = loc.status == LOC_OK
+        c = loc.node if centres is None else np.asarray(centres, np.int32).reshape(-1, 3)
+        if c.shape != loc.node.shape:
+            raise SweepError(f"joint_update: centres of shape {c.shape}, expected {loc.node.shape}")
+        c = np.where(ok[:, None], c, 0).astype(np.int32)   # an event that is not OK has no rows
+        with ctx.freeze_rays(c) as rs:
+            obs = p.T.astype(np.float64)
+            with np.errstate(invalid="ignore"):
+                residual = (obs - loc.origin_time[None, :]) - rs.tt.astype(np.float64)
+            rows = np.isfinite(obs) & (rs.status == RAY_OK) & ok[None, :]
+            d = hypocentre_partials(ctx, c).transpose(1, 0, 2)[rows]     # [m, 3] in q order
+            h = np.concatenate([hypo_scale * d, np.full((len(d), 1), np.float64(origin_scale))], axis=1)
+            sol = rs.lsqr(residual[rows], rows, hypo=h, damp=damp, smooth=smooth, atol=atol, btol=btol,
+                          iter_lim=iter_lim)
+    residual = np.where(rows, residual, np.nan)
+    return JointUpdate(sol.x.astype(np.float32).reshape(np.shape(slowness)), hypo_scale * sol.hypo[:, :3],
+                       origin_scale * sol.hypo[:, 3], np.where(ok[:, None], c, -1).astype(np.int32), loc.origin_time, residual, rows, sol.istop, sol.itn,
+                       sol.r1norm, sol.r2norm, sol.anorm, sol.acond, sol.arnorm, sol.xnorm)
 
 
 def locate_events(slowness, star, stations, picks, *, delta: float = 10.0, device: int | None = None,

@@ -1614,7 +1614,7 @@ __global__ void grad_finish_kernel(const long long* __restrict__ acc, float* __r
 }
 
 // ---------------------------------------------------------------------------------------
-// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr; DESIGN §3.11)
+// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr / _hypo; DESIGN §3.11, §3.14)
 // ---------------------------------------------------------------------------------------
 // The vector passes of one LSQR iteration, every one float64 with DADD / DMUL only (no division or square root: the
 // host forms the reciprocals and roots).  A pass that needs a norm squares its outputs and sums every block of
@@ -1720,6 +1720,29 @@ __device__ __forceinline__ double lsqr_dt(const LsqrArgs& a, long long j) {
   return __dmul_rn(a.smooth, acc);
 }
 
+// Row i < m of the hypocentre columns (sweeptt_rayset_lsqr_hypo), added to g = float64(io[q]) of ray q = row[i] left
+// to right: fl(fl(fl(fl(g + h_i0 v_r0) + h_i1 v_r1) + h_i2 v_r2) + h_i3 v_r3), r = q % nrec, v_rc = v[D + 4r + c].
+__device__ __forceinline__ double hypo_av(const LsqrArgs& a, long long i, long long q, double g) {
+  const double* h = a.h + 4 * i;
+  const double* vr = a.v + (long long)a.nx * a.ny * a.nz + 4 * (q % a.nrec);
+#pragma unroll
+  for (int c = 0; c < 4; ++c) g = __dadd_rn(g, __dmul_rn(h[c], vr[c]));
+  return g;
+}
+
+// Hypocentre column k = 4r + c of A^T u: acc = +0, then acc = fl(acc + fl(h_ic u_i)) over the selected rows i of
+// receiver r in increasing i.
+__device__ __forceinline__ double hypo_atu(const LsqrArgs& a, long long k) {
+  const long long r = k >> 2;
+  const int c = (int)(k & 3);
+  double acc = 0.0;
+  for (long long p = a.hoff[r]; p < a.hoff[r + 1]; ++p) {
+    const long long i = a.hrow[p];
+    acc = __dadd_rn(acc, __dmul_rn(a.h[4 * i + c], a.u[i]));
+  }
+  return acc;
+}
+
 // Partials of sumsq(p[0 .. n)).
 __global__ void __launch_bounds__(LSQR_THREADS) lsqr_sumsq_kernel(const double* __restrict__ p, long long n,
                                                                   double* __restrict__ part) {
@@ -1732,9 +1755,11 @@ __global__ void lsqr_to_f32_kernel(const double* __restrict__ v, float* __restri
     stage[i] = __double2float_rn(v[i]);
 }
 
-// Pass C: u = A v - alpha u, A v = [float64(io[row[i]]); D v], and the partials of sumsq(u).
+// Pass C: u = A v - alpha u, A v = [float64(io[row[i]]); D v], and the partials of sumsq(u).  With hypocentre
+// columns hypo_u_kernel has already formed the G rows, and only their squares are taken here.
 __global__ void __launch_bounds__(LSQR_THREADS) lsqr_u_kernel(const LsqrArgs a, double alpha) {
   lsqr_blocks(a.m + a.mD, a.part, [&](long long i) {
+    if (i < a.m && a.nh) return lsqr_sq(a.u[i]);  // hypo_u_kernel has formed the G rows
     const double av = i < a.m ? (double)a.io[a.row[i]] : lsqr_d_row(a, i - a.m);
     const double u = __dsub_rn(av, __dmul_rn(alpha, a.u[i]));
     a.u[i] = u;
@@ -1761,9 +1786,12 @@ __global__ void __launch_bounds__(LSQR_THREADS) lsqr_scale_u_kernel(const LsqrAr
 }
 
 // Pass F: v = A^T u - beta v, A^T u = fl(float64(grad) + D^T u_D) (the D term only with smoothing; grad = the set's
-// rounded back-projection in stage), and the partials of sumsq(v).
+// rounded back-projection in stage) over the box, and the partials of sumsq(v) over the box and the hypocentre columns
+// (formed by hypo_v_kernel before this pass).
 __global__ void __launch_bounds__(LSQR_THREADS) lsqr_v_kernel(const LsqrArgs a, double beta) {
-  lsqr_blocks((long long)a.nx * a.ny * a.nz, a.part, [&](long long j) {
+  const long long D = (long long)a.nx * a.ny * a.nz;
+  lsqr_blocks(D + a.nh, a.part, [&](long long j) {
+    if (j >= D) return lsqr_sq(a.v[j]);  // hypo_v_kernel has formed the hypocentre columns
     double g = (double)a.stage[j];
     if (a.smooth > 0.0) g = __dadd_rn(g, lsqr_dt(a, j));
     const double v = __dsub_rn(g, __dmul_rn(beta, a.v[j]));
@@ -1777,9 +1805,26 @@ __global__ void lsqr_scale_kernel(double* __restrict__ p, long long n, double s)
     p[i] = __dmul_rn(s, p[i]);
 }
 
+// The hypocentre passes (sweeptt_rayset_lsqr_hypo; DESIGN §3.14), launched before lsqr_u_kernel / lsqr_v_kernel and
+// only when nh > 0.  They are kernels of their own so that the plain solve's passes keep their registers.
+// Pass C, rows i < m: u = fl(hypo_av(i) - fl(alpha u)).
+__global__ void __launch_bounds__(LSQR_THREADS) hypo_u_kernel(const LsqrArgs a, double alpha) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < a.m; i += (long long)gridDim.x * blockDim.x) {
+    const long long q = a.row[i];
+    a.u[i] = __dsub_rn(hypo_av(a, i, q, (double)a.io[q]), __dmul_rn(alpha, a.u[i]));
+  }
+}
+
+// Pass F, columns D + k, k < nh: v = fl(hypo_atu(k) - fl(beta v)).
+__global__ void __launch_bounds__(LSQR_THREADS) hypo_v_kernel(const LsqrArgs a, double beta) {
+  double* v = a.v + (long long)a.nx * a.ny * a.nz;
+  for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < a.nh; k += (long long)gridDim.x * blockDim.x)
+    v[k] = __dsub_rn(hypo_atu(a, k), __dmul_rn(beta, v[k]));
+}
+
 // Step 7: dk = inv_rho * w (only its sumsq partials are kept), x = x + t1 w, w = v + t2 w.
 __global__ void __launch_bounds__(LSQR_THREADS) lsqr_xw_kernel(const LsqrArgs a, double t1, double t2, double inv_rho) {
-  lsqr_blocks((long long)a.nx * a.ny * a.nz, a.part, [&](long long j) {
+  lsqr_blocks((long long)a.nx * a.ny * a.nz + a.nh, a.part, [&](long long j) {
     const double w = a.w[j];
     const double dk = __dmul_rn(inv_rho, w);
     a.x[j] = __dadd_rn(a.x[j], __dmul_rn(t1, w));
@@ -2813,6 +2858,10 @@ cudaError_t launch_lsqr_to_f32(const double* v, float* stage, long long n, cudaS
 
 cudaError_t launch_lsqr_u(const LsqrArgs& a, double alpha, cudaStream_t stream, int* launches) {
   const long long n = a.m + a.mD;
+  if (a.nh && a.m) {
+    hypo_u_kernel<<<1184, LSQR_THREADS, 0, stream>>>(a, alpha);
+    ++*launches;
+  }
   if (n > 0) lsqr_u_kernel<<<lsqr_grid(n, a.ctas), LSQR_THREADS, 0, stream>>>(a, alpha);
   return lsqr_finish(a.part, n, stream, launches);
 }
@@ -2823,7 +2872,11 @@ cudaError_t launch_lsqr_scale_u(const LsqrArgs& a, double inv_beta, cudaStream_t
 }
 
 cudaError_t launch_lsqr_v(const LsqrArgs& a, double beta, cudaStream_t stream, int* launches) {
-  const long long n = (long long)a.nx * a.ny * a.nz;
+  const long long n = (long long)a.nx * a.ny * a.nz + a.nh;
+  if (a.nh) {
+    hypo_v_kernel<<<1184, LSQR_THREADS, 0, stream>>>(a, beta);
+    ++*launches;
+  }
   lsqr_v_kernel<<<lsqr_grid(n, a.ctas), LSQR_THREADS, 0, stream>>>(a, beta);
   return lsqr_finish(a.part, n, stream, launches);
 }
@@ -2834,7 +2887,7 @@ cudaError_t launch_lsqr_scale(double* p, long long n, double s, cudaStream_t str
 }
 
 cudaError_t launch_lsqr_xw(const LsqrArgs& a, double t1, double t2, double inv_rho, cudaStream_t stream, int* launches) {
-  const long long n = (long long)a.nx * a.ny * a.nz;
+  const long long n = (long long)a.nx * a.ny * a.nz + a.nh;
   lsqr_xw_kernel<<<lsqr_grid(n, a.ctas), LSQR_THREADS, 0, stream>>>(a, t1, t2, inv_rho);
   return lsqr_finish(a.part, n, stream, launches);
 }

@@ -170,9 +170,10 @@ cudaError_t launch_rayset_walk(bool backproject, const RaySetArgs& s, int device
 // grad (dense, caller axes) := acc * 2^E rounded once to float32.
 cudaError_t launch_grad_finish(const long long* acc, float* dense, BoxGeom g, int E, cudaStream_t stream);
 
-// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr).  float64 vectors: u over the m selected rows of G then
-// the mD rows of the smoothing operator D, x / v / w over the dense caller-FLOATBOX box.  A launcher whose pass ends
-// in a norm leaves sumsq of the pass's outputs in part[0] (the fixed-order block tree, kernels.cu) and adds its
+// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr / sweeptt_rayset_lsqr_hypo).  float64 vectors: u over
+// the m selected rows of G then the mD rows of the smoothing operator D, x / v / w over the dense caller-FLOATBOX box
+// (D nodes) then the nh hypocentre columns, 4 per receiver (nh = 0 for sweeptt_rayset_lsqr).  A launcher whose pass
+// ends in a norm leaves sumsq of the pass's outputs in part[0] (the fixed-order block tree, kernels.cu) and adds its
 // launches to *launches; the others are one launch each.
 struct LsqrArgs {
   long long m, mD;             // rows of G selected, rows of D (0 without smoothing)
@@ -180,12 +181,17 @@ struct LsqrArgs {
   double smooth;
   const long long* row;        // [m] ray of every selected row
   double* u;                   // [m + mD]
-  double* x;                   // [D]
-  double* v;                   // [D]
-  double* w;                   // [D]
+  double* x;                   // [D + nh]
+  double* v;                   // [D + nh]
+  double* w;                   // [D + nh]
+  long long nh;                // hypocentre columns: column D + 4r + c is coefficient c of receiver r; 0 = none
+  long long nrec;              // receivers of the set: row i is on receiver row[i] % nrec
+  const double* h;             // [4m] the hypocentre coefficients of every selected row (nh > 0)
+  const long long* hoff;       // [nrec + 1] the selected rows of receiver r are hrow[hoff[r] .. hoff[r+1])
+  const long long* hrow;       // [m] those rows, in increasing order for every receiver
   float* io;                   // the set's per-ray floats (projections in, weights out)
   float* stage;                // the set's dense float32 box
-  double* part;                // block sums: ceil(max(m + mD, D) / 2048) doubles
+  double* part;                // block sums: ceil(max(m + mD, D + nh) / 2048) doubles
   unsigned* wmax;              // bits of max |W| of pass D (zeroed by the caller)
   int ctas;                    // CTAs that share the blocks of a first-level reduction (the result does not depend on it)
 };

@@ -2214,7 +2214,7 @@ extern "C" int sweeptt_rayset_backproject(sweeptt_rayset* r, const float* weight
 }
 
 // ---------------------------------------------------------------------------------------
-// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr; DESIGN §3.11)
+// LSQR over a ray set (include/sweeptt.h, sweeptt_rayset_lsqr / sweeptt_rayset_lsqr_hypo; DESIGN §3.11, §3.14)
 // ---------------------------------------------------------------------------------------
 // The vectors stay on the device; the host runs scipy's scalar recurrences (this file is built with
 // -ffp-contract=off, so they round exactly as numpy's scalars do) and reads four scalars per iteration.
@@ -2317,39 +2317,49 @@ void sym_ortho(double a, double b, double* c, double* s, double* rr) {
 
 // A norm that is not finite would make x NaN and every stopping test false, so the loop would run to iter_lim and
 // report NaN: the call fails instead (returning frees the workspace; x_out and the set are not touched).
-int lsqr_not_finite(const char* norm, double value, int itn) {
-  return fail("sweeptt_rayset_lsqr: %s is not finite (%g) at iteration %d", norm, value, itn);
+int lsqr_not_finite(const char* who, const char* norm, double value, int itn) {
+  return fail("%s: %s is not finite (%g) at iteration %d", who, norm, value, itn);
 }
 
-}  // namespace
-
-extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const double* b,
-                                   const sweeptt_lsqr_opts* opts, double* x_out, sweeptt_lsqr_info* info,
-                                   sweeptt_stats* stats) {
-  if (!r) return fail("null ray set");
-  if (stats) std::memset(stats, 0, sizeof *stats);
-  if (!b || !opts || !x_out) return fail("sweeptt_rayset_lsqr: b, opts and x_out are required");
+// The solve of both entry points: h == nullptr is sweeptt_rayset_lsqr (no hypocentre columns), else
+// sweeptt_rayset_lsqr_hypo with 4 columns per receiver (the pointers checked by the caller).
+int rayset_lsqr(const char* who, sweeptt_rayset* r, const uint8_t* rows, const double* b, const double* h,
+                const sweeptt_lsqr_opts* opts, double* x_out, double* hypo_out, sweeptt_lsqr_info* info,
+                sweeptt_stats* stats) {
   if (opts->struct_size != (int)sizeof *opts)
-    return fail("sweeptt_rayset_lsqr: opts->struct_size is %d, expected %d", opts->struct_size, (int)sizeof *opts);
+    return fail("%s: opts->struct_size is %d, expected %d", who, opts->struct_size, (int)sizeof *opts);
   if (info && info->struct_size != (int)sizeof *info)
-    return fail("sweeptt_rayset_lsqr: info->struct_size is %d, expected %d", info->struct_size, (int)sizeof *info);
+    return fail("%s: info->struct_size is %d, expected %d", who, info->struct_size, (int)sizeof *info);
   const double damp = opts->damp, smooth = opts->smooth;
-  if (!std::isfinite(damp) || damp < 0) return fail("sweeptt_rayset_lsqr: damp must be finite and >= 0");
-  if (!std::isfinite(smooth) || smooth < 0) return fail("sweeptt_rayset_lsqr: smooth must be finite and >= 0");
+  if (!std::isfinite(damp) || damp < 0) return fail("%s: damp must be finite and >= 0", who);
+  if (!std::isfinite(smooth) || smooth < 0) return fail("%s: smooth must be finite and >= 0", who);
   if (!(opts->atol >= 0) || !(opts->btol >= 0) || !(opts->conlim >= 0))
-    return fail("sweeptt_rayset_lsqr: atol, btol and conlim must be >= 0");
-  if (opts->iter_lim < 0) return fail("sweeptt_rayset_lsqr: iter_lim must be >= 0");
-  if (!std::isfinite(r->hd_max)) return fail("sweeptt_rayset_lsqr: the star's edge lengths are not finite");
+    return fail("%s: atol, btol and conlim must be >= 0", who);
+  if (opts->iter_lim < 0) return fail("%s: iter_lim must be >= 0", who);
+  if (!std::isfinite(r->hd_max)) return fail("%s: the star's edge lengths are not finite", who);
   std::vector<long long> row;
   for (long long q = 0; q < r->nrays; ++q) {
     const bool sel = rows ? rows[q] != 0 : r->status[q] == SWEEPTT_RAY_OK;
     if (!sel) continue;
-    if (r->status[q] != SWEEPTT_RAY_OK) return fail("sweeptt_rayset_lsqr: rows selects ray %lld, which is not OK", q);
+    if (r->status[q] != SWEEPTT_RAY_OK) return fail("%s: rows selects ray %lld, which is not OK", who, q);
     row.push_back(q);
   }
   const long long m = (long long)row.size();
   for (long long i = 0; i < m; ++i)
-    if (!std::isfinite(b[i])) return fail("sweeptt_rayset_lsqr: b[%lld] is not finite", i);
+    if (!std::isfinite(b[i])) return fail("%s: b[%lld] is not finite", who, i);
+  // the hypocentre columns: 4 per receiver, and every receiver's selected rows as a CSR in increasing i
+  const long long nrec = r->nrec, nh = h ? 4 * nrec : 0;
+  std::vector<long long> hoff, hrow;
+  if (h) {
+    for (long long i = 0; i < 4 * m; ++i)
+      if (!std::isfinite(h[i])) return fail("%s: h[%lld] is not finite", who, i);
+    hoff.assign(nrec + 1, 0);
+    hrow.resize(m);
+    for (long long i = 0; i < m; ++i) ++hoff[row[i] % nrec + 1];
+    for (long long k = 0; k < nrec; ++k) hoff[k + 1] += hoff[k];
+    std::vector<long long> next(hoff.begin(), hoff.end() - 1);
+    for (long long i = 0; i < m; ++i) hrow[next[row[i] % nrec]++] = i;
+  }
 
   const BoxGeom& g = r->g;
   const long long nx = g.nx, ny = g.ny, nz = g.nz;  // kernel axes: the caller's through perm
@@ -2362,33 +2372,42 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
   const long long D = S.D;
   const long long mD = smooth > 0 ? (cd[0] - 1) * cd[1] * cd[2] + cd[0] * (cd[1] - 1) * cd[2] + cd[0] * cd[1] * (cd[2] - 1) : 0;
   const long long mu = m + mD;
-  const long long nblk = (std::max({mu, D, 1LL}) + 2047) / 2048;
+  const long long nx_all = D + nh;  // x, v and w: the box, then the hypocentre columns
+  const long long nblk = (std::max({mu, nx_all, 1LL}) + 2047) / 2048;
+  const long long hbytes = h ? 32 * m + 8 * m + 8 * (nrec + 1) : 0;  // h, hrow, hoff
   CK(cudaSetDevice(r->device));
   cudaStream_t st = S.st;
   {
-    const size_t bytes = 8 * (size_t)mu + 24 * (size_t)D + 8 * (size_t)m + 8 * (size_t)(nblk + 1);
+    const size_t bytes = 8 * (size_t)mu + 24 * (size_t)nx_all + 8 * (size_t)m + 8 * (size_t)(nblk + 1) + (size_t)hbytes;
     const cudaError_t e = cudaMalloc(&S.dev, bytes);
     if (e != cudaSuccess) {
       cudaGetLastError();
       S.dev = nullptr;
-      return fail("sweeptt_rayset_lsqr: no device memory for the %.3f GB workspace (%s)", bytes / 1e9, cudaGetErrorString(e));
+      return fail("%s: no device memory for the %.3f GB workspace (%s)", who, bytes / 1e9, cudaGetErrorString(e));
     }
     const cudaError_t eh = cudaMallocHost(&S.host, 32);
     if (eh != cudaSuccess) {
       cudaGetLastError();
       S.host = nullptr;
-      return fail("sweeptt_rayset_lsqr: no page-locked host memory (%s)", cudaGetErrorString(eh));
+      return fail("%s: no page-locked host memory (%s)", who, cudaGetErrorString(eh));
     }
   }
   LsqrArgs& a = S.a;
   double* p = static_cast<double*>(S.dev);
   a.u = p; p += mu;
-  a.x = p; p += D;
-  a.v = p; p += D;
-  a.w = p; p += D;
+  a.x = p; p += nx_all;
+  a.v = p; p += nx_all;
+  a.w = p; p += nx_all;
   a.row = reinterpret_cast<long long*>(p); p += m;
   a.part = p; p += nblk;
-  a.wmax = reinterpret_cast<unsigned*>(p);
+  a.wmax = reinterpret_cast<unsigned*>(p); p += 1;
+  if (h) {
+    a.h = p; p += 4 * m;
+    a.hrow = reinterpret_cast<long long*>(p); p += m;
+    a.hoff = reinterpret_cast<long long*>(p);
+  }
+  a.nh = nh;
+  a.nrec = nrec;
   a.m = m;
   a.mD = mD;
   a.nx = (int)cd[0]; a.ny = (int)cd[1]; a.nz = (int)cd[2];
@@ -2403,10 +2422,17 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
     CK(cudaMemcpyAsync(a.u, b, 8 * (size_t)m, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(const_cast<long long*>(a.row), row.data(), 8 * (size_t)m, cudaMemcpyHostToDevice, st));
   }
+  if (h) {
+    if (m) {
+      CK(cudaMemcpyAsync(const_cast<double*>(a.h), h, 32 * (size_t)m, cudaMemcpyHostToDevice, st));
+      CK(cudaMemcpyAsync(const_cast<long long*>(a.hrow), hrow.data(), 8 * (size_t)m, cudaMemcpyHostToDevice, st));
+    }
+    CK(cudaMemcpyAsync(const_cast<long long*>(a.hoff), hoff.data(), 8 * (size_t)(nrec + 1), cudaMemcpyHostToDevice, st));
+  }
   CK(cudaStreamSynchronize(st));  // pageable sources: the copies are complete
   const double h2d_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_h2d).count();
   if (mD) CK(cudaMemsetAsync(a.u + m, 0, 8 * (size_t)mD, st));
-  CK(cudaMemsetAsync(a.x, 0, 8 * (size_t)D, st));
+  CK(cudaMemsetAsync(a.x, 0, 8 * (size_t)nx_all, st));
 
   // scipy's lsqr, x0 = None, calc_var = False
   const double eps = std::numeric_limits<double>::epsilon();
@@ -2420,22 +2446,22 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
   double bnorm, alfa = 0, beta;
   CK(launch_lsqr_sumsq(a.u, m, a.part, a.ctas, st, &S.launches));
   if (!S.read_norm(&bnorm)) return 0;
-  if (!std::isfinite(bnorm)) return fail("sweeptt_rayset_lsqr: ‖b‖² overflows (its sum of squares is +inf)");
+  if (!std::isfinite(bnorm)) return fail("%s: ‖b‖² overflows (its sum of squares is +inf)", who);
   beta = bnorm;
   if (beta > 0) {
     if (!S.backproject(1 / beta)) return 0;
-    CK(cudaMemsetAsync(a.v, 0, 8 * (size_t)D, st));
+    CK(cudaMemsetAsync(a.v, 0, 8 * (size_t)nx_all, st));
     CK(launch_lsqr_v(a, 0.0, st, &S.launches));  // v = A^T u (- 0 * 0)
     if (!S.read_norm(&alfa)) return 0;
-    if (!std::isfinite(alfa)) return lsqr_not_finite("alfa = ‖v‖", alfa, itn);
+    if (!std::isfinite(alfa)) return lsqr_not_finite(who, "alfa = ‖v‖", alfa, itn);
   } else {
-    CK(cudaMemsetAsync(a.v, 0, 8 * (size_t)D, st));
+    CK(cudaMemsetAsync(a.v, 0, 8 * (size_t)nx_all, st));
   }
   if (alfa > 0) {
-    CK(launch_lsqr_scale(a.v, D, 1 / alfa, st));
+    CK(launch_lsqr_scale(a.v, nx_all, 1 / alfa, st));
     ++S.launches;
   }
-  CK(cudaMemcpyAsync(a.w, a.v, 8 * (size_t)D, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(a.w, a.v, 8 * (size_t)nx_all, cudaMemcpyDeviceToDevice, st));
   double rhobar = alfa, phibar = beta, rnorm = beta, r1norm = rnorm, r2norm = rnorm, arnorm = alfa * beta;
 
   const bool solved = arnorm == 0;  // scipy returns x = 0 before its loop
@@ -2444,15 +2470,15 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
     if (!S.project()) return 0;
     CK(launch_lsqr_u(a, alfa, st, &S.launches));
     if (!S.read_norm(&beta)) return 0;
-    if (!std::isfinite(beta)) return lsqr_not_finite("beta = ‖u‖", beta, itn);
+    if (!std::isfinite(beta)) return lsqr_not_finite(who, "beta = ‖u‖", beta, itn);
     if (beta > 0) {
       if (!S.backproject(1 / beta)) return 0;
       anorm = std::sqrt(anorm * anorm + alfa * alfa + beta * beta + dampsq);
       CK(launch_lsqr_v(a, beta, st, &S.launches));
       if (!S.read_norm(&alfa)) return 0;
-      if (!std::isfinite(alfa)) return lsqr_not_finite("alfa = ‖v‖", alfa, itn);
+      if (!std::isfinite(alfa)) return lsqr_not_finite(who, "alfa = ‖v‖", alfa, itn);
       if (alfa > 0) {
-        CK(launch_lsqr_scale(a.v, D, 1 / alfa, st));
+        CK(launch_lsqr_scale(a.v, nx_all, 1 / alfa, st));
         ++S.launches;
       }
     }
@@ -2528,9 +2554,10 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
   CK(cudaEventRecord(r->ev1, st));
   const auto t_x = std::chrono::steady_clock::now();
   CK(cudaMemcpyAsync(x_out, a.x, 8 * (size_t)D, cudaMemcpyDeviceToHost, st));
+  if (nh) CK(cudaMemcpyAsync(hypo_out, a.x + D, 8 * (size_t)nh, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   S.d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_x).count();
-  S.d2h_bytes += 8 * D;
+  S.d2h_bytes += 8 * nx_all;
   float ms = 0;
   CK(cudaEventElapsedTime(&ms, r->ev0, r->ev1));
   if (info) {
@@ -2549,11 +2576,32 @@ extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const
     stats->kernel_launches = S.launches;
     stats->devices_used = 1;
     stats->h2d_ms = h2d_ms;
-    stats->h2d_bytes = 16 * m;
+    stats->h2d_bytes = 16 * m + hbytes;
     stats->d2h_ms = S.d2h_ms;
     stats->d2h_bytes = S.d2h_bytes;
   }
   return 1;
+}
+
+}  // namespace
+
+extern "C" int sweeptt_rayset_lsqr(sweeptt_rayset* r, const uint8_t* rows, const double* b,
+                                   const sweeptt_lsqr_opts* opts, double* x_out, sweeptt_lsqr_info* info,
+                                   sweeptt_stats* stats) {
+  if (!r) return fail("null ray set");
+  if (stats) std::memset(stats, 0, sizeof *stats);
+  if (!b || !opts || !x_out) return fail("sweeptt_rayset_lsqr: b, opts and x_out are required");
+  return rayset_lsqr("sweeptt_rayset_lsqr", r, rows, b, nullptr, opts, x_out, nullptr, info, stats);
+}
+
+extern "C" int sweeptt_rayset_lsqr_hypo(sweeptt_rayset* r, const uint8_t* rows, const double* b, const double* h,
+                                        const sweeptt_lsqr_opts* opts, double* x_out, double* hypo_out,
+                                        sweeptt_lsqr_info* info, sweeptt_stats* stats) {
+  if (!r) return fail("null ray set");
+  if (stats) std::memset(stats, 0, sizeof *stats);
+  if (!b || !h || !opts || !x_out || !hypo_out)
+    return fail("sweeptt_rayset_lsqr_hypo: b, h, opts, x_out and hypo_out are required");
+  return rayset_lsqr("sweeptt_rayset_lsqr_hypo", r, rows, b, h, opts, x_out, hypo_out, info, stats);
 }
 
 // ---------------------------------------------------------------------------------------
